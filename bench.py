@@ -15,9 +15,11 @@ roofline block (K/V bytes / event time / measured HBM peak), an end-to-end figur
 ``dist.online_eval_sharded`` (host means in, host regret curves out) and the reference's own
 deploy_online_vec + BanditTransformerController timed on the host cores at reduced N.
 
-    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--workload collect|online_eval]
+    python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--workload collect|online_eval] [--dump-outputs DIR]
 
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
+Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.  --dump-outputs DIR writes what the
+collection's last timed step returned as DIR/<name>.npy (see dump_outputs), so that two builds can be compared
+output for output: with the same arguments the inputs are identical from run to run.
 """
 import argparse
 import json
@@ -38,6 +40,7 @@ UNIT = "env-steps/s"
 OE_ENVS = int(os.environ.get("DPT_BENCH_OE_ENVS", 10000))    # BASELINE configs[3]: 10k envs
 OE_LAYERS, OE_EMBD = 4, 32
 OE_METRIC = "online-eval trajs/sec (deploy_online_vec, GPT-2 embd=32 layer=4 head=1 controller, H=500 dim=5)"
+DUMP_ENVS = 2048     # envs in the --dump-outputs sample: 2048 x H=500 x 32 B = 31 MiB of the 2 GB a step writes
 
 
 def workload_name(n_gpus):
@@ -215,6 +218,24 @@ def time_events(torch, fn, reps, warm):
     return [ev[i].elapsed_time(ev[i + 1]) for i in range(reps)], ev[0].elapsed_time(ev[reps])
 
 
+def dump_outputs(path, out, stats):
+    """Writes what one bandit_rollin step returned as path/<name>.npy: the four fp32 context arrays [n, H, *] at a fixed
+    sample of DUMP_ENVS envs of this rank's shard (np.random.RandomState(0), in ascending env order; every env when the
+    shard is smaller) and, when the step accumulated them, its float64 return statistics [3]."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    first = next(iter(out.values()))
+    n = first.shape[0]
+    idx = np.sort(np.random.RandomState(0).choice(n, min(n, DUMP_ENVS), replace=False))
+    rows = torch.as_tensor(idx, device=first.device)
+    arrays = {name: t.index_select(0, rows) for name, t in out.items()}
+    if stats is not None:
+        arrays["return_stats"] = stats
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
+
+
 def other_workloads(kernels, torch):
     """The other BASELINE.json configs on one GPU (informational; CUDA events, 3 warm-up + 5 timed runs each)."""
     import numpy as np
@@ -309,7 +330,8 @@ def online_eval_block(args, torch, dist, rank, world, dev, pool):
     model = Transformer({"horizon": H, "state_dim": 1, "action_dim": DIM, "n_layer": OE_LAYERS, "n_embd": OE_EMBD, "n_head": 1,
                          "dropout": 0.0, "test": True})
     peak = float(load_peaks().get("hbm_gbs", 6650.0))
-    reps = int(os.environ.get("DPT_BENCH_OE_STEPS", 3))
+    # --steps sets the timed passes when this block is the line's headline; as the secondary block it keeps its own count
+    reps = args.steps if args.workload == "online_eval" else int(os.environ.get("DPT_BENCH_OE_STEPS", 3))
     block = {"metric": OE_METRIC, "unit": "trajs/s", "H": H, "dim": DIM, "var": VAR, "sample": True, "steps": reps, "warmup": 3,
              "model": "GPT-2 trunk embd=32 layer=4 head=1, random init (torch.manual_seed(0)), one token-forward per env-step on a per-env K/V cache",
              "l2": "K/V caches of a pass (%.2f GB fp32 / %.2f GB bf16 per 10k envs) exceed the 126 MB L2; no flush" % (
@@ -399,7 +421,14 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=None)
     ap.add_argument("--no-other", action="store_true", help="skip the secondary workloads (configs 2-4)")
     ap.add_argument("--no-online-eval", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the collection's last timed step (rank 0's shard) "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU collection's outputs; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
@@ -407,7 +436,6 @@ def main():
         run_reference(args, rank)
         return
     args.warmup = max(args.warmup, 3)   # timing rule: at least 3 warm-up steps (the JSON line reports the value used)
-    args.steps = max(args.steps, 1)
 
     # CPU legs first (rank 0, N=1 only), before the GPU is busy: bounded samples on all host cores
     cpu_baseline, cpu_other, pool = None, None, None
@@ -487,6 +515,8 @@ def main():
     barrier()
     if sampler:
         sampler.stop()
+    if args.dump_outputs and rank == 0:   # `out` still holds the last timed step's outputs
+        dump_outputs(args.dump_outputs, out, stats[args.warmup + args.steps - 1] if gather_mode != "none" else None)
     total_ms = ev[0].elapsed_time(end_ev)
     per = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)

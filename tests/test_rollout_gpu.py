@@ -596,3 +596,32 @@ def test_bench_own_arm_contract(dpt):
     e = r["e2e"]
     assert e["unit"] == r["unit"] and 0 < e["value"] < r["value"] and e["h2d_bytes_per_step"] > 0 and e["d2h_bytes_per_step"] > 0
     assert {"sm_mhz", "sm_max_mhz", "reasons"} <= set(r["clocks"])
+
+
+def test_bench_dump_outputs(dpt, tmp_path):
+    """`bench.py --dump-outputs DIR` writes the last timed step's outputs: the sampled envs equal a direct bandit_rollin at
+    that step's seed (warm-up + --steps - 1), float32 / float64 only, 64 MB at most."""
+    import os
+    import subprocess
+    import sys
+    import bench
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    warmup, steps = 3, 2
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", str(warmup),
+                          "--no-cpu-baseline", "--no-other", "--no-online-eval", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    files = sorted(os.listdir(tmp_path))
+    assert files == ["context_actions.npy", "context_next_states.npy", "context_rewards.npy", "context_states.npy", "return_stats.npy"]
+    got = {f[:-4]: np.load(tmp_path / f) for f in files}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert sum(a.nbytes for a in got.values()) <= 64 << 20
+    N = bench.ENVS_PER_GPU
+    idx = np.sort(np.random.RandomState(0).choice(N, min(N, bench.DUMP_ENVS), replace=False))
+    means, _, _ = dpt.kernels.bandit_sample_means(N, bench.DIM, 0, 0)
+    stats = torch.zeros(3, dtype=torch.float64, device="cuda")
+    want = dpt.kernels.bandit_rollin(means, bench.H, bench.VAR, warmup + steps - 1, 0, stats=stats)
+    rows = torch.as_tensor(idx, device="cuda")
+    for k, t in want.items():
+        assert np.array_equal(got[k], _np(t.index_select(0, rows))), k
+    assert np.allclose(got["return_stats"], _np(stats), rtol=1e-9)
