@@ -25,19 +25,21 @@ int sm_count() {
   return cached;
 }
 
-int pick_envs_per_cta(int N, int slots, int min_e, int max_e) {
+int pick_envs_per_cta(int N, int slots, int min_e, int max_e, int step) {
   if (min_e < 1) min_e = 1;
   if (max_e < min_e) max_e = min_e;
   if (slots < 1) slots = 1;
   int best = -1;
   double best_eff = -1.0;
   for (int e = max_e; e >= min_e; --e) {
+    if (step > 1 && e % step) continue;
     const long grid = ((long)N + e - 1) / e;
     const long waves = (grid + slots - 1) / slots;
     if (waves < 3 && e > min_e) continue;           // too coarse: keep shrinking e
     const double eff = (double)grid / (double)(waves * slots);
     if (eff > best_eff + 1e-9) best_eff = eff, best = e;
   }
+  if (best < 0 && step > 1) return pick_envs_per_cta(N, slots, min_e, max_e, 1);   // no multiple of step qualifies
   return best < 0 ? min_e : best;
 }
 

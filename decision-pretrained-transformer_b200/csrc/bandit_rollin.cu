@@ -8,14 +8,16 @@
 //      as numpy (no FMA contraction), turned into integer thresholds so the per-step categorical
 //      draw is (d-1) integer compares and bit-exact against the oracle;
 //   2. meanwhile the other warps stream the constant context_states / context_next_states (== 1);
-//   3. step loop: each warp takes 64-step chunks; a lane owns two consecutive steps and makes
-//      ONE Philox4x32-10 call for them (2 categorical uniforms + 1 Box-Muller pair).  Rewards go
-//      out as one coalesced float2 per lane; the one-hot action rows (d floats per step, 20 B for
-//      d=5) are re-tiled across the warp with shuffles of a 2d-bit one-hot mask so that every
-//      store is a full, 16 B-aligned float4 of a contiguous 64*d*4-byte run.
+//   3. step loop: each warp takes 128-step ranges of one env; a lane owns a step quad and makes
+//      two Philox4x32-10 calls for it (one per step pair: 2 categorical uniforms + 1 Box-Muller
+//      pair each, round keys from the constant bank).  Rewards go out as one float4 per lane
+//      (512 B per warp store); the quad's one-hot rows (4d floats = d float4) are re-tiled across
+//      the warp by shuffling the quads' 4d-bit strings, one 16-entry table lookup per float4
+//      (onehot_quad_store, shared with the online loop's context expansion).
 // HBM traffic is write-only: 4*(2+d+1) B per env-step (32 B for d=5), inputs are < 0.1 B/step.
 #include <string.h>
 
+#include <type_traits>
 #include <unordered_map>
 
 #include "common.cuh"
@@ -35,6 +37,7 @@ struct RollinParams {
   float var;
   int rtype;  // DPT_REWARD_*
   Key key;
+  RoundKeys rk;  // key schedule of `key` (fast path: round keys from the constant bank)
   uint64_t env_id0;
   int N, H, d, envs_per_cta;
   float *ctx_s, *ctx_a, *ctx_ns, *ctx_r;
@@ -189,23 +192,36 @@ __device__ __forceinline__ int argmax_first(const float* m, int D) {
 
 // ---------------------------------------------------------------------------------------------
 // Fast path: compile-time d (2d <= 32), H % 4 == 0, 16 B-aligned outputs.
+// A warp task is one env x 128 steps; lane l owns the step quad 4l .. 4l + 3 (never partial: H % 4 == 0, only the last range
+// of an env is ragged, predicated per quad).  Per lane and task: two Philox calls (step pairs 2l, 2l + 1 of the range: the
+// same counters as the generic path), one float4 of rewards (512 B per warp store) and D float4 of one-hot rows from the
+// quad's 4D-bit string (onehot_quad_store).
 // ---------------------------------------------------------------------------------------------
+// Resident CTAs per SM the fast kernel is compiled for: 5 up to d = 5 (48 registers; left to itself ptxas takes 50-64 and the SM
+// holds 4 CTAs: 0.320 against 0.292 ms at 125k x 500, d = 5); d = 6 .. 10: 4 (<= 64 registers); d = 16: 2 (<= 128; at 3 the
+// Philox instantiations spill).  No instantiation spills.
+#ifndef DPT_RB_MINB
+#define DPT_RB_MINB (D <= 5 ? 5 : D <= 10 ? 4 : 2)
+#endif
 template <int D, int MODE, int RT>   // RT: DPT_REWARD_* (compile-time: the kernel sits at the issue / HBM balance point)
-__global__ void __launch_bounds__(RB_THREADS) bandit_rollin_fast(const RollinParams p) {
+__global__ void __launch_bounds__(RB_THREADS, DPT_RB_MINB) bandit_rollin_fast(const RollinParams p) {
   using thr_t = typename Thr<MODE>::type;
+  using qbits_t = typename std::conditional<(4 * D > 32), uint64_t, uint32_t>::type;   // a quad's one-hot bit string
+  __shared__ float4 s_nib[16];
   __shared__ float s_means[RB_MAX_ENVS][D];
   __shared__ thr_t s_thr[RB_MAX_ENVS][D];
-  __shared__ uint32_t s_optmask[RB_MAX_ENVS];   // one-hot bits of the optimal arm in both halves of a step pair
+  __shared__ qbits_t s_optmask[RB_MAX_ENVS];   // one-hot bits of the optimal arm in all four steps of a quad
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int env0 = blockIdx.x * p.envs_per_cta;
   const int ne = min(p.envs_per_cta, p.N - env0);
   const int H = p.H;
 
   if (warp == 0) {
+    onehot_nib_init(s_nib, lane);
     if (lane < ne) {
       rollin_setup_env<MODE, D>(p, env0 + lane, D, s_means[lane], s_thr[lane]);
-      const int oa = argmax_first(s_means[lane], D);
-      s_optmask[lane] = (1u << oa) | (1u << (D + oa));
+      const qbits_t o = (qbits_t)1 << argmax_first(s_means[lane], D);
+      s_optmask[lane] = o | (o << D) | (o << (2 * D)) | (o << (3 * D));
     }
   } else {  // bandit state is the constant [1] (envs/bandit_env.py:38): dx = 1
     const size_t b = (size_t)env0 * H, e = (size_t)(env0 + ne) * H;
@@ -214,11 +230,11 @@ __global__ void __launch_bounds__(RB_THREADS) bandit_rollin_fast(const RollinPar
   }
   __syncthreads();
 
-  const int chunks = (H + 63) >> 6;
+  const int chunks = (H + 127) >> 7;
   const bool inj_actions = (MODE == MODE_INJECT) && p.in.actions != nullptr;
   float2 st_r = make_float2(0.f, 0.f), st_r2 = make_float2(0.f, 0.f);   // per pair component, packed f32x2 updates
   int st_opt = 0;
-  // (env, chunk) of this warp's task: task index t = warp + i * RB_WARPS = e * chunks + c, advanced by the
+  // (env, range) of this warp's task: task index t = warp + i * RB_WARPS = e * chunks + c, advanced by the
   // constant (de, dc) = divmod(RB_WARPS, chunks) with one predicated carry -- no division, no data-dependent loop
   const int de = RB_WARPS / chunks, dc = RB_WARPS - de * chunks;
   int e = warp / chunks, c = warp - e * chunks;
@@ -228,78 +244,72 @@ __global__ void __launch_bounds__(RB_THREADS) bandit_rollin_fast(const RollinPar
       if (e >= ne) break;
     }
     const int env = env0 + e;
-    const int h0 = c * 64 + 2 * lane;
+    const int h0 = c * 128 + 4 * lane;
+    const bool valid = h0 < H;
     const size_t row = (size_t)env * H + h0;
-    int a0 = 0, a1 = 0;
-    float z0 = 0.f, z1 = 0.f;
+    int a[4] = {0, 0, 0, 0};
+    float z[4] = {0.f, 0.f, 0.f, 0.f};
     if (MODE != MODE_INJECT) {
-      const uint4 w = philox_words(p.key, p.env_id0 + (uint64_t)env, (uint32_t)(c * 32 + lane), STREAM_ROLLIN_STEP);
-      const uint32_t k0 = w.x >> 1, k1 = w.y >> 1;
+      const uint64_t gid = p.env_id0 + (uint64_t)env;
+      const uint4 w0 = philox_words(p.rk, gid, (uint32_t)(h0 >> 1), STREAM_ROLLIN_STEP);
+      const uint4 w1 = philox_words(p.rk, gid, (uint32_t)(h0 >> 1) + 1u, STREAM_ROLLIN_STEP);
+      const uint32_t k[4] = {w0.x >> 1, w0.y >> 1, w1.x >> 1, w1.y >> 1};
+      // a = #{j : k >= t_j}.  k < 2^31 and t_j <= 2^31, so k - t_j fits in 32 bits and its sign bit is (k < t_j): one
+      // subtract and one shift-add per compare
 #pragma unroll
       for (int j = 0; j < D - 1; ++j) {
         const uint32_t t = s_thr[e][j];
-        a0 += (k0 >= t);
-        a1 += (k1 >= t);
-      }
-      if (RT == DPT_REWARD_GAUSSIAN)
-        box_muller(w.z, w.w, z0, z1);
-      else
-        z0 = u24(w.z), z1 = u24(w.w);
-      if (MODE == MODE_PHILOX_DUMP && h0 < H) {
-        if (p.out.u) {
-          p.out.u[row] = (double)k0 * 4.656612873077392578125e-10;
-          p.out.u[row + 1] = (double)k1 * 4.656612873077392578125e-10;
-        }
-        if (p.out.z) p.out.z[row] = z0, p.out.z[row + 1] = z1;
-        if (p.out.actions) p.out.actions[row] = a0, p.out.actions[row + 1] = a1;
-      }
-    } else if (h0 < H) {
-      if (inj_actions) {
-        a0 = p.in.actions[row];
-        a1 = p.in.actions[row + 1];
-      } else {  // searchsorted(cdf, u, side='right') = #{j : cdf_j <= u}
-        const double u0 = p.in.u[row], u1 = p.in.u[row + 1];
 #pragma unroll
-        for (int j = 0; j < D - 1; ++j) {
-          const double t = s_thr[e][j];
-          a0 += (t <= u0);
-          a1 += (t <= u1);
+        for (int u = 0; u < 4; ++u) a[u] -= (int)((k[u] - t) >> 31);
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) a[u] += D - 1;
+      if (RT == DPT_REWARD_GAUSSIAN) {
+        box_muller(w0.z, w0.w, z[0], z[1]);
+        box_muller(w1.z, w1.w, z[2], z[3]);
+      } else {
+        z[0] = u24(w0.z), z[1] = u24(w0.w), z[2] = u24(w1.z), z[3] = u24(w1.w);
+      }
+      if (MODE == MODE_PHILOX_DUMP && valid) {
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+          if (p.out.u) p.out.u[row + u] = (double)k[u] * 4.656612873077392578125e-10;
+          if (p.out.z) p.out.z[row + u] = z[u];
+          if (p.out.actions) p.out.actions[row + u] = a[u];
         }
       }
-      z0 = p.in.z[row];
-      z1 = p.in.z[row + 1];
-    }
-    // r = means[a] + var * z   (envs/bandit_env.py:59)
-    {
-      const float m0 = s_means[e][a0], m1 = s_means[e][a1];
-      const bool gauss = RT == DPT_REWARD_GAUSSIAN;   // else Bernoulli(mean): envs/bandit_env.py:61
-      const float r0 = gauss ? fmaf(p.var, z0, m0) : (z0 < m0 ? 1.f : 0.f);
-      const float r1 = gauss ? fmaf(p.var, z1, m1) : (z1 < m1 ? 1.f : 0.f);
-      st_stream_if(h0 < H, reinterpret_cast<float2*>(p.ctx_r + row), make_float2(r0, r1));
-      if (p.stats && h0 < H) {
-        const float2 rr = make_float2(r0, r1);
-        st_r = add2(st_r, rr);
-        st_r2 = fma2(rr, rr, st_r2);
+    } else if (valid) {
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        if (inj_actions) {
+          a[u] = p.in.actions[row + u];
+        } else {  // searchsorted(cdf, u, side='right') = #{j : cdf_j <= u}
+          const double uu = p.in.u[row + u];
+#pragma unroll
+          for (int j = 0; j < D - 1; ++j) a[u] += (s_thr[e][j] <= uu);
+        }
+        z[u] = p.in.z[row + u];
       }
     }
-    // one-hot rows: lane l holds flat elements [2D*l, 2D*(l+1)) of this chunk as a 2D-bit mask
-    const uint32_t m = (1u << a0) | (1u << (D + a1));
-    if (p.stats && h0 < H) st_opt += __popc(m & s_optmask[e]);
-    float4* abase = reinterpret_cast<float4*>(p.ctx_a + ((size_t)env * H + (size_t)c * 64) * D);
-    const int n_valid4 = (min(64, H - c * 64) * D) >> 2;
+    // r = means[a] + var * z   (envs/bandit_env.py:59); else Bernoulli(mean): envs/bandit_env.py:61
+    float r[4];
+    qbits_t bq = 0;
 #pragma unroll
-    for (int it = 0; it < (16 * D + 31) / 32; ++it) {
-      const int q = it * 32 + lane;
-      const int e0 = 4 * q;
-      const int l0 = e0 / (2 * D);
-      const int off = e0 - l0 * (2 * D);
-      const uint32_t mlo = __shfl_sync(0xffffffffu, m, l0 & 31);
-      const uint32_t mhi = __shfl_sync(0xffffffffu, m, (l0 + 1) & 31);
-      const uint32_t bits = (uint32_t)(((((uint64_t)mhi) << (2 * D)) | mlo) >> off);
-      const float4 v = make_float4((bits & 1u) ? 1.f : 0.f, (bits & 2u) ? 1.f : 0.f, (bits & 4u) ? 1.f : 0.f,
-                                   (bits & 8u) ? 1.f : 0.f);
-      st_stream_if(q < n_valid4, abase + q, v);
+    for (int u = 0; u < 4; ++u) {
+      const float m = s_means[e][a[u]];
+      r[u] = RT == DPT_REWARD_GAUSSIAN ? fmaf(p.var, z[u], m) : (z[u] < m ? 1.f : 0.f);
+      bq |= ((qbits_t)1 << a[u]) << (u * D);
     }
+    st_stream_if(valid, reinterpret_cast<float4*>(p.ctx_r + row), make_float4(r[0], r[1], r[2], r[3]));
+    if (p.stats && valid) {
+      const float2 r01 = make_float2(r[0], r[1]), r23 = make_float2(r[2], r[3]);
+      st_r = add2(add2(st_r, r01), r23);
+      st_r2 = fma2(r23, r23, fma2(r01, r01, st_r2));
+      st_opt += 4 * D > 32 ? __popcll((uint64_t)(bq & s_optmask[e])) : __popc((uint32_t)(bq & s_optmask[e]));
+    }
+    const int nq = min(32, (H - c * 128) >> 2);
+    onehot_quad_store<D>(reinterpret_cast<float4*>(p.ctx_a + ((size_t)env * H + (size_t)c * 128) * D), bq, lane, nq * D, s_nib,
+                         [](int) {});
   }
   if (p.stats) reduce_stats(p, st_r.x + st_r.y, st_r2.x + st_r2.y, (float)st_opt);
 }
@@ -407,20 +417,29 @@ template <int MODE>
 static void launch_mode(RollinParams p, bool fast, cudaStream_t st) {
   // envs per CTA: up to 32, few enough that the grid covers the machine >= 3 times, and chosen so that the
   // last wave is nearly full (the kernel's real occupancy decides what a wave is)
-  auto go = [&](auto kern) {
-    const int per_sm = resident_ctas(kern);
-    p.envs_per_cta = pick_envs_per_cta(p.N, sm_count() * per_sm, 1, RB_MAX_ENVS);
+  auto go = [&](auto kern, int step, int min_e) {
+    const int slots = sm_count() * resident_ctas(kern);
+    p.envs_per_cta = pick_envs_per_cta(p.N, slots, min_e, RB_MAX_ENVS, step);
+    if (min_e > 1 && (p.N + p.envs_per_cta - 1) / p.envs_per_cta < 3 * slots)   // small N: spread the envs over the machine
+      p.envs_per_cta = pick_envs_per_cta(p.N, slots, 1, RB_MAX_ENVS);
     const int grid = (p.N + p.envs_per_cta - 1) / p.envs_per_cta;
     kern<<<grid, RB_THREADS, 0, st>>>(p);
   };
   if (fast) {
+    // envs per CTA a multiple of `step`: the CTA's (env, 128-step range) tasks then split evenly over its warps (125k x 500:
+    // 0.307 -> 0.292 ms); and at least 4 tasks per warp, or the per-CTA setup is paid for too little work (100k x 200, d = 10:
+    // the fullest last wave alone picks 4 envs per CTA, one task per warp, 0.242 ms against 0.173 for the 64-step kernel)
+    const int chunks = (p.H + 127) >> 7;
+    int step = 1;
+    while ((step * chunks) % RB_WARPS) ++step;
+    const int min_e = (4 * RB_WARPS / chunks + step - 1) / step * step;
     switch (p.d) {
 #define DPT_CASE(DD)                                                   \
   case DD:                                                             \
     if (p.rtype == DPT_REWARD_GAUSSIAN)                                \
-      go(bandit_rollin_fast<DD, MODE, DPT_REWARD_GAUSSIAN>);           \
+      go(bandit_rollin_fast<DD, MODE, DPT_REWARD_GAUSSIAN>, step, min_e);  \
     else                                                               \
-      go(bandit_rollin_fast<DD, MODE, DPT_REWARD_BERNOULLI>);          \
+      go(bandit_rollin_fast<DD, MODE, DPT_REWARD_BERNOULLI>, step, min_e); \
     return;
       DPT_CASE(2)
       DPT_CASE(3)
@@ -435,7 +454,7 @@ static void launch_mode(RollinParams p, bool fast, cudaStream_t st) {
         break;
     }
   }
-  go(bandit_rollin_generic<MODE>);
+  go(bandit_rollin_generic<MODE>, 1, 1);
 }
 
 }  // namespace dpt
@@ -460,6 +479,7 @@ static int bandit_rollin_impl(const float* means, float var, int reward_type, ui
   p.var = var;
   p.rtype = reward_type;
   p.key = Key{(uint32_t)seed, (uint32_t)(seed >> 32)};
+  p.rk = round_keys(p.key);
   p.env_id0 = env_id0;
   p.N = N, p.H = H, p.d = d;
   p.ctx_s = ctx_states, p.ctx_a = ctx_actions, p.ctx_ns = ctx_next_states, p.ctx_r = ctx_rewards;

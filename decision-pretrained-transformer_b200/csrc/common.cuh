@@ -20,7 +20,8 @@ int bandit_rollin_compact(const float* means, float var, uint64_t seed, uint64_t
                           float* ctx_rewards, void* stream);
 // Envs per CTA such that the grid (ceil(N / e) CTAs, `slots` resident at a time) ends close to a whole number
 // of waves: among e in [min_e, max_e] with at least 3 waves, the one with the fullest last wave (ties: larger e).
-int pick_envs_per_cta(int N, int slots, int min_e, int max_e);
+// step > 1: only multiples of step are candidates; when none of them qualifies, the rule above without step.
+int pick_envs_per_cta(int N, int slots, int min_e, int max_e, int step = 1);
 
 #define DPT_CHECK_ARG(cond, ...)                \
   do {                                          \
@@ -89,6 +90,34 @@ __device__ __forceinline__ void fill_range(float* base, size_t begin, size_t end
   float4* p = reinterpret_cast<float4*>(base + b4);
   const size_t n4 = (e4 - b4) >> 2;
   for (size_t i = tid; i < n4; i += nthreads) st_stream(p + i, v4);
+}
+
+// One-hot rows from bit strings.  s_nib[t] holds the 4-bit pattern t as four 0 / 1 floats; threads 0 .. 15 fill it.
+__device__ __forceinline__ void onehot_nib_init(float4* s_nib, int t) {
+  if (t < 16) s_nib[t] = make_float4((t & 1) ? 1.f : 0.f, (t & 2) ? 1.f : 0.f, (t & 4) ? 1.f : 0.f, (t & 8) ? 1.f : 0.f);
+}
+
+// The one-hot rows of a warp task of 32 step quads (lane = quad), D floats per step.  Lane l passes its quad's 4D-bit string `bq`
+// (bit u * D + j: step u took arm j), so a quad's rows are exactly D float4 and float4 g of the task is nibble g % D of quad
+// g / D's string: D stores per lane, each one shuffle, one shift and one table lookup, 512 B per warp and store.  Float4s at
+// g >= nvalid (past the end of the row) are not stored.  per_it(it) runs after store `it`: independent work to interleave.
+template <int D, typename F>
+__device__ __forceinline__ void onehot_quad_store(float4* abase, uint64_t bq, int lane, int nvalid, const float4* s_nib, F&& per_it) {
+  const uint32_t blo = (uint32_t)bq, bhi = (uint32_t)(bq >> 32);
+#pragma unroll
+  for (int it = 0; it < D; ++it) {
+    const int g = it * 32 + lane;
+    const int src = g / D, f = g - src * D;
+    uint32_t w = __shfl_sync(0xffffffffu, blo, src);
+    if (4 * D > 32) {
+      const uint32_t wh = __shfl_sync(0xffffffffu, bhi, src);
+      w = (uint32_t)((((uint64_t)wh << 32) | w) >> (4 * f));
+    } else {
+      w >>= 4 * f;
+    }
+    st_stream_if(g < nvalid, abase + g, s_nib[w & 15u]);
+    per_it(it);
+  }
 }
 #endif
 

@@ -42,7 +42,7 @@ __global__ void __launch_bounds__(OL_THREADS) online_loop_kernel(const OnlinePar
   WarpTile& tile = tiles[warp];
   float(*s_means)[DMAX] = reinterpret_cast<float(*)[DMAX]>(s_means_all) + warp * 32;
   const int env0w = (blockIdx.x * nwarps + warp) * 32;  // first env of this warp
-  if (tid < 16) s_nib[tid] = make_float4((tid & 1) ? 1.f : 0.f, (tid & 2) ? 1.f : 0.f, (tid & 4) ? 1.f : 0.f, (tid & 8) ? 1.f : 0.f);
+  onehot_nib_init(s_nib, tid);
   const int env = env0w + lane;
   const bool live = env < p.N;
   const int N = p.N, H = p.H, d = p.d;

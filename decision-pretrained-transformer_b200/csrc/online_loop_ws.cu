@@ -545,7 +545,7 @@ __global__ void __launch_bounds__(WS_NCONS * 32, ws_min_blocks<DMAX, KIND>()) on
   Cons* cons = reinterpret_cast<Cons*>(smem_raw);
   double* s_arms = reinterpret_cast<double*>(smem_raw + sizeof(Cons) * WS_NCONS);   // [d][LIN_AW] (LinUCB)
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid < 16) s_nib[tid] = make_float4((tid & 1) ? 1.f : 0.f, (tid & 2) ? 1.f : 0.f, (tid & 4) ? 1.f : 0.f, (tid & 8) ? 1.f : 0.f);
+  onehot_nib_init(s_nib, tid);
   if (KIND == K_LINUCB2)
     for (int j = tid; j < p.d; j += blockDim.x) lin_arm_row(s_arms + LIN_AW * j, p.arms[2 * j], p.arms[2 * j + 1]);
   __syncthreads();
@@ -624,10 +624,7 @@ __global__ void __launch_bounds__(EX_WARPS * 32, DPT_EX_MINB) online_expand_kern
   DPT_TL(10);
   __shared__ float4 s_nib[16];   // 4-bit pattern -> four 0/1 floats
   __shared__ uint32_t s_arm[EX_WARPS][EX_Q][33];   // per warp: arms words [quad][env], read back by lane = quad (conflict-free)
-  if (threadIdx.x < 16) {
-    const int t = threadIdx.x;
-    s_nib[t] = make_float4((t & 1) ? 1.f : 0.f, (t & 2) ? 1.f : 0.f, (t & 4) ? 1.f : 0.f, (t & 8) ? 1.f : 0.f);
-  }
+  onehot_nib_init(s_nib, threadIdx.x);
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int N = p.N, H = p.H;
@@ -690,24 +687,10 @@ __global__ void __launch_bounds__(EX_WARPS * 32, DPT_EX_MINB) online_expand_kern
       const double v = __shfl_up_sync(0xffffffffu, sc, o);
       if (lane >= o) sc += v;
     };
-    // one-hot rows: the task's 32 quads are 32 D float4; float4 g is nibble g % D of the bit string of quad g / D
-    float4* abase = reinterpret_cast<float4*>(p.ctx_a + row * D);
-    const uint32_t blo = (uint32_t)bq, bhi = (uint32_t)(bq >> 32);
-    const int nvalid = nq * D;
-#pragma unroll
-    for (int it = 0; it < D; ++it) {
-      const int g = it * 32 + lane;
-      const int src = g / D, f = g - src * D;
-      uint32_t w = __shfl_sync(0xffffffffu, blo, src);
-      if (4 * D > 32) {
-        const uint32_t wh = __shfl_sync(0xffffffffu, bhi, src);
-        w = (uint32_t)((((uint64_t)wh << 32) | w) >> (4 * f));
-      } else {
-        w >>= 4 * f;
-      }
-      st_stream_if(g < nvalid, abase + g, s_nib[w & 15u]);
+    // one-hot rows: the task's 32 quads are 32 D float4
+    onehot_quad_store<D>(reinterpret_cast<float4*>(p.ctx_a + row * D), bq, lane, nq * D, s_nib, [&](int it) {
       if (REG && it < 5) scan_round(1 << it);
-    }
+    });
     if (REG) {
 #pragma unroll
       for (int it = D; it < 5; ++it) scan_round(1 << it);

@@ -24,24 +24,49 @@ struct Key {
   uint32_t k0, k1;
 };
 
+// The key schedule written out: round r uses (k0 + r * 0x9E3779B9, k1 + r * 0xBB67AE85).  Computed on the host into a kernel
+// parameter, the round keys sit in the constant bank and each round's XOR takes them as an operand instead of recomputing the
+// schedule in the kernel's loop.
+struct RoundKeys {
+  uint32_t k0[10], k1[10];
+};
+__host__ __device__ inline RoundKeys round_keys(Key key) {
+  RoundKeys rk;
+  for (int r = 0; r < 10; ++r) rk.k0[r] = key.k0 + (uint32_t)r * 0x9E3779B9u, rk.k1[r] = key.k1 + (uint32_t)r * 0xBB67AE85u;
+  return rk;
+}
+
+__device__ __forceinline__ void philox_round(uint32_t& c0, uint32_t& c1, uint32_t& c2, uint32_t& c3, uint32_t k0, uint32_t k1) {
+  const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+  const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+  c0 = hi1 ^ c1 ^ k0;
+  c1 = lo1;
+  c2 = hi0 ^ c3 ^ k1;
+  c3 = lo0;
+}
+
 __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, Key key) {
   uint32_t k0 = key.k0, k1 = key.k1;
 #pragma unroll
   for (int r = 0; r < 10; ++r) {
-    uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-    uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-    c0 = hi1 ^ c1 ^ k0;
-    c1 = lo1;
-    c2 = hi0 ^ c3 ^ k1;
-    c3 = lo0;
+    philox_round(c0, c1, c2, c3, k0, k1);
     k0 += 0x9E3779B9u;
     k1 += 0xBB67AE85u;
   }
   return make_uint4(c0, c1, c2, c3);
 }
 
+__device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, const RoundKeys& rk) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) philox_round(c0, c1, c2, c3, rk.k0[r], rk.k1[r]);
+  return make_uint4(c0, c1, c2, c3);
+}
+
 __device__ __forceinline__ uint4 philox_words(Key key, uint64_t env, uint32_t index, uint32_t stream) {
   return philox4x32_10(index, (uint32_t)env, (uint32_t)(env >> 32), stream, key);
+}
+__device__ __forceinline__ uint4 philox_words(const RoundKeys& rk, uint64_t env, uint32_t index, uint32_t stream) {
+  return philox4x32_10(index, (uint32_t)env, (uint32_t)(env >> 32), stream, rk);
 }
 
 __device__ __forceinline__ uint32_t word_of(uint4 w, int i) {
