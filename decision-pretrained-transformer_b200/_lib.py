@@ -10,7 +10,7 @@ from ctypes import (POINTER, Structure, c_char_p, c_double, c_float, c_int, c_in
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DPT_B200_LIB") or os.path.join(_HERE, "libdpt_b200.so")   # override: A/B builds of the same ABI
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 OK, ERR_INVALID_ARG, ERR_CUDA, ERR_UNSUPPORTED = 0, -1, -2, -3
 
@@ -69,6 +69,14 @@ class ExploreDump(Structure):
                 ("logits_exploiter", c_void_p)]
 
 
+class OfflineParams(Structure):
+    _fields_ = [("N", c_int), ("d", c_int), ("H_stride", c_int), ("K", c_int), ("horizons_host", c_void_p), ("ctrl_mask", c_int),
+                ("lcb_const", c_double), ("thmp_std", c_double), ("thmp_prior_mean", c_double), ("thmp_prior_var", c_double),
+                ("n_draws", c_int), ("arms", c_void_p), ("lin_d", c_int), ("linreg_const", c_double),
+                ("learner_logits", c_void_p), ("logits_T", c_int), ("seed", c_uint64), ("env_id0", c_uint64),
+                ("inject_z", c_void_p), ("dump_z", c_void_p)]
+
+
 # name -> (restype, argtypes); every symbol include/dpt_b200.h declares
 PROTOTYPES = {
     "dpt_version": (c_int, []),
@@ -106,6 +114,7 @@ PROTOTYPES = {
     "dpt_online_loop": (c_int, [c_int, c_double, c_double, c_double, c_void_p, c_void_p, c_int, c_double, c_int, c_uint64,
                                 c_uint64, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                 c_void_p, POINTER(OnlineInject), POINTER(OnlineDump), c_void_p]),
+    "dpt_offline_eval": (c_int, [POINTER(OfflineParams), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "dpt_debug_umma_gemm": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "dpt_gpt2_create": (c_int, [POINTER(Gpt2Weights), POINTER(c_void_p), c_void_p]),
     "dpt_gpt2_destroy": (c_int, [c_void_p]),

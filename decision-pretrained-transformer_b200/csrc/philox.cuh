@@ -18,6 +18,7 @@ enum : uint32_t {
   STREAM_DARKROOM_QUERY = 4,  // query state per sample
   STREAM_ENV_REWARD = 5,      // env.step reward noise (index = step pair)
   STREAM_CTRL = 6,            // controller draws
+  STREAM_OFFLINE = 7,         // offline evaluation: Thompson sample=False draws (index = (slot * n_draws + draw) * ceil(d/4) + block)
 };
 
 struct Key {

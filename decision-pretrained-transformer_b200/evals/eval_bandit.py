@@ -173,9 +173,91 @@ def offline(eval_trajs, model, n_eval, horizon, var, bandit_type="uniform", np_r
     return baselines
 
 
-def offline_graph(eval_trajs, model, n_eval, horizon, var, bandit_type="uniform"):
+def _offline_context(batch_or_trajs, means, n_eval=None):
+    """(means [N,d], context dict of fp32 device tensors [N,H,.]) from a device batch (e.g. collect_data.collect_bandit's
+    dict, used as is) or from the reference's list of traj dicts (stacked once)."""
+    dev = kernels._dev()
+    if isinstance(batch_or_trajs, dict):
+        ctx = {k: batch_or_trajs[k] for k in ("context_states", "context_actions", "context_next_states", "context_rewards")}
+        if means is None:
+            means = batch_or_trajs["means"]
+    else:
+        trajs = list(batch_or_trajs)[:n_eval]
+        f = lambda k, tail: torch.as_tensor(np.stack([np.asarray(t[k], dtype=np.float32).reshape((-1,) + tail) for t in trajs])).to(dev)  # noqa: E731
+        d = np.asarray(trajs[0]["context_actions"]).shape[-1]
+        ctx = {"context_states": f("context_states", (1,)), "context_actions": f("context_actions", (d,)),
+               "context_next_states": f("context_next_states", (1,)), "context_rewards": f("context_rewards", (1,))}
+        if means is None:
+            means = np.stack([np.asarray(t["means"], dtype=np.float64) for t in trajs])
+    means = torch.as_tensor(means).to(device=dev, dtype=torch.float32) if not torch.is_tensor(means) else means.to(dev).float()
+    return means, ctx
+
+
+def learner_logits(model, ctx, T):
+    """Logits of every context prefix 0..T-1 in one forward: row h-1 of the test=False forward over ``ctx[:, :T]``
+    attends to the query token and the first h transitions at the same positions as the reference's test=True forward
+    on ``ctx[:, :h]`` (models/net.py:41-60).  [N, T, d] fp32."""
+    N = ctx["context_actions"].shape[0]
+    dev = ctx["context_actions"].device
+    was_test = model.test
+    model.test = False
+    try:
+        x = {k: v[:, :T] for k, v in ctx.items()}
+        x["query_states"] = torch.ones((N, 1), dtype=torch.float32, device=dev)   # the bandit state is the constant [1]
+        return model.forward(x)
+    finally:
+        model.test = was_test
+
+
+def offline_device(batch_or_trajs, means, horizons, model=None, var=None, seed=None, env_id0=0, per_env=True, inject=None,
+                   dump=False, n_eval=None, ctrls=("opt", "emp", "lcb", "thmp")):
+    """``offline`` for every horizon in ``horizons`` at once, on the device (dpt_offline_eval): one pass over the
+    context gives the noise-free reward of Opt, EmpMean, LCB(0.8), Thompson(sample=False, prior 0.5 / (1/12),
+    std = var) and, with a model, the transformer (one test=False forward over max(horizons) rows).
+
+    batch_or_trajs: a dict of device tensors with context_* [N,H,.] (and ``means`` when ``means`` is None), e.g.
+    collect_data.collect_bandit's output, or the reference's list of traj dicts.  inject: {'z': f64 [K,100,N,d]} the
+    Thompson normals in the reference's order; dump=True returns the normals used.  Returns kernels.offline_eval's dict
+    (sums [K,6,2], rewards [K,6,N] when per_env, slots kernels.OFFLINE_SLOTS) plus 'horizons', 'n_envs' and 'ctrls'
+    (the slots that were computed)."""
+    if var is None:
+        raise ValueError("offline_device: var (the Thompson std, as in offline()) is required")
+    means, ctx = _offline_context(batch_or_trajs, means, n_eval)
+    hz = np.asarray(horizons, dtype=np.int64).reshape(-1)
+    ctrls = tuple(ctrls)
+    logits = None
+    if model is not None:
+        ctrls = ctrls + ("lnr",)
+        logits = learner_logits(model, ctx, int(hz.max()))
+    key = rng.next_key() if seed is None else seed
+    out = kernels.offline_eval(means, ctx["context_actions"], ctx["context_rewards"], hz, ctrls, lcb_const=.8, thmp_std=var,
+                               thmp_prior_mean=0.5, thmp_prior_var=1 / 12.0, n_draws=100, learner_logits=logits, seed=key,
+                               env_id0=env_id0, per_env=per_env, inject=inject, dump=dump)
+    out["horizons"], out["n_envs"] = hz, means.shape[0]
+    out["ctrls"] = ("opt",) + tuple(c for c in ctrls if c != "opt")
+    return out
+
+
+def _names(ctrls):
+    return [c for c in ("opt", "emp", "lnr", "lcb", "thmp", "linreg") if c in ctrls]   # the reference's dict order
+
+
+def offline_graph_device(batch_or_trajs, means, horizon, model=None, var=None, seed=None, env_id0=0, n_eval=None):
+    """``offline_graph`` from one dpt_offline_eval launch over np.linspace(1, horizon, 50, dtype=int).  Returns
+    (horizons [50], {name: regret of the mean per horizon}) with sums over envs left on the device until the end."""
+    horizons = np.linspace(1, horizon, 50, dtype=int)
+    out = offline_device(batch_or_trajs, means, horizons, model, var, seed, env_id0, per_env=False, n_eval=n_eval)
+    s = out["sums"].cpu().numpy()
+    regrets = {k: s[:, kernels.OFFLINE_SLOTS.index(k), 0] / out["n_envs"] for k in _names(out["ctrls"]) if k != "opt"}
+    return horizons, regrets
+
+
+def offline_graph(eval_trajs, model, n_eval, horizon, var, bandit_type="uniform", fused=False):
     """evals/eval_bandit.py:304-335 without plotting: suboptimality against dataset size.  Returns
-    (horizons [50], {name: regret-of-the-mean per horizon})."""
+    (horizons [50], {name: regret-of-the-mean per horizon}).  fused=True computes the same curves from one
+    offline_eval launch (``offline_graph_device``) instead of 50 ``offline`` calls."""
+    if fused:
+        return offline_graph_device(eval_trajs, None, horizon, model, var, n_eval=n_eval)
     horizons = np.linspace(1, horizon, 50, dtype=int)
     all_means = []
     for h in horizons:

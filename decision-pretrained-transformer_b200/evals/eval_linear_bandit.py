@@ -3,10 +3,11 @@
 offline evaluation (:202-330) on the first ``horizon`` rows of each eval trajectory."""
 import numpy as np
 
+from .. import kernels, rng
 from ..ctrls.ctrl_bandit import (BanditTransformerController, EmpMeanPolicy, LinUCBPolicy, OptPolicy,  # noqa: F401
                                  ThompsonSamplingPolicy)
 from ..envs.bandit_env import BanditEnvVec, LinearBanditEnv
-from .eval_bandit import deploy_online, deploy_online_vec, deploy_online_vec_device, regret_stats  # noqa: F401
+from .eval_bandit import _offline_context, deploy_online, deploy_online_vec, deploy_online_vec_device, learner_logits, regret_stats  # noqa: F401
 
 
 def online(eval_trajs, model, n_eval, horizon, var):
@@ -60,9 +61,53 @@ def offline(eval_trajs, model, n_eval, horizon, var):
     return baselines
 
 
-def offline_graph(eval_trajs, model, n_eval, horizon, var):
+def offline_device(batch_or_trajs, means, horizons, model=None, var=None, arms=None, seed=None, env_id0=0, per_env=True,
+                   inject=None, dump=False, n_eval=None):
+    """``offline`` for every horizon in ``horizons`` at once, on the device (dpt_offline_eval): Opt, Thompson
+    (sample=False, prior 0 / 1, std = var), LinReg (LinUCB with const 0 on ``arms`` [d, lin_d], lin_d <= 8; taken from
+    the trajs when not given) and, with a model, the transformer.  Arguments and result as eval_bandit.offline_device."""
+    if var is None:
+        raise ValueError("offline_device: var (the Thompson std, as in offline()) is required")
+    if arms is None:
+        arms = batch_or_trajs["arms"] if isinstance(batch_or_trajs, dict) else batch_or_trajs[0]["arms"]
+    means, ctx = _offline_context(batch_or_trajs, means, n_eval)
+    hz = np.asarray(horizons, dtype=np.int64).reshape(-1)
+    ctrls = ("opt", "thmp", "linreg")
+    logits = None
+    if model is not None:
+        ctrls = ctrls + ("lnr",)
+        logits = learner_logits(model, ctx, int(hz.max()))
+    key = rng.next_key() if seed is None else seed
+    out = kernels.offline_eval(means, ctx["context_actions"], ctx["context_rewards"], hz, ctrls, thmp_std=var,
+                               thmp_prior_mean=0.0, thmp_prior_var=1.0, n_draws=100, arms=np.asarray(arms, dtype=np.float64),
+                               linreg_const=0.0, learner_logits=logits, seed=key, env_id0=env_id0, per_env=per_env,
+                               inject=inject, dump=dump)
+    out["horizons"], out["n_envs"], out["ctrls"] = hz, means.shape[0], ctrls
+    return out
+
+
+def offline_graph_device(batch_or_trajs, means, horizon, model=None, var=None, arms=None, seed=None, env_id0=0, n_eval=None):
+    """``offline_graph`` from one dpt_offline_eval launch over every dataset size 1..horizon.  Returns
+    (horizons, {name: (mean, sem) of opt - name per horizon}); sem is NaN for a single env, like the default path."""
+    horizons = np.linspace(1, horizon, horizon, dtype=int)
+    out = offline_device(batch_or_trajs, means, horizons, model, var, arms, seed, env_id0, per_env=False, n_eval=n_eval)
+    s, n = out["sums"].cpu().numpy(), out["n_envs"]
+    res = {}
+    for k in ("lnr", "thmp", "linreg"):                          # the reference's dict order
+        if k in out["ctrls"]:
+            s1, s2 = s[:, kernels.OFFLINE_SLOTS.index(k), 0], s[:, kernels.OFFLINE_SLOTS.index(k), 1]
+            mean = s1 / n
+            sem = np.sqrt(np.maximum(s2 - s1 * mean, 0.0) / (n - 1)) / np.sqrt(n) if n > 1 else np.full(len(horizons), np.nan)
+            res[k] = (mean, sem)
+    return horizons, res
+
+
+def offline_graph(eval_trajs, model, n_eval, horizon, var, fused=False):
     """evals/eval_linear_bandit.py:289-330 without plotting: suboptimality for every dataset size 1..horizon.
-    Returns (horizons, {name: (mean, sem) of opt - name per horizon})."""
+    Returns (horizons, {name: (mean, sem) of opt - name per horizon}).  fused=True computes the same from one
+    offline_eval launch (``offline_graph_device``) instead of ``horizon`` ``offline`` calls."""
+    if fused:
+        return offline_graph_device(eval_trajs, None, horizon, model, var, n_eval=n_eval)
     horizons = np.linspace(1, horizon, horizon, dtype=int)
     sub_mean, sub_sem = {}, {}
     for h in horizons:

@@ -340,3 +340,87 @@ def darkroom_policy_rollout(logits, goals, dim, horizon, sample, seed, env_id0=0
                                             ptr(out["rewards"]), ptr(out["returns"]), ptr(inj), ptr(out.get("u")), stream_ptr()),
           "dpt_darkroom_policy_rollout")
     return out
+
+
+# ------------------------------------------------------------------ offline evaluation ---------
+OFFLINE_SLOTS = ("opt", "emp", "lcb", "thmp", "linreg", "lnr")   # slot order of dpt_offline_eval (DPT_OFFLINE_*)
+
+
+def _rows(t, N, d):
+    """(tensor, row stride in steps) of a [N, T, d] context tensor or a [:, :T] view of one, without a copy when the
+    rows are laid out as [N, H_stride, d]."""
+    if t.dim() == 2:
+        t = t.unsqueeze(-1)
+    if t.stride(-1) == 1 and t.stride(1) == d and t.stride(0) % d == 0 and t.stride(0) // d >= t.shape[1]:
+        return t, t.stride(0) // d
+    t = t.contiguous()
+    return t, t.shape[1]
+
+
+def offline_eval(means, ctx_actions, ctx_rewards, horizons, ctrls=("opt", "emp", "lcb", "thmp"), lcb_const=0.8,
+                 thmp_std=0.3, thmp_prior_mean=0.5, thmp_prior_var=1 / 12.0, n_draws=100, arms=None, linreg_const=0.0,
+                 learner_logits=None, seed=0, env_id0=0, per_env=True, inject=None, dump=False, sums=None):
+    """Offline evaluation of every horizon in ``horizons`` in one launch (dpt_offline_eval).
+
+    means [N,d], ctx_actions [N,H,d] one-hot and ctx_rewards [N,H(,1)] fp32 device tensors (views ``[:, :h]`` of a
+    larger buffer pass without a copy); horizons: ints in [1, H], any order, duplicates allowed.  ``ctrls`` picks slots
+    of OFFLINE_SLOTS: 'linreg' needs ``arms`` [d, lin_d], 'lnr' needs ``learner_logits`` [N, T >= max(horizons), d]
+    (the test=False forward).  inject: {'z': f64 [K, n_draws, N, d]} Thompson normals; dump=True returns them as
+    out['noise']['z'].  ``sums`` may be a caller's f64 [K, 6, 2] tensor to accumulate into (shards).
+    Returns dict: sums [K, 6, 2] f64 (sum over envs of max mean - reward and its square; unselected slots stay 0),
+    rewards [K, 6, N] f64 when per_env (unselected slots 0)."""
+    import numpy as np
+    dev = _dev(means.device if torch.is_tensor(means) and means.is_cuda else None)
+    means = _as(means, F32, dev)
+    N, d = means.shape
+    hz = np.ascontiguousarray(np.asarray(horizons, dtype=np.int64).reshape(-1)).astype(np.int32)
+    K = hz.shape[0]
+    unknown = set(ctrls) - set(OFFLINE_SLOTS)
+    if unknown:
+        raise ValueError("offline_eval: unknown controllers %s (slots: %s)" % (sorted(unknown), OFFLINE_SLOTS))
+    mask = sum(1 << OFFLINE_SLOTS.index(c) for c in ctrls)
+    ca, cr, hs = None, None, 1
+    if ctx_actions is not None:
+        ca = ctx_actions if torch.is_tensor(ctx_actions) and ctx_actions.device == dev and ctx_actions.dtype == F32 else _as(ctx_actions, F32, dev)
+        cr = ctx_rewards if torch.is_tensor(ctx_rewards) and ctx_rewards.device == dev and ctx_rewards.dtype == F32 else _as(ctx_rewards, F32, dev)
+        if K and int(hz.max()) > ca.shape[1]:
+            raise ValueError("offline_eval: horizon %d > context length %d" % (int(hz.max()), ca.shape[1]))
+        ca, hs = _rows(ca, N, d)
+        cr, hr = _rows(cr, N, 1)
+        if hr != hs:
+            ca, cr, hs = ca.contiguous(), cr.contiguous(), ca.shape[1]
+    elif K:
+        hs = int(hz.max())
+    out = {"sums": sums if sums is not None else torch.zeros((K, len(OFFLINE_SLOTS), 2), dtype=F64, device=dev)}
+    if per_env:
+        out["rewards"] = torch.zeros((K, len(OFFLINE_SLOTS), N), dtype=F64, device=dev)
+    keep = []
+    prm = _lib.OfflineParams()
+    prm.N, prm.d, prm.H_stride, prm.K = N, d, hs, K
+    prm.horizons_host = hz.ctypes.data
+    prm.ctrl_mask = mask
+    prm.lcb_const = float(lcb_const)
+    prm.thmp_std, prm.thmp_prior_mean, prm.thmp_prior_var = float(thmp_std), float(thmp_prior_mean), float(thmp_prior_var)
+    prm.n_draws = int(n_draws)
+    if arms is not None:
+        arms_t = _as(arms, F64, dev)
+        keep.append(arms_t)
+        prm.arms, prm.lin_d = arms_t.data_ptr(), arms_t.shape[1]
+    prm.linreg_const = float(linreg_const)
+    if learner_logits is not None:
+        lg = learner_logits.to(device=dev, dtype=F32).contiguous()
+        keep.append(lg)
+        prm.learner_logits, prm.logits_T = lg.data_ptr(), lg.shape[1]
+    prm.seed, prm.env_id0 = int(seed), int(env_id0)
+    if inject is not None and inject.get("z") is not None:
+        z = _as(inject["z"], F64, dev)
+        assert z.shape == (K, int(n_draws), N, d), z.shape
+        keep.append(z)
+        prm.inject_z = z.data_ptr()
+    if dump:
+        out["noise"] = {"z": torch.empty((K, int(n_draws), N, d), dtype=F64, device=dev)}
+        prm.dump_z = out["noise"]["z"].data_ptr()
+    check(lib().dpt_offline_eval(ctypes.byref(prm), ptr(means), ca.data_ptr() if ca is not None else None,
+                                 cr.data_ptr() if cr is not None else None, ptr(out["sums"]), ptr(out.get("rewards")),
+                                 stream_ptr()), "dpt_offline_eval")
+    return out

@@ -35,7 +35,7 @@ extern "C" {
 #define DPT_ERR_CUDA (-2)
 #define DPT_ERR_UNSUPPORTED (-3)
 
-#define DPT_ABI_VERSION 3
+#define DPT_ABI_VERSION 4
 
 /* reward_type of the bandit entry points (envs/bandit_env.py:56-63, envs/gpu_bandit_env.py:53-63):
  * 0 'uniform'  : r = means[a] + var * z, z ~ N(0,1);
@@ -238,6 +238,58 @@ int dpt_online_loop(int ctrl_kind, double p0, double p1, double p2, const float*
                     float* ctx_actions, float* ctx_next_states, float* ctx_rewards, float* cum_means,
                     double* regret_sums, const dpt_online_inject_t* inject, const dpt_online_dump_t* dump,
                     void* stream);
+
+/* ---------------------------------------------------------------- L2: offline evaluation ----
+ * evals/eval_bandit.py:214-335 (offline / offline_graph) and evals/eval_linear_bandit.py:202-330 for a whole horizon list
+ * in ONE launch: for every env and every entry k of horizons_host, each selected controller sees the first h = horizons[k]
+ * context rows and plays one noise-free pull (BanditEnvVec.deploy_eval, envs/bandit_env.py:115-123: reward = means[a]).
+ * The context is read once (one warp per env, horizons visited in ascending order).
+ * Slots (bit c of ctrl_mask selects slot c; the output layout always has DPT_OFFLINE_NSLOTS slots):
+ *   0 opt    OptPolicy: the first best arm
+ *   1 emp    EmpMeanPolicy(online=False): argmax b / max(1, n)
+ *   2 lcb    PessMeanPolicy (ctrls/ctrl_bandit.py:255-314): argmax b/max(1,n) - lcb_const/max(1, sqrt(n))
+ *   3 thmp   ThompsonSamplingPolicy(sample=False) :122-251: posterior from (thmp_std, prior_mean, prior_var), n_draws
+ *            float64 draws mu + sqrt(v) z, argmax of each, the arm that won most often
+ *   4 linreg LinUCBPolicy(const = linreg_const) :447-528: arms f64 [d, lin_d], theta = (I + sum_a n_a x_a x_a^T)^-1 sum_a b_a x_a,
+ *            value theta.x + c sqrt(x^T Sigma^-1 x)
+ *   5 lnr    BanditTransformerController(sample=False): argmax of row h-1 of learner_logits [N, logits_T, d] fp32, the
+ *            test=False forward over the full context (row h-1 attends to the same tokens as the test=True forward on
+ *            context[:, :h])
+ * Every argmax takes the first maximum.  Inputs: means [N,d] fp32, ctx_actions [N,H_stride,d] fp32 one-hot (the arm of a
+ * step is the first max of its row), ctx_rewards [N,H_stride] fp32; horizons_host is a HOST array [K], each in [1, H_stride],
+ * any order, duplicates allowed.  Outputs: sums f64 [K, NSLOTS, 2] += over envs of (max mean - reward, its square) for the
+ * selected slots (zeroed by the caller, accumulated with atomics, so shards may share it; other slots are not written);
+ * rewards f64 [K, NSLOTS, N] (NULL = skip; only selected slots are written).  Thompson normals: Philox, key = seed,
+ * counter ((k * n_draws + draw) * ceil(d/4) + block, global env id, STREAM 7), 4 normals per block; inject_z / dump_z f64
+ * [K, n_draws, N, d] (the reference's np.random.normal order per horizon; local env index).  The (horizon, slot) schedule
+ * is copied to stream-ordered device scratch from pageable host memory, so the call is not graph-capturable. */
+#define DPT_OFFLINE_OPT 0
+#define DPT_OFFLINE_EMP 1
+#define DPT_OFFLINE_LCB 2
+#define DPT_OFFLINE_THMP 3
+#define DPT_OFFLINE_LINREG 4
+#define DPT_OFFLINE_LNR 5
+#define DPT_OFFLINE_NSLOTS 6
+
+typedef struct {
+  int N, d, H_stride, K;
+  const int32_t* horizons_host;  /* [K] */
+  int ctrl_mask;
+  double lcb_const;
+  double thmp_std, thmp_prior_mean, thmp_prior_var;
+  int n_draws;
+  const double* arms;            /* [d, lin_d] */
+  int lin_d;
+  double linreg_const;
+  const float* learner_logits;   /* [N, logits_T, d] */
+  int logits_T;
+  uint64_t seed, env_id0;
+  const double* inject_z;        /* [K, n_draws, N, d] or NULL */
+  double* dump_z;                /* [K, n_draws, N, d] or NULL */
+} dpt_offline_params_t;
+
+int dpt_offline_eval(const dpt_offline_params_t* params, const float* means, const float* ctx_actions,
+                     const float* ctx_rewards, double* sums, double* rewards, void* stream);
 
 /* ---------------------------------------------------------------- M1: Transformer ----------
  * models/net.py:9-60 (GPT2Model trunk with n_head = 1, embed_transition, pred_actions).
