@@ -15,6 +15,7 @@ from .ctrls import ctrl_bandit, ctrl_darkroom   # noqa: F401
 from .evals import eval_bandit, eval_linear_bandit, eval_darkroom, eval_interactive_bandit   # noqa: F401
 from . import models, dataset             # noqa: F401
 from .models import net                   # noqa: F401
+from . import train                       # noqa: F401
 
 __all__ = ["seed", "kernels", "envs", "collect_data", "install_dropin"]
 

@@ -10,7 +10,7 @@ from ctypes import (POINTER, Structure, c_char_p, c_double, c_float, c_int, c_in
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DPT_B200_LIB") or os.path.join(_HERE, "libdpt_b200.so")   # override: A/B builds of the same ABI
-ABI_VERSION = 4
+ABI_VERSION = 5
 
 OK, ERR_INVALID_ARG, ERR_CUDA, ERR_UNSUPPORTED = 0, -1, -2, -3
 
@@ -46,6 +46,15 @@ class Gpt2Weights(Structure):
                 ("n_positions", c_int),
                 ("wpe", c_void_p), ("embed_w", c_void_p), ("embed_b", c_void_p), ("pred_w", c_void_p),
                 ("pred_b", c_void_p), ("lnf_w", c_void_p), ("lnf_b", c_void_p),
+                ("ln1_w", POINTER(c_void_p)), ("ln1_b", POINTER(c_void_p)), ("attn_w", POINTER(c_void_p)),
+                ("attn_b", POINTER(c_void_p)), ("proj_w", POINTER(c_void_p)), ("proj_b", POINTER(c_void_p)),
+                ("ln2_w", POINTER(c_void_p)), ("ln2_b", POINTER(c_void_p)), ("fc_w", POINTER(c_void_p)),
+                ("fc_b", POINTER(c_void_p)), ("fc2_w", POINTER(c_void_p)), ("fc2_b", POINTER(c_void_p))]
+
+
+class Gpt2Grads(Structure):
+    _fields_ = [("wpe", c_void_p), ("embed_w", c_void_p), ("embed_b", c_void_p), ("pred_w", c_void_p), ("pred_b", c_void_p),
+                ("lnf_w", c_void_p), ("lnf_b", c_void_p),
                 ("ln1_w", POINTER(c_void_p)), ("ln1_b", POINTER(c_void_p)), ("attn_w", POINTER(c_void_p)),
                 ("attn_b", POINTER(c_void_p)), ("proj_w", POINTER(c_void_p)), ("proj_b", POINTER(c_void_p)),
                 ("ln2_w", POINTER(c_void_p)), ("ln2_b", POINTER(c_void_p)), ("fc_w", POINTER(c_void_p)),
@@ -121,6 +130,11 @@ PROTOTYPES = {
     "dpt_gpt2_forward_workspace_bytes": (c_uint64, [c_void_p, c_int, c_int, c_int]),
     "dpt_gpt2_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
                                  c_int, c_int, c_int, c_void_p, c_void_p, c_uint64, c_void_p]),
+    "dpt_gpt2_train_workspace_bytes": (c_uint64, [POINTER(Gpt2Weights), c_int, c_int]),
+    "dpt_gpt2_train_forward": (c_int, [POINTER(Gpt2Weights), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int,
+                                       c_int, c_void_p, c_void_p, c_uint64, c_void_p]),
+    "dpt_gpt2_train_backward": (c_int, [POINTER(Gpt2Weights), c_void_p, c_int, c_int, c_int, POINTER(Gpt2Grads), c_void_p,
+                                        c_uint64, c_void_p]),
     "dpt_darkroom_policy_rollout": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_uint64, c_uint64, c_int64,
                                             c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                             c_void_p]),

@@ -7,8 +7,14 @@
 // LDS.128 (all threads of a warp read the same address) and keeps 32 outputs in registers.  Attention is a
 // per-row online softmax over the keys <= t (K/V rows broadcast from shared memory).  Compared with the
 // token-sequential kernel there is no K/V traffic to HBM and all tokens of a sequence advance in parallel.
+//
+// SAVE = true is the forward of training (gpt2_train.cu): the same arithmetic on the parameter tensors as they are
+// (embed_transition.weight [E, din], pred_actions.weight [du, E] instead of the handle's transposed copies), and
+// every row also stores what the backward needs (TrainSave, layout TA_* / TF_* in gpt2_model.cuh).  Its logits are
+// bit-identical to SAVE = false.
 #include "common.cuh"
 #include "gpt2_model.cuh"
+#include "gpt2_fp32.cuh"
 
 namespace dpt {
 
@@ -20,50 +26,8 @@ constexpr int DF_WFC2 = DF_WFC + 32 * 128;     // [128][32]
 constexpr int DF_K = DF_WFC2 + 128 * 32;       // [THREADS][32], then V [THREADS][32]
 constexpr int df_floats(int threads) { return DF_K + 2 * threads * 32; }   // 80 KB / 112 KB / 176 KB
 
-__device__ __forceinline__ float2 ffma2_(float2 a, float2 b, float2 c) {
-  float2 d;
-  asm("fma.rn.f32x2 %0, %1, %2, %3;"
-      : "=l"(reinterpret_cast<unsigned long long&>(d))
-      : "l"(reinterpret_cast<unsigned long long&>(a)), "l"(reinterpret_cast<unsigned long long&>(b)),
-        "l"(reinterpret_cast<unsigned long long&>(c)));
-  return d;
-}
-
-// acc[0..31] += sum_i xs[i] * W[i][col0 .. col0+31],  W in shared memory with row stride `ld` floats
-template <int IN>
-__device__ __forceinline__ void row_matvec32(const float* xs, const float* W, int ld, int col0, float2* acc) {
-#pragma unroll 4
-  for (int i = 0; i < IN; ++i) {
-    const float2 xx = make_float2(xs[i], xs[i]);
-    const float4* row = reinterpret_cast<const float4*>(W + i * ld + col0);
-#pragma unroll
-    for (int o = 0; o < 8; ++o) {
-      const float4 w = row[o];
-      acc[2 * o] = ffma2_(xx, make_float2(w.x, w.y), acc[2 * o]);
-      acc[2 * o + 1] = ffma2_(xx, make_float2(w.z, w.w), acc[2 * o + 1]);
-    }
-  }
-}
-
-__device__ __forceinline__ void ln_row_f(const float* x, const float* w, const float* b, float* y) {
-  float mean = 0.f;
-#pragma unroll
-  for (int c = 0; c < G_E; ++c) mean += x[c];
-  mean *= (1.0f / G_E);
-  float var = 0.f;
-#pragma unroll
-  for (int c = 0; c < G_E; ++c) var = fmaf(x[c] - mean, x[c] - mean, var);
-  const float rs = 1.0f / sqrtf(var * (1.0f / G_E) + 1e-5f);
-#pragma unroll
-  for (int c = 0; c < G_E; ++c) y[c] = (x[c] - mean) * rs * __ldg(w + c) + __ldg(b + c);
-}
-
-__device__ __forceinline__ float gelu_new_f(float x) {
-  return 0.5f * x * (1.0f + tanhf(0.7978845608028654f * (x + 0.044715f * x * x * x)));
-}
-
-template <int DF_THREADS>
-__global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const DenseParams p) {
+template <int DF_THREADS, bool SAVE = false>
+__global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const DenseParams p, const TrainSave sv = TrainSave{}) {
   constexpr int DF_V = DF_K + DF_THREADS * 32;
   extern __shared__ __align__(16) float sm[];
   const int tid = threadIdx.x;
@@ -89,17 +53,19 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
         tok[2 * dx + du] = p.cr[row];
       }
     }
+    if (SAVE && valid) store32_(sv.fin + ((size_t)b * S + tid) * TF_STRIDE + TF_TOK, tok);
 #pragma unroll
     for (int c = 0; c < G_E; ++c) x[c] = valid ? __ldg(m.embed_b + c) + __ldg(m.wpe + (size_t)tid * G_E + c) : 0.f;
     for (int i = 0; i < din; ++i) {
       const float tv = tok[i];
 #pragma unroll
-      for (int c = 0; c < G_E; ++c) x[c] = fmaf(tv, __ldg(m.embed_wT + i * G_E + c), x[c]);
+      for (int c = 0; c < G_E; ++c) x[c] = fmaf(tv, __ldg(SAVE ? m.embed_wT + c * din + i : m.embed_wT + i * G_E + c), x[c]);
     }
   }
 
   for (int l = 0; l < m.L; ++l) {
     const LayerW& w = m.layer[l];
+    float* const rec = SAVE && valid ? sv.act + (((size_t)l * p.B + b) * S + tid) * TA_STRIDE : nullptr;   // SAVE: this row's record
     __syncthreads();   // previous layer's readers of the weights / K / V are done
     {
       auto cp = [&](const float* src, int off, int n) {
@@ -116,7 +82,14 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
     float y[G_E];
     float2 acc[16];
     // ---- LN1, then k and v rows -> shared memory, q stays in registers ----
-    ln_row_f(x, w.ln1_w, w.ln1_b, y);
+    if (SAVE) {
+      if (valid) store32_(rec + TA_XIN, x);
+      float st[2];
+      ln_row_f<true>(x, w.ln1_w, w.ln1_b, y, st);
+      if (valid) rec[TA_MU1] = st[0], rec[TA_RS1] = st[1];
+    } else {
+      ln_row_f(x, w.ln1_w, w.ln1_b, y);
+    }
 #pragma unroll
     for (int part = 1; part <= 2; ++part) {      // 1: k, 2: v
 #pragma unroll
@@ -125,6 +98,11 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
       float4* dst = reinterpret_cast<float4*>(sm + (part == 1 ? DF_K : DF_V) + tid * G_E);
 #pragma unroll
       for (int o = 0; o < 8; ++o) dst[o] = make_float4(acc[2 * o].x, acc[2 * o].y, acc[2 * o + 1].x, acc[2 * o + 1].y);
+      if (SAVE && valid) {
+        float4* g4 = reinterpret_cast<float4*>(rec + (part == 1 ? TA_K : TA_V));
+#pragma unroll
+        for (int o = 0; o < 8; ++o) g4[o] = make_float4(acc[2 * o].x, acc[2 * o].y, acc[2 * o + 1].x, acc[2 * o + 1].y);
+      }
     }
     float q[G_E];
 #pragma unroll
@@ -132,6 +110,7 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
     row_matvec32<G_E>(y, sm + DF_WQKV, 96, 0, acc);
 #pragma unroll
     for (int o = 0; o < 16; ++o) q[2 * o] = acc[o].x * 0.17677669529663687f, q[2 * o + 1] = acc[o].y * 0.17677669529663687f;
+    if (SAVE && valid) store32_(rec + TA_Q, q);
     __syncthreads();
     // ---- causal attention of row tid: online softmax over keys 0..tid ----
     {
@@ -172,6 +151,7 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
       const float inv = 1.0f / lsum;
 #pragma unroll
       for (int o = 0; o < 16; ++o) y[2 * o] = acc[o].x * inv, y[2 * o + 1] = acc[o].y * inv;
+      if (SAVE && valid) store32_(rec + TA_O, y), rec[TA_LSE] = mx + logf(lsum);
     }
     // ---- x += o Wproj + b ----
 #pragma unroll
@@ -180,7 +160,14 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
 #pragma unroll
     for (int o = 0; o < 16; ++o) x[2 * o] += acc[o].x, x[2 * o + 1] += acc[o].y;
     // ---- MLP: 4 slices of 32 hidden units, each consumed by fc2 as soon as it is activated ----
-    ln_row_f(x, w.ln2_w, w.ln2_b, y);
+    if (SAVE) {
+      if (valid) store32_(rec + TA_XMID, x);
+      float st[2];
+      ln_row_f<true>(x, w.ln2_w, w.ln2_b, y, st);
+      if (valid) rec[TA_MU2] = st[0], rec[TA_RS2] = st[1];
+    } else {
+      ln_row_f(x, w.ln2_w, w.ln2_b, y);
+    }
     float2 out2[16];
 #pragma unroll
     for (int o = 0; o < 16; ++o) out2[o] = make_float2(__ldg(w.fc2_b + 2 * o), __ldg(w.fc2_b + 2 * o + 1));
@@ -189,6 +176,11 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
 #pragma unroll
       for (int o = 0; o < 16; ++o) acc[o] = make_float2(__ldg(w.fc_b + part * 32 + 2 * o), __ldg(w.fc_b + part * 32 + 2 * o + 1));
       row_matvec32<G_E>(y, sm + DF_WFC, 128, part * 32, acc);
+      if (SAVE && valid) {
+        float4* h4 = reinterpret_cast<float4*>(rec + TA_H + part * 32);
+#pragma unroll
+        for (int o = 0; o < 8; ++o) h4[o] = make_float4(acc[2 * o].x, acc[2 * o].y, acc[2 * o + 1].x, acc[2 * o + 1].y);
+      }
       float g[G_E];
 #pragma unroll
       for (int o = 0; o < 16; ++o) g[2 * o] = gelu_new_f(acc[o].x), g[2 * o + 1] = gelu_new_f(acc[o].y);
@@ -198,6 +190,13 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
     for (int o = 0; o < 16; ++o) x[2 * o] += out2[o].x, x[2 * o + 1] += out2[o].y;
   }
 
+  if (SAVE && valid) {   // final residual and ln_f statistics of every row (rows without logits get gradient 0 there)
+    float* f = sv.fin + ((size_t)b * S + tid) * TF_STRIDE;
+    store32_(f + TF_X, x);
+    float y[G_E], st[2];
+    ln_row_f<true>(x, m.lnf_w, m.lnf_b, y, st);
+    f[TF_MU] = st[0], f[TF_RS] = st[1];
+  }
   if (p.test ? (tid == p.T) : (tid >= 1 && tid <= p.T)) {
     float y[G_E];
     ln_row_f(x, m.lnf_w, m.lnf_b, y);
@@ -205,18 +204,18 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
     for (int j = 0; j < du; ++j) {
       float lg = __ldg(m.pred_b + j);
 #pragma unroll
-      for (int c = 0; c < G_E; ++c) lg = fmaf(y[c], __ldg(m.pred_wT + c * du + j), lg);
+      for (int c = 0; c < G_E; ++c) lg = fmaf(y[c], __ldg(SAVE ? m.pred_wT + j * G_E + c : m.pred_wT + c * du + j), lg);
       o[j] = lg;
     }
   }
 }
 
-template <int THREADS>
-static cudaError_t launch_df(const DenseParams& p, cudaStream_t st) {
+template <int THREADS, bool SAVE = false>
+static cudaError_t launch_df(const DenseParams& p, cudaStream_t st, const TrainSave& sv = TrainSave{}) {
   const int smem = df_floats(THREADS) * (int)sizeof(float);
-  cudaError_t e = cudaFuncSetAttribute(gpt2_dense_fp32_kernel<THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  cudaError_t e = cudaFuncSetAttribute(gpt2_dense_fp32_kernel<THREADS, SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;
-  gpt2_dense_fp32_kernel<THREADS><<<p.B, THREADS, smem, st>>>(p);
+  gpt2_dense_fp32_kernel<THREADS, SAVE><<<p.B, THREADS, smem, st>>>(p, sv);
   return cudaGetLastError();
 }
 
@@ -225,6 +224,17 @@ int gpt2_dense_fp32_launch(const DenseParams& p, cudaStream_t st) {
   cudaError_t e = S <= 128 ? launch_df<128>(p, st) : S <= 256 ? launch_df<256>(p, st) : launch_df<512>(p, st);
   if (e != cudaSuccess) {
     set_error("gpt2_dense_fp32 launch failed: %s", cudaGetErrorString(e));
+    return DPT_ERR_CUDA;
+  }
+  return DPT_OK;
+}
+
+int gpt2_train_forward_launch(const DenseParams& p, const TrainSave& sv, cudaStream_t st) {
+  const int S = p.T + 1;
+  cudaError_t e = S <= 128 ? launch_df<128, true>(p, st, sv) : S <= 256 ? launch_df<256, true>(p, st, sv)
+                                                                         : launch_df<512, true>(p, st, sv);
+  if (e != cudaSuccess) {
+    set_error("gpt2_train_forward launch failed: %s", cudaGetErrorString(e));
     return DPT_ERR_CUDA;
   }
   return DPT_OK;

@@ -60,6 +60,26 @@ struct DenseParams {
 int gpt2_dense_launch(const DenseParams& p, cudaStream_t st);        // gpt2_dense.cu (tcgen05, bf16 operands)
 int gpt2_dense_long_launch(const DenseParams& p, cudaStream_t st);   // gpt2_dense.cu (tcgen05, 129..512 tokens)
 int gpt2_dense_fp32_launch(const DenseParams& p, cudaStream_t st);   // gpt2_dense_fp32.cu (CUDA cores, fp32)
+
+// Activations the training forward saves for the backward (gpt2_train.cu), fp32.  act: [L][B][S][TA_STRIDE], one record
+// per layer and row (S = T + 1 rows, row 0 = query token); fin: [B][S][TF_STRIDE], the input token, the final residual
+// and the ln_f statistics.
+constexpr int TA_XIN = 0;      // residual input of the layer [32]
+constexpr int TA_Q = 32;       // q * 1/sqrt(32) [32]
+constexpr int TA_K = 64;       // [32]
+constexpr int TA_V = 96;       // [32]
+constexpr int TA_O = 128;      // attention output (input of attn.c_proj) [32]
+constexpr int TA_XMID = 160;   // residual after attention [32]
+constexpr int TA_H = 192;      // mlp.c_fc pre-activation [128]
+constexpr int TA_MU1 = 320, TA_RS1 = 321, TA_LSE = 322, TA_MU2 = 323, TA_RS2 = 324;
+constexpr int TA_STRIDE = 328;
+constexpr int TF_X = 0, TF_TOK = 32, TF_MU = 64, TF_RS = 65, TF_STRIDE = 68;   // TF_TOK: the input token, zero-padded
+struct TrainSave {
+  float *act, *fin;
+};
+// the dense fp32 forward with SAVE = true: DenseParams::m holds the parameter tensors' own pointers (embed_wT =
+// embed_transition.weight [E, din], pred_wT = pred_actions.weight [du, E]); share must be 1
+int gpt2_train_forward_launch(const DenseParams& p, const TrainSave& sv, cudaStream_t st);
 void gpt2_pack_wimg(const float* attn_w, const float* proj_w, const float* fc_w, const float* fc2_w, unsigned char* img,
                     cudaStream_t st);
 }  // namespace dpt

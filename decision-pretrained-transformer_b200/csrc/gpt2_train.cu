@@ -1,0 +1,636 @@
+// Training of the GPT-2 (models/net.py:9-60) in fp32 on the CUDA cores, sequences of <= 512 tokens.
+//
+//   dpt_gpt2_train_forward : the dense fp32 forward (gpt2_dense_fp32.cu, SAVE = true) on the parameter tensors as
+//                            they are -- no handle, no repack -- which also stores each row's activations (TA_* / TF_*).
+//   dpt_gpt2_train_backward: three launches on the caller's stream.
+//     1. gpt2_train_backward_kernel: one CTA per sequence, thread t = token row t (as the forward), layers in reverse.
+//        It computes every row's data gradients and writes, per layer and row, the operand pairs of the weight
+//        gradients (GR_* / GF_*).  Causal attention is flash-attention-2 style from the saved log-sum-exp:
+//        D_i = dO_i . O_i, a query-side pass for dQ (K, V in shared memory) and key-side passes for dV and dK
+//        (Q, dO, lse, D in shared memory).
+//     2. weight_grad_partial_kernel: every weight gradient is a sum over the B*S rows of an outer product
+//        A_r^T G_r (or of A_r * G_r for LayerNorm weights; biases: of G_r).  The rows are cut into NC fixed chunks;
+//        CTA (tile, chunk) writes its 32 x 32 tile's chunk sum to slot `chunk` of the partial buffer.
+//     3. weight_grad_reduce_kernel sums the NC slots in chunk order into the gradient tensors; wpe_grad_kernel sums
+//        the position gradients over the batch in sequence order (rows past T are zero).
+//   Every sum has a fixed order, so two identical calls give bit-identical gradients.
+#include <algorithm>
+
+#include "common.cuh"
+#include "gpt2_model.cuh"
+#include "gpt2_fp32.cuh"
+
+namespace dpt {
+
+// per layer and row: what the weight-gradient reduction reads, [L][B][S][GR_STRIDE]
+constexpr int GR_DX = 0;       // gradient of the layer's output residual [32]   (G of mlp.c_proj + bias)
+constexpr int GR_G = 32;       // gelu_new(h) [128]                                (A of mlp.c_proj)
+constexpr int GR_DH = 160;     // gradient of h [128]                              (G of mlp.c_fc + bias)
+constexpr int GR_Y2 = 288;     // ln_2 output [32]                                 (A of mlp.c_fc)
+constexpr int GR_XH2 = 320;    // ln_2 normalised input [32]                       (A of ln_2.weight)
+constexpr int GR_DY2 = 352;    // gradient of the ln_2 output [32]                 (G of ln_2)
+constexpr int GR_DXM = 384;    // gradient of the post-attention residual [32]     (G of attn.c_proj + bias)
+constexpr int GR_DQKV = 416;   // gradient of q, k, v (unscaled q) [96]            (G of attn.c_attn + bias)
+constexpr int GR_Y1 = 512;     // ln_1 output [32]                                 (A of attn.c_attn)
+constexpr int GR_XH1 = 544;    // [32]                                             (A of ln_1.weight)
+constexpr int GR_DY1 = 576;    // [32]                                             (G of ln_1)
+constexpr int GR_STRIDE = 608;
+// per row, once: [B][S][GF_STRIDE]
+constexpr int GF_DLOG = 0;     // gradient of the logits, zero-padded to 32        (G of pred_actions + bias)
+constexpr int GF_YF = 32;      // ln_f output                                      (A of pred_actions)
+constexpr int GF_XHF = 64;     // ln_f normalised input                            (A of ln_f.weight)
+constexpr int GF_DYF = 96;     // gradient of the ln_f output                      (G of ln_f)
+constexpr int GF_DX0 = 128;    // gradient of the embedded token (G of embed_transition + bias, and of wpe)
+constexpr int GF_STRIDE = 160;
+
+// backward shared memory (floats): transposed layer weights, then two [THREADS][32] row arrays and [THREADS][2]
+constexpr int DB_WQKVT = 0;                      // [96][32]  = attn_w^T
+constexpr int DB_WPROJT = DB_WQKVT + 96 * 32;    // [32][32]  = proj_w^T
+constexpr int DB_WFCT = DB_WPROJT + 32 * 32;     // [128][32] = fc_w^T
+constexpr int DB_WFC2T = DB_WFCT + 128 * 32;     // [32][128] = fc2_w^T
+constexpr int DB_X1 = DB_WFC2T + 32 * 128;
+constexpr int db_floats(int threads) { return DB_X1 + 2 * threads * 32 + 2 * threads; }   // 84 KB / 120 KB / 184 KB
+
+constexpr float ATT_SCALE = 0.17677669529663687f;   // 1 / sqrt(32)
+
+struct TrainModel {   // the parameter tensors (reference layouts)
+  int L, dx, du, din, n_pos;
+  const float *wpe, *embed_w, *embed_b, *pred_w, *pred_b, *lnf_w, *lnf_b;
+  const float *ln1_w[G_MAX_L], *ln1_b[G_MAX_L], *attn_w[G_MAX_L], *attn_b[G_MAX_L], *proj_w[G_MAX_L], *proj_b[G_MAX_L];
+  const float *ln2_w[G_MAX_L], *ln2_b[G_MAX_L], *fc_w[G_MAX_L], *fc_b[G_MAX_L], *fc2_w[G_MAX_L], *fc2_b[G_MAX_L];
+};
+
+struct BackParams {
+  TrainModel m;
+  const float* dout;
+  int B, T, test;
+  const float *act, *fin;
+  float *grec, *gfin;
+};
+
+// dx += d LayerNorm(x)/dx applied to dy, from the normalised input xh, rstd rs and the LN weight w
+__device__ __forceinline__ void ln_back_(const float* xh, float rs, const float* dy, const float* w, float* dx) {
+  float m1 = 0.f, m2 = 0.f;
+#pragma unroll
+  for (int c = 0; c < G_E; ++c) {
+    const float d = dy[c] * __ldg(w + c);
+    m1 += d;
+    m2 = fmaf(d, xh[c], m2);
+  }
+  m1 *= (1.0f / G_E), m2 *= (1.0f / G_E);
+#pragma unroll
+  for (int c = 0; c < G_E; ++c) dx[c] += rs * (dy[c] * __ldg(w + c) - m1 - xh[c] * m2);
+}
+
+__device__ __forceinline__ void acc_to_(const float2* acc, float* v) {
+#pragma unroll
+  for (int o = 0; o < 16; ++o) v[2 * o] = acc[o].x, v[2 * o + 1] = acc[o].y;
+}
+
+__device__ __forceinline__ float dot32_(const float* a, const float* b_sm) {
+  const float4* b4 = reinterpret_cast<const float4*>(b_sm);
+  float2 d0 = make_float2(0.f, 0.f), d1 = make_float2(0.f, 0.f);
+#pragma unroll
+  for (int o = 0; o < 8; ++o) {
+    const float4 bb = b4[o];
+    d0 = ffma2_(make_float2(a[4 * o], a[4 * o + 1]), make_float2(bb.x, bb.y), d0);
+    d1 = ffma2_(make_float2(a[4 * o + 2], a[4 * o + 3]), make_float2(bb.z, bb.w), d1);
+  }
+  return (d0.x + d0.y) + (d1.x + d1.y);
+}
+
+// acc[0..31] += s * v_sm[0..31]
+__device__ __forceinline__ void axpy32_(float s, const float* v_sm, float2* acc) {
+  const float2 ss = make_float2(s, s);
+  const float4* v4 = reinterpret_cast<const float4*>(v_sm);
+#pragma unroll
+  for (int o = 0; o < 8; ++o) {
+    const float4 vv = v4[o];
+    acc[2 * o] = ffma2_(ss, make_float2(vv.x, vv.y), acc[2 * o]);
+    acc[2 * o + 1] = ffma2_(ss, make_float2(vv.z, vv.w), acc[2 * o + 1]);
+  }
+}
+
+template <int THREADS>
+__global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const BackParams p) {
+  extern __shared__ __align__(16) float sm[];
+  float* const X1 = sm + DB_X1;
+  float* const X2 = sm + DB_X1 + THREADS * 32;
+  float* const SV = sm + DB_X1 + 2 * THREADS * 32;
+  const TrainModel& m = p.m;
+  const int tid = threadIdx.x, b = blockIdx.x;
+  const int S = p.T + 1, du = m.du;
+  const bool valid = tid < S;
+  const int row = valid ? tid : S - 1;   // rows past the sequence load a valid row and store nothing
+  const size_t r = (size_t)b * S + row;
+  const size_t NR = (size_t)p.B * S;
+
+  float dx[G_E];
+  // ---- pred_actions and ln_f ----
+  {
+    const float* f = p.fin + r * TF_STRIDE;
+    float xh[G_E], dl[G_E], dy[G_E];
+    load32_(xh, f + TF_X);
+    const float mu = f[TF_MU], rs = f[TF_RS];
+#pragma unroll
+    for (int c = 0; c < G_E; ++c) xh[c] = (xh[c] - mu) * rs, dl[c] = 0.f, dy[c] = 0.f;
+    const bool has_out = p.test ? row == p.T : row >= 1;
+    if (has_out) {
+      const float* d = p.test ? p.dout + (size_t)b * du : p.dout + ((size_t)b * p.T + (row - 1)) * du;
+      for (int j = 0; j < du; ++j) {
+        const float g = d[j];
+        dl[j] = g;
+#pragma unroll
+        for (int c = 0; c < G_E; ++c) dy[c] = fmaf(g, __ldg(m.pred_w + j * G_E + c), dy[c]);
+      }
+    }
+#pragma unroll
+    for (int c = 0; c < G_E; ++c) dx[c] = 0.f;
+    ln_back_(xh, rs, dy, m.lnf_w, dx);
+    if (valid) {
+      float* g = p.gfin + r * GF_STRIDE;
+      store32_(g + GF_DLOG, dl), store32_(g + GF_XHF, xh), store32_(g + GF_DYF, dy);
+#pragma unroll
+      for (int c = 0; c < G_E; ++c) dl[c] = fmaf(xh[c], __ldg(m.lnf_w + c), __ldg(m.lnf_b + c));
+      store32_(g + GF_YF, dl);
+    }
+  }
+
+  for (int l = m.L - 1; l >= 0; --l) {
+    __syncthreads();   // the previous layer's readers of the weights and row arrays are done
+    for (int i = tid; i < 32 * 96; i += THREADS) sm[DB_WQKVT + (i % 96) * 32 + i / 96] = __ldg(m.attn_w[l] + i);
+    for (int i = tid; i < 32 * 32; i += THREADS) sm[DB_WPROJT + (i % 32) * 32 + i / 32] = __ldg(m.proj_w[l] + i);
+    for (int i = tid; i < 32 * 128; i += THREADS) sm[DB_WFCT + (i % 128) * 32 + i / 128] = __ldg(m.fc_w[l] + i);
+    for (int i = tid; i < 128 * 32; i += THREADS) sm[DB_WFC2T + (i % 32) * 128 + i / 32] = __ldg(m.fc2_w[l] + i);
+    const float* a = p.act + ((size_t)l * NR + r) * TA_STRIDE;
+    float* g = p.grec + ((size_t)l * NR + r) * GR_STRIDE;
+    if (valid) store32_(g + GR_DX, dx);
+    __syncthreads();
+    float2 acc[16];
+    // ---- MLP: x_out = x_mid + fc2(gelu_new(fc(ln_2(x_mid)))) ----
+    float dxm[G_E];   // becomes the gradient of x_mid
+    {
+      float xh[G_E], dy[G_E];
+      load32_(xh, a + TA_XMID);
+      const float mu = a[TA_MU2], rs = a[TA_RS2];
+#pragma unroll
+      for (int c = 0; c < G_E; ++c) xh[c] = (xh[c] - mu) * rs;
+      if (valid) {
+        float y[G_E];
+#pragma unroll
+        for (int c = 0; c < G_E; ++c) y[c] = fmaf(xh[c], __ldg(m.ln2_w[l] + c), __ldg(m.ln2_b[l] + c));
+        store32_(g + GR_Y2, y), store32_(g + GR_XH2, xh);
+      }
+      float2 dy2[16];
+#pragma unroll
+      for (int o = 0; o < 16; ++o) dy2[o] = make_float2(0.f, 0.f);
+#pragma unroll 1
+      for (int part = 0; part < 4; ++part) {
+#pragma unroll
+        for (int o = 0; o < 16; ++o) acc[o] = make_float2(0.f, 0.f);
+        row_matvec32<G_E>(dx, sm + DB_WFC2T, 128, part * 32, acc);   // d gelu(h)
+        float h[G_E], dh[G_E];
+        load32_(h, a + TA_H + part * 32);
+        acc_to_(acc, dh);
+#pragma unroll
+        for (int c = 0; c < G_E; ++c) {
+          const float x = h[c], x2 = x * x;
+          const float t = tanhf(0.7978845608028654f * (x + 0.044715f * x2 * x));
+          h[c] = 0.5f * x * (1.0f + t);
+          const float dg = 0.5f * (1.0f + t) + 0.5f * x * (1.0f - t * t) * 0.7978845608028654f * (1.0f + 3.0f * 0.044715f * x2);
+          dh[c] *= dg;
+        }
+        if (valid) store32_(g + GR_G + part * 32, h), store32_(g + GR_DH + part * 32, dh);
+        row_matvec32<G_E>(dh, sm + DB_WFCT + part * 32 * 32, 32, 0, dy2);
+      }
+      acc_to_(dy2, dy);
+      if (valid) store32_(g + GR_DY2, dy);
+#pragma unroll
+      for (int c = 0; c < G_E; ++c) dxm[c] = dx[c];
+      ln_back_(xh, rs, dy, m.ln2_w[l], dxm);
+    }
+    if (valid) store32_(g + GR_DXM, dxm);
+    // ---- attention: x_mid = x_in + proj(softmax(q k^T) v) ----
+    float dO[G_E];
+#pragma unroll
+    for (int o = 0; o < 16; ++o) acc[o] = make_float2(0.f, 0.f);
+    row_matvec32<G_E>(dxm, sm + DB_WPROJT, 32, 0, acc);
+    acc_to_(acc, dO);
+    float Dm;
+    {
+      float o_[G_E];
+      load32_(o_, a + TA_O);
+      Dm = 0.f;
+#pragma unroll
+      for (int c = 0; c < G_E; ++c) Dm = fmaf(dO[c], o_[c], Dm);
+    }
+    const float lse = a[TA_LSE];
+    {   // K, V rows -> shared memory
+      float t[G_E];
+      load32_(t, a + TA_K);
+      store32_(X1 + tid * G_E, t);
+      load32_(t, a + TA_V);
+      store32_(X2 + tid * G_E, t);
+    }
+    __syncthreads();
+    const int jmax = __shfl_sync(0xffffffffu, tid, 31);   // last row of this warp: warp-uniform trip counts
+    const int jmin = tid & ~31;                           // first row of this warp
+    float dqk[G_E];   // dq (unscaled), later dk
+    {
+      float q[G_E];
+      load32_(q, a + TA_Q);
+#pragma unroll
+      for (int o = 0; o < 16; ++o) acc[o] = make_float2(0.f, 0.f);
+      for (int j = 0; j <= jmax; ++j) {
+        const float s = dot32_(q, X1 + j * G_E);
+        if (j <= tid) {
+          const float pr = expf(s - lse);
+          const float ds = pr * (dot32_(dO, X2 + j * G_E) - Dm);
+          axpy32_(ds, X1 + j * G_E, acc);
+        }
+      }
+#pragma unroll
+      for (int o = 0; o < 16; ++o) dqk[2 * o] = acc[o].x * ATT_SCALE, dqk[2 * o + 1] = acc[o].y * ATT_SCALE;
+    }
+    if (valid) store32_(g + GR_DQKV, dqk);
+    float dy1[G_E];
+#pragma unroll
+    for (int o = 0; o < 16; ++o) acc[o] = make_float2(0.f, 0.f);
+    row_matvec32<G_E>(dqk, sm + DB_WQKVT, 32, 0, acc);
+    __syncthreads();   // K, V readers done
+    {   // Q, dO, lse, D -> shared memory
+      float t[G_E];
+      load32_(t, a + TA_Q);
+      store32_(X1 + tid * G_E, t);
+      store32_(X2 + tid * G_E, dO);
+      SV[2 * tid] = lse, SV[2 * tid + 1] = Dm;
+    }
+    __syncthreads();
+    {
+      float k[G_E];
+      load32_(k, a + TA_K);
+      // dv_j = sum_{i >= j} P_ij dO_i
+      float2 dv[16];
+#pragma unroll
+      for (int o = 0; o < 16; ++o) dv[o] = make_float2(0.f, 0.f);
+      for (int i = jmin; i < S; ++i) {
+        const float s = dot32_(k, X1 + i * G_E);
+        if (i >= tid) axpy32_(expf(s - SV[2 * i]), X2 + i * G_E, dv);
+      }
+      acc_to_(dv, dO);   // dO is not needed any more: it holds dv
+      if (valid) store32_(g + GR_DQKV + 64, dO);
+      row_matvec32<G_E>(dO, sm + DB_WQKVT + 64 * 32, 32, 0, acc);
+      // dk_j = sum_{i >= j} P_ij (dO_i . v_j - D_i) q_i
+      float v[G_E];
+      load32_(v, a + TA_V);
+      float2 dk[16];
+#pragma unroll
+      for (int o = 0; o < 16; ++o) dk[o] = make_float2(0.f, 0.f);
+      for (int i = jmin; i < S; ++i) {
+        const float s = dot32_(k, X1 + i * G_E);
+        if (i >= tid) {
+          const float ds = expf(s - SV[2 * i]) * (dot32_(v, X2 + i * G_E) - SV[2 * i + 1]);
+          axpy32_(ds, X1 + i * G_E, dk);
+        }
+      }
+      acc_to_(dk, dqk);
+      if (valid) store32_(g + GR_DQKV + 32, dqk);
+      row_matvec32<G_E>(dqk, sm + DB_WQKVT + 32 * 32, 32, 0, acc);
+    }
+    acc_to_(acc, dy1);
+    // ---- ln_1 ----
+    {
+      float xh[G_E];
+      load32_(xh, a + TA_XIN);
+      const float mu = a[TA_MU1], rs = a[TA_RS1];
+#pragma unroll
+      for (int c = 0; c < G_E; ++c) xh[c] = (xh[c] - mu) * rs;
+      if (valid) {
+        float y[G_E];
+#pragma unroll
+        for (int c = 0; c < G_E; ++c) y[c] = fmaf(xh[c], __ldg(m.ln1_w[l] + c), __ldg(m.ln1_b[l] + c));
+        store32_(g + GR_Y1, y), store32_(g + GR_XH1, xh), store32_(g + GR_DY1, dy1);
+      }
+#pragma unroll
+      for (int c = 0; c < G_E; ++c) dx[c] = dxm[c];
+      ln_back_(xh, rs, dy1, m.ln1_w[l], dx);
+    }
+  }
+  if (valid) store32_(p.gfin + r * GF_STRIDE + GF_DX0, dx);
+}
+
+// ---- weight gradients: fixed-chunk partial sums, then a fixed-order reduction ----
+struct RJob {
+  const float *A, *G;   // row r of the operands at A + r * sa, G + r * sg
+  int sa, sg, nin, nout;
+  int diag;             // 0: W[i][o] = sum_r A[r][i] G[r][o]; 1: W[c] = sum_r A[r][c] G[r][c] (nin = nout = 32)
+  int trans;            // W is stored [nout][nin] (nn.Linear) instead of [nin][nout] (Conv1D)
+  int woff, boff;       // flat offsets of the weight and of the bias (sum_r G[r][o]) in a partial slot
+};
+struct RTile {
+  short job, i0, o0;
+};
+constexpr int R_MAX_JOBS = 6 * G_MAX_L + 3;
+constexpr int R_MAX_TILES = 14 * G_MAX_L + 3;
+struct RParams {
+  RJob job[R_MAX_JOBS];
+  RTile tile[R_MAX_TILES];
+  int NR, CH, P;
+  float* part;   // [NC][P]
+};
+struct RSeg {
+  float* dst;
+  int off, n;
+};
+constexpr int R_MAX_SEGS = 2 * R_MAX_JOBS;
+struct RSegs {
+  RSeg seg[R_MAX_SEGS];
+  int NC, P;
+  const float* part;
+};
+
+__global__ void __launch_bounds__(256) weight_grad_partial_kernel(const RParams p) {
+  __shared__ __align__(16) float As[32][32];
+  __shared__ __align__(16) float Gs[32][32];
+  __shared__ float red[2][8][32];
+  const RTile t = p.tile[blockIdx.x];
+  const RJob& j = p.job[t.job];
+  const int tid = threadIdx.x, chunk = blockIdx.y;
+  const int r0 = chunk * p.CH, r1 = min(p.NR, r0 + p.CH);
+  const int lr = tid >> 3, l4 = (tid & 7) * 4;   // loader: row, 4 columns
+  const int i = tid >> 3, o4 = (tid & 7) * 4;    // outer product: input i, outputs o4..o4+3
+  const int dc = tid & 31, dg = tid >> 5;        // diagonal: column, row group
+  float4 acc = make_float4(0.f, 0.f, 0.f, 0.f), bacc = acc;
+  float dacc = 0.f, dbacc = 0.f;
+  for (int rb = r0; rb < r1; rb += 32) {
+    const int rr = rb + lr;
+    float4 av = make_float4(0.f, 0.f, 0.f, 0.f), gv = av;
+    if (rr < r1) {
+      av = *reinterpret_cast<const float4*>(j.A + (size_t)rr * j.sa + t.i0 + l4);
+      gv = *reinterpret_cast<const float4*>(j.G + (size_t)rr * j.sg + t.o0 + l4);
+    }
+    __syncthreads();
+    *reinterpret_cast<float4*>(&As[lr][l4]) = av;
+    *reinterpret_cast<float4*>(&Gs[lr][l4]) = gv;
+    __syncthreads();
+    if (!j.diag) {
+#pragma unroll 8
+      for (int k = 0; k < 32; ++k) {
+        const float a = As[k][i];
+        const float4 gg = *reinterpret_cast<const float4*>(&Gs[k][o4]);
+        acc.x = fmaf(a, gg.x, acc.x), acc.y = fmaf(a, gg.y, acc.y), acc.z = fmaf(a, gg.z, acc.z), acc.w = fmaf(a, gg.w, acc.w);
+        bacc.x += gg.x, bacc.y += gg.y, bacc.z += gg.z, bacc.w += gg.w;
+      }
+    } else {
+#pragma unroll
+      for (int k = dg; k < 32; k += 8) dacc = fmaf(As[k][dc], Gs[k][dc], dacc), dbacc += Gs[k][dc];
+    }
+  }
+  float* part = p.part + (size_t)chunk * p.P;
+  if (!j.diag) {
+    const float v[4] = {acc.x, acc.y, acc.z, acc.w}, bv[4] = {bacc.x, bacc.y, bacc.z, bacc.w};
+    const int gi = t.i0 + i;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const int go = t.o0 + o4 + e;
+      if (gi < j.nin && go < j.nout) part[j.woff + (j.trans ? go * j.nin + gi : gi * j.nout + go)] = v[e];
+      if (i == 0 && t.i0 == 0 && go < j.nout) part[j.boff + go] = bv[e];
+    }
+  } else {
+    red[0][dg][dc] = dacc, red[1][dg][dc] = dbacc;
+    __syncthreads();
+    if (tid < 32) {
+      float s = 0.f, sb = 0.f;
+#pragma unroll
+      for (int k = 0; k < 8; ++k) s += red[0][k][tid], sb += red[1][k][tid];
+      part[j.woff + tid] = s, part[j.boff + tid] = sb;
+    }
+  }
+}
+
+__global__ void __launch_bounds__(256) weight_grad_reduce_kernel(const RSegs s) {
+  const RSeg& g = s.seg[blockIdx.y];
+  const int e = blockIdx.x * 256 + threadIdx.x;
+  if (e >= g.n) return;
+  const float* src = s.part + g.off + e;
+  float acc = 0.f;
+  for (int c = 0; c < s.NC; ++c) acc += src[(size_t)c * s.P];
+  g.dst[e] = acc;
+}
+
+__global__ void wpe_grad_kernel(const float* gfin, int B, int S, int n_pos, float* dwpe) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n_pos * G_E) return;
+  const int t = e / G_E, c = e % G_E;
+  float acc = 0.f;
+  if (t < S)
+    for (int b = 0; b < B; ++b) acc += gfin[((size_t)b * S + t) * GF_STRIDE + GF_DX0 + c];
+  dwpe[e] = acc;
+}
+
+// ---- host side ----
+struct TrainLayout {
+  int L, S, din, du, NC, CH, P;
+  size_t NR, act, fin, grec, gfin, part, total;   // offsets in floats
+};
+
+static int params_per_slot(int L, int din, int du) {
+  const int per_layer = 32 * 96 + 96 + 32 * 32 + 32 + 32 * 128 + 128 + 128 * 32 + 32 + 4 * 32;
+  const int p = L * per_layer + 32 * du + du + 2 * 32 + 32 * din + 32;
+  return (p + 3) & ~3;
+}
+
+static TrainLayout train_layout(int L, int din, int du, int B, int T) {
+  TrainLayout t{};
+  t.L = L, t.S = T + 1, t.din = din, t.du = du;
+  t.NR = (size_t)B * t.S;
+  // chunks of >= 256 rows, at most 256 of them; the chunking depends on the shape only (determinism)
+  t.NC = (int)std::min<size_t>(256, (t.NR + 255) / 256);
+  if (t.NC < 1) t.NC = 1;
+  t.CH = (int)((((t.NR + t.NC - 1) / t.NC) + 31) / 32 * 32);
+  t.NC = (int)((t.NR + t.CH - 1) / t.CH);
+  if (t.NC < 1) t.NC = 1;
+  t.P = params_per_slot(L, din, du);
+  size_t o = 0;
+  t.act = o, o += (size_t)L * t.NR * TA_STRIDE;
+  t.fin = o, o += t.NR * TF_STRIDE;
+  t.grec = o, o += (size_t)L * t.NR * GR_STRIDE;
+  t.gfin = o, o += t.NR * GF_STRIDE;
+  t.part = o, o += (size_t)t.NC * t.P;
+  t.total = o;
+  return t;
+}
+
+static int check_model(const char* fn, const dpt_gpt2_weights_t* w, int B, int T) {
+  DPT_CHECK_ARG(w, "%s: null weights", fn);
+  if (w->n_embd != G_E) {
+    set_error("%s: n_embd=%d, training supports n_embd == %d", fn, w->n_embd, G_E);
+    return DPT_ERR_UNSUPPORTED;
+  }
+  if (w->n_layer < 1 || w->n_layer > G_MAX_L) {
+    set_error("%s: n_layer=%d outside [1,%d]", fn, w->n_layer, G_MAX_L);
+    return DPT_ERR_UNSUPPORTED;
+  }
+  const int din = 2 * w->state_dim + w->action_dim + 1;
+  DPT_CHECK_ARG(w->state_dim >= 1 && w->action_dim >= 1 && din <= 32,
+                "%s: token width 2*state_dim+action_dim+1 = %d must be <= 32", fn, din);
+  DPT_CHECK_ARG(B >= 0 && T >= 0, "%s: B=%d T=%d", fn, B, T);
+  if (T + 1 > 512) {
+    set_error("%s: T=%d, training supports sequences of <= 512 tokens (T <= 511)", fn, T);
+    return DPT_ERR_UNSUPPORTED;
+  }
+  DPT_CHECK_ARG(T + 1 <= w->n_positions, "%s: sequence %d exceeds n_positions %d", fn, T + 1, w->n_positions);
+  DPT_CHECK_ARG(w->wpe && w->embed_w && w->embed_b && w->pred_w && w->pred_b && w->lnf_w && w->lnf_b && w->ln1_w && w->ln1_b &&
+                    w->attn_w && w->attn_b && w->proj_w && w->proj_b && w->ln2_w && w->ln2_b && w->fc_w && w->fc_b &&
+                    w->fc2_w && w->fc2_b,
+                "%s: null weight pointer", fn);
+  for (int l = 0; l < w->n_layer; ++l)
+    DPT_CHECK_ARG(w->ln1_w[l] && w->ln1_b[l] && w->attn_w[l] && w->attn_b[l] && w->proj_w[l] && w->proj_b[l] && w->ln2_w[l] &&
+                      w->ln2_b[l] && w->fc_w[l] && w->fc_b[l] && w->fc2_w[l] && w->fc2_b[l],
+                  "%s: null layer %d weight", fn, l);
+  return DPT_OK;
+}
+
+}  // namespace dpt
+
+using namespace dpt;
+
+extern "C" uint64_t dpt_gpt2_train_workspace_bytes(const dpt_gpt2_weights_t* w, int B, int T) {
+  if (!w || B <= 0 || T < 0 || w->n_layer < 1) return 0;
+  return train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T).total * sizeof(float);
+}
+
+extern "C" int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, const float* query_states, const float* ctx_states,
+                                      const float* ctx_actions, const float* ctx_next_states, const float* ctx_rewards, int B,
+                                      int T, int T_stride, int test, float* out, void* workspace, uint64_t workspace_bytes,
+                                      void* stream) {
+  const char* fn = "dpt_gpt2_train_forward";
+  int rc = check_model(fn, w, B, T);
+  if (rc != DPT_OK) return rc;
+  DPT_CHECK_ARG(T_stride >= T, "%s: T_stride=%d < T=%d", fn, T_stride, T);
+  if (B == 0) return DPT_OK;
+  DPT_CHECK_ARG(query_states && out && (T == 0 || (ctx_states && ctx_actions && ctx_next_states && ctx_rewards)),
+                "%s: null input or output pointer", fn);
+  DPT_CHECK_ARG(workspace && workspace_bytes >= dpt_gpt2_train_workspace_bytes(w, B, T) && aligned16(workspace),
+                "%s: workspace of %llu B, needs %llu B (16 B aligned)", fn, (unsigned long long)workspace_bytes,
+                (unsigned long long)dpt_gpt2_train_workspace_bytes(w, B, T));
+  const TrainLayout lay = train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T);
+  DenseParams dp{};
+  Gpt2Dev& d = dp.m;
+  d.L = w->n_layer, d.dx = w->state_dim, d.du = w->action_dim, d.din = lay.din, d.H = w->horizon, d.n_pos = w->n_positions;
+  d.wpe = w->wpe, d.embed_wT = w->embed_w, d.embed_b = w->embed_b, d.pred_wT = w->pred_w, d.pred_b = w->pred_b;
+  d.lnf_w = w->lnf_w, d.lnf_b = w->lnf_b;
+  for (int l = 0; l < d.L; ++l) {
+    LayerW& lw = d.layer[l];
+    lw.ln1_w = w->ln1_w[l], lw.ln1_b = w->ln1_b[l], lw.attn_w = w->attn_w[l], lw.attn_b = w->attn_b[l];
+    lw.proj_w = w->proj_w[l], lw.proj_b = w->proj_b[l], lw.ln2_w = w->ln2_w[l], lw.ln2_b = w->ln2_b[l];
+    lw.fc_w = w->fc_w[l], lw.fc_b = w->fc_b[l], lw.fc2_w = w->fc2_w[l], lw.fc2_b = w->fc2_b[l];
+    DPT_CHECK_ARG(aligned16(lw.attn_w) && aligned16(lw.proj_w) && aligned16(lw.fc_w) && aligned16(lw.fc2_w),
+                  "%s: layer %d matrices must be 16 B aligned", fn, l);
+  }
+  dp.query = query_states, dp.cs = ctx_states, dp.ca = ctx_actions, dp.cns = ctx_next_states, dp.cr = ctx_rewards;
+  dp.B = B, dp.T = T, dp.Ts = T_stride, dp.test = test ? 1 : 0, dp.share = 1, dp.out = out;
+  float* ws = static_cast<float*>(workspace);
+  TrainSave sv{ws + lay.act, ws + lay.fin};
+  return gpt2_train_forward_launch(dp, sv, (cudaStream_t)stream);
+}
+
+template <int THREADS>
+static cudaError_t launch_back(const BackParams& p, cudaStream_t st) {
+  const int smem = db_floats(THREADS) * (int)sizeof(float);
+  cudaError_t e = cudaFuncSetAttribute(gpt2_train_backward_kernel<THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e != cudaSuccess) return e;
+  gpt2_train_backward_kernel<THREADS><<<p.B, THREADS, smem, st>>>(p);
+  return cudaGetLastError();
+}
+
+extern "C" int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float* dout, int B, int T, int test,
+                                       const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream) {
+  const char* fn = "dpt_gpt2_train_backward";
+  int rc = check_model(fn, w, B, T);
+  if (rc != DPT_OK) return rc;
+  if (B == 0) return DPT_OK;
+  DPT_CHECK_ARG(dout && grads, "%s: null dout or grads", fn);
+  DPT_CHECK_ARG(workspace && workspace_bytes >= dpt_gpt2_train_workspace_bytes(w, B, T) && aligned16(workspace),
+                "%s: workspace of %llu B, needs %llu B (16 B aligned)", fn, (unsigned long long)workspace_bytes,
+                (unsigned long long)dpt_gpt2_train_workspace_bytes(w, B, T));
+  const int L = w->n_layer;
+  const dpt_gpt2_grads_t* g = grads;
+  DPT_CHECK_ARG(g->wpe && g->embed_w && g->embed_b && g->pred_w && g->pred_b && g->lnf_w && g->lnf_b && g->ln1_w && g->ln1_b &&
+                    g->attn_w && g->attn_b && g->proj_w && g->proj_b && g->ln2_w && g->ln2_b && g->fc_w && g->fc_b &&
+                    g->fc2_w && g->fc2_b,
+                "%s: null gradient pointer", fn);
+  for (int l = 0; l < L; ++l)
+    DPT_CHECK_ARG(g->ln1_w[l] && g->ln1_b[l] && g->attn_w[l] && g->attn_b[l] && g->proj_w[l] && g->proj_b[l] && g->ln2_w[l] &&
+                      g->ln2_b[l] && g->fc_w[l] && g->fc_b[l] && g->fc2_w[l] && g->fc2_b[l],
+                  "%s: null layer %d gradient", fn, l);
+  const TrainLayout lay = train_layout(L, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T);
+  float* ws = static_cast<float*>(workspace);
+  cudaStream_t st = (cudaStream_t)stream;
+
+  BackParams bp{};
+  TrainModel& m = bp.m;
+  m.L = L, m.dx = w->state_dim, m.du = w->action_dim, m.din = lay.din, m.n_pos = w->n_positions;
+  m.wpe = w->wpe, m.embed_w = w->embed_w, m.embed_b = w->embed_b, m.pred_w = w->pred_w, m.pred_b = w->pred_b;
+  m.lnf_w = w->lnf_w, m.lnf_b = w->lnf_b;
+  for (int l = 0; l < L; ++l) {
+    m.ln1_w[l] = w->ln1_w[l], m.ln1_b[l] = w->ln1_b[l], m.attn_w[l] = w->attn_w[l], m.attn_b[l] = w->attn_b[l];
+    m.proj_w[l] = w->proj_w[l], m.proj_b[l] = w->proj_b[l], m.ln2_w[l] = w->ln2_w[l], m.ln2_b[l] = w->ln2_b[l];
+    m.fc_w[l] = w->fc_w[l], m.fc_b[l] = w->fc_b[l], m.fc2_w[l] = w->fc2_w[l], m.fc2_b[l] = w->fc2_b[l];
+  }
+  bp.dout = dout, bp.B = B, bp.T = T, bp.test = test ? 1 : 0;
+  bp.act = ws + lay.act, bp.fin = ws + lay.fin, bp.grec = ws + lay.grec, bp.gfin = ws + lay.gfin;
+  const int S = T + 1;
+  cudaError_t e = S <= 128 ? launch_back<128>(bp, st) : S <= 256 ? launch_back<256>(bp, st) : launch_back<512>(bp, st);
+  if (e != cudaSuccess) {
+    set_error("%s: backward launch failed: %s", fn, cudaGetErrorString(e));
+    return DPT_ERR_CUDA;
+  }
+
+  // weight-gradient jobs (operands in the workspace) and the gradient tensors they reduce into
+  RParams rp{};
+  RSegs rs{};
+  int nj = 0, nt = 0, ns = 0, off = 0;
+  auto job = [&](const float* A, int sa, const float* G, int sg, int nin, int nout, int diag, int trans, float* dw, float* db) {
+    RJob& j = rp.job[nj];
+    j.A = A, j.G = G, j.sa = sa, j.sg = sg, j.nin = nin, j.nout = nout, j.diag = diag, j.trans = trans;
+    const int nw = diag ? nout : nin * nout;
+    j.woff = off, rs.seg[ns++] = RSeg{dw, off, nw}, off += nw;
+    j.boff = off, rs.seg[ns++] = RSeg{db, off, nout}, off += nout;
+    if (diag) {
+      rp.tile[nt++] = RTile{(short)nj, 0, 0};
+    } else {
+      for (int i0 = 0; i0 < nin; i0 += 32)
+        for (int o0 = 0; o0 < nout; o0 += 32) rp.tile[nt++] = RTile{(short)nj, (short)i0, (short)o0};
+    }
+    ++nj;
+  };
+  const size_t NR = lay.NR;
+  for (int l = 0; l < L; ++l) {
+    const float* a = ws + lay.act + (size_t)l * NR * TA_STRIDE;
+    const float* gr = ws + lay.grec + (size_t)l * NR * GR_STRIDE;
+    job(gr + GR_G, GR_STRIDE, gr + GR_DX, GR_STRIDE, G_FF, G_E, 0, 0, g->fc2_w[l], g->fc2_b[l]);
+    job(gr + GR_Y2, GR_STRIDE, gr + GR_DH, GR_STRIDE, G_E, G_FF, 0, 0, g->fc_w[l], g->fc_b[l]);
+    job(gr + GR_XH2, GR_STRIDE, gr + GR_DY2, GR_STRIDE, G_E, G_E, 1, 0, g->ln2_w[l], g->ln2_b[l]);
+    job(a + TA_O, TA_STRIDE, gr + GR_DXM, GR_STRIDE, G_E, G_E, 0, 0, g->proj_w[l], g->proj_b[l]);
+    job(gr + GR_Y1, GR_STRIDE, gr + GR_DQKV, GR_STRIDE, G_E, 3 * G_E, 0, 0, g->attn_w[l], g->attn_b[l]);
+    job(gr + GR_XH1, GR_STRIDE, gr + GR_DY1, GR_STRIDE, G_E, G_E, 1, 0, g->ln1_w[l], g->ln1_b[l]);
+  }
+  const float* gf = ws + lay.gfin;
+  job(gf + GF_YF, GF_STRIDE, gf + GF_DLOG, GF_STRIDE, G_E, lay.du, 0, 1, g->pred_w, g->pred_b);
+  job(gf + GF_XHF, GF_STRIDE, gf + GF_DYF, GF_STRIDE, G_E, G_E, 1, 0, g->lnf_w, g->lnf_b);
+  job(ws + lay.fin + TF_TOK, TF_STRIDE, gf + GF_DX0, GF_STRIDE, lay.din, G_E, 0, 1, g->embed_w, g->embed_b);
+  if (off > lay.P) {
+    set_error("%s: internal: %d gradient entries exceed the partial slot of %d", fn, off, lay.P);
+    return DPT_ERR_CUDA;
+  }
+  rp.NR = (int)NR, rp.CH = lay.CH, rp.P = lay.P, rp.part = ws + lay.part;
+  weight_grad_partial_kernel<<<dim3(nt, lay.NC), 256, 0, st>>>(rp);
+  int maxn = 0;
+  for (int s = 0; s < ns; ++s) maxn = std::max(maxn, rs.seg[s].n);
+  rs.NC = lay.NC, rs.P = lay.P, rs.part = ws + lay.part;
+  weight_grad_reduce_kernel<<<dim3((maxn + 255) / 256, ns), 256, 0, st>>>(rs);
+  wpe_grad_kernel<<<(w->n_positions * G_E + 255) / 256, 256, 0, st>>>(ws + lay.gfin, B, S, w->n_positions, g->wpe);
+  DPT_LAUNCH_CHECK();
+  return DPT_OK;
+}

@@ -7,8 +7,10 @@ key layout (HuggingFace GPT2Model under ``transformer.``, ``embed_transition.*``
 so checkpoints written by the reference's train.py load unchanged.  As in the reference, ``n_head``
 from the config is ignored: the trunk always has ONE head (models/net.py:29), head_dim = n_embd.
 
-The forward pass is dpt_gpt2_forward (hand-written CUDA, fp32); this class holds no HuggingFace
-dependency and no autograd path -- training is out of scope of the rollout hot path.
+``forward`` is dpt_gpt2_forward (hand-written CUDA, fp32) under ``torch.no_grad()``.  ``forward_train`` is the
+same computation with a gradient: dpt_gpt2_train_forward / dpt_gpt2_train_backward (hand-written CUDA, fp32) read
+the parameter tensors in place, and autograd receives a gradient for every parameter except ``transformer.wte``
+(which the model never reads, as in the reference).  The class holds no HuggingFace dependency.
 """
 import ctypes
 
@@ -179,6 +181,39 @@ class Transformer(nn.Module):
               "dpt_gpt2_forward")
         return out
 
+    # ---- training: models/net.py:41-60 with a gradient ----------------------------------------
+    def _train_params(self):
+        """The parameters forward_train differentiates, in the order of dpt_gpt2_weights_t (transformer.wte excluded)."""
+        t = self.transformer
+        ps = [t.wpe.weight, self.embed_transition.weight, self.embed_transition.bias, self.pred_actions.weight,
+              self.pred_actions.bias, t.ln_f.weight, t.ln_f.bias]
+        for f in _LAYER_FIELDS:
+            ps += [f(b) for b in t.h]
+        return ps
+
+    def forward_train(self, x):
+        """``forward(x)`` with an autograd graph: returns ``preds[:, -1, :]`` (test) or ``preds[:, 1:, :]`` with a
+        ``grad_fn``; ``backward`` fills ``.grad`` of every parameter except ``transformer.wte``.  The logits are
+        bit-identical to ``forward(x)``.  The context inputs get no gradient.  fp32, sequences of <= 512 tokens."""
+        if self.dropout > 0:
+            raise NotImplementedError("forward_train: dropout=%g, the fused training path has no dropout" % self.dropout)
+        dev = kernels._dev()
+        if next(self.parameters()).device != dev:
+            self.to(dev)
+        f = lambda t: t.to(device=dev, dtype=torch.float32)   # noqa: E731
+        q = f(x["query_states"]).contiguous()
+        cs, ca, cns, cr = f(x["context_states"]), f(x["context_actions"]), f(x["context_next_states"]), f(x["context_rewards"])
+        B, T = ca.shape[0], ca.shape[1]
+        assert q.shape[0] == B, "query_states and the context disagree on the batch size"
+        # context views [:, :h] of a [B,H,.] buffer are passed with their row stride, without a copy
+        stride = ca.stride(0) // max(1, ca.shape[2]) if T > 0 else 0
+        ok = T > 0 and stride >= T and all(t.stride(-1) == 1 and t.stride(1) == t.shape[2] and t.stride(0) == stride * t.shape[2]
+                                           for t in (cs, ca, cns, cr.reshape(B, T, 1) if cr.dim() == 2 else cr))
+        if not ok:
+            cs, ca, cns, cr = cs.contiguous(), ca.contiguous(), cns.contiguous(), cr.contiguous()
+            stride = T
+        return _TrainFn.apply(self, (q, cs, ca, cns, cr, B, T, stride), *self._train_params())
+
     # ---- step-by-step K/V-cached decode (callers that choose the pulled arm themselves) -------------
     def decoder(self, n_seqs, max_transitions=None):
         """A K/V-cached incremental view of ``forward(...)[:, -1]`` for loops that are driven from outside (the rollout
@@ -236,6 +271,73 @@ class Transformer(nn.Module):
         if noise is not None:
             out["noise"] = noise
         return out
+
+
+_LAYER_FIELDS = (lambda b: b.ln_1.weight, lambda b: b.ln_1.bias, lambda b: b.attn.c_attn.weight, lambda b: b.attn.c_attn.bias,
+                 lambda b: b.attn.c_proj.weight, lambda b: b.attn.c_proj.bias, lambda b: b.ln_2.weight, lambda b: b.ln_2.bias,
+                 lambda b: b.mlp.c_fc.weight, lambda b: b.mlp.c_fc.bias, lambda b: b.mlp.c_proj.weight, lambda b: b.mlp.c_proj.bias)
+_LAYER_NAMES = ("ln1_w", "ln1_b", "attn_w", "attn_b", "proj_w", "proj_b", "ln2_w", "ln2_b", "fc_w", "fc_b", "fc2_w", "fc2_b")
+_TOP_NAMES = ("wpe", "embed_w", "embed_b", "pred_w", "pred_b", "lnf_w", "lnf_b")
+
+
+def _pointer_struct(cls, model, tensors, keep, **extra):
+    """dpt_gpt2_weights_t / dpt_gpt2_grads_t over `tensors` (ordered as Transformer._train_params)."""
+    L = model.n_layer
+    for t in tensors:
+        if t.dtype != torch.float32 or not t.is_contiguous() or not t.is_cuda:
+            raise ValueError("forward_train needs contiguous fp32 CUDA parameters")
+    kw = {n: t.data_ptr() for n, t in zip(_TOP_NAMES, tensors)}
+    for i, n in enumerate(_LAYER_NAMES):
+        a = (ctypes.c_void_p * L)(*[t.data_ptr() for t in tensors[7 + i * L:7 + (i + 1) * L]])
+        keep.append(a)
+        kw[n] = ctypes.cast(a, ctypes.POINTER(ctypes.c_void_p))
+    kw.update(extra)
+    return cls(**kw)
+
+
+def _weights_struct(model, params, keep):
+    return _pointer_struct(_lib.Gpt2Weights, model, params, keep, horizon=model.horizon, state_dim=model.state_dim,
+                           action_dim=model.action_dim, n_layer=model.n_layer, n_embd=model.n_embd,
+                           n_positions=model.transformer.wpe.weight.shape[0])
+
+
+class _TrainFn(torch.autograd.Function):
+    """dpt_gpt2_train_forward / dpt_gpt2_train_backward.  The workspace holds the saved activations between the two."""
+
+    @staticmethod
+    def forward(ctx, model, inputs, *params):
+        q, cs, ca, cns, cr, B, T, stride = inputs
+        dev = q.device
+        keep = []
+        w = _weights_struct(model, params, keep)
+        out = torch.empty((B, model.action_dim) if model.test else (B, T, model.action_dim), dtype=torch.float32, device=dev)
+        nbytes = lib().dpt_gpt2_train_workspace_bytes(ctypes.byref(w), B, T)
+        ws = torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=dev)
+        check(lib().dpt_gpt2_train_forward(ctypes.byref(w), q.data_ptr(), cs.data_ptr() if T else None, ca.data_ptr() if T else None,
+                                           cns.data_ptr() if T else None, cr.data_ptr() if T else None, B, T, stride,
+                                           1 if model.test else 0, out.data_ptr(), ws.data_ptr(), ws.numel(), stream_ptr()),
+              "dpt_gpt2_train_forward")
+        ctx.model, ctx.ws, ctx.B, ctx.T, ctx.test = model, ws, B, T, model.test
+        ctx.save_for_backward(*params)
+        return out
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dout):
+        params = ctx.saved_tensors
+        grads = [torch.empty_like(p) for p in params]
+        if ctx.B == 0:
+            for g in grads:
+                g.zero_()
+            return (None, None, *grads)
+        keep = []
+        w = _weights_struct(ctx.model, params, keep)
+        g = _pointer_struct(_lib.Gpt2Grads, ctx.model, grads, keep)
+        dout = dout.to(torch.float32).contiguous()
+        check(lib().dpt_gpt2_train_backward(ctypes.byref(w), dout.data_ptr(), ctx.B, ctx.T, 1 if ctx.test else 0, ctypes.byref(g),
+                                            ctx.ws.data_ptr(), ctx.ws.numel(), stream_ptr()), "dpt_gpt2_train_backward")
+        ctx.ws = None
+        return (None, None, *grads)
 
 
 class _Decoder:

@@ -35,7 +35,7 @@ extern "C" {
 #define DPT_ERR_CUDA (-2)
 #define DPT_ERR_UNSUPPORTED (-3)
 
-#define DPT_ABI_VERSION 4
+#define DPT_ABI_VERSION 5
 
 /* reward_type of the bandit entry points (envs/bandit_env.py:56-63, envs/gpu_bandit_env.py:53-63):
  * 0 'uniform'  : r = means[a] + var * z, z ~ N(0,1);
@@ -340,6 +340,45 @@ uint64_t dpt_gpt2_forward_workspace_bytes(const dpt_gpt2_t* m, int B, int T, int
 int dpt_gpt2_forward(dpt_gpt2_t* m, const float* query_states, const float* ctx_states, const float* ctx_actions,
                      const float* ctx_next_states, const float* ctx_rewards, int B, int T, int T_stride, int ctx_share,
                      int test, int precision, float* out, void* workspace, uint64_t workspace_bytes, void* stream);
+
+/* Training (train.py:252-331 with Transformer.forward, models/net.py:41-60): fp32, sequences of <= 512 tokens, the
+ * parameter tensors read in place through dpt_gpt2_weights_t (no handle, no repack, no host synchronisation).
+ * dpt_gpt2_train_forward computes the same logits as dpt_gpt2_forward(precision = 0), bit for bit, and saves the
+ * activations the backward needs in `workspace` (dpt_gpt2_train_workspace_bytes(w, B, T) bytes, 16 B aligned, the same
+ * buffer for both calls).  dpt_gpt2_train_backward takes dout, the gradient of the logits ([B,du] if test, else
+ * [B,T,du]), and OVERWRITES every gradient of `grads` (transformer.wte is not an input and has none): weight gradients
+ * are sums over all B*(T+1) rows reduced in a fixed order (two identical calls give bit-identical gradients); wpe's
+ * gradient has n_positions rows, zero past row T.  The context inputs get no gradient.  B = 0 is a no-op.  n_embd != 32,
+ * n_layer > 8 and T + 1 > 512 return DPT_ERR_UNSUPPORTED. */
+typedef struct {
+  float* wpe;
+  float* embed_w;
+  float* embed_b;
+  float* pred_w;
+  float* pred_b;
+  float* lnf_w;
+  float* lnf_b;
+  /* per layer arrays of n_layer pointers (HOST arrays of DEVICE pointers), as in dpt_gpt2_weights_t */
+  float* const* ln1_w;
+  float* const* ln1_b;
+  float* const* attn_w;
+  float* const* attn_b;
+  float* const* proj_w;
+  float* const* proj_b;
+  float* const* ln2_w;
+  float* const* ln2_b;
+  float* const* fc_w;
+  float* const* fc_b;
+  float* const* fc2_w;
+  float* const* fc2_b;
+} dpt_gpt2_grads_t;
+
+uint64_t dpt_gpt2_train_workspace_bytes(const dpt_gpt2_weights_t* w, int B, int T);
+int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, const float* query_states, const float* ctx_states,
+                           const float* ctx_actions, const float* ctx_next_states, const float* ctx_rewards, int B, int T,
+                           int T_stride, int test, float* out, void* workspace, uint64_t workspace_bytes, void* stream);
+int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float* dout, int B, int T, int test,
+                            const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream);
 
 /* Fused bandit online loop with the transformer controller: evals/eval_bandit.py:56-103 +
  * ctrls/ctrl_bandit.py:383-444 (BanditTransformerController, sample != 0 -> softmax + categorical
