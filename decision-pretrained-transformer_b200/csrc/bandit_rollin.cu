@@ -200,11 +200,10 @@ __device__ __forceinline__ int argmax_first(const float* m, int D) {
 // Resident CTAs per SM the fast kernel is compiled for: 5 up to d = 5 (48 registers; left to itself ptxas takes 50-64 and the SM
 // holds 4 CTAs: 0.320 against 0.292 ms at 125k x 500, d = 5); d = 6 .. 10: 4 (<= 64 registers); d = 16: 2 (<= 128; at 3 the
 // Philox instantiations spill).  No instantiation spills.
-#ifndef DPT_RB_MINB
-#define DPT_RB_MINB (D <= 5 ? 5 : D <= 10 ? 4 : 2)
-#endif
+template <int D>
+constexpr int rb_min_blocks() { return D <= 5 ? 5 : D <= 10 ? 4 : 2; }
 template <int D, int MODE, int RT>   // RT: DPT_REWARD_* (compile-time: the kernel sits at the issue / HBM balance point)
-__global__ void __launch_bounds__(RB_THREADS, DPT_RB_MINB) bandit_rollin_fast(const RollinParams p) {
+__global__ void __launch_bounds__(RB_THREADS, rb_min_blocks<D>()) bandit_rollin_fast(const RollinParams p) {
   using thr_t = typename Thr<MODE>::type;
   using qbits_t = typename std::conditional<(4 * D > 32), uint64_t, uint32_t>::type;   // a quad's one-hot bit string
   __shared__ float4 s_nib[16];

@@ -23,18 +23,12 @@
 #include <cuda_bf16.h>
 
 #include <algorithm>
-#include <cstdlib>
-
 #include <type_traits>
 
 #include "common.cuh"
 #include "philox.cuh"
 
 #include "gpt2_model.cuh"
-
-#ifndef DPT_GPT2_KPRED
-#define DPT_GPT2_KPRED 0   // register-staged K loads: 1 = predicate the rows past the last key (measured below)
-#endif
 
 namespace dpt {
 
@@ -154,15 +148,8 @@ __global__ void pack_wfrag_kernel(const float* __restrict__ W, uint4* __restrict
 }
 
 // resident CTAs per SM the online-loop kernels are compiled for (register cap = 65536 / (128 * n)); measured on B200
-#ifndef DPT_GPT2_MINB_F32
-#define DPT_GPT2_MINB_F32 9   // 56 registers: 221 ms at C4 against 241 ms (8) / 226 ms (7) / 270 ms (10)
-#endif
-#ifndef DPT_GPT2_MINB_BF16
-#define DPT_GPT2_MINB_BF16 6
-#endif
-#ifndef DPT_GPT2_BF16_PREFETCH_V
-#define DPT_GPT2_BF16_PREFETCH_V 0   // measured: 161 ms with, 155 ms without (C4, bf16 K/V)
-#endif
+constexpr int GPT2_MINB_F32 = 9;   // 56 registers: 221 ms at C4 against 241 ms (8) / 226 ms (7) / 270 ms (10)
+constexpr int GPT2_MINB_BF16 = 6;
 
 // WS: the projections run on the tensor cores from bf16 weight fragments in shared memory (`wf`, all layers)
 template <bool BF16, bool WS = false>
@@ -203,20 +190,15 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
       // cached keys 0..pos-1, 32 per tile: 8 row loads in flight per lane.  TAIL = the last, partial tile: load instruction i
       // covers keys k0 + 4 i .. k0 + 4 i + 3 of all key groups, so instructions past the last key are skipped with a
       // WARP-UNIFORM predicate (round 2: the padded rows of the last tile were 4.7 % of the kernel's DRAM traffic; per-lane
-      // predication of every tile, DPT_GPT2_KPRED, cost more issue than the bytes saved)
+      // predication of every tile, which skips 3-5 % of the K/V traffic at H = 500, cost more issue than the bytes saved)
       auto k_tile = [&](const int k0, auto tail_tag) {
         constexpr bool TAIL = decltype(tail_tag)::value;
         const int r = pos - k0;
         if (pos <= PF_MAX_POS && k0 + PF_AHEAD * 32 < pos) prefetch_l2(K + (size_t)(k0 + PF_AHEAD * 32 + lane) * G_E);
         float4 kk[8];
   #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-#if DPT_GPT2_KPRED   // rows >= pos are not read (3-5 % of the K/V traffic at H = 500)
-          kk[i] = (k0 + 4 * i + g < pos) ? __ldcg(K4 + (size_t)(k0 + 4 * i + g) * 8) : make_float4(0.f, 0.f, 0.f, 0.f);
-#else
+        for (int i = 0; i < 8; ++i)
           kk[i] = (!TAIL || 4 * i < r) ? __ldcg(K4 + (size_t)(k0 + 4 * i + g) * 8) : make_float4(0.f, 0.f, 0.f, 0.f);   // in bounds (Tpad % 32 == 0)
-#endif
-        }
         float pv[8];
   #pragma unroll
         for (int i = 0; i < 8; ++i) pv[i] = fmaf(q4.x, kk[i].x, fmaf(q4.y, kk[i].y, fmaf(q4.z, kk[i].z, q4.w * kk[i].w)));
@@ -339,17 +321,9 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
         const int r = pos - k0;
         uint4 kk[8];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-#if DPT_GPT2_KPRED   // rows >= pos are not read (~6 % of the K/V traffic at H = 500)
-          kk[i] = (k0 + 8 * i + g < pos) ? __ldcg(K8 + (size_t)(k0 + 8 * i + g) * 4) : make_uint4(0u, 0u, 0u, 0u);
-#else
+        for (int i = 0; i < 8; ++i)
           kk[i] = (!TAIL || 8 * i < r) ? __ldcg(K8 + (size_t)(k0 + 8 * i + g) * 4) : make_uint4(0u, 0u, 0u, 0u);   // in bounds (Tpad % 64 == 0)
-#endif
-        }
-        // the V blocks of the same 64 keys (4 KB = one 128 B line per lane) start their trip from HBM to L2 now; the
-        // P V pass below then waits an L2 rather than a DRAM latency (this mode is latency-, not bandwidth-bound)
-        if (DPT_GPT2_BF16_PREFETCH_V && k0 + 16 * (lane >> 3) < pos)
-          prefetch_l2(reinterpret_cast<const unsigned char*>(V) + (size_t)(k0 >> 4) * 1024 + lane * 128);
+        // (an L2 prefetch of the same 64 keys' V blocks here was measured slower: 161 ms with, 155 ms without, C4)
         // scores^T = K q^T: 16 keys are the rows of the A tile (octets 2m and 2m + 1), q is column 0 of B
 #pragma unroll
         for (int mt = 0; mt < 4; ++mt) {
@@ -466,21 +440,16 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
 // stream keeps flowing through the softmax between the K and the V pass and through the projections / MLP between
 // layers -- with register-staged loads (token_forward above) a warp has nothing in flight during those phases.
 // ---------------------------------------------------------------------------------------------
-#ifndef DPT_GPT2_TMA_WARPS
-#define DPT_GPT2_TMA_WARPS 4
-#endif
-#ifndef DPT_GPT2_TMA_MINB
-#define DPT_GPT2_TMA_MINB 5   // 96 registers: 20 warps per SM with a 2-deep ring (measured best at 10k envs: 210 ms; 4 CTAs / 128 regs: 257 ms)
-#endif
-constexpr int KV_MAX_STAGES = 8;   // ring depth is a launch parameter: as deep as shared memory allows for the CTAs that must be resident
+constexpr int TMA_WARPS = 4;
+constexpr int TMA_MINB = 5;   // 96 registers: 20 warps per SM with a 2-deep ring (measured best at 10k envs: 210 ms; 4 CTAs / 128 regs: 257 ms)
+constexpr int KV_STAGES = 2;  // ring depth: measured at 1250 and 10000 envs, 2 stages beat 3, 4 and 6 (DESIGN.md)
 constexpr int KV_TILE_BYTES = 32 * G_E * 4;   // 32 keys x 32 channels fp32
 
 __device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 struct KvRing {
   uint32_t stage0, bar0;        // shared addresses: stage s at stage0 + s * KV_TILE_BYTES, its mbarrier at bar0 + 8 s
-  uint32_t S;                   // ring depth (2 .. KV_MAX_STAGES)
-  uint32_t is, ip;              // stage the next issued tile goes to, and (unused by the producer) its lap
+  uint32_t is;                  // stage the next issued tile goes to
   uint32_t cs, cp;              // stage of the next tile to consume, and the parity of its mbarrier phase
   int cl, ckv, ct;              // cursor of the next tile to issue: layer, K (0) / V (1), tile
   int nt, pos, L, Tpad;
@@ -499,7 +468,7 @@ struct KvRing {
                    "r"(bar)
                    : "memory");
     }
-    if (++is == S) is = 0;
+    if (++is == KV_STAGES) is = 0;
     if (++ct == nt) {
       ct = 0;
       if (++ckv == 2) ckv = 0, ++cl;
@@ -509,7 +478,7 @@ struct KvRing {
   __device__ __forceinline__ void begin_token(int pos_, int lane) {
     pos = pos_, nt = (pos_ + 31) >> 5;
     cl = nt ? 0 : L, ckv = 0, ct = 0;
-    for (uint32_t i = 0; i < S; ++i) issue_next(lane);
+    for (int i = 0; i < KV_STAGES; ++i) issue_next(lane);
   }
   // wait for the next tile in sequence; returns its shared-memory address as a generic pointer
   __device__ __forceinline__ const float4* acquire() {
@@ -523,7 +492,7 @@ struct KvRing {
   // every lane has finished reading the tile: its stage is free for the next copy
   __device__ __forceinline__ void release(int lane) {
     __syncwarp();
-    if (++cs == S) cs = 0, cp ^= 1u;
+    if (++cs == KV_STAGES) cs = 0, cp ^= 1u;
     issue_next(lane);
   }
 };
@@ -767,7 +736,6 @@ struct OnlineGptParams {
   Key key;
   uint64_t env_id0;
   int N, H, Tpad;
-  int kv_stages;   // depth of the per-warp bulk-async K/V ring (TMA kernel)
   void* kv;
   float *ctx_s, *ctx_a, *ctx_ns, *ctx_r, *cum_means;
   double* regret;
@@ -777,17 +745,13 @@ struct OnlineGptParams {
 
 // WS (precision 1): ONE CTA of GW_WARPS warps per SM shares the bf16 weight fragments of all layers in shared memory
 // (24 KB per layer) and every warp runs its env's projections on the tensor cores from there.
-#ifndef DPT_GPT2_GW_WARPS
-#define DPT_GPT2_GW_WARPS 24
-#endif
-constexpr int GW_WARPS = DPT_GPT2_GW_WARPS;
+constexpr int GW_WARPS = 24;
 constexpr int GW_THREADS = GW_WARPS * 32;
 
-constexpr int TMA_WARPS = DPT_GPT2_TMA_WARPS;
 // TMA (precision 0 only): the fp32 K/V stream is staged through a per-warp ring of bulk-async copies (KvRing)
 template <bool BF16, bool WS, bool TMA = false>
 __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_THREADS),
-                                  WS ? 1 : (TMA ? DPT_GPT2_TMA_MINB : (BF16 ? DPT_GPT2_MINB_BF16 : DPT_GPT2_MINB_F32)))
+                                  WS ? 1 : (TMA ? TMA_MINB : (BF16 ? GPT2_MINB_BF16 : GPT2_MINB_F32)))
     gpt2_online_kernel(const OnlineGptParams p) {
   extern __shared__ __align__(128) float g_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -798,18 +762,16 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
   if constexpr (TMA) {   // [warps][KV_STAGES] tiles of 4 KB | [warps][KV_STAGES] mbarriers | per-warp scratch
     const int nw = blockDim.x >> 5;
     unsigned char* base = reinterpret_cast<unsigned char*>(g_smem);
-    const int S = p.kv_stages;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(base + (size_t)nw * S * KV_TILE_BYTES);
-    if (threadIdx.x < nw * S)
+    uint64_t* bars = reinterpret_cast<uint64_t*>(base + (size_t)nw * KV_STAGES * KV_TILE_BYTES);
+    if (threadIdx.x < nw * KV_STAGES)
       asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(bars + threadIdx.x)) : "memory");
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
-    ring.S = (uint32_t)S;
-    ring.stage0 = smem_addr(base + (size_t)warp * S * KV_TILE_BYTES);
-    ring.bar0 = smem_addr(bars + warp * S);
-    ring.is = ring.ip = ring.cs = ring.cp = 0;
+    ring.stage0 = smem_addr(base + (size_t)warp * KV_STAGES * KV_TILE_BYTES);
+    ring.bar0 = smem_addr(bars + warp * KV_STAGES);
+    ring.is = ring.cs = ring.cp = 0;
     ring.L = m.L, ring.Tpad = p.Tpad;
-    scratch = reinterpret_cast<float*>(bars + ((nw * S + 1) & ~1));   // keep the per-warp scratch 16 B aligned
+    scratch = reinterpret_cast<float*>(bars + ((nw * KV_STAGES + 1) & ~1));   // keep the per-warp scratch 16 B aligned
   }
   if constexpr (WS) {
     uint4* dst = reinterpret_cast<uint4*>(g_smem);
@@ -937,7 +899,7 @@ struct ExploreParams {
   dpt_explore_dump_t out;
 };
 
-__global__ void __launch_bounds__(G_THREADS, DPT_GPT2_MINB_F32) gpt2_explore_exploit_kernel(const ExploreParams p) {
+__global__ void __launch_bounds__(G_THREADS, GPT2_MINB_F32) gpt2_explore_exploit_kernel(const ExploreParams p) {
   extern __shared__ __align__(128) float g_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int env = blockIdx.x * G_WARPS + warp;
@@ -1265,24 +1227,15 @@ extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double va
     DPT_LAUNCH_CHECK();
     return DPT_OK;
   }
-  static const int use_tma = [] {
-    const char* e = getenv("DPT_GPT2_TMA");
-    return e ? atoi(e) : -1;
-  }();
-  // fp32 K/V staged by bulk-async copies (cp.async.bulk + mbarrier ring per warp).  DPT_GPT2_TMA: 1 = always, 0 = never,
-  // unset = when the batch leaves warp slots empty (fewer than ~36 env-warps per SM): there the register-staged kernel
-  // cannot keep enough bytes in flight (0.43 of the HBM bound at 1250 envs) and a deep ring can (0.8+)
+  // fp32 K/V staged by bulk-async copies (cp.async.bulk + mbarrier ring per warp) when the batch leaves warp slots empty
+  // (fewer than ~36 env-warps per SM): there the register-staged kernel cannot keep enough bytes in flight (0.43 of the HBM
+  // bound at 1250 envs) and a ring can (0.8+)
   const long env_warps_per_sm = ((long)N + sm_count() - 1) / sm_count();
-  const bool tma = !precision && (use_tma == 1 || (use_tma < 0 && env_warps_per_sm <= 24));
-  if (tma) {
+  if (!precision && env_warps_per_sm <= 24) {
     // CTA size: small batches get small CTAs so that the SMs carry equal numbers of warps (1250 envs = 8.4 warps per SM:
     // 4-warp CTAs would put 12 warps on some SMs and 8 on the others)
-    int nw = env_warps_per_sm <= 12 ? 1 : (env_warps_per_sm <= 20 ? 2 : TMA_WARPS);
-    if (const char* e = getenv("DPT_GPT2_TMA_WARPS")) nw = std::max(1, std::min(TMA_WARPS, atoi(e)));   // (measurement override)
-    int S = 2;   // measured at 1250 and 10000 envs: 2 stages beat 3, 4 and 6 (DESIGN.md)
-    if (const char* e = getenv("DPT_GPT2_KV_STAGES")) S = std::max(2, std::min(KV_MAX_STAGES, atoi(e)));   // (measurement override)
-    p.kv_stages = S;
-    const size_t smem_tma = (size_t)nw * (S * (KV_TILE_BYTES + 8) + per_warp) + 8;
+    const int nw = env_warps_per_sm <= 12 ? 1 : (env_warps_per_sm <= 20 ? 2 : TMA_WARPS);
+    const size_t smem_tma = (size_t)nw * (KV_STAGES * (KV_TILE_BYTES + 8) + per_warp) + 8;
     int rc = launch_smem((const void*)gpt2_online_kernel<false, false, true>, smem_tma);
     if (rc != DPT_OK) return rc;
     gpt2_online_kernel<false, false, true><<<(N + nw - 1) / nw, nw * 32, smem_tma, (cudaStream_t)stream>>>(p);

@@ -7,7 +7,6 @@
 #include <atomic>
 #include <chrono>
 #include <cstdlib>
-#include <cstring>
 #include <condition_variable>
 #include <memory>
 #include <mutex>
@@ -17,14 +16,7 @@
 #include "common.cuh"
 
 namespace dpt {
-static int host_chunk_envs() {
-  static const int v = [] {
-    const char* e = getenv("DPT_HOST_CHUNK_ENVS");
-    const int n = e ? atoi(e) : 0;
-    return n >= 256 ? n : 8192;
-  }();
-  return v;
-}
+constexpr int HOST_CHUNK_ENVS = 8192;   // envs per pipeline chunk
 
 struct ChunkLayout {
   size_t means, s, a, ns, r, total;  // float offsets
@@ -50,7 +42,7 @@ extern "C" uint64_t dpt_bandit_rollin_host_last_d2h_bytes(void) { return t_last_
 
 extern "C" uint64_t dpt_bandit_rollin_host_scratch_bytes(int N, int H, int d) {
   if (N <= 0 || H <= 0 || d <= 0) return 0;
-  const int C = N < host_chunk_envs() ? N : host_chunk_envs();
+  const int C = N < HOST_CHUNK_ENVS ? N : HOST_CHUNK_ENVS;
   return 2 * chunk_layout(C, H, d).total * sizeof(float);
 }
 
@@ -63,14 +55,9 @@ extern "C" uint64_t dpt_bandit_rollin_host_scratch_bytes(int N, int H, int d) {
 // bit-identical results (the same Philox counters; tests/test_rollout_gpu.py::test_bandit_rollin_host_path).
 namespace {
 constexpr int HOST_PARTS = 16;  // host jobs per chunk and phase
-
-// DPT_HOST_COMPACT: "auto" (default: a chunk goes compact whenever the host workers are about to run dry, otherwise by
-// DMA -- self-balancing between PCIe and the host cores), "0" (all chunks by DMA) or "1" (all compact).
-int compact_policy() {
-  const char* e = getenv("DPT_HOST_COMPACT");
-  if (!e || !strcmp(e, "auto")) return -1;
-  return atoi(e) != 0;
-}
+// compact chunks queued for the host before a chunk goes by DMA; measured on a 16-core host: 1: 2.8, 2: 3.4, 3: 4.4,
+// 4: 4.9, 6: 5.0 G env-steps/s
+constexpr int HOST_BACKLOG = 4;
 
 // Host-side writers use non-temporal stores: the output arrays are written once and never read here, and a normal
 // store would first pull every cache line in from DRAM (read-for-ownership), doubling the memory traffic that
@@ -429,7 +416,7 @@ static int rollin_host_impl(const float* means_host, float var, uint64_t seed, u
   DPT_CHECK_ARG(scratch && scratch_bytes >= dpt_bandit_rollin_host_scratch_bytes(N, H, d),
                 "dpt_bandit_rollin_host: scratch too small (%llu < %llu bytes)", (unsigned long long)scratch_bytes,
                 (unsigned long long)dpt_bandit_rollin_host_scratch_bytes(N, H, d));
-  const int C = N < host_chunk_envs() ? N : host_chunk_envs();
+  const int C = N < HOST_CHUNK_ENVS ? N : HOST_CHUNK_ENVS;
   const ChunkLayout L = chunk_layout(C, H, d);
   cudaStream_t cs = (cudaStream_t)stream;
   struct Res {   // the pipeline's own stream and events: released on every return path
@@ -466,7 +453,7 @@ static int rollin_host_impl(const float* means_host, float var, uint64_t seed, u
   jobs.compact.assign(jobs.K, 0);
   jobs.enqueued.reset(new std::atomic<int>[jobs.K]);
   jobs.phase1_left.reset(new std::atomic<int>[jobs.K]);
-  const int policy = wide ? 1 : ((jobs.K >= 4 && d <= 255) ? compact_policy() : 0);
+  const bool balance = !wide && jobs.K >= 4 && d <= 255;   // wide: every chunk compact; few chunks or d > 255: every chunk by DMA
   for (int kk = 0; kk < jobs.K; ++kk) {
     jobs.enqueued[kk].store(0);
     jobs.phase1_left[kk].store(HOST_PARTS);
@@ -478,10 +465,6 @@ static int rollin_host_impl(const float* means_host, float var, uint64_t seed, u
   HostPool& pool = HostPool::get();
   const int n_workers = (int)std::min<size_t>((size_t)pool.capacity(), std::max<size_t>(1, total_rows >> 18));
   pool.start(&jobs, n_workers);
-  static const int backlog = [] {
-    const char* e = getenv("DPT_HOST_BACKLOG");
-    return std::max(1, e ? atoi(e) : 4);   // measured on a 16-core host: 1: 2.8, 2: 3.4, 3: 4.4, 4: 4.9, 6: 5.0 G env-steps/s
-  }();
   int rc = DPT_OK;
   int k = 0;
   uint64_t d2h_bytes = 0;
@@ -495,11 +478,11 @@ static int rollin_host_impl(const float* means_host, float var, uint64_t seed, u
     };
     if (k >= 2) ck(cudaEventSynchronize(freed[b]));    // buffer b's previous D2H has drained (host-side pacing)
     // kind of this chunk: compact when the host workers would otherwise run out of expansion work
-    // auto: the host cores expand compact chunks (5 B per step over PCIe) as fast as they can -- with the table-driven
+    // balance: the host cores expand compact chunks (5 B per step over PCIe) as fast as they can -- with the table-driven
     // expansion that alone reaches the host's measured store bandwidth on a 16-core box -- and a chunk goes by DMA
-    // (24 B per step over PCIe, 8 B per step of host work) only while more than `backlog` compact chunks are queued
+    // (24 B per step over PCIe, 8 B per step of host work) only while more than HOST_BACKLOG compact chunks are queued
     // for the host, i.e. when the cores, not PCIe, are what the pipeline waits for (few cores per rank at 8 GPUs)
-    jobs.compact[k] = policy < 0 ? (jobs.compact_parts_pending.load() < backlog * HOST_PARTS) : (char)policy;
+    jobs.compact[k] = wide || (balance && jobs.compact_parts_pending.load() < HOST_BACKLOG * HOST_PARTS);
     if (jobs.compact[k]) jobs.compact_parts_pending.fetch_add(HOST_PARTS);
     ck(cudaMemcpyAsync(buf + L.means, means_host + (size_t)e0 * d, sizeof(float) * n * d, cudaMemcpyHostToDevice, cs));
     const size_t row = (size_t)e0 * H, nrow = (size_t)n * H;

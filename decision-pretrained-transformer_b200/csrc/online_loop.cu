@@ -16,8 +16,6 @@
 // A thread's own rows are strided by H*d*4 B, so rows are staged per warp in shared memory (1 B per
 // action, 4 B per reward, 32 envs x 32 steps) and flushed as contiguous, 16 B-aligned float4 runs
 // (32 steps * d * 4 B per env).
-#include <cstdlib>
-
 #include <atomic>
 
 #include "online_loop.cuh"
@@ -474,16 +472,11 @@ extern "C" int dpt_online_loop(int ctrl_kind, double p0, double p1, double p2, c
   cudaStream_t st = (cudaStream_t)stream;
   // Every warp adds its 32 envs' partial sums to the same [H,4] block, tile by tile and nearly in lockstep:
   // spread them over replicated accumulators (stream-ordered scratch, <= 4 MB) and fold the replicas afterwards.
-  // DPT_OL_IMPL: 0 / unset = online_loop_ws.cu where it applies (d <= 10, lin_d == 2): the split pipeline (controller kernel, then
-  // context expansion) for Opt / EmpMean / UCB and for small batches, the single fused kernel for Thompson / LinUCB at large batches
-  // (their controller chains are long enough to hide the fused kernel's scattered stores: 100k x 200, d = 10: 0.50 / 0.65 ms fused
-  // against 0.56 / 0.71 ms split); 2 = always fused, 3 = always split, 1 = always the general kernel
-  static const int env_impl = [] {
-    const char* s = getenv("DPT_OL_IMPL");
-    return s ? atoi(s) : 0;
-  }();
-  const int ovr = g_online_impl.load(std::memory_order_relaxed);
-  const int impl = ovr >= 0 ? ovr : env_impl;
+  // Automatic choice (dpt_debug_online_impl -1 / 0): online_loop_ws.cu where it applies (d <= 10, lin_d == 2): the split pipeline
+  // (controller kernel, then context expansion) for Opt / EmpMean / UCB and for small batches, the single fused kernel for Thompson /
+  // LinUCB at large batches (their controller chains are long enough to hide the fused kernel's scattered stores: 100k x 200,
+  // d = 10: 0.50 / 0.65 ms fused against 0.56 / 0.71 ms split); 2 = always fused, 3 = always split, 1 = always the general kernel
+  const int impl = g_online_impl.load(std::memory_order_relaxed);
   const bool ws = impl != 1 && online_ws_supported(ctrl_kind, p);
   double* reps = nullptr;
   unsigned char* scratch = nullptr;

@@ -30,28 +30,10 @@
 
 namespace dpt {
 
-#ifndef DPT_WS_WT5
-#define DPT_WS_WT5 32
-#endif
-#ifndef DPT_WS_WT10
-#define DPT_WS_WT10 16
-#endif
-#ifndef DPT_WS_STAGGER
-#define DPT_WS_STAGGER 0   // measured: no gain (opt 0.668 -> 0.673 ms, Thompson 0.79 -> 1.01 ms)
-#endif
-#ifndef DPT_WS_FILL_TILE
-#define DPT_WS_FILL_TILE 0
-#endif
-#ifndef DPT_WS_SKIP
-#define DPT_WS_SKIP 0   // measurement builds: 1 = no one-hot stores, 2 = no constant-column fill, 4 = no reward stores
-#endif
-#ifndef DPT_WS_NCONS
-#define DPT_WS_NCONS 4
-#endif
 // steps per staging tile (multiple of 4): 32 at d <= 5, 16 at d <= 10 (shared memory per warp: 32 warps must stay resident)
 template <int DMAX>
-constexpr int ws_wt() { return DMAX <= 5 ? DPT_WS_WT5 : DPT_WS_WT10; }
-constexpr int WS_NCONS = DPT_WS_NCONS; // warps per CTA
+constexpr int ws_wt() { return DMAX <= 5 ? 32 : 16; }
+constexpr int WS_NCONS = 4; // warps per CTA
 
 template <int DMAX>
 struct alignas(16) WsTile {
@@ -63,29 +45,6 @@ struct alignas(16) WsTile {
   uint32_t bits[32][BROW];   // one-hot rows of each step quad as a bit string (DMAX bits per step): nibble f of quad q is
                              // float4 q DMAX + f of the env's run of T d floats
 };
-
-// Measurement builds (-DDPT_TIMELINE): first-CTA-start / last-CTA-end of every kernel of a pass on the GPU's global timer,
-// the stand-in for a timeline profiler on a box without nsys (scripts/ol_timeline.py)
-#ifdef DPT_TIMELINE
-__device__ unsigned long long g_tl[64][2];
-struct TlScope {
-  int id;
-  static __device__ __forceinline__ unsigned long long now() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-  }
-  __device__ __forceinline__ explicit TlScope(int i) : id(i) {
-    if (threadIdx.x == 0) atomicMin(&g_tl[id][0], now());
-  }
-  __device__ __forceinline__ ~TlScope() {
-    if (threadIdx.x == 0) atomicMax(&g_tl[id][1], now());
-  }
-};
-#define DPT_TL(id) TlScope tl_scope_(id)
-#else
-#define DPT_TL(id)
-#endif
 
 struct WsNoTile {};
 
@@ -198,8 +157,7 @@ struct WsKernel {
                                                bool bits_ok, bool vec_r, int lane) {
     const int H = p.H, d = p.d;
     // rewards: T * 4 B per env and tile
-    if (DPT_WS_SKIP & 4) {
-    } else if (vec_r) {
+    if (vec_r) {
 #pragma unroll
       for (int it = 0; it < WQ; ++it) {
         const int e = it * (32 / WQ) + lane / WQ, q = lane % WQ;
@@ -217,7 +175,6 @@ struct WsKernel {
       }
     }
     // one-hot rows
-    if (DPT_WS_SKIP & 1) return;   // (measurement builds only)
     if (bits_ok) {   // d == DMAX and T % 4 == 0: float4 g of an env's run of T*d floats is nibble g % DMAX of step quad g / DMAX
       // lane = (env of a group of 4, 8 consecutive float4): every store covers whole 128 B lines of 4 envs
       const int nbn = (T >> 2) * DMAX;                 // float4 per env in this tile
@@ -456,19 +413,15 @@ struct WsKernel {
     const int env0 = env - lane, nl = min(32, N - env0);
     const bool bits_ok = p.vec && d == DMAX && (H % 4 == 0);
     const bool vec_r = (H % 4 == 0) && (reinterpret_cast<uintptr_t>(p.ctx_r) & 15) == 0;
-    if (stage && !DPT_WS_FILL_TILE && !(DPT_WS_SKIP & 2)) {   // constant states (bandit dx = 1): this warp's envs are one contiguous run
+    if (stage) {   // constant states (bandit dx = 1): this warp's envs are one contiguous run
       fill_range(p.ctx_s, (size_t)env0 * H, (size_t)(env0 + nl) * H, 1.0f, lane, 32);
       fill_range(p.ctx_ns, (size_t)env0 * H, (size_t)(env0 + nl) * H, 1.0f, lane, 32);
     }
     Tile& tl = cs.tile;
     SplitLane sl{};   // (the fused kernel uses the regret carries only)
     if (p.creg_carry) sl.creg_out = p.creg_carry + env, sl.mmax = (double)mmax;
-    // Warps start with first tiles of different lengths (WT/4 .. WT steps by warp index), so that the warps of an SM
-    // are in different phases: while some drain a tile (store bursts) the others run their controllers
-    int T = WT;
-    if (DPT_WS_STAGGER) T = (((env0 >> 5) & 3) + 1) * (WT / 4);
-    for (int h0 = 0; h0 < H; h0 += T, T = WT) {
-      T = min(T, H - h0);
+    for (int h0 = 0, T; h0 < H; h0 += T) {
+      T = min(WT, H - h0);
       const int nq = T >> 2;
 #pragma unroll 1
       for (int q = 0; q < nq; ++q)
@@ -477,13 +430,6 @@ struct WsKernel {
       if (stage) {
         __syncwarp();
         flush(p, tl, s_nib, env0, nl, h0, T, bits_ok, vec_r, lane);
-        if (DPT_WS_FILL_TILE) {   // the constant state columns of this tile: T * 4 B per env and array
-          for (int i = lane; i < nl * T; i += 32) {
-            const int e = i / T, t = i - e * T;
-            st_stream(p.ctx_s + (size_t)(env0 + e) * H + h0 + t, 1.0f);
-            st_stream(p.ctx_ns + (size_t)(env0 + e) * H + h0 + t, 1.0f);
-          }
-        }
         __syncwarp();
       }
     }
@@ -576,18 +522,11 @@ __global__ void __launch_bounds__(WS_NCONS * 32, ws_min_blocks<DMAX, KIND>()) on
 // wave), Thompson at d = 10 (40 float64 statistics in registers) 4
 template <int DMAX, int KIND>
 constexpr int ctrl_min_blocks() { return (DMAX > 5 && KIND == K_THOMPSON) ? 4 : 6; }
-#ifndef DPT_CTRL_MINB
-#define DPT_CTRL_MINB (ctrl_min_blocks<DMAX, KIND>())
-#endif
-#ifndef DPT_EX_MINB
-#define DPT_EX_MINB (REG ? (D > 5 ? 5 : 6) : 8)   // the 12 float64 accumulators of REG need 80 registers (96 at d = 10)
-#endif
 template <int DMAX, int KIND, bool IO>
-__global__ void __launch_bounds__(WS_NCONS * 32, DPT_CTRL_MINB) online_ctrl_kernel(const OnlineParams p, const double* __restrict__ tab,
+__global__ void __launch_bounds__(WS_NCONS * 32, ctrl_min_blocks<DMAX, KIND>()) online_ctrl_kernel(const OnlineParams p, const double* __restrict__ tab,
                                                                                                    const SplitArgs sa) {
   using K = WsKernel<DMAX, KIND, IO, true>;
   using Cons = typename K::Cons;
-  DPT_TL(1);
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Cons* cons = reinterpret_cast<Cons*>(smem_raw);
   double* s_arms = reinterpret_cast<double*>(smem_raw + sizeof(Cons) * WS_NCONS);   // [d][LIN_AW] (LinUCB)
@@ -604,6 +543,9 @@ __global__ void __launch_bounds__(WS_NCONS * 32, DPT_CTRL_MINB) online_ctrl_kern
 constexpr int EX_WARPS = 4;
 constexpr int EX_Q = 32;      // step quads per warp task (lane = quad): 128 steps
 constexpr int EX_TASKS = 32;  // envs per warp: the 32 arms words a lane gathers are one 128 B line
+// resident CTAs per SM the fast expander is compiled for: the 12 float64 accumulators of REG need 80 registers (96 at d = 10)
+template <int D, bool REG>
+constexpr int ex_min_blocks() { return REG ? (D > 5 ? 5 : 6) : 8; }
 
 // Fast expander: compile-time d, H % 4 == 0, 16 B-aligned context rows.  A warp task is one env x 32 step quads (lane = quad); a
 // warp walks up to 32 consecutive envs at a fixed 128-step range.  Its arms words arrive as coalesced [quad][env] rows (one line
@@ -619,9 +561,8 @@ constexpr int EX_TASKS = 32;  // envs per warp: the 32 arms words a lane gathers
 // warp's envs, so the sums over envs are thread-local float64 accumulators; the cumulative regret of a step is the carry the
 // controller left for this 128-step range + a warp scan over the quads + the prefix inside the quad.
 template <int D, bool INJ, bool REG>
-__global__ void __launch_bounds__(EX_WARPS * 32, DPT_EX_MINB) online_expand_kernel(const OnlineParams p, const uint32_t* __restrict__ arms4,
-                                                                                   const double* __restrict__ creg_in, int nqt, int ngy) {
-  DPT_TL(10);
+__global__ void __launch_bounds__(EX_WARPS * 32, ex_min_blocks<D, REG>()) online_expand_kernel(const OnlineParams p, const uint32_t* __restrict__ arms4,
+                                                                                               const double* __restrict__ creg_in, int nqt, int ngy) {
   __shared__ float4 s_nib[16];   // 4-bit pattern -> four 0/1 floats
   __shared__ uint32_t s_arm[EX_WARPS][EX_Q][33];   // per warp: arms words [quad][env], read back by lane = quad (conflict-free)
   onehot_nib_init(s_nib, threadIdx.x);
@@ -712,7 +653,6 @@ __global__ void __launch_bounds__(EX_WARPS * 32, DPT_EX_MINB) online_expand_kern
 // Generic expander: any d <= 10, any H, any alignment; lane = step quad, scalar stores (odd shapes only)
 __global__ void __launch_bounds__(EX_WARPS * 32) online_expand_generic_kernel(const OnlineParams p, const uint32_t* __restrict__ arms4, int q_lo,
                                                                               int q_hi) {
-  DPT_TL(10);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int N = p.N, H = p.H, d = p.d;
   const int env = blockIdx.x * EX_WARPS + warp;
@@ -741,7 +681,6 @@ __global__ void __launch_bounds__(EX_WARPS * 32) online_expand_generic_kernel(co
 
 // constant states (bandit dx = 1, envs/bandit_env.py:38): context_states = context_next_states = 1
 __global__ void __launch_bounds__(256) ones_fill_kernel(float* __restrict__ a, float* __restrict__ b, size_t n) {
-  DPT_TL(0);
   const size_t per = ((n + gridDim.x - 1) / gridDim.x + 3) & ~size_t(3);
   const size_t lo = min(n, per * blockIdx.x), hi = min(n, lo + per);
   fill_range(a, lo, hi, 1.0f, threadIdx.x, 256);
@@ -759,7 +698,6 @@ constexpr int RP_T = 16;      // steps per tile: 32 envs x 16 steps (6.5 KB of s
 __global__ void __launch_bounds__(RP_WARPS * 32, 6) regret_pass_kernel(const float* __restrict__ cum_means, const float* __restrict__ means, int N,
                                                                        int H, int d, double* __restrict__ reps, int n_reps,
                                                                        const double* __restrict__ creg_in) {
-  DPT_TL(20);
   // blockIdx.y = a 128-step range; its starting cumulative regret per env is what the loop kernel left in creg_in [range][N].
   // (Measured, 100k x 500: one warp per 32 envs over all H 0.09 ms; ranges -- 4x the warps -- the same; 4 env blocks per warp
   // with the sums meeting in shared memory -- 4x fewer atomics -- 0.11 ms: neither parallelism nor the atomics bound it.)
@@ -816,7 +754,6 @@ __global__ void __launch_bounds__(RP_WARPS * 32, 6) regret_pass_kernel(const flo
 // regret[h] += (S1, S2, C1, C2)[h]: S1, S2, C2 folded over the replicas in a fixed order; the sum over envs of the cumulative
 // regret is linear in the per-step sums, C1[h] = sum_{h' <= h} S1[h'], so it is a prefix over steps (one block, carry per chunk)
 __global__ void __launch_bounds__(1024) regret_finish_kernel(const double* __restrict__ reps, int n_reps, int H, double* __restrict__ regret) {
-  DPT_TL(30);
   __shared__ double s_warp[32];
   __shared__ double s_carry;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1017,7 +954,8 @@ static cudaError_t launch_split_kind(int kind, const OnlineParams& p, double* ta
   }
 }
 
-// the split pipeline (default); fused = true: the single fused kernel of this file's first half (DPT_OL_IMPL=2, A/B measurements)
+// the split pipeline; fused = true: the single fused kernel of this file's first half (dpt_online_loop picks one by controller
+// kind and batch size)
 cudaError_t launch_online_ws(int kind, const OnlineParams& p, double* tab, double* regret_out, cudaStream_t st, bool fused) {
   if (!online_ws_supported(kind, p)) return cudaErrorNotSupported;
   if (!fused) return p.d <= 5 ? launch_split_kind<5>(kind, p, tab, regret_out, st) : launch_split_kind<10>(kind, p, tab, regret_out, st);
@@ -1041,18 +979,6 @@ cudaError_t launch_online_ws(int kind, const OnlineParams& p, double* tab, doubl
 }  // namespace dpt
 
 using namespace dpt;
-
-#ifdef DPT_TIMELINE
-// copies the [64][2] stamps to the host (after a device synchronise) and re-arms them
-extern "C" int dpt_debug_timeline(unsigned long long* out) {
-  DPT_CUDA(cudaDeviceSynchronize());
-  DPT_CUDA(cudaMemcpyFromSymbol(out, g_tl, sizeof(unsigned long long) * 128));
-  unsigned long long init[64][2];
-  for (auto& r : init) r[0] = ~0ull, r[1] = 0ull;
-  DPT_CUDA(cudaMemcpyToSymbol(g_tl, init, sizeof(init)));
-  return DPT_OK;
-}
-#endif
 
 extern "C" int dpt_selftest_div(const double* a, const int* n, int count, int* mismatches, void* stream) {
   DPT_CHECK_ARG(a && n && mismatches && count >= 0, "dpt_selftest_div: bad arguments");

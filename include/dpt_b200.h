@@ -115,7 +115,7 @@ int dpt_peer_buffer_zero(void* dev_ptr, uint64_t bytes, void* stream);  /* cudaM
  * dpt_bandit_rollin_host_scratch_bytes(...) bytes) for double-buffered chunks so the D2H copies
  * overlap the kernel; the constant state columns (bandit state == [1]) are written by host threads
  * instead of crossing PCIe, and a self-balancing share of the chunks comes back as arm index + reward (5 B per step)
- * and is expanded to the one-hot fp32 layout by the same host threads (DPT_HOST_COMPACT=auto|0|1).  Results are
+ * and is expanded to the one-hot fp32 layout by the same host threads.  Results are
  * identical whichever way a chunk travels.  Synchronises `stream` before returning. */
 uint64_t dpt_bandit_rollin_host_scratch_bytes(int N, int H, int d);
 int dpt_bandit_rollin_host(const float* means_host, float var, uint64_t seed, uint64_t env_id0, int N, int H, int d,
@@ -199,9 +199,9 @@ int dpt_arm_stats(const float* ctx_actions, const float* ctx_rewards, int N, int
 int dpt_selftest_div(const double* a, const int32_t* n, int count, int32_t* mismatches, void* stream);
 /* Which implementation dpt_online_loop uses for shapes the fast kernels cover (d <= 10; LinUCB: lin_d == 2), for A/B
  * measurements and for the parity test that runs every implementation on the same inputs (no reference counterpart):
- * 0 = automatic (the default: split pipeline -- controller kernel, then context expansion -- or the single fused kernel,
- * by controller kind and batch size), 1 = general kernel, 2 = fused kernel, 3 = split pipeline; -1 = back to the
- * DPT_OL_IMPL environment variable (what a fresh process uses).  Returns the previous setting. */
+ * 0 = automatic (split pipeline -- controller kernel, then context expansion -- or the single fused kernel, by
+ * controller kind and batch size), 1 = general kernel, 2 = fused kernel, 3 = split pipeline; -1 = automatic as well
+ * (the setting a fresh process starts with).  Returns the previous setting. */
 int dpt_debug_online_impl(int impl);
 
 /* ---------------------------------------------------------------- L1: deploy_online_vec ----
