@@ -26,6 +26,16 @@ def shard_range(n_total, rank, world_size):
     return lo, lo + base + (1 if rank < rem else 0)
 
 
+def microbatch_shard(n_total, mb, rank, world_size):
+    """Micro-batch m covers the global items ``[m*mb, min(n_total, (m+1)*mb))``; rank r owns the contiguous micro-batch
+    range ``shard_range(M, r, world_size)`` of the M = ceil(n_total / mb).  Returns (m_lo, m_hi, lo, hi): its micro-batches
+    and the global item range they cover (empty, lo == hi, when the rank owns none)."""
+    if mb < 1:
+        raise ValueError("micro-batch size must be >= 1 (got %d)" % mb)
+    m_lo, m_hi = shard_range(-(-n_total // mb), rank, world_size)
+    return m_lo, m_hi, min(n_total, m_lo * mb), min(n_total, m_hi * mb)
+
+
 def all_gather_stats(local, group=None):
     """All-gather a small per-rank statistics tensor -> [world, ...] (same on every rank)."""
     rank, ws = world()
@@ -69,19 +79,17 @@ def regret_stats_from_sums(sums, n_envs):
     return {"mean": m, "sem": se, "regret_mean": cm, "regret_sem": cse}
 
 
-class PeerGather:
-    """Per-rank gather buffers [slots, world, width] float64, mutually mapped over CUDA IPC.
+class PeerBuffer:
+    """One device buffer per rank (``nbytes`` of it on this rank, zero-filled; the size may differ between ranks), mapped
+    into every rank's address space over CUDA IPC: ``peer_ptrs[r]`` is rank r's buffer as seen from this rank (its own
+    buffer at r == rank).  Kernels read or store through these pointers over NVLink; ordering against the other ranks is
+    the caller's job (stream synchronise + barrier).  ``rank_world``: (rank, world size) to use instead of ``world()``;
+    (0, 1) is a buffer of this process alone, with no exchange, even inside a process group."""
 
-    Rank r's kernels store their statistics for slot s straight into element [s, r, :] of EVERY rank's
-    buffer over NVLink (dpt_bandit_rollin_p2p): an all-gather with no collective launch.  Readers must
-    order themselves after all ranks' launches (stream synchronise + barrier), then ``read()``."""
-
-    def __init__(self, slots, width=3):
+    def __init__(self, nbytes, rank_world=None):
         import ctypes
         from ._lib import check, lib
-        self.rank, self.world = world()
-        self.slots, self.width = slots, width
-        self.data_bytes = slots * self.world * width * 8
+        self.rank, self.world = world() if rank_world is None else rank_world
         self.ptr = ctypes.c_void_p()
         self.peer_ptrs, self._opened = [], []
         self._ctypes = ctypes
@@ -90,7 +98,7 @@ class PeerGather:
         # (a rank that raised on its own would leave the others blocked in the next collective)
         err = None
         try:
-            check(lib().dpt_peer_buffer_create(self.data_bytes + 256, ctypes.byref(self.ptr), handle), "dpt_peer_buffer_create")
+            check(lib().dpt_peer_buffer_create(nbytes, ctypes.byref(self.ptr), handle), "dpt_peer_buffer_create")
         except Exception as e:   # noqa: BLE001
             err = str(e)
         handles = [bytes(handle) if err is None else None]
@@ -119,6 +127,36 @@ class PeerGather:
             if not all(oks):
                 self.close()
                 raise RuntimeError("CUDA IPC peer mapping failed on some rank: %s" % err)
+
+    def local_f32(self, n):
+        """The first ``n`` floats of this rank's own buffer as a float32 torch tensor (a view: no copy, no ownership; valid
+        until ``close``)."""
+        class _View:
+            __cuda_array_interface__ = {"shape": (n,), "typestr": "<f4", "data": (self.ptr.value, False), "version": 3,
+                                        "strides": None}
+        return torch.as_tensor(_View(), device=torch.device("cuda", torch.cuda.current_device()))
+
+    def close(self):
+        from ._lib import lib
+        for pp in self._opened:
+            lib().dpt_peer_buffer_close(pp)
+        self._opened = []
+        if self.ptr is not None and self.ptr.value:
+            lib().dpt_peer_buffer_destroy(self.ptr)
+        self.ptr = None
+
+
+class PeerGather(PeerBuffer):
+    """Per-rank gather buffers [slots, world, width] float64, mutually mapped over CUDA IPC.
+
+    Rank r's kernels store their statistics for slot s straight into element [s, r, :] of EVERY rank's
+    buffer over NVLink (dpt_bandit_rollin_p2p): an all-gather with no collective launch.  Readers must
+    order themselves after all ranks' launches (stream synchronise + barrier), then ``read()``."""
+
+    def __init__(self, slots, width=3):
+        self.slots, self.width = slots, width
+        self.data_bytes = slots * world()[1] * width * 8
+        super().__init__(self.data_bytes + 256)
         self.counter_ptr = self.ptr.value + self.data_bytes          # uint32 done-counter of this rank's launches
 
     def dst_array(self, slot):
@@ -141,15 +179,6 @@ class PeerGather:
         out = np.empty((self.slots, self.world, self.width), dtype=np.float64)
         check(lib().dpt_peer_buffer_read(self.ptr, out.ctypes.data, self.data_bytes, stream_ptr()), "dpt_peer_buffer_read")
         return out
-
-    def close(self):
-        from ._lib import lib
-        for pp in self._opened:
-            lib().dpt_peer_buffer_close(pp)
-        self._opened = []
-        if self.ptr is not None and self.ptr.value:
-            lib().dpt_peer_buffer_destroy(self.ptr)
-        self.ptr = None
 
 
 # ------------------------------------------------------------------ sharded entry points -------
@@ -221,3 +250,14 @@ def collect_darkroom_sharded(goals_total, dim, horizon, seed, rollin_type="unifo
     tot = all_reduce_sums(local).cpu().numpy()
     batch["env_range"] = (lo, hi)
     return batch, {"mean_reward": float(tot[0] / max(tot[1], 1.0)), "env_steps": int(tot[1])}
+
+
+def train_interactive_sharded(model, dim, n_envs_total, K, n_iters, mb=1024, **kw):
+    """``train.train_interactive`` over all ranks (one process per GPU): rank r rolls out and differentiates its contiguous
+    range of micro-batches (``microbatch_shard``; Philox counters use global env ids, so its contexts are slices of the
+    one-GPU rollout), keeps their gradient slots in a ``PeerBuffer``, and every rank sums all slots in micro-batch order
+    (``dpt_ordered_sum_f32`` over the peer mappings) before its AdamW step.  The weights after every iteration are
+    bit-identical on every rank and to the one-GPU run, for any world size.  Same arguments and return value."""
+    from . import train
+    rank, ws = world()
+    return train._interactive(model, dim, n_envs_total, K, n_iters, mb, rank, ws, **kw)

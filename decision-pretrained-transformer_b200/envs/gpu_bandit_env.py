@@ -84,23 +84,26 @@ class GPUBanditEnv(BaseEnv):
         return res
 
     # ---- interactive rollouts (train_interactive.py:97-134, rollout half) ----------------------------
-    def rollout(self, model, K=None, sample=True):
+    def rollout(self, model, K=None, sample=True, logits=True):
         """The K-step interactive rollout of the reference's on-policy trainers in ONE fused launch: at each
         step the transformer sees the context so far (K/V-cached), an action is drawn from its logits, the env
         steps, the row is appended.  Returns the four context tensors [n_envs,K,.] (device, fp32), the logits
-        the model produced at every step [K,n_envs,du] and ``target = opt_a_index`` (:134).  Training itself
-        (backward through the last forward) is out of scope: a trainer re-runs ``model(batch)`` on
-        ``context[:, :K-1]`` with its own autograd-enabled model to get ``last_logits`` with gradients."""
+        the model produced at every step [K,n_envs,du] (not written with ``logits=False``; the rollout is the same)
+        and ``target = opt_a_index`` (:134).  The gradient half (train_interactive.py:134-139) re-runs the model on
+        ``context[:, :K-1]`` with a gradient: ``train.train_interactive`` does both halves."""
         K = self.H if K is None else K
         with torch.cuda.device(self._device):
             key = (self._key ^ 0x2545F4914F6CDD1D) + 0x9E3779B97F4A7C15 * self._rollouts & 0xFFFFFFFFFFFFFFFF
             out = model.online_loop(self.means, K, float(self.var), sample, key, self._env_id0,
-                                    materialise=True, regret=False, dump=True, reward_type=self.type)
+                                    materialise=True, regret=False, dump=logits, reward_type=self.type)
         self._draws += K
         self._rollouts += 1
-        return {"context_states": out["context_states"], "context_actions": out["context_actions"],
-                "context_next_states": out["context_next_states"], "context_rewards": out["context_rewards"],
-                "logits": out["noise"]["logits"], "target": self.opt_a_index}
+        res = {"context_states": out["context_states"], "context_actions": out["context_actions"],
+               "context_next_states": out["context_next_states"], "context_rewards": out["context_rewards"]}
+        if logits:
+            res["logits"] = out["noise"]["logits"]
+        res["target"] = self.opt_a_index
+        return res
 
     @torch.no_grad()
     def rollout_explorer_exploiter(self, explorer, exploiter, K=None, fused=True, inject=None, dump=False):

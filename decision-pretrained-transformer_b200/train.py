@@ -9,6 +9,10 @@ len(dataset).  The forward of training is ``model.forward_train`` (hand-written 
 Unlike the reference's DataLoader, batches are gathered on the device from ``Dataset.dataset`` with a seeded
 permutation (and, with ``Dataset.shuffle``, a seeded per-item context permutation), and the losses stay on the
 device until one host read per epoch.  There is no argparse, plotting or checkpoint naming.
+
+``train_interactive`` is the on-policy trainer of the reference's train_interactive.py (:97-139): every iteration rolls
+out a fresh ``GPUBanditEnv`` with the current model and takes one AdamW step on the cross-entropy of the last logits
+against the optimal arm.  ``dist.train_interactive_sharded`` runs the same code over a box's GPUs.
 """
 import torch
 import torch.nn.functional as F
@@ -85,3 +89,149 @@ def train(model, train_dataset, test_dataset, num_epochs, batch_size=64, lr=1e-3
         test_loss.append(losses[0])
         train_loss.append(losses[1])
     return train_loss, test_loss, optimizer
+
+
+def interactive_loss(last_logits, target, n_envs):
+    """train_interactive.py's loss: the mean over the iteration's ``n_envs`` envs of the cross-entropy of the last logits
+    against the optimal arm index.  It is written as the sum over the rows given divided by ``n_envs``, so that the losses
+    (and gradients) of the micro-batches add up to those of the whole batch."""
+    return F.cross_entropy(last_logits, target, reduction="sum") / n_envs
+
+
+def train_interactive(model, dim, n_envs, K, n_iters, mb=1024, var=0.0, env_type="uniform", seed=0, lr=1e-3,
+                      weight_decay=1e-4, optimizer=None, timings=None):
+    """On-policy training (train_interactive.py:97-139) on one GPU.  Iteration ``it``:
+
+    1. ``env = GPUBanditEnv(dim, n_envs, K, var, env_type, seed=rng.key_for(seed, it))``;
+    2. ``env.rollout(model, K, sample=True)``: the fused K-step rollout with the current weights (``model.precision``);
+    3. the last logits on ``context[:, :K-1]`` with a gradient (``dpt_gpt2_train_forward``, last position, whatever
+       ``model.test`` says), ``interactive_loss`` against ``env.opt_a_index`` and ``dpt_gpt2_train_backward``, one
+       micro-batch of ``mb`` envs at a time (micro-batch m is envs ``[m*mb, min(n_envs, (m+1)*mb))``), each into its own
+       gradient slot;
+    4. the slots summed in micro-batch order into the parameters' ``.grad`` (one flat buffer; ``transformer.wte`` gets
+       none), then ``optimizer.step()`` (default ``torch.optim.AdamW(lr, weight_decay)``).
+
+    With ``mb >= n_envs`` an iteration is exactly ``env.rollout`` + ``forward_train`` + ``interactive_loss`` + ``backward``
+    + ``step``.  The result does not depend on how the micro-batches are spread over GPUs (``dist.train_interactive_sharded``),
+    only on ``mb``.  fp32 training, ``dropout == 0`` and K <= 512 (the limits of ``forward_train``).  ``n_envs == 0`` runs
+    nothing.  ``timings``: a list that receives, per iteration, the CUDA-event milliseconds of the rollout, the forward and
+    backward of all micro-batches, the exchange (host barrier to the end of the sum), the optimizer and the whole iteration.
+    Returns ``(losses, optimizer)``: the per-iteration losses (one host read at the end) and the optimizer."""
+    return _interactive(model, dim, n_envs, K, n_iters, mb, 0, 1, var=var, env_type=env_type, seed=seed, lr=lr,
+                        weight_decay=weight_decay, optimizer=optimizer, timings=timings)
+
+
+def _agree(err, ws):
+    """Every rank learns whether any rank failed (so that no rank is left blocked in a collective); raises if one did."""
+    bad = []
+    if ws > 1:
+        import torch.distributed as tdist
+        msgs = [None] * ws
+        tdist.all_gather_object(msgs, None if err is None else "%s: %s" % (type(err).__name__, err))
+        bad = [(r, m) for r, m in enumerate(msgs) if m is not None]
+    if err is not None:
+        raise err
+    if bad:
+        raise RuntimeError("train_interactive failed on rank %d: %s" % bad[0])
+
+
+def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type="uniform", seed=0, lr=1e-3,
+                 weight_decay=1e-4, optimizer=None, timings=None):
+    """train_interactive on rank ``rank`` of ``ws`` (ws == 1: the one-GPU trainer; see dist.train_interactive_sharded)."""
+    import ctypes
+    from . import _lib, dist as D, kernels, rng
+    from ._lib import check, lib, stream_ptr
+    from .envs.gpu_bandit_env import GPUBanditEnv
+    from .models import net
+    if model.dropout > 0:
+        raise NotImplementedError("train_interactive: dropout=%g, the fused training path has no dropout" % model.dropout)
+    if K < 1:
+        raise ValueError("train_interactive: K=%d, the rollout needs at least one step" % K)
+    dev = kernels._dev()
+    if next(model.parameters()).device != dev:
+        model.to(dev)
+    if optimizer is None:
+        optimizer = torch.optim.AdamW(model.parameters(), lr=lr, weight_decay=weight_decay)
+    m_lo, m_hi, lo, hi = D.microbatch_shard(n_envs, mb, rank, ws)
+    M = -(-n_envs // mb)
+    if M == 0:
+        return [], optimizer
+    params = model._train_params()
+    sizes = [p.numel() for p in params]
+    offs = [sum(sizes[:i]) for i in range(len(sizes))]
+    P = sum(sizes) + 1                 # a slot: every trained parameter (_train_params order), then the micro-batch's loss
+    Ps = (P + 3) & ~3                  # slot stride: 16 B aligned slots
+    T, du, st = K - 1, model.action_dim, stream_ptr()
+    # the train kernels' shape checks (n_embd, n_layer, sequence length) before any rollout: a B = 0 call only validates
+    check(lib().dpt_gpt2_train_forward(ctypes.byref(net._weights_struct(model, params, [])), None, None, None, None, None, 0,
+                                       T, K, 1, None, None, 0, st), "dpt_gpt2_train_forward")
+    n_local, n_mb = hi - lo, m_hi - m_lo
+    peer = D.PeerBuffer(max(n_mb, 1) * Ps * 4, (rank, ws))
+    try:
+        slots = peer.local_f32(max(n_mb, 1) * Ps).view(-1, Ps)
+        grad_slots = [[slots[j, o:o + n].view_as(p) for p, o, n in zip(params, offs, sizes)] for j in range(n_mb)]
+        owner_lo = [D.microbatch_shard(n_envs, mb, r, ws)[:2] for r in range(ws)]
+        src = (ctypes.c_void_p * M)(*[peer.peer_ptrs[r] + (m - a) * Ps * 4 for r, (a, b) in enumerate(owner_lo)
+                                      for m in range(a, b)])
+        flat = torch.zeros(Ps, dtype=torch.float32, device=dev)
+        for p, o, n in zip(params, offs, sizes):
+            p.grad = flat[o:o + n].view_as(p)
+        losses = torch.zeros(n_iters, dtype=torch.float32, device=dev)
+        if n_local:
+            q = torch.ones((min(mb, n_local), model.state_dim), dtype=torch.float32, device=dev)
+            wbytes = int(lib().dpt_gpt2_train_workspace_bytes(ctypes.byref(net._weights_struct(model, params, [])),
+                                                               min(mb, n_local), T))
+            work = torch.empty((max(wbytes, 16),), dtype=torch.uint8, device=dev)
+        for it in range(n_iters):
+            ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)] if timings is not None else []
+            mark = lambda i: ev and ev[i].record()   # noqa: E731
+            err = None
+            try:
+                mark(0)
+                if n_local:
+                    env = GPUBanditEnv(dim, n_local, K, var, env_type, device=dev, seed=rng.key_for(seed, it), env_id0=lo)
+                    ro = env.rollout(model, K, sample=True, logits=False)
+                    mark(1)
+                    keep = []
+                    w = net._weights_struct(model, params, keep)
+                    ctx = [ro[k] for k in _CTX]
+                    for j in range(n_mb):
+                        a, b = j * mb, min(n_local, (j + 1) * mb)
+                        out = torch.empty((b - a, du), dtype=torch.float32, device=dev)
+                        cp = [c[a:b].data_ptr() if T else None for c in ctx]
+                        check(lib().dpt_gpt2_train_forward(ctypes.byref(w), q.data_ptr(), *cp, b - a, T, K, 1, out.data_ptr(),
+                                                           work.data_ptr(), work.numel(), st), "dpt_gpt2_train_forward")
+                        lg = out.requires_grad_()
+                        with torch.enable_grad():
+                            loss = interactive_loss(lg, ro["target"][a:b], n_envs)
+                            dout, = torch.autograd.grad(loss, lg)
+                        g = net._pointer_struct(_lib.Gpt2Grads, model, grad_slots[j], keep)
+                        check(lib().dpt_gpt2_train_backward(ctypes.byref(w), dout.contiguous().data_ptr(), b - a, T, 1,
+                                                            ctypes.byref(g), work.data_ptr(), work.numel(), st),
+                              "dpt_gpt2_train_backward")
+                        slots[j, P - 1].copy_(loss.detach())
+                else:
+                    mark(1)
+                mark(2)
+                torch.cuda.current_stream().synchronize()   # this rank's slots are written ...
+            except Exception as e:   # noqa: BLE001
+                err = e
+            _agree(err, ws)                                 # ... and so are every rank's (the exchange is a barrier)
+            try:
+                check(lib().dpt_ordered_sum_f32(src, M, Ps, flat.data_ptr(), st), "dpt_ordered_sum_f32")
+                mark(3)
+                losses[it].copy_(flat[P - 1])
+                optimizer.step()
+                mark(4)
+                torch.cuda.current_stream().synchronize()
+            except Exception as e:   # noqa: BLE001
+                err = e
+            _agree(err, ws)                                 # no rank rewrites its slots before every rank has summed them
+            if ev:
+                timings.append({"rollout": ev[0].elapsed_time(ev[1]), "fwd_bwd": ev[1].elapsed_time(ev[2]),
+                                "exchange": ev[2].elapsed_time(ev[3]), "optimizer": ev[3].elapsed_time(ev[4]),
+                                "total": ev[0].elapsed_time(ev[4])})
+        return losses.tolist(), optimizer
+    finally:
+        torch.cuda.current_stream().synchronize()           # nothing in flight uses the slots when they are freed
+        peer.close()

@@ -35,7 +35,7 @@ extern "C" {
 #define DPT_ERR_CUDA (-2)
 #define DPT_ERR_UNSUPPORTED (-3)
 
-#define DPT_ABI_VERSION 5
+#define DPT_ABI_VERSION 6
 
 /* reward_type of the bandit entry points (envs/bandit_env.py:56-63, envs/gpu_bandit_env.py:53-63):
  * 0 'uniform'  : r = means[a] + var * z, z ~ N(0,1);
@@ -379,6 +379,14 @@ int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, const float* query_state
                            int T_stride, int test, float* out, void* workspace, uint64_t workspace_bytes, void* stream);
 int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float* dout, int B, int T, int test,
                             const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream);
+
+/* Ordered multi-source sum (the gradient exchange of the data-parallel interactive trainer, train_interactive.py:97-139;
+ * the reference is single-GPU): dst[i] = (((src[0][i] + src[1][i]) + ...) + src[M-1][i]) for i < n, fp32, added in
+ * source order whatever the launch geometry, so every rank that sums the same M slots gets the same bits.  src is a HOST
+ * array of M device pointers; each may be local or a peer mapping opened with dpt_peer_buffer_open (read with ordinary
+ * loads).  No source may alias dst.  M = 0 or n = 0 is a no-op; negative M or n and null pointers return
+ * DPT_ERR_INVALID_ARG.  The caller orders the call after every writer of the sources (stream sync + barrier). */
+int dpt_ordered_sum_f32(const float* const* src, int M, int64_t n, float* dst, void* stream);
 
 /* Fused bandit online loop with the transformer controller: evals/eval_bandit.py:56-103 +
  * ctrls/ctrl_bandit.py:383-444 (BanditTransformerController, sample != 0 -> softmax + categorical

@@ -1,0 +1,42 @@
+"""Multi-GPU tier of the interactive trainer: spawns scripts/interactive_train_check.py under torch.distributed.run over
+EVERY visible GPU (skipped below 2 GPUs), and with two ranks sharing one GPU (the sharded code path, CUDA IPC slots and
+the ordered sum included, on any GPU box).  After 3 iterations of dist.train_interactive_sharded the weights of every rank
+must be bit-identical to each other and to a world-size-1 run of the same problem, for N divisible by mb * world, a ragged
+last micro-batch, ranks without a micro-batch, and shards whose rollout takes another decode kernel than the one-GPU run."""
+import os
+import socket
+import subprocess
+import sys
+
+import pytest
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+
+def _check(ranks, gpus):
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        port = s.getsockname()[1]
+    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(ranks), "--master-addr",
+           "127.0.0.1", "--master-port", str(port), os.path.join(ROOT, "scripts", "interactive_train_check.py")]
+    env = dict(os.environ)
+    if gpus == 1:        # the first visible GPU only: the ranks share it
+        env["CUDA_VISIBLE_DEVICES"] = os.environ.get("CUDA_VISIBLE_DEVICES", "0").split(",")[0]
+    r =subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True, timeout=900, env=env)
+    print(r.stdout[-3000:])
+    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
+    assert "interactive_train_check world=%d gpus=%d: OK" % (ranks, gpus) in r.stdout, r.stdout[-3000:]
+
+
+@pytest.mark.gpu
+def test_sharded_weights_equal_the_single_gpu_run():
+    import torch
+    n = torch.cuda.device_count()
+    if n < 2:
+        pytest.skip("needs >= 2 GPUs (found %d)" % n)
+    _check(n, n)
+
+
+@pytest.mark.gpu
+def test_two_ranks_on_one_gpu():
+    _check(2, 1)
