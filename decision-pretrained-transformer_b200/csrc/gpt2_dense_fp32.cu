@@ -8,10 +8,11 @@
 // per-row online softmax over the keys <= t (K/V rows broadcast from shared memory).  Compared with the
 // token-sequential kernel there is no K/V traffic to HBM and all tokens of a sequence advance in parallel.
 //
-// SAVE = true is the forward of training (gpt2_train.cu): the same arithmetic on the parameter tensors as they are
-// (embed_transition.weight [E, din], pred_actions.weight [du, E] instead of the handle's transposed copies), and
-// every row also stores what the backward needs (TrainSave, layout TA_* / TF_* in gpt2_model.cuh).  Its logits are
-// bit-identical to SAVE = false.
+// SAVE = true is the forward of training (gpt2_train_forward_kernel, called from gpt2_train.cu): the same rows
+// (dense_fp32_rows) on the parameter tensors as they are (embed_transition.weight [E, din], pred_actions.weight [du, E]
+// instead of the handle's transposed copies), and every row also stores what the backward needs (TrainSave, layout
+// TA_* / TF_* in gpt2_model.cuh).  Its logits are bit-identical to SAVE = false.  A training launch covers a population
+// of same-shape models: CTA (b, member = blockIdx.y), each member with its own parameters, inputs, logits and save area.
 #include "common.cuh"
 #include "gpt2_model.cuh"
 #include "gpt2_fp32.cuh"
@@ -26,16 +27,16 @@ constexpr int DF_WFC2 = DF_WFC + 32 * 128;     // [128][32]
 constexpr int DF_K = DF_WFC2 + 128 * 32;       // [THREADS][32], then V [THREADS][32]
 constexpr int df_floats(int threads) { return DF_K + 2 * threads * 32; }   // 80 KB / 112 KB / 176 KB
 
-template <int DF_THREADS, bool SAVE = false>
-__global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const DenseParams p, const TrainSave sv = TrainSave{}) {
+// The rows of sequence b.  W is Gpt2Dev (SAVE = false: the handle's transposed embed / pred copies) or TrainW
+// (SAVE = true: the parameter tensors); sh gives L, dx, du, din; p the inputs, the output and B, T, Ts, test, share.
+// tid = threadIdx.x and b are read by the kernel, which knows the range of threadIdx.x from its launch bounds.
+template <int DF_THREADS, bool SAVE, class W, class Sh, class P>
+__device__ __forceinline__ void dense_fp32_rows(const int tid, const int b, const W& m, const Sh& sh, const P& p, const TrainSave& sv) {
   constexpr int DF_V = DF_K + DF_THREADS * 32;
   extern __shared__ __align__(16) float sm[];
-  const int tid = threadIdx.x;
-  const int b = blockIdx.x;
-  const Gpt2Dev& m = p.m;
   const int S = p.T + 1;
   const bool valid = tid < S;
-  const int dx = m.dx, du = m.du, din = m.din;
+  const int dx = sh.dx, du = sh.du, din = sh.din;
 
   float x[G_E];
   {
@@ -59,12 +60,17 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
     for (int i = 0; i < din; ++i) {
       const float tv = tok[i];
 #pragma unroll
-      for (int c = 0; c < G_E; ++c) x[c] = fmaf(tv, __ldg(SAVE ? m.embed_wT + c * din + i : m.embed_wT + i * G_E + c), x[c]);
+      for (int c = 0; c < G_E; ++c) {
+        const float* e;
+        if constexpr (SAVE) e = m.embed_w + c * din + i;
+        else e = m.embed_wT + i * G_E + c;
+        x[c] = fmaf(tv, __ldg(e), x[c]);
+      }
     }
   }
 
-  for (int l = 0; l < m.L; ++l) {
-    const LayerW& w = m.layer[l];
+  for (int l = 0; l < sh.L; ++l) {
+    const auto& w = m.layer[l];
     float* const rec = SAVE && valid ? sv.act + (((size_t)l * p.B + b) * S + tid) * TA_STRIDE : nullptr;   // SAVE: this row's record
     __syncthreads();   // previous layer's readers of the weights / K / V are done
     {
@@ -204,18 +210,42 @@ __global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const Dense
     for (int j = 0; j < du; ++j) {
       float lg = __ldg(m.pred_b + j);
 #pragma unroll
-      for (int c = 0; c < G_E; ++c) lg = fmaf(y[c], __ldg(SAVE ? m.pred_wT + j * G_E + c : m.pred_wT + c * du + j), lg);
+      for (int c = 0; c < G_E; ++c) {
+        const float* e;
+        if constexpr (SAVE) e = m.pred_w + j * G_E + c;
+        else e = m.pred_wT + c * du + j;
+        lg = fmaf(y[c], __ldg(e), lg);
+      }
       o[j] = lg;
     }
   }
 }
 
-template <int THREADS, bool SAVE = false>
-static cudaError_t launch_df(const DenseParams& p, cudaStream_t st, const TrainSave& sv = TrainSave{}) {
+// inference (dpt_gpt2_forward, precision 0): one CTA per sequence
+template <int DF_THREADS, bool SAVE = false>
+__global__ void __launch_bounds__(DF_THREADS) gpt2_dense_fp32_kernel(const DenseParams p, const TrainSave sv = TrainSave{}) {
+  static_assert(!SAVE, "the forward of training is gpt2_train_forward_kernel");
+  dense_fp32_rows<DF_THREADS, false>(threadIdx.x, blockIdx.x, p.m, p.m, p, sv);
+}
+
+// the forward of training: CTA (b, member), member = blockIdx.y reads its own parameters, inputs, logits and save area
+template <int DF_THREADS, int NM>
+__global__ void __launch_bounds__(DF_THREADS) gpt2_train_forward_kernel(const __grid_constant__ TrainFwdParams<NM> p) {
+  const TrainFwdMember& mb = p.mem[NM == 1 ? 0 : blockIdx.y];
+  struct {
+    const float *query, *cs, *ca, *cns, *cr;
+    float* out;
+    int B, T, Ts, test, share;
+  } io{mb.query, mb.cs, mb.ca, mb.cns, mb.cr, mb.out, p.B, p.T, p.Ts, p.test, 1};
+  dense_fp32_rows<DF_THREADS, true>(threadIdx.x, blockIdx.x, mb.w, p, io, mb.sv);
+}
+
+template <int THREADS>
+static cudaError_t launch_df(const DenseParams& p, cudaStream_t st) {
   const int smem = df_floats(THREADS) * (int)sizeof(float);
-  cudaError_t e = cudaFuncSetAttribute(gpt2_dense_fp32_kernel<THREADS, SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  cudaError_t e = cudaFuncSetAttribute(gpt2_dense_fp32_kernel<THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;
-  gpt2_dense_fp32_kernel<THREADS, SAVE><<<p.B, THREADS, smem, st>>>(p, sv);
+  gpt2_dense_fp32_kernel<THREADS><<<p.B, THREADS, smem, st>>>(p);
   return cudaGetLastError();
 }
 
@@ -229,15 +259,27 @@ int gpt2_dense_fp32_launch(const DenseParams& p, cudaStream_t st) {
   return DPT_OK;
 }
 
-int gpt2_train_forward_launch(const DenseParams& p, const TrainSave& sv, cudaStream_t st) {
+template <int THREADS, int NM>
+static cudaError_t launch_train_fwd(const TrainFwdParams<NM>& p, int n, cudaStream_t st) {
+  const int smem = df_floats(THREADS) * (int)sizeof(float);
+  cudaError_t e = cudaFuncSetAttribute(gpt2_train_forward_kernel<THREADS, NM>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  if (e != cudaSuccess) return e;
+  gpt2_train_forward_kernel<THREADS, NM><<<dim3(p.B, n), THREADS, smem, st>>>(p);
+  return cudaGetLastError();
+}
+
+template <int NM>
+int gpt2_train_forward_launch(const TrainFwdParams<NM>& p, int n, cudaStream_t st) {
   const int S = p.T + 1;
-  cudaError_t e = S <= 128 ? launch_df<128, true>(p, st, sv) : S <= 256 ? launch_df<256, true>(p, st, sv)
-                                                                         : launch_df<512, true>(p, st, sv);
+  cudaError_t e = S <= 128 ? launch_train_fwd<128>(p, n, st) : S <= 256 ? launch_train_fwd<256>(p, n, st)
+                                                                         : launch_train_fwd<512>(p, n, st);
   if (e != cudaSuccess) {
     set_error("gpt2_train_forward launch failed: %s", cudaGetErrorString(e));
     return DPT_ERR_CUDA;
   }
   return DPT_OK;
 }
+template int gpt2_train_forward_launch<1>(const TrainFwdParams<1>&, int, cudaStream_t);
+template int gpt2_train_forward_launch<TRAIN_POP_MAX>(const TrainFwdParams<TRAIN_POP_MAX>&, int, cudaStream_t);
 
 }  // namespace dpt

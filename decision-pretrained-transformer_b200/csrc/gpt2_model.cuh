@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "../../include/dpt_b200.h"
+
 namespace dpt {
 
 constexpr int G_E = 32;
@@ -77,9 +79,33 @@ constexpr int TF_X = 0, TF_TOK = 32, TF_MU = 64, TF_RS = 65, TF_STRIDE = 68;   /
 struct TrainSave {
   float *act, *fin;
 };
-// the dense fp32 forward with SAVE = true: DenseParams::m holds the parameter tensors' own pointers (embed_wT =
-// embed_transition.weight [E, din], pred_wT = pred_actions.weight [du, E]); share must be 1
-int gpt2_train_forward_launch(const DenseParams& p, const TrainSave& sv, cudaStream_t st);
+
+// Training reads the parameter tensors in place (reference layouts: embed_w = embed_transition.weight [E, din], pred_w =
+// pred_actions.weight [du, E]).  A population of same-shape models runs in one launch: CTA (b, member = blockIdx.y).
+// The per-member tables travel in the kernel parameters, so a launch needs no upload and stays graph-capturable; at
+// ~0.9 KB per member, TRAIN_POP_MAX members fit the 32 764 B parameter limit.
+constexpr int TRAIN_POP_MAX = DPT_GPT2_POPULATION_MAX;
+struct TrainLayerW {
+  const float *ln1_w, *ln1_b, *attn_w, *attn_b, *proj_w, *proj_b, *ln2_w, *ln2_b, *fc_w, *fc_b, *fc2_w, *fc2_b;
+};
+struct TrainW {
+  const float *wpe, *embed_w, *embed_b, *pred_w, *pred_b, *lnf_w, *lnf_b;
+  TrainLayerW layer[G_MAX_L];
+};
+struct TrainFwdMember {
+  TrainW w;
+  const float *query, *cs, *ca, *cns, *cr;
+  float* out;
+  TrainSave sv;
+};
+template <int NM>   // NM: member capacity of the launch (1 for the one-model entry points, else TRAIN_POP_MAX)
+struct TrainFwdParams {
+  int L, dx, du, din, B, T, Ts, test;
+  TrainFwdMember mem[NM];
+};
+// the dense fp32 forward that also saves the activations (gpt2_dense_fp32.cu), members mem[0 .. n)
+template <int NM>
+int gpt2_train_forward_launch(const TrainFwdParams<NM>& p, int n, cudaStream_t st);
 void gpt2_pack_wimg(const float* attn_w, const float* proj_w, const float* fc_w, const float* fc2_w, unsigned char* img,
                     cudaStream_t st);
 }  // namespace dpt

@@ -14,6 +14,12 @@
 //     3. weight_grad_reduce_kernel sums the NC slots in chunk order into the gradient tensors; wpe_grad_kernel sums
 //        the position gradients over the batch in sequence order (rows past T are zero).
 //   Every sum has a fixed order, so two identical calls give bit-identical gradients.
+//
+// Population training (dpt_gpt2_train_population_*): n same-shape models in the same launches.  Every kernel takes its
+// member from the grid (forward / backward: blockIdx.y, partial sums and reduction: blockIdx.z, wpe: blockIdx.y); member i
+// uses workspace region i (train_layout(...).total floats each) and its own pointer table in the kernel parameters.  The
+// chunking depends on B and T only, so each member runs exactly the arithmetic of the one-model call; the one-model entry
+// points are the n = 1 case (kernels instantiated with a member capacity NM of 1, so their parameter blocks stay small).
 #include <algorithm>
 
 #include "common.cuh"
@@ -53,19 +59,16 @@ constexpr int db_floats(int threads) { return DB_X1 + 2 * threads * 32 + 2 * thr
 
 constexpr float ATT_SCALE = 0.17677669529663687f;   // 1 / sqrt(32)
 
-struct TrainModel {   // the parameter tensors (reference layouts)
-  int L, dx, du, din, n_pos;
-  const float *wpe, *embed_w, *embed_b, *pred_w, *pred_b, *lnf_w, *lnf_b;
-  const float *ln1_w[G_MAX_L], *ln1_b[G_MAX_L], *attn_w[G_MAX_L], *attn_b[G_MAX_L], *proj_w[G_MAX_L], *proj_b[G_MAX_L];
-  const float *ln2_w[G_MAX_L], *ln2_b[G_MAX_L], *fc_w[G_MAX_L], *fc_b[G_MAX_L], *fc2_w[G_MAX_L], *fc2_b[G_MAX_L];
-};
-
-struct BackParams {
-  TrainModel m;
+struct BackMember {   // one member of the population: its parameter tensors, dout and workspace region
+  TrainW w;
   const float* dout;
-  int B, T, test;
   const float *act, *fin;
   float *grec, *gfin;
+};
+template <int NM>
+struct BackParams {
+  int L, du, B, T, test;
+  BackMember mem[NM];
 };
 
 // dx += d LayerNorm(x)/dx applied to dy, from the normalised input xh, rstd rs and the LN weight w
@@ -111,15 +114,17 @@ __device__ __forceinline__ void axpy32_(float s, const float* v_sm, float2* acc)
   }
 }
 
-template <int THREADS>
-__global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const BackParams p) {
+// CTA (b, member = blockIdx.y)
+template <int THREADS, int NM>
+__global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const __grid_constant__ BackParams<NM> p) {
   extern __shared__ __align__(16) float sm[];
   float* const X1 = sm + DB_X1;
   float* const X2 = sm + DB_X1 + THREADS * 32;
   float* const SV = sm + DB_X1 + 2 * THREADS * 32;
-  const TrainModel& m = p.m;
+  const BackMember& mb = p.mem[NM == 1 ? 0 : blockIdx.y];
+  const TrainW& m = mb.w;
   const int tid = threadIdx.x, b = blockIdx.x;
-  const int S = p.T + 1, du = m.du;
+  const int S = p.T + 1, du = p.du;
   const bool valid = tid < S;
   const int row = valid ? tid : S - 1;   // rows past the sequence load a valid row and store nothing
   const size_t r = (size_t)b * S + row;
@@ -128,7 +133,7 @@ __global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const Back
   float dx[G_E];
   // ---- pred_actions and ln_f ----
   {
-    const float* f = p.fin + r * TF_STRIDE;
+    const float* f = mb.fin + r * TF_STRIDE;
     float xh[G_E], dl[G_E], dy[G_E];
     load32_(xh, f + TF_X);
     const float mu = f[TF_MU], rs = f[TF_RS];
@@ -136,7 +141,7 @@ __global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const Back
     for (int c = 0; c < G_E; ++c) xh[c] = (xh[c] - mu) * rs, dl[c] = 0.f, dy[c] = 0.f;
     const bool has_out = p.test ? row == p.T : row >= 1;
     if (has_out) {
-      const float* d = p.test ? p.dout + (size_t)b * du : p.dout + ((size_t)b * p.T + (row - 1)) * du;
+      const float* d = p.test ? mb.dout + (size_t)b * du : mb.dout + ((size_t)b * p.T + (row - 1)) * du;
       for (int j = 0; j < du; ++j) {
         const float g = d[j];
         dl[j] = g;
@@ -148,7 +153,7 @@ __global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const Back
     for (int c = 0; c < G_E; ++c) dx[c] = 0.f;
     ln_back_(xh, rs, dy, m.lnf_w, dx);
     if (valid) {
-      float* g = p.gfin + r * GF_STRIDE;
+      float* g = mb.gfin + r * GF_STRIDE;
       store32_(g + GF_DLOG, dl), store32_(g + GF_XHF, xh), store32_(g + GF_DYF, dy);
 #pragma unroll
       for (int c = 0; c < G_E; ++c) dl[c] = fmaf(xh[c], __ldg(m.lnf_w + c), __ldg(m.lnf_b + c));
@@ -156,14 +161,15 @@ __global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const Back
     }
   }
 
-  for (int l = m.L - 1; l >= 0; --l) {
+  for (int l = p.L - 1; l >= 0; --l) {
+    const TrainLayerW& lw = m.layer[l];
     __syncthreads();   // the previous layer's readers of the weights and row arrays are done
-    for (int i = tid; i < 32 * 96; i += THREADS) sm[DB_WQKVT + (i % 96) * 32 + i / 96] = __ldg(m.attn_w[l] + i);
-    for (int i = tid; i < 32 * 32; i += THREADS) sm[DB_WPROJT + (i % 32) * 32 + i / 32] = __ldg(m.proj_w[l] + i);
-    for (int i = tid; i < 32 * 128; i += THREADS) sm[DB_WFCT + (i % 128) * 32 + i / 128] = __ldg(m.fc_w[l] + i);
-    for (int i = tid; i < 128 * 32; i += THREADS) sm[DB_WFC2T + (i % 32) * 128 + i / 32] = __ldg(m.fc2_w[l] + i);
-    const float* a = p.act + ((size_t)l * NR + r) * TA_STRIDE;
-    float* g = p.grec + ((size_t)l * NR + r) * GR_STRIDE;
+    for (int i = tid; i < 32 * 96; i += THREADS) sm[DB_WQKVT + (i % 96) * 32 + i / 96] = __ldg(lw.attn_w + i);
+    for (int i = tid; i < 32 * 32; i += THREADS) sm[DB_WPROJT + (i % 32) * 32 + i / 32] = __ldg(lw.proj_w + i);
+    for (int i = tid; i < 32 * 128; i += THREADS) sm[DB_WFCT + (i % 128) * 32 + i / 128] = __ldg(lw.fc_w + i);
+    for (int i = tid; i < 128 * 32; i += THREADS) sm[DB_WFC2T + (i % 32) * 128 + i / 32] = __ldg(lw.fc2_w + i);
+    const float* a = mb.act + ((size_t)l * NR + r) * TA_STRIDE;
+    float* g = mb.grec + ((size_t)l * NR + r) * GR_STRIDE;
     if (valid) store32_(g + GR_DX, dx);
     __syncthreads();
     float2 acc[16];
@@ -178,7 +184,7 @@ __global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const Back
       if (valid) {
         float y[G_E];
 #pragma unroll
-        for (int c = 0; c < G_E; ++c) y[c] = fmaf(xh[c], __ldg(m.ln2_w[l] + c), __ldg(m.ln2_b[l] + c));
+        for (int c = 0; c < G_E; ++c) y[c] = fmaf(xh[c], __ldg(lw.ln2_w + c), __ldg(lw.ln2_b + c));
         store32_(g + GR_Y2, y), store32_(g + GR_XH2, xh);
       }
       float2 dy2[16];
@@ -207,7 +213,7 @@ __global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const Back
       if (valid) store32_(g + GR_DY2, dy);
 #pragma unroll
       for (int c = 0; c < G_E; ++c) dxm[c] = dx[c];
-      ln_back_(xh, rs, dy, m.ln2_w[l], dxm);
+      ln_back_(xh, rs, dy, lw.ln2_w, dxm);
     }
     if (valid) store32_(g + GR_DXM, dxm);
     // ---- attention: x_mid = x_in + proj(softmax(q k^T) v) ----
@@ -308,15 +314,15 @@ __global__ void __launch_bounds__(THREADS) gpt2_train_backward_kernel(const Back
       if (valid) {
         float y[G_E];
 #pragma unroll
-        for (int c = 0; c < G_E; ++c) y[c] = fmaf(xh[c], __ldg(m.ln1_w[l] + c), __ldg(m.ln1_b[l] + c));
+        for (int c = 0; c < G_E; ++c) y[c] = fmaf(xh[c], __ldg(lw.ln1_w + c), __ldg(lw.ln1_b + c));
         store32_(g + GR_Y1, y), store32_(g + GR_XH1, xh), store32_(g + GR_DY1, dy1);
       }
 #pragma unroll
       for (int c = 0; c < G_E; ++c) dx[c] = dxm[c];
-      ln_back_(xh, rs, dy1, m.ln1_w[l], dx);
+      ln_back_(xh, rs, dy1, lw.ln1_w, dx);
     }
   }
-  if (valid) store32_(p.gfin + r * GF_STRIDE + GF_DX0, dx);
+  if (valid) store32_(mb.gfin + r * GF_STRIDE + GF_DX0, dx);
 }
 
 // ---- weight gradients: fixed-chunk partial sums, then a fixed-order reduction ----
@@ -332,23 +338,37 @@ struct RTile {
 };
 constexpr int R_MAX_JOBS = 6 * G_MAX_L + 3;
 constexpr int R_MAX_TILES = 14 * G_MAX_L + 3;
-struct RParams {
+struct RParams {   // the operands of member 0; member z's are at the same offsets in its workspace region (+ z * mstride)
   RJob job[R_MAX_JOBS];
   RTile tile[R_MAX_TILES];
   int NR, CH, P;
+  size_t mstride;
   float* part;   // [NC][P]
 };
 struct RSeg {
-  float* dst;
   int off, n;
 };
 constexpr int R_MAX_SEGS = 2 * R_MAX_JOBS;
+template <int NM>
 struct RSegs {
   RSeg seg[R_MAX_SEGS];
   int NC, P;
+  size_t mstride;
   const float* part;
+  float* dst[NM][R_MAX_SEGS];   // per member: the gradient tensor of each segment
 };
+template <int NM>
+struct WpeParams {
+  const float* gfin;
+  size_t mstride;
+  int B, S, n_pos;
+  float* dwpe[NM];
+};
+static_assert(sizeof(TrainFwdParams<TRAIN_POP_MAX>) <= 32764 && sizeof(BackParams<TRAIN_POP_MAX>) <= 32764 &&
+                  sizeof(RSegs<TRAIN_POP_MAX>) <= 32764 && sizeof(RParams) <= 32764,
+              "the per-member tables of TRAIN_POP_MAX members must fit the kernel parameter limit");
 
+// CTA (tile, chunk, member)
 __global__ void __launch_bounds__(256) weight_grad_partial_kernel(const RParams p) {
   __shared__ __align__(16) float As[32][32];
   __shared__ __align__(16) float Gs[32][32];
@@ -356,6 +376,9 @@ __global__ void __launch_bounds__(256) weight_grad_partial_kernel(const RParams 
   const RTile t = p.tile[blockIdx.x];
   const RJob& j = p.job[t.job];
   const int tid = threadIdx.x, chunk = blockIdx.y;
+  const size_t moff = (size_t)blockIdx.z * p.mstride;
+  const float* const A = j.A + moff;
+  const float* const G = j.G + moff;
   const int r0 = chunk * p.CH, r1 = min(p.NR, r0 + p.CH);
   const int lr = tid >> 3, l4 = (tid & 7) * 4;   // loader: row, 4 columns
   const int i = tid >> 3, o4 = (tid & 7) * 4;    // outer product: input i, outputs o4..o4+3
@@ -366,8 +389,8 @@ __global__ void __launch_bounds__(256) weight_grad_partial_kernel(const RParams 
     const int rr = rb + lr;
     float4 av = make_float4(0.f, 0.f, 0.f, 0.f), gv = av;
     if (rr < r1) {
-      av = *reinterpret_cast<const float4*>(j.A + (size_t)rr * j.sa + t.i0 + l4);
-      gv = *reinterpret_cast<const float4*>(j.G + (size_t)rr * j.sg + t.o0 + l4);
+      av = *reinterpret_cast<const float4*>(A + (size_t)rr * j.sa + t.i0 + l4);
+      gv = *reinterpret_cast<const float4*>(G + (size_t)rr * j.sg + t.o0 + l4);
     }
     __syncthreads();
     *reinterpret_cast<float4*>(&As[lr][l4]) = av;
@@ -386,7 +409,7 @@ __global__ void __launch_bounds__(256) weight_grad_partial_kernel(const RParams 
       for (int k = dg; k < 32; k += 8) dacc = fmaf(As[k][dc], Gs[k][dc], dacc), dbacc += Gs[k][dc];
     }
   }
-  float* part = p.part + (size_t)chunk * p.P;
+  float* part = p.part + moff + (size_t)chunk * p.P;
   if (!j.diag) {
     const float v[4] = {acc.x, acc.y, acc.z, acc.w}, bv[4] = {bacc.x, bacc.y, bacc.z, bacc.w};
     const int gi = t.i0 + i;
@@ -408,24 +431,31 @@ __global__ void __launch_bounds__(256) weight_grad_partial_kernel(const RParams 
   }
 }
 
-__global__ void __launch_bounds__(256) weight_grad_reduce_kernel(const RSegs s) {
+// CTA (x, segment, member)
+template <int NM>
+__global__ void __launch_bounds__(256) weight_grad_reduce_kernel(const __grid_constant__ RSegs<NM> s) {
   const RSeg& g = s.seg[blockIdx.y];
+  const int mz = NM == 1 ? 0 : blockIdx.z;
   const int e = blockIdx.x * 256 + threadIdx.x;
   if (e >= g.n) return;
-  const float* src = s.part + g.off + e;
+  const float* src = s.part + (size_t)mz * s.mstride + g.off + e;
   float acc = 0.f;
   for (int c = 0; c < s.NC; ++c) acc += src[(size_t)c * s.P];
-  g.dst[e] = acc;
+  s.dst[mz][blockIdx.y][e] = acc;
 }
 
-__global__ void wpe_grad_kernel(const float* gfin, int B, int S, int n_pos, float* dwpe) {
+// CTA (x, member)
+template <int NM>
+__global__ void wpe_grad_kernel(const __grid_constant__ WpeParams<NM> p) {
+  const int mz = NM == 1 ? 0 : blockIdx.y;
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= n_pos * G_E) return;
+  if (e >= p.n_pos * G_E) return;
   const int t = e / G_E, c = e % G_E;
+  const float* gfin = p.gfin + (size_t)mz * p.mstride;
   float acc = 0.f;
-  if (t < S)
-    for (int b = 0; b < B; ++b) acc += gfin[((size_t)b * S + t) * GF_STRIDE + GF_DX0 + c];
-  dwpe[e] = acc;
+  if (t < p.S)
+    for (int b = 0; b < p.B; ++b) acc += gfin[((size_t)b * p.S + t) * GF_STRIDE + GF_DX0 + c];
+  p.dwpe[mz][e] = acc;
 }
 
 // ---- host side ----
@@ -461,142 +491,145 @@ static TrainLayout train_layout(int L, int din, int du, int B, int T) {
   return t;
 }
 
-static int check_model(const char* fn, const dpt_gpt2_weights_t* w, int B, int T) {
-  DPT_CHECK_ARG(w, "%s: null weights", fn);
+// `mem`: the member's index in a population call (its messages name it), -1 for the one-model entry points
+static int check_model(const char* fn, int mem, const dpt_gpt2_weights_t* w, int B, int T) {
+  char who[96];
+  if (mem < 0) snprintf(who, sizeof who, "%s", fn);
+  else snprintf(who, sizeof who, "%s: member %d", fn, mem);
+  DPT_CHECK_ARG(w, "%s: null weights", who);
   if (w->n_embd != G_E) {
-    set_error("%s: n_embd=%d, training supports n_embd == %d", fn, w->n_embd, G_E);
+    set_error("%s: n_embd=%d, training supports n_embd == %d", who, w->n_embd, G_E);
     return DPT_ERR_UNSUPPORTED;
   }
   if (w->n_layer < 1 || w->n_layer > G_MAX_L) {
-    set_error("%s: n_layer=%d outside [1,%d]", fn, w->n_layer, G_MAX_L);
+    set_error("%s: n_layer=%d outside [1,%d]", who, w->n_layer, G_MAX_L);
     return DPT_ERR_UNSUPPORTED;
   }
   const int din = 2 * w->state_dim + w->action_dim + 1;
   DPT_CHECK_ARG(w->state_dim >= 1 && w->action_dim >= 1 && din <= 32,
-                "%s: token width 2*state_dim+action_dim+1 = %d must be <= 32", fn, din);
-  DPT_CHECK_ARG(B >= 0 && T >= 0, "%s: B=%d T=%d", fn, B, T);
+                "%s: token width 2*state_dim+action_dim+1 = %d must be <= 32", who, din);
+  DPT_CHECK_ARG(B >= 0 && T >= 0, "%s: B=%d T=%d", who, B, T);
   if (T + 1 > 512) {
-    set_error("%s: T=%d, training supports sequences of <= 512 tokens (T <= 511)", fn, T);
+    set_error("%s: T=%d, training supports sequences of <= 512 tokens (T <= 511)", who, T);
     return DPT_ERR_UNSUPPORTED;
   }
-  DPT_CHECK_ARG(T + 1 <= w->n_positions, "%s: sequence %d exceeds n_positions %d", fn, T + 1, w->n_positions);
+  DPT_CHECK_ARG(T + 1 <= w->n_positions, "%s: sequence %d exceeds n_positions %d", who, T + 1, w->n_positions);
   DPT_CHECK_ARG(w->wpe && w->embed_w && w->embed_b && w->pred_w && w->pred_b && w->lnf_w && w->lnf_b && w->ln1_w && w->ln1_b &&
                     w->attn_w && w->attn_b && w->proj_w && w->proj_b && w->ln2_w && w->ln2_b && w->fc_w && w->fc_b &&
                     w->fc2_w && w->fc2_b,
-                "%s: null weight pointer", fn);
+                "%s: null weight pointer", who);
   for (int l = 0; l < w->n_layer; ++l)
     DPT_CHECK_ARG(w->ln1_w[l] && w->ln1_b[l] && w->attn_w[l] && w->attn_b[l] && w->proj_w[l] && w->proj_b[l] && w->ln2_w[l] &&
                       w->ln2_b[l] && w->fc_w[l] && w->fc_b[l] && w->fc2_w[l] && w->fc2_b[l],
-                  "%s: null layer %d weight", fn, l);
+                  "%s: null layer %d weight", who, l);
   return DPT_OK;
 }
 
-}  // namespace dpt
-
-using namespace dpt;
-
-extern "C" uint64_t dpt_gpt2_train_workspace_bytes(const dpt_gpt2_weights_t* w, int B, int T) {
-  if (!w || B <= 0 || T < 0 || w->n_layer < 1) return 0;
-  return train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T).total * sizeof(float);
+// The checks of a population call: 0 <= n <= TRAIN_POP_MAX, every member valid (check_model) and of member 0's shape.
+// Returns DPT_OK with *done = true when there is nothing to compute (n = 0 or B = 0).
+static int check_population(const char* fn, const dpt_gpt2_weights_t* w, int n, int B, int T, bool* done) {
+  *done = true;
+  DPT_CHECK_ARG(n >= 0 && n <= TRAIN_POP_MAX, "%s: n_models=%d outside [0,%d]", fn, n, TRAIN_POP_MAX);
+  if (n == 0) return DPT_OK;
+  DPT_CHECK_ARG(w, "%s: null weights", fn);
+  for (int i = 0; i < n; ++i) {
+    const int rc = check_model(fn, n == 1 ? -1 : i, w + i, B, T);
+    if (rc != DPT_OK) return rc;
+    const struct { const char* name; int v, v0; } f[] = {{"n_layer", w[i].n_layer, w[0].n_layer},
+                                                         {"state_dim", w[i].state_dim, w[0].state_dim},
+                                                         {"action_dim", w[i].action_dim, w[0].action_dim},
+                                                         {"n_positions", w[i].n_positions, w[0].n_positions}};
+    for (const auto& x : f)
+      DPT_CHECK_ARG(x.v == x.v0, "%s: member %d has %s=%d, member 0 has %d (members must share one shape)", fn, i, x.name,
+                    x.v, x.v0);
+  }
+  *done = B == 0;
+  return DPT_OK;
 }
 
-extern "C" int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, const float* query_states, const float* ctx_states,
-                                      const float* ctx_actions, const float* ctx_next_states, const float* ctx_rewards, int B,
-                                      int T, int T_stride, int test, float* out, void* workspace, uint64_t workspace_bytes,
-                                      void* stream) {
-  const char* fn = "dpt_gpt2_train_forward";
-  int rc = check_model(fn, w, B, T);
-  if (rc != DPT_OK) return rc;
-  DPT_CHECK_ARG(T_stride >= T, "%s: T_stride=%d < T=%d", fn, T_stride, T);
-  if (B == 0) return DPT_OK;
-  DPT_CHECK_ARG(query_states && out && (T == 0 || (ctx_states && ctx_actions && ctx_next_states && ctx_rewards)),
-                "%s: null input or output pointer", fn);
-  DPT_CHECK_ARG(workspace && workspace_bytes >= dpt_gpt2_train_workspace_bytes(w, B, T) && aligned16(workspace),
-                "%s: workspace of %llu B, needs %llu B (16 B aligned)", fn, (unsigned long long)workspace_bytes,
-                (unsigned long long)dpt_gpt2_train_workspace_bytes(w, B, T));
-  const TrainLayout lay = train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T);
-  DenseParams dp{};
-  Gpt2Dev& d = dp.m;
-  d.L = w->n_layer, d.dx = w->state_dim, d.du = w->action_dim, d.din = lay.din, d.H = w->horizon, d.n_pos = w->n_positions;
-  d.wpe = w->wpe, d.embed_wT = w->embed_w, d.embed_b = w->embed_b, d.pred_wT = w->pred_w, d.pred_b = w->pred_b;
+static TrainW train_w(const dpt_gpt2_weights_t* w) {
+  TrainW d{};
+  d.wpe = w->wpe, d.embed_w = w->embed_w, d.embed_b = w->embed_b, d.pred_w = w->pred_w, d.pred_b = w->pred_b;
   d.lnf_w = w->lnf_w, d.lnf_b = w->lnf_b;
-  for (int l = 0; l < d.L; ++l) {
-    LayerW& lw = d.layer[l];
+  for (int l = 0; l < w->n_layer; ++l) {
+    TrainLayerW& lw = d.layer[l];
     lw.ln1_w = w->ln1_w[l], lw.ln1_b = w->ln1_b[l], lw.attn_w = w->attn_w[l], lw.attn_b = w->attn_b[l];
     lw.proj_w = w->proj_w[l], lw.proj_b = w->proj_b[l], lw.ln2_w = w->ln2_w[l], lw.ln2_b = w->ln2_b[l];
     lw.fc_w = w->fc_w[l], lw.fc_b = w->fc_b[l], lw.fc2_w = w->fc2_w[l], lw.fc2_b = w->fc2_b[l];
-    DPT_CHECK_ARG(aligned16(lw.attn_w) && aligned16(lw.proj_w) && aligned16(lw.fc_w) && aligned16(lw.fc2_w),
-                  "%s: layer %d matrices must be 16 B aligned", fn, l);
   }
-  dp.query = query_states, dp.cs = ctx_states, dp.ca = ctx_actions, dp.cns = ctx_next_states, dp.cr = ctx_rewards;
-  dp.B = B, dp.T = T, dp.Ts = T_stride, dp.test = test ? 1 : 0, dp.share = 1, dp.out = out;
-  float* ws = static_cast<float*>(workspace);
-  TrainSave sv{ws + lay.act, ws + lay.fin};
-  return gpt2_train_forward_launch(dp, sv, (cudaStream_t)stream);
+  return d;
 }
 
-template <int THREADS>
-static cudaError_t launch_back(const BackParams& p, cudaStream_t st) {
+static uint64_t member_bytes(const dpt_gpt2_weights_t* w, int B, int T) {
+  return train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T).total * sizeof(float);
+}
+
+template <int NM>
+static int population_forward(const char* fn, const dpt_gpt2_weights_t* w, int n, const float* const* query,
+                              const float* const* cs, const float* const* ca, const float* const* cns, const float* const* cr,
+                              int B, int T, int T_stride, int test, float* const* out, float* ws, cudaStream_t st) {
+  const TrainLayout lay = train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T);
+  TrainFwdParams<NM> p{};
+  p.L = w->n_layer, p.dx = w->state_dim, p.du = w->action_dim, p.din = lay.din;
+  p.B = B, p.T = T, p.Ts = T_stride, p.test = test ? 1 : 0;
+  for (int i = 0; i < n; ++i) {
+    TrainFwdMember& m = p.mem[i];
+    m.w = train_w(w + i);
+    for (int l = 0; l < p.L; ++l) {
+      const TrainLayerW& lw = m.w.layer[l];
+      DPT_CHECK_ARG(aligned16(lw.attn_w) && aligned16(lw.proj_w) && aligned16(lw.fc_w) && aligned16(lw.fc2_w),
+                    "%s: layer %d matrices must be 16 B aligned", fn, l);
+    }
+    m.query = query[i], m.cs = T ? cs[i] : nullptr, m.ca = T ? ca[i] : nullptr, m.cns = T ? cns[i] : nullptr;
+    m.cr = T ? cr[i] : nullptr, m.out = out[i];
+    float* mws = ws + (size_t)i * lay.total;
+    m.sv = TrainSave{mws + lay.act, mws + lay.fin};
+  }
+  return gpt2_train_forward_launch<NM>(p, n, st);
+}
+
+template <int THREADS, int NM>
+static cudaError_t launch_back(const BackParams<NM>& p, int n, cudaStream_t st) {
   const int smem = db_floats(THREADS) * (int)sizeof(float);
-  cudaError_t e = cudaFuncSetAttribute(gpt2_train_backward_kernel<THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  cudaError_t e = cudaFuncSetAttribute(gpt2_train_backward_kernel<THREADS, NM>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;
-  gpt2_train_backward_kernel<THREADS><<<p.B, THREADS, smem, st>>>(p);
+  gpt2_train_backward_kernel<THREADS, NM><<<dim3(p.B, n), THREADS, smem, st>>>(p);
   return cudaGetLastError();
 }
 
-extern "C" int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float* dout, int B, int T, int test,
-                                       const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream) {
-  const char* fn = "dpt_gpt2_train_backward";
-  int rc = check_model(fn, w, B, T);
-  if (rc != DPT_OK) return rc;
-  if (B == 0) return DPT_OK;
-  DPT_CHECK_ARG(dout && grads, "%s: null dout or grads", fn);
-  DPT_CHECK_ARG(workspace && workspace_bytes >= dpt_gpt2_train_workspace_bytes(w, B, T) && aligned16(workspace),
-                "%s: workspace of %llu B, needs %llu B (16 B aligned)", fn, (unsigned long long)workspace_bytes,
-                (unsigned long long)dpt_gpt2_train_workspace_bytes(w, B, T));
+template <int NM>
+static int population_backward(const char* fn, const dpt_gpt2_weights_t* w, int n, const float* const* dout, int B, int T,
+                               int test, const dpt_gpt2_grads_t* grads, float* ws, cudaStream_t st) {
   const int L = w->n_layer;
-  const dpt_gpt2_grads_t* g = grads;
-  DPT_CHECK_ARG(g->wpe && g->embed_w && g->embed_b && g->pred_w && g->pred_b && g->lnf_w && g->lnf_b && g->ln1_w && g->ln1_b &&
-                    g->attn_w && g->attn_b && g->proj_w && g->proj_b && g->ln2_w && g->ln2_b && g->fc_w && g->fc_b &&
-                    g->fc2_w && g->fc2_b,
-                "%s: null gradient pointer", fn);
-  for (int l = 0; l < L; ++l)
-    DPT_CHECK_ARG(g->ln1_w[l] && g->ln1_b[l] && g->attn_w[l] && g->attn_b[l] && g->proj_w[l] && g->proj_b[l] && g->ln2_w[l] &&
-                      g->ln2_b[l] && g->fc_w[l] && g->fc_b[l] && g->fc2_w[l] && g->fc2_b[l],
-                  "%s: null layer %d gradient", fn, l);
   const TrainLayout lay = train_layout(L, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T);
-  float* ws = static_cast<float*>(workspace);
-  cudaStream_t st = (cudaStream_t)stream;
-
-  BackParams bp{};
-  TrainModel& m = bp.m;
-  m.L = L, m.dx = w->state_dim, m.du = w->action_dim, m.din = lay.din, m.n_pos = w->n_positions;
-  m.wpe = w->wpe, m.embed_w = w->embed_w, m.embed_b = w->embed_b, m.pred_w = w->pred_w, m.pred_b = w->pred_b;
-  m.lnf_w = w->lnf_w, m.lnf_b = w->lnf_b;
-  for (int l = 0; l < L; ++l) {
-    m.ln1_w[l] = w->ln1_w[l], m.ln1_b[l] = w->ln1_b[l], m.attn_w[l] = w->attn_w[l], m.attn_b[l] = w->attn_b[l];
-    m.proj_w[l] = w->proj_w[l], m.proj_b[l] = w->proj_b[l], m.ln2_w[l] = w->ln2_w[l], m.ln2_b[l] = w->ln2_b[l];
-    m.fc_w[l] = w->fc_w[l], m.fc_b[l] = w->fc_b[l], m.fc2_w[l] = w->fc2_w[l], m.fc2_b[l] = w->fc2_b[l];
+  const size_t NR = lay.NR;
+  BackParams<NM> bp{};
+  bp.L = L, bp.du = w->action_dim, bp.B = B, bp.T = T, bp.test = test ? 1 : 0;
+  for (int i = 0; i < n; ++i) {
+    BackMember& m = bp.mem[i];
+    float* mws = ws + (size_t)i * lay.total;
+    m.w = train_w(w + i);
+    m.dout = dout[i];
+    m.act = mws + lay.act, m.fin = mws + lay.fin, m.grec = mws + lay.grec, m.gfin = mws + lay.gfin;
   }
-  bp.dout = dout, bp.B = B, bp.T = T, bp.test = test ? 1 : 0;
-  bp.act = ws + lay.act, bp.fin = ws + lay.fin, bp.grec = ws + lay.grec, bp.gfin = ws + lay.gfin;
   const int S = T + 1;
-  cudaError_t e = S <= 128 ? launch_back<128>(bp, st) : S <= 256 ? launch_back<256>(bp, st) : launch_back<512>(bp, st);
+  cudaError_t e = S <= 128 ? launch_back<128>(bp, n, st) : S <= 256 ? launch_back<256>(bp, n, st) : launch_back<512>(bp, n, st);
   if (e != cudaSuccess) {
     set_error("%s: backward launch failed: %s", fn, cudaGetErrorString(e));
     return DPT_ERR_CUDA;
   }
 
-  // weight-gradient jobs (operands in the workspace) and the gradient tensors they reduce into
+  // weight-gradient jobs (operands in member 0's workspace region) and, per member, the gradient tensors they reduce into
   RParams rp{};
-  RSegs rs{};
+  RSegs<NM> rs{};
+  WpeParams<NM> wp{};
   int nj = 0, nt = 0, ns = 0, off = 0;
-  auto job = [&](const float* A, int sa, const float* G, int sg, int nin, int nout, int diag, int trans, float* dw, float* db) {
+  auto job = [&](const float* A, int sa, const float* G, int sg, int nin, int nout, int diag, int trans) {
     RJob& j = rp.job[nj];
     j.A = A, j.G = G, j.sa = sa, j.sg = sg, j.nin = nin, j.nout = nout, j.diag = diag, j.trans = trans;
     const int nw = diag ? nout : nin * nout;
-    j.woff = off, rs.seg[ns++] = RSeg{dw, off, nw}, off += nw;
-    j.boff = off, rs.seg[ns++] = RSeg{db, off, nout}, off += nout;
+    j.woff = off, rs.seg[ns++] = RSeg{off, nw}, off += nw;
+    j.boff = off, rs.seg[ns++] = RSeg{off, nout}, off += nout;
     if (diag) {
       rp.tile[nt++] = RTile{(short)nj, 0, 0};
     } else {
@@ -605,32 +638,138 @@ extern "C" int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float*
     }
     ++nj;
   };
-  const size_t NR = lay.NR;
   for (int l = 0; l < L; ++l) {
     const float* a = ws + lay.act + (size_t)l * NR * TA_STRIDE;
     const float* gr = ws + lay.grec + (size_t)l * NR * GR_STRIDE;
-    job(gr + GR_G, GR_STRIDE, gr + GR_DX, GR_STRIDE, G_FF, G_E, 0, 0, g->fc2_w[l], g->fc2_b[l]);
-    job(gr + GR_Y2, GR_STRIDE, gr + GR_DH, GR_STRIDE, G_E, G_FF, 0, 0, g->fc_w[l], g->fc_b[l]);
-    job(gr + GR_XH2, GR_STRIDE, gr + GR_DY2, GR_STRIDE, G_E, G_E, 1, 0, g->ln2_w[l], g->ln2_b[l]);
-    job(a + TA_O, TA_STRIDE, gr + GR_DXM, GR_STRIDE, G_E, G_E, 0, 0, g->proj_w[l], g->proj_b[l]);
-    job(gr + GR_Y1, GR_STRIDE, gr + GR_DQKV, GR_STRIDE, G_E, 3 * G_E, 0, 0, g->attn_w[l], g->attn_b[l]);
-    job(gr + GR_XH1, GR_STRIDE, gr + GR_DY1, GR_STRIDE, G_E, G_E, 1, 0, g->ln1_w[l], g->ln1_b[l]);
+    job(gr + GR_G, GR_STRIDE, gr + GR_DX, GR_STRIDE, G_FF, G_E, 0, 0);
+    job(gr + GR_Y2, GR_STRIDE, gr + GR_DH, GR_STRIDE, G_E, G_FF, 0, 0);
+    job(gr + GR_XH2, GR_STRIDE, gr + GR_DY2, GR_STRIDE, G_E, G_E, 1, 0);
+    job(a + TA_O, TA_STRIDE, gr + GR_DXM, GR_STRIDE, G_E, G_E, 0, 0);
+    job(gr + GR_Y1, GR_STRIDE, gr + GR_DQKV, GR_STRIDE, G_E, 3 * G_E, 0, 0);
+    job(gr + GR_XH1, GR_STRIDE, gr + GR_DY1, GR_STRIDE, G_E, G_E, 1, 0);
   }
   const float* gf = ws + lay.gfin;
-  job(gf + GF_YF, GF_STRIDE, gf + GF_DLOG, GF_STRIDE, G_E, lay.du, 0, 1, g->pred_w, g->pred_b);
-  job(gf + GF_XHF, GF_STRIDE, gf + GF_DYF, GF_STRIDE, G_E, G_E, 1, 0, g->lnf_w, g->lnf_b);
-  job(ws + lay.fin + TF_TOK, TF_STRIDE, gf + GF_DX0, GF_STRIDE, lay.din, G_E, 0, 1, g->embed_w, g->embed_b);
+  job(gf + GF_YF, GF_STRIDE, gf + GF_DLOG, GF_STRIDE, G_E, lay.du, 0, 1);
+  job(gf + GF_XHF, GF_STRIDE, gf + GF_DYF, GF_STRIDE, G_E, G_E, 1, 0);
+  job(ws + lay.fin + TF_TOK, TF_STRIDE, gf + GF_DX0, GF_STRIDE, lay.din, G_E, 0, 1);
   if (off > lay.P) {
     set_error("%s: internal: %d gradient entries exceed the partial slot of %d", fn, off, lay.P);
     return DPT_ERR_CUDA;
   }
-  rp.NR = (int)NR, rp.CH = lay.CH, rp.P = lay.P, rp.part = ws + lay.part;
-  weight_grad_partial_kernel<<<dim3(nt, lay.NC), 256, 0, st>>>(rp);
+  for (int i = 0; i < n; ++i) {   // the segments in job order: per layer fc2, fc, ln_2, proj, attn, ln_1 (w, b), then the top
+    const dpt_gpt2_grads_t* g = grads + i;
+    float** d = rs.dst[i];
+    int k = 0;
+    for (int l = 0; l < L; ++l) {
+      d[k++] = g->fc2_w[l], d[k++] = g->fc2_b[l], d[k++] = g->fc_w[l], d[k++] = g->fc_b[l];
+      d[k++] = g->ln2_w[l], d[k++] = g->ln2_b[l], d[k++] = g->proj_w[l], d[k++] = g->proj_b[l];
+      d[k++] = g->attn_w[l], d[k++] = g->attn_b[l], d[k++] = g->ln1_w[l], d[k++] = g->ln1_b[l];
+    }
+    d[k++] = g->pred_w, d[k++] = g->pred_b, d[k++] = g->lnf_w, d[k++] = g->lnf_b, d[k++] = g->embed_w, d[k++] = g->embed_b;
+    wp.dwpe[i] = g->wpe;
+  }
+  rp.NR = (int)NR, rp.CH = lay.CH, rp.P = lay.P, rp.mstride = lay.total, rp.part = ws + lay.part;
+  weight_grad_partial_kernel<<<dim3(nt, lay.NC, n), 256, 0, st>>>(rp);
   int maxn = 0;
   for (int s = 0; s < ns; ++s) maxn = std::max(maxn, rs.seg[s].n);
-  rs.NC = lay.NC, rs.P = lay.P, rs.part = ws + lay.part;
-  weight_grad_reduce_kernel<<<dim3((maxn + 255) / 256, ns), 256, 0, st>>>(rs);
-  wpe_grad_kernel<<<(w->n_positions * G_E + 255) / 256, 256, 0, st>>>(ws + lay.gfin, B, S, w->n_positions, g->wpe);
+  rs.NC = lay.NC, rs.P = lay.P, rs.mstride = lay.total, rs.part = ws + lay.part;
+  weight_grad_reduce_kernel<NM><<<dim3((maxn + 255) / 256, ns, n), 256, 0, st>>>(rs);
+  wp.gfin = ws + lay.gfin, wp.mstride = lay.total, wp.B = B, wp.S = S, wp.n_pos = w->n_positions;
+  wpe_grad_kernel<NM><<<dim3((w->n_positions * G_E + 255) / 256, n), 256, 0, st>>>(wp);
   DPT_LAUNCH_CHECK();
   return DPT_OK;
+}
+
+// the argument checks and launches shared by the one-model and the population entry points (one = the one-model call)
+static int train_forward(const char* fn, bool one, const dpt_gpt2_weights_t* w, int n, const float* const* query,
+                         const float* const* cs, const float* const* ca, const float* const* cns, const float* const* cr, int B,
+                         int T, int T_stride, int test, float* const* out, void* workspace, uint64_t workspace_bytes,
+                         void* stream) {
+  bool done;
+  int rc = check_population(fn, w, n, B, T, &done);
+  if (rc != DPT_OK) return rc;
+  if (n == 0) return DPT_OK;
+  DPT_CHECK_ARG(T_stride >= T, "%s: T_stride=%d < T=%d", fn, T_stride, T);
+  if (done) return DPT_OK;
+  DPT_CHECK_ARG(query && out && (T == 0 || (cs && ca && cns && cr)), "%s: null input or output pointer array", fn);
+  for (int i = 0; i < n; ++i)
+    DPT_CHECK_ARG(query[i] && out[i] && (T == 0 || (cs[i] && ca[i] && cns[i] && cr[i])),
+                  one ? "%s: null input or output pointer" : "%s: member %d: null input or output pointer", fn, i);
+  const uint64_t need = (uint64_t)n * member_bytes(w, B, T);
+  DPT_CHECK_ARG(workspace && workspace_bytes >= need && aligned16(workspace), "%s: workspace of %llu B, needs %llu B (16 B aligned)",
+                fn, (unsigned long long)workspace_bytes, (unsigned long long)need);
+  float* ws = static_cast<float*>(workspace);
+  cudaStream_t st = (cudaStream_t)stream;
+  return n == 1 ? population_forward<1>(fn, w, n, query, cs, ca, cns, cr, B, T, T_stride, test, out, ws, st)
+                : population_forward<TRAIN_POP_MAX>(fn, w, n, query, cs, ca, cns, cr, B, T, T_stride, test, out, ws, st);
+}
+
+static int train_backward(const char* fn, bool one, const dpt_gpt2_weights_t* w, int n, const float* const* dout, int B, int T,
+                          int test, const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream) {
+  bool done;
+  int rc = check_population(fn, w, n, B, T, &done);
+  if (rc != DPT_OK || done) return rc;
+  DPT_CHECK_ARG(dout && grads, "%s: null dout or grads", fn);
+  const uint64_t need = (uint64_t)n * member_bytes(w, B, T);
+  DPT_CHECK_ARG(workspace && workspace_bytes >= need && aligned16(workspace), "%s: workspace of %llu B, needs %llu B (16 B aligned)",
+                fn, (unsigned long long)workspace_bytes, (unsigned long long)need);
+  const int L = w->n_layer;
+  for (int i = 0; i < n; ++i) {
+    const dpt_gpt2_grads_t* g = grads + i;
+    DPT_CHECK_ARG(dout[i], one ? "%s: null dout or grads" : "%s: member %d: null dout", fn, i);
+    DPT_CHECK_ARG(g->wpe && g->embed_w && g->embed_b && g->pred_w && g->pred_b && g->lnf_w && g->lnf_b && g->ln1_w && g->ln1_b &&
+                      g->attn_w && g->attn_b && g->proj_w && g->proj_b && g->ln2_w && g->ln2_b && g->fc_w && g->fc_b &&
+                      g->fc2_w && g->fc2_b,
+                  one ? "%s: null gradient pointer" : "%s: member %d: null gradient pointer", fn, i);
+    for (int l = 0; l < L; ++l)
+      DPT_CHECK_ARG(g->ln1_w[l] && g->ln1_b[l] && g->attn_w[l] && g->attn_b[l] && g->proj_w[l] && g->proj_b[l] && g->ln2_w[l] &&
+                        g->ln2_b[l] && g->fc_w[l] && g->fc_b[l] && g->fc2_w[l] && g->fc2_b[l],
+                    "%s: member %d: null layer %d gradient", fn, i, l);
+  }
+  float* ws = static_cast<float*>(workspace);
+  cudaStream_t st = (cudaStream_t)stream;
+  return n == 1 ? population_backward<1>(fn, w, n, dout, B, T, test, grads, ws, st)
+                : population_backward<TRAIN_POP_MAX>(fn, w, n, dout, B, T, test, grads, ws, st);
+}
+
+}  // namespace dpt
+
+using namespace dpt;
+
+extern "C" uint64_t dpt_gpt2_train_population_workspace_bytes(const dpt_gpt2_weights_t* w, int n_models, int B, int T) {
+  if (!w || n_models <= 0 || n_models > TRAIN_POP_MAX || B <= 0 || T < 0 || w->n_layer < 1) return 0;
+  return (uint64_t)n_models * member_bytes(w, B, T);
+}
+
+extern "C" uint64_t dpt_gpt2_train_workspace_bytes(const dpt_gpt2_weights_t* w, int B, int T) {
+  return dpt_gpt2_train_population_workspace_bytes(w, 1, B, T);
+}
+
+extern "C" int dpt_gpt2_train_population_forward(const dpt_gpt2_weights_t* w, int n_models, const float* const* query_states,
+                                                 const float* const* ctx_states, const float* const* ctx_actions,
+                                                 const float* const* ctx_next_states, const float* const* ctx_rewards, int B,
+                                                 int T, int T_stride, int test, float* const* out, void* workspace,
+                                                 uint64_t workspace_bytes, void* stream) {
+  return train_forward("dpt_gpt2_train_population_forward", false, w, n_models, query_states, ctx_states, ctx_actions,
+                       ctx_next_states, ctx_rewards, B, T, T_stride, test, out, workspace, workspace_bytes, stream);
+}
+
+extern "C" int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, const float* query_states, const float* ctx_states,
+                                      const float* ctx_actions, const float* ctx_next_states, const float* ctx_rewards, int B,
+                                      int T, int T_stride, int test, float* out, void* workspace, uint64_t workspace_bytes,
+                                      void* stream) {
+  return train_forward("dpt_gpt2_train_forward", true, w, 1, &query_states, &ctx_states, &ctx_actions, &ctx_next_states,
+                       &ctx_rewards, B, T, T_stride, test, &out, workspace, workspace_bytes, stream);
+}
+
+extern "C" int dpt_gpt2_train_population_backward(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B,
+                                                  int T, int test, const dpt_gpt2_grads_t* grads, void* workspace,
+                                                  uint64_t workspace_bytes, void* stream) {
+  return train_backward("dpt_gpt2_train_population_backward", false, w, n_models, dout, B, T, test, grads, workspace,
+                        workspace_bytes, stream);
+}
+
+extern "C" int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float* dout, int B, int T, int test,
+                                       const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream) {
+  return train_backward("dpt_gpt2_train_backward", true, w, 1, &dout, B, T, test, grads, workspace, workspace_bytes, stream);
 }

@@ -194,25 +194,9 @@ class Transformer(nn.Module):
     def forward_train(self, x):
         """``forward(x)`` with an autograd graph: returns ``preds[:, -1, :]`` (test) or ``preds[:, 1:, :]`` with a
         ``grad_fn``; ``backward`` fills ``.grad`` of every parameter except ``transformer.wte``.  The logits are
-        bit-identical to ``forward(x)``.  The context inputs get no gradient.  fp32, sequences of <= 512 tokens."""
-        if self.dropout > 0:
-            raise NotImplementedError("forward_train: dropout=%g, the fused training path has no dropout" % self.dropout)
-        dev = kernels._dev()
-        if next(self.parameters()).device != dev:
-            self.to(dev)
-        f = lambda t: t.to(device=dev, dtype=torch.float32)   # noqa: E731
-        q = f(x["query_states"]).contiguous()
-        cs, ca, cns, cr = f(x["context_states"]), f(x["context_actions"]), f(x["context_next_states"]), f(x["context_rewards"])
-        B, T = ca.shape[0], ca.shape[1]
-        assert q.shape[0] == B, "query_states and the context disagree on the batch size"
-        # context views [:, :h] of a [B,H,.] buffer are passed with their row stride, without a copy
-        stride = ca.stride(0) // max(1, ca.shape[2]) if T > 0 else 0
-        ok = T > 0 and stride >= T and all(t.stride(-1) == 1 and t.stride(1) == t.shape[2] and t.stride(0) == stride * t.shape[2]
-                                           for t in (cs, ca, cns, cr.reshape(B, T, 1) if cr.dim() == 2 else cr))
-        if not ok:
-            cs, ca, cns, cr = cs.contiguous(), ca.contiguous(), cns.contiguous(), cr.contiguous()
-            stride = T
-        return _TrainFn.apply(self, (q, cs, ca, cns, cr, B, T, stride), *self._train_params())
+        bit-identical to ``forward(x)``.  The context inputs get no gradient.  fp32, sequences of <= 512 tokens.
+        This is the one-member case of ``forward_train_population``."""
+        return forward_train_population([self], [x])[0]
 
     # ---- step-by-step K/V-cached decode (callers that choose the pulled arm themselves) -------------
     def decoder(self, n_seqs, max_transitions=None):
@@ -301,43 +285,132 @@ def _weights_struct(model, params, keep):
                            n_positions=model.transformer.wpe.weight.shape[0])
 
 
-class _TrainFn(torch.autograd.Function):
-    """dpt_gpt2_train_forward / dpt_gpt2_train_backward.  The workspace holds the saved activations between the two."""
+def _train_inputs(x, dev):
+    """(q, cs, ca, cns, cr, B, T, stride) of a batch dict; context views [:, :h] of a [B,H,.] buffer keep their row
+    stride, other layouts are made contiguous."""
+    f = lambda t: t.to(device=dev, dtype=torch.float32)   # noqa: E731
+    q = f(x["query_states"]).contiguous()
+    cs, ca, cns, cr = f(x["context_states"]), f(x["context_actions"]), f(x["context_next_states"]), f(x["context_rewards"])
+    B, T = ca.shape[0], ca.shape[1]
+    assert q.shape[0] == B, "query_states and the context disagree on the batch size"
+    stride = ca.stride(0) // max(1, ca.shape[2]) if T > 0 else 0
+    ok = T > 0 and stride >= T and all(t.stride(-1) == 1 and t.stride(1) == t.shape[2] and t.stride(0) == stride * t.shape[2]
+                                       for t in (cs, ca, cns, cr.reshape(B, T, 1) if cr.dim() == 2 else cr))
+    if not ok:
+        cs, ca, cns, cr = cs.contiguous(), ca.contiguous(), cns.contiguous(), cr.contiguous()
+        stride = T
+    return [q, cs, ca, cns, cr, B, T, stride]
+
+
+_MEMBER_FIELDS = ("n_layer", "state_dim", "action_dim", "horizon", "test")
+
+
+def forward_train_population(models, batches):
+    """``[m.forward_train(x) for m, x in zip(models, batches)]`` in the same kernel launches: member i's logits, and
+    after ``backward`` the ``.grad`` of its parameters, are bit-identical to training it alone.  The members are
+    same-shape Transformers (``n_layer``, ``state_dim``, ``action_dim``, ``horizon`` and ``test`` agree, else
+    ``ValueError``) on one device, and the batches share B and T.  All members' parameters go through ONE autograd
+    Function; a member whose logits get no gradient keeps ``.grad`` as it was, as if it had not been trained.  At most
+    ``POPULATION_MAX`` members per call are launched together; larger populations are cut into such calls."""
+    models, batches = list(models), list(batches)
+    if len(models) != len(batches):
+        raise ValueError("forward_train_population: %d models and %d batches" % (len(models), len(batches)))
+    if not models:
+        return []
+    m0 = models[0]
+    devs = [next(m.parameters()).device for m in models]
+    for i, m in enumerate(models):
+        if m.dropout > 0:
+            raise NotImplementedError("forward_train: dropout=%g, the fused training path has no dropout" % m.dropout)
+        for f in _MEMBER_FIELDS:
+            if getattr(m, f) != getattr(m0, f):
+                raise ValueError("forward_train_population: member %d has %s=%r, member 0 has %r"
+                                 % (i, f, getattr(m, f), getattr(m0, f)))
+        if devs[i] != devs[0]:
+            raise ValueError("forward_train_population: member %d is on %s, member 0 on %s" % (i, devs[i], devs[0]))
+    dev = kernels._dev()
+    if devs[0] != dev:
+        for m in models:
+            m.to(dev)
+    ins = [_train_inputs(x, dev) for x in batches]
+    for i, x in enumerate(ins):
+        if x[5:7] != ins[0][5:7]:
+            raise ValueError("forward_train_population: batch %d has B, T = %d, %d, batch 0 has %d, %d"
+                             % (i, x[5], x[6], ins[0][5], ins[0][6]))
+    if len({x[7] for x in ins}) > 1:   # one context row stride per call
+        for x in ins:
+            x[1:5] = [t.contiguous() for t in x[1:5]]
+            x[7] = x[6]
+    out = []
+    for a in range(0, len(models), POPULATION_MAX):
+        ms = models[a:a + POPULATION_MAX]
+        params = [p for m in ms for p in m._train_params()]
+        out += list(_PopulationTrainFn.apply(ms, ins[a:a + POPULATION_MAX], *params))
+    return out
+
+
+POPULATION_MAX = 32   # DPT_GPT2_POPULATION_MAX: members per population launch
+
+
+class _PopulationTrainFn(torch.autograd.Function):
+    """dpt_gpt2_train_population_forward / _backward over k members (k = 1: the one-model path).  One workspace holds
+    every member's saved activations between the two."""
 
     @staticmethod
-    def forward(ctx, model, inputs, *params):
-        q, cs, ca, cns, cr, B, T, stride = inputs
-        dev = q.device
+    def forward(ctx, models, inputs, *params):
+        ctx.set_materialize_grads(False)
+        k, m0 = len(models), models[0]
+        B, T, stride = inputs[0][5:8]
+        dev = inputs[0][0].device
+        n = len(params) // k
         keep = []
-        w = _weights_struct(model, params, keep)
-        out = torch.empty((B, model.action_dim) if model.test else (B, T, model.action_dim), dtype=torch.float32, device=dev)
-        nbytes = lib().dpt_gpt2_train_workspace_bytes(ctypes.byref(w), B, T)
+        w = (_lib.Gpt2Weights * k)(*[_weights_struct(m, params[i * n:(i + 1) * n], keep) for i, m in enumerate(models)])
+        outs = [torch.empty((B, m0.action_dim) if m0.test else (B, T, m0.action_dim), dtype=torch.float32, device=dev)
+                for _ in range(k)]
+        nbytes = lib().dpt_gpt2_train_population_workspace_bytes(w, k, B, T)
         ws = torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=dev)
-        check(lib().dpt_gpt2_train_forward(ctypes.byref(w), q.data_ptr(), cs.data_ptr() if T else None, ca.data_ptr() if T else None,
-                                           cns.data_ptr() if T else None, cr.data_ptr() if T else None, B, T, stride,
-                                           1 if model.test else 0, out.data_ptr(), ws.data_ptr(), ws.numel(), stream_ptr()),
-              "dpt_gpt2_train_forward")
-        ctx.model, ctx.ws, ctx.B, ctx.T, ctx.test = model, ws, B, T, model.test
+        arr = lambda ts: (ctypes.c_void_p * k)(*[t.data_ptr() if T else None for t in ts])   # noqa: E731
+        qs = (ctypes.c_void_p * k)(*[x[0].data_ptr() for x in inputs])
+        check(lib().dpt_gpt2_train_population_forward(w, k, qs, *[arr([x[j] for x in inputs]) for j in range(1, 5)], B, T, stride,
+                                                      1 if m0.test else 0, (ctypes.c_void_p * k)(*[o.data_ptr() for o in outs]),
+                                                      ws.data_ptr(), ws.numel(), stream_ptr()),
+              "dpt_gpt2_train_forward" if k == 1 else "dpt_gpt2_train_population_forward")
+        ctx.models, ctx.ws, ctx.B, ctx.T, ctx.test, ctx.out_shape = models, ws, B, T, m0.test, outs[0].shape
         ctx.save_for_backward(*params)
-        return out
+        return tuple(outs)
 
     @staticmethod
     @torch.autograd.function.once_differentiable
-    def backward(ctx, dout):
+    def backward(ctx, *douts):
         params = ctx.saved_tensors
-        grads = [torch.empty_like(p) for p in params]
+        models, k = ctx.models, len(ctx.models)
+        n = len(params) // k
+        dev = params[0].device
+        grads = []
+        for i in range(k):   # one buffer per member, a view per parameter
+            ps = params[i * n:(i + 1) * n]
+            flat = torch.empty(sum(p.numel() for p in ps), dtype=torch.float32, device=dev)
+            o = 0
+            for p in ps:
+                grads.append(flat[o:o + p.numel()].view_as(p))
+                o += p.numel()
         if ctx.B == 0:
             for g in grads:
                 g.zero_()
-            return (None, None, *grads)
-        keep = []
-        w = _weights_struct(ctx.model, params, keep)
-        g = _pointer_struct(_lib.Gpt2Grads, ctx.model, grads, keep)
-        dout = dout.to(torch.float32).contiguous()
-        check(lib().dpt_gpt2_train_backward(ctypes.byref(w), dout.data_ptr(), ctx.B, ctx.T, 1 if ctx.test else 0, ctypes.byref(g),
-                                            ctx.ws.data_ptr(), ctx.ws.numel(), stream_ptr()), "dpt_gpt2_train_backward")
+        else:
+            keep = []
+            w = (_lib.Gpt2Weights * k)(*[_weights_struct(m, params[i * n:(i + 1) * n], keep) for i, m in enumerate(models)])
+            gs = (_lib.Gpt2Grads * k)(*[_pointer_struct(_lib.Gpt2Grads, m, grads[i * n:(i + 1) * n], keep)
+                                        for i, m in enumerate(models)])
+            # a member whose logits got no gradient runs on a zero dout; its gradients are dropped below
+            ds = [torch.zeros(ctx.out_shape, dtype=torch.float32, device=dev) if d is None else d.to(torch.float32).contiguous()
+                  for d in douts]
+            check(lib().dpt_gpt2_train_population_backward(w, k, (ctypes.c_void_p * k)(*[d.data_ptr() for d in ds]), ctx.B,
+                                                           ctx.T, 1 if ctx.test else 0, gs, ctx.ws.data_ptr(), ctx.ws.numel(),
+                                                           stream_ptr()),
+                  "dpt_gpt2_train_backward" if k == 1 else "dpt_gpt2_train_population_backward")
         ctx.ws = None
-        return (None, None, *grads)
+        return (None, None, *[None if douts[i // n] is None else g for i, g in enumerate(grads)])
 
 
 class _Decoder:

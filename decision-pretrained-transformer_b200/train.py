@@ -5,6 +5,7 @@
 weight_decay)``, batch 64, and the sum-reduced cross-entropy of the logits of every context row against the
 optimal action.  Both epoch losses are reported as the reference reports them: sum of the batch losses / horizon /
 len(dataset).  The forward of training is ``model.forward_train`` (hand-written CUDA forward and backward).
+``train_population`` trains k same-shape models at once, each bit-identical to ``train`` on it alone.
 
 Unlike the reference's DataLoader, batches are gathered on the device from ``Dataset.dataset`` with a seeded
 permutation (and, with ``Dataset.shuffle``, a seeded per-item context permutation), and the losses stay on the
@@ -64,30 +65,137 @@ def batches(dataset, batch_size, generator, shuffle_items=None):
 def train(model, train_dataset, test_dataset, num_epochs, batch_size=64, lr=1e-3, weight_decay=1e-4, seed=None,
           optimizer=None):
     """The reference's epoch loop.  Returns ``(train_loss, test_loss, optimizer)``: per-epoch lists of floats and the
-    AdamW optimizer (its ``state_dict`` is the reference's)."""
-    dev = train_dataset.dataset["context_actions"].device
-    if next(model.parameters()).device != dev:
-        model.to(dev)
-    if optimizer is None:
-        optimizer = torch.optim.AdamW(model.parameters(), lr=lr, weight_decay=weight_decay)
-    gen = torch.Generator(device=dev)
-    if seed is None:
-        gen.seed()
+    AdamW optimizer (its ``state_dict`` is the reference's).  This is the one-member case of ``train_population``."""
+    tr, te, optimizer = train_population([model], train_dataset, test_dataset, num_epochs, batch_size, lr, weight_decay,
+                                         [seed], optimizer)
+    return tr[0], te[0], optimizer
+
+
+def train_population_step(models, optimizer, batches, loss_fn=ce_sum_loss):
+    """One optimizer step of every member: ``forward_train_population``, the loss of each member on its own batch, one
+    backward and ``optimizer.step()``.  Member i's gradient is the one ``train_step(models[i], ..., batches[i])`` computes,
+    bit for bit.  With the default loss the cross-entropy runs once on the stacked logits (per-row reduction, then a sum
+    per member), so a member's loss value can differ from ``train_step``'s in the last bits (within 1e-6 relative); with
+    one member, or another ``loss_fn``, each member's loss is ``loss_fn(pred, batch)`` as in ``train_step``.  Returns the
+    losses as one device tensor [k] (no host synchronisation)."""
+    from .models.net import forward_train_population
+    optimizer.zero_grad()
+    preds = forward_train_population(models, batches)
+    if loss_fn is ce_sum_loss and len(preds) > 1:
+        pred = torch.stack(preds)
+        du, k = pred.shape[-1], pred.shape[0]
+        target = torch.stack([b["optimal_actions"] for b in batches])
+        if pred.dim() == 4:
+            target = target.unsqueeze(2).expand(-1, -1, pred.shape[2], -1)
+        losses = F.cross_entropy(pred.reshape(-1, du), target.reshape(-1, du), reduction="none").view(k, -1).sum(1)
     else:
-        gen.manual_seed(seed)
-    horizon = model.horizon
-    train_loss, test_loss = [], []
+        losses = torch.stack([loss_fn(p, b) for p, b in zip(preds, batches)])
+    losses.sum().backward()
+    optimizer.step()
+    return losses.detach()
+
+
+def _per_member(v, k, name):
+    v = list(v) if isinstance(v, (list, tuple)) else [v] * k
+    if len(v) != k:
+        raise ValueError("train_population: %d values of %s for %d models" % (len(v), name, k))
+    return v
+
+
+def _population_batches(datasets, batch_size, gens):
+    """``batches(datasets[i], batch_size, gens[i])`` of every member, step by step: yields a list of k batch dicts.  Each
+    member draws from its own generator in the order ``batches`` does, so its batches are the ones ``train`` gathers.
+    Members that share a dataset are gathered with one index per key (and one context permutation gather)."""
+    k = len(datasets)
+    groups = {}
+    for i, d in enumerate(datasets):
+        groups.setdefault(id(d), []).append(i)
+    data0 = datasets[0].dataset
+    n = data0["context_actions"].shape[0]
+    dev = data0["context_actions"].device
+    orders = [torch.randperm(n, generator=g, device=g.device).to(dev) for g in gens]
+    for a in range(0, n, batch_size):
+        out = [None] * k
+        for members in groups.values():
+            ds = datasets[members[0]]
+            data = ds.dataset
+            idx = [orders[i][a:a + batch_size] for i in members]
+            nb = idx[0].shape[0]
+            cat = torch.cat(idx) if len(idx) > 1 else idx[0]
+            b = {key: data[key][cat] for key in _KEYS}
+            if ds.shuffle:
+                H = b["context_actions"].shape[1]
+                perm = [torch.argsort(torch.rand((nb, H), generator=gens[i], device=gens[i].device).to(dev), dim=1) for i in members]
+                perm = torch.cat(perm) if len(perm) > 1 else perm[0]
+                for key in _CTX:
+                    b[key] = torch.gather(b[key], 1, perm.unsqueeze(-1).expand(-1, -1, b[key].shape[-1]))
+            for j, i in enumerate(members):
+                out[i] = {key: v[j * nb:(j + 1) * nb] for key, v in b.items()} if len(members) > 1 else b
+        yield out
+
+
+def train_population(models, train_datasets, test_datasets, num_epochs, batch_size=64, lr=1e-3, weight_decay=1e-4, seeds=None,
+                     optimizer=None):
+    """``train`` of k same-shape models at once (``forward_train_population``): the members' forward and backward run in
+    the same kernel launches, their batches are gathered together and their AdamW updates go through one optimizer.
+
+    ``train_datasets`` / ``test_datasets``: one ``Dataset`` shared by every member or a list of k; all datasets of one
+    split have the same length, so that the members' steps line up.  ``lr``, ``weight_decay`` and ``seeds``: a scalar or
+    a list of k.  The default optimizer is one ``torch.optim.AdamW`` with a parameter group per distinct (lr,
+    weight_decay); AdamW's update is elementwise, so the grouping does not change any weight.
+
+    Member i ends bit-identical to ``train(models[i], train_i, test_i, num_epochs, batch_size, lr_i, weight_decay_i,
+    seed=seeds[i])``: the same weights and the same AdamW state of its parameters.  Its test losses are bit for bit
+    ``train``'s (the same per-member computation); its train losses are summed from the stacked cross-entropy of
+    ``train_population_step`` and match ``train``'s within 1e-6 relative (bit for bit when k = 1).  Returns
+    ``(train_loss, test_loss, optimizer)``: ``train_loss[i][e]`` and ``test_loss[i][e]`` are floats."""
+    models = list(models)
+    k = len(models)
+    if k == 0:
+        return [], [], optimizer
+    trs, tes = _per_member(train_datasets, k, "train_datasets"), _per_member(test_datasets, k, "test_datasets")
+    lrs, wds = _per_member(lr, k, "lr"), _per_member(weight_decay, k, "weight_decay")
+    seeds = _per_member(seeds, k, "seeds")
+    for split, ds in (("train", trs), ("test", tes)):
+        for i, d in enumerate(ds):
+            if len(d) != len(ds[0]):
+                raise ValueError("train_population: %s dataset of member %d has %d items, member 0's has %d"
+                                 % (split, i, len(d), len(ds[0])))
+    dev = trs[0].dataset["context_actions"].device
+    for m in models:
+        if next(m.parameters()).device != dev:
+            m.to(dev)
+    if optimizer is None:
+        groups = {}
+        for m, a, b in zip(models, lrs, wds):
+            groups.setdefault((a, b), []).extend(m.parameters())
+        optimizer = torch.optim.AdamW([{"params": ps, "lr": a, "weight_decay": b} for (a, b), ps in groups.items()])
+    gens = []
+    for s in seeds:
+        g = torch.Generator(device=dev)
+        if s is None:
+            g.seed()
+        else:
+            g.manual_seed(s)
+        gens.append(g)
+    horizon = models[0].horizon
+    train_loss, test_loss = [[] for _ in range(k)], [[] for _ in range(k)]
     for _ in range(num_epochs):
         with torch.no_grad():
-            te = torch.zeros((), dtype=torch.float32, device=dev)
-            for b in batches(test_dataset, batch_size, gen):
-                te += ce_sum_loss(model(b), b)
-        tr = torch.zeros((), dtype=torch.float32, device=dev)
-        for b in batches(train_dataset, batch_size, gen):
-            tr += train_step(model, optimizer, b)
-        losses = torch.stack([te / horizon / len(test_dataset), tr / horizon / len(train_dataset)]).tolist()   # one host read
-        test_loss.append(losses[0])
-        train_loss.append(losses[1])
+            te = [torch.zeros((), dtype=torch.float32, device=dev) for _ in range(k)]
+            for bs in _population_batches(tes, batch_size, gens):
+                for i, (m, b) in enumerate(zip(models, bs)):
+                    te[i] += ce_sum_loss(m(b), b)
+        tr = torch.zeros((k,), dtype=torch.float32, device=dev)
+        for bs in _population_batches(trs, batch_size, gens):
+            if k == 1:
+                tr[0] += train_step(models[0], optimizer, bs[0])
+            else:
+                tr += train_population_step(models, optimizer, bs)
+        losses = torch.stack([torch.stack(te) / horizon / len(tes[0]), tr / horizon / len(trs[0])]).tolist()   # one host read
+        for i in range(k):
+            test_loss[i].append(losses[0][i])
+            train_loss[i].append(losses[1][i])
     return train_loss, test_loss, optimizer
 
 

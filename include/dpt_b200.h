@@ -35,7 +35,7 @@ extern "C" {
 #define DPT_ERR_CUDA (-2)
 #define DPT_ERR_UNSUPPORTED (-3)
 
-#define DPT_ABI_VERSION 6
+#define DPT_ABI_VERSION 7
 
 /* reward_type of the bandit entry points (envs/bandit_env.py:56-63, envs/gpu_bandit_env.py:53-63):
  * 0 'uniform'  : r = means[a] + var * z, z ~ N(0,1);
@@ -379,6 +379,28 @@ int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, const float* query_state
                            int T_stride, int test, float* out, void* workspace, uint64_t workspace_bytes, void* stream);
 int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float* dout, int B, int T, int test,
                             const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream);
+
+/* Population training: n_models same-shape models (members share n_layer, state_dim, action_dim and n_positions) trained
+ * in the same launches, each exactly as dpt_gpt2_train_forward / dpt_gpt2_train_backward would train it alone: member i's
+ * logits and gradients are bit-identical to the one-model calls on its own weights, inputs and dout (same row chunking,
+ * same fixed-order sums).  w and grads are arrays of n_models structs; query_states, ctx_*, out and dout are HOST arrays
+ * of n_models DEVICE pointers, with the shapes of the one-model calls; B, T, T_stride and test are shared.  The workspace
+ * holds one member region after another: dpt_gpt2_train_population_workspace_bytes(w, n_models, B, T) =
+ * n_models * dpt_gpt2_train_workspace_bytes(w, B, T) bytes, 16 B aligned, the same buffer for both calls.  The per-member
+ * tables travel in the kernel parameters: no host synchronisation, no upload, capturable in a CUDA graph.
+ * 1 <= n_models <= DPT_GPT2_POPULATION_MAX per call; n_models = 0 or B = 0 is a no-op.  n_models < 0 or above the limit,
+ * null pointers and a member of another shape (the message names the member and the field) return DPT_ERR_INVALID_ARG;
+ * n_embd != 32, n_layer > 8 and T + 1 > 512 return DPT_ERR_UNSUPPORTED. */
+#define DPT_GPT2_POPULATION_MAX 32
+uint64_t dpt_gpt2_train_population_workspace_bytes(const dpt_gpt2_weights_t* w, int n_models, int B, int T);
+int dpt_gpt2_train_population_forward(const dpt_gpt2_weights_t* w, int n_models, const float* const* query_states,
+                                      const float* const* ctx_states, const float* const* ctx_actions,
+                                      const float* const* ctx_next_states, const float* const* ctx_rewards, int B, int T,
+                                      int T_stride, int test, float* const* out, void* workspace, uint64_t workspace_bytes,
+                                      void* stream);
+int dpt_gpt2_train_population_backward(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B, int T,
+                                       int test, const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes,
+                                       void* stream);
 
 /* Ordered multi-source sum (the gradient exchange of the data-parallel interactive trainer, train_interactive.py:97-139;
  * the reference is single-GPU): dst[i] = (((src[0][i] + src[1][i]) + ...) + src[M-1][i]) for i < n, fp32, added in

@@ -100,7 +100,7 @@ def kernel_split(fwd, opt, b, steps=5):
             TR.ce_sum_loss(fwd(b), b).backward()
             opt.step()
         torch.cuda.synchronize()
-    groups = {"forward": ["gpt2_dense_fp32_kernel"], "backward": ["gpt2_train_backward_kernel"],
+    groups = {"forward": ["gpt2_train_forward_kernel"], "backward": ["gpt2_train_backward_kernel"],
               "reduction": ["weight_grad_partial_kernel", "weight_grad_reduce_kernel", "wpe_grad_kernel"]}
     out = {k: 0.0 for k in list(groups) + ["other"]}
     for e in prof.key_averages():
