@@ -9,14 +9,22 @@ len(dataset).  The forward of training is ``model.forward_train`` (hand-written 
 
 Unlike the reference's DataLoader, batches are gathered on the device from ``Dataset.dataset`` with a seeded
 permutation (and, with ``Dataset.shuffle``, a seeded per-item context permutation), and the losses stay on the
-device until one host read per epoch.  There is no argparse, plotting or checkpoint naming.
+device until one host read per epoch.  There is no argparse or plotting.
+
+Every trainer can write a training-state file at epoch (iteration) boundaries and resume from it (``state_path``,
+``save_every``, ``resume``); a resumed run ends bit-identical to the run that was never interrupted (``checkpoint``).
+``train`` and ``train_population`` also write the reference's weight files (``weights_dir``, ``stems``).
 
 ``train_interactive`` is the on-policy trainer of the reference's train_interactive.py (:97-139): every iteration rolls
 out a fresh ``GPUBanditEnv`` with the current model and takes one AdamW step on the cross-entropy of the last logits
 against the optimal arm.  ``dist.train_interactive_sharded`` runs the same code over a box's GPUs.
 """
+import os
+
 import torch
 import torch.nn.functional as F
+
+from . import checkpoint as C
 
 _CTX = ("context_states", "context_actions", "context_next_states", "context_rewards")
 _KEYS = _CTX + ("query_states", "optimal_actions")
@@ -63,11 +71,13 @@ def batches(dataset, batch_size, generator, shuffle_items=None):
 
 
 def train(model, train_dataset, test_dataset, num_epochs, batch_size=64, lr=1e-3, weight_decay=1e-4, seed=None,
-          optimizer=None):
+          optimizer=None, *, state_path=None, save_every=50, resume=False, weights_dir=None, stems=None):
     """The reference's epoch loop.  Returns ``(train_loss, test_loss, optimizer)``: per-epoch lists of floats and the
-    AdamW optimizer (its ``state_dict`` is the reference's).  This is the one-member case of ``train_population``."""
-    tr, te, optimizer = train_population([model], train_dataset, test_dataset, num_epochs, batch_size, lr, weight_decay,
-                                         [seed], optimizer)
+    AdamW optimizer (its ``state_dict`` is the reference's).  This is the one-member case of ``train_population``, whose
+    docstring describes the checkpoint arguments; ``stems`` is one stem here."""
+    tr, te, optimizer = _population("train", [model], train_dataset, test_dataset, num_epochs, batch_size, lr, weight_decay,
+                                    [seed], optimizer, state_path, save_every, resume, weights_dir,
+                                    None if stems is None else [stems])
     return tr[0], te[0], optimizer
 
 
@@ -135,7 +145,7 @@ def _population_batches(datasets, batch_size, gens):
 
 
 def train_population(models, train_datasets, test_datasets, num_epochs, batch_size=64, lr=1e-3, weight_decay=1e-4, seeds=None,
-                     optimizer=None):
+                     optimizer=None, *, state_path=None, save_every=50, resume=False, weights_dir=None, stems=None):
     """``train`` of k same-shape models at once (``forward_train_population``): the members' forward and backward run in
     the same kernel launches, their batches are gathered together and their AdamW updates go through one optimizer.
 
@@ -148,7 +158,27 @@ def train_population(models, train_datasets, test_datasets, num_epochs, batch_si
     seed=seeds[i])``: the same weights and the same AdamW state of its parameters.  Its test losses are bit for bit
     ``train``'s (the same per-member computation); its train losses are summed from the stacked cross-entropy of
     ``train_population_step`` and match ``train``'s within 1e-6 relative (bit for bit when k = 1).  Returns
-    ``(train_loss, test_loss, optimizer)``: ``train_loss[i][e]`` and ``test_loss[i][e]`` are floats."""
+    ``(train_loss, test_loss, optimizer)``: ``train_loss[i][e]`` and ``test_loss[i][e]`` are floats.
+
+    Checkpoints (all off by default):
+
+    - ``state_path``: the training state (``checkpoint``) is written there after every epoch e with
+      ``(e + 1) % save_every == 0`` and after the last epoch (``save_every=10`` is the reference's linear-bandit cadence).
+    - ``resume=True``: if ``state_path`` exists, the models, the optimizer (built as without it, then
+      ``load_state_dict``) and the batch generators are restored from it and training continues at its next epoch;
+      otherwise training starts from scratch.  ``num_epochs`` stays the total, and the loss lists returned are the full
+      ones.  The result is bit-identical to the call that was never interrupted.  A state that does not match the call
+      (model configs, member count, ``batch_size``, lr, weight_decay, seeds, dataset lengths, shuffle flags and sharing,
+      optimizer groups) raises ``ValueError`` before anything is modified.
+    - ``weights_dir`` with ``stems`` (k distinct stems, e.g. from ``utils.build_bandit_model_filename``): member i's
+      ``state_dict`` goes to ``{weights_dir}/{stems[i]}_epoch{e + 1}.pt`` at the same epochs and to
+      ``{weights_dir}/{stems[i]}.pt`` at the end (``checkpoint.save_weights``), as the reference's train.py writes them."""
+    return _population("population", models, train_datasets, test_datasets, num_epochs, batch_size, lr, weight_decay, seeds,
+                       optimizer, state_path, save_every, resume, weights_dir, stems)
+
+
+def _population(kind, models, train_datasets, test_datasets, num_epochs, batch_size, lr, weight_decay, seeds, optimizer,
+                state_path, save_every, resume, weights_dir, stems):
     models = list(models)
     k = len(models)
     if k == 0:
@@ -156,6 +186,11 @@ def train_population(models, train_datasets, test_datasets, num_epochs, batch_si
     trs, tes = _per_member(train_datasets, k, "train_datasets"), _per_member(test_datasets, k, "test_datasets")
     lrs, wds = _per_member(lr, k, "lr"), _per_member(weight_decay, k, "weight_decay")
     seeds = _per_member(seeds, k, "seeds")
+    _check_saving(state_path, save_every, resume)
+    if weights_dir is not None:
+        stems = _per_member(stems, k, "stems")
+        if None in stems or len(set(stems)) != k:
+            raise ValueError("train_population: weights_dir needs %d distinct stems, got %r" % (k, stems))
     for split, ds in (("train", trs), ("test", tes)):
         for i, d in enumerate(ds):
             if len(d) != len(ds[0]):
@@ -180,7 +215,12 @@ def train_population(models, train_datasets, test_datasets, num_epochs, batch_si
         gens.append(g)
     horizon = models[0].horizon
     train_loss, test_loss = [[] for _ in range(k)], [[] for _ in range(k)]
-    for _ in range(num_epochs):
+    args = C.train_args(batch_size, lrs, wds, seeds, trs, tes, dev)
+    e0 = 0
+    if resume and os.path.exists(state_path):
+        e0, hist = C.load_state(state_path, kind, models, optimizer, args, num_epochs, gens)
+        train_loss, test_loss = hist["train_loss"], hist["test_loss"]
+    for e in range(e0, num_epochs):
         with torch.no_grad():
             te = [torch.zeros((), dtype=torch.float32, device=dev) for _ in range(k)]
             for bs in _population_batches(tes, batch_size, gens):
@@ -196,7 +236,25 @@ def train_population(models, train_datasets, test_datasets, num_epochs, batch_si
         for i in range(k):
             test_loss[i].append(losses[0][i])
             train_loss[i].append(losses[1][i])
+        # weight files first: a state written after them means they are on disk, and a resume rewrites them otherwise
+        if weights_dir is not None and (e + 1) % save_every == 0:
+            for m, stem in zip(models, stems):
+                C.save_weights(m, weights_dir, stem, e + 1)
+        if state_path is not None and ((e + 1) % save_every == 0 or e + 1 == num_epochs):
+            C.save_state(state_path, C.training_state(kind, models, optimizer, args, e + 1,
+                                                      {"train_loss": train_loss, "test_loss": test_loss}, gens))
+    if weights_dir is not None:
+        for m, stem in zip(models, stems):
+            C.save_weights(m, weights_dir, stem)
     return train_loss, test_loss, optimizer
+
+
+def _check_saving(state_path, save_every, resume):
+    if save_every < 1:
+        raise ValueError("save_every=%r, it must be >= 1" % (save_every,))
+    if resume and state_path is None:
+        raise ValueError("resume=True needs a state_path")
+
 
 
 def interactive_loss(last_logits, target, n_envs):
@@ -207,7 +265,7 @@ def interactive_loss(last_logits, target, n_envs):
 
 
 def train_interactive(model, dim, n_envs, K, n_iters, mb=1024, var=0.0, env_type="uniform", seed=0, lr=1e-3,
-                      weight_decay=1e-4, optimizer=None, timings=None):
+                      weight_decay=1e-4, optimizer=None, timings=None, *, state_path=None, save_every=50, resume=False):
     """On-policy training (train_interactive.py:97-139) on one GPU.  Iteration ``it``:
 
     1. ``env = GPUBanditEnv(dim, n_envs, K, var, env_type, seed=rng.key_for(seed, it))``;
@@ -224,9 +282,16 @@ def train_interactive(model, dim, n_envs, K, n_iters, mb=1024, var=0.0, env_type
     only on ``mb``.  fp32 training, ``dropout == 0`` and K <= 512 (the limits of ``forward_train``).  ``n_envs == 0`` runs
     nothing.  ``timings``: a list that receives, per iteration, the CUDA-event milliseconds of the rollout, the forward and
     backward of all micro-batches, the exchange (host barrier to the end of the sum), the optimizer and the whole iteration.
-    Returns ``(losses, optimizer)``: the per-iteration losses (one host read at the end) and the optimizer."""
+    Returns ``(losses, optimizer)``: the per-iteration losses (one host read at the end) and the optimizer.
+
+    ``state_path``, ``save_every`` and ``resume`` work as in ``train_population``, per iteration: the state is written
+    after every iteration it with ``(it + 1) % save_every == 0`` and after the last one, and a resumed call continues at
+    the saved iteration with its keys ``rng.key_for(seed, it)``; ``n_iters`` stays the total.  The arguments a resume must
+    repeat are ``dim``, ``n_envs``, ``K``, ``mb``, ``var``, ``env_type``, ``seed``, ``lr`` and ``weight_decay``, not the
+    world size: a state saved by ``dist.train_interactive_sharded`` at one world size resumes at any other."""
     return _interactive(model, dim, n_envs, K, n_iters, mb, 0, 1, var=var, env_type=env_type, seed=seed, lr=lr,
-                        weight_decay=weight_decay, optimizer=optimizer, timings=timings)
+                        weight_decay=weight_decay, optimizer=optimizer, timings=timings, state_path=state_path,
+                        save_every=save_every, resume=resume)
 
 
 def _agree(err, ws):
@@ -244,7 +309,7 @@ def _agree(err, ws):
 
 
 def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type="uniform", seed=0, lr=1e-3,
-                 weight_decay=1e-4, optimizer=None, timings=None):
+                 weight_decay=1e-4, optimizer=None, timings=None, state_path=None, save_every=50, resume=False):
     """train_interactive on rank ``rank`` of ``ws`` (ws == 1: the one-GPU trainer; see dist.train_interactive_sharded)."""
     import ctypes
     from . import _lib, dist as D, kernels, rng
@@ -255,6 +320,7 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
         raise NotImplementedError("train_interactive: dropout=%g, the fused training path has no dropout" % model.dropout)
     if K < 1:
         raise ValueError("train_interactive: K=%d, the rollout needs at least one step" % K)
+    _check_saving(state_path, save_every, resume)
     dev = kernels._dev()
     if next(model.parameters()).device != dev:
         model.to(dev)
@@ -273,6 +339,17 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
     # the train kernels' shape checks (n_embd, n_layer, sequence length) before any rollout: a B = 0 call only validates
     check(lib().dpt_gpt2_train_forward(ctypes.byref(net._weights_struct(model, params, [])), None, None, None, None, None, 0,
                                        T, K, 1, None, None, 0, st), "dpt_gpt2_train_forward")
+    args = C.interactive_args(dim, n_envs, K, mb, var, env_type, seed, lr, weight_decay)
+    it0, done = 0, []
+    if resume:   # every rank reads the same file; all raise if one fails to
+        err = None
+        try:
+            if os.path.exists(state_path):
+                it0, hist = C.load_state(state_path, "interactive", [model], optimizer, args, n_iters)
+                done = hist["losses"]
+        except Exception as e:   # noqa: BLE001
+            err = e
+        _agree(err, ws)
     n_local, n_mb = hi - lo, m_hi - m_lo
     peer = D.PeerBuffer(max(n_mb, 1) * Ps * 4, (rank, ws))
     try:
@@ -285,12 +362,13 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
         for p, o, n in zip(params, offs, sizes):
             p.grad = flat[o:o + n].view_as(p)
         losses = torch.zeros(n_iters, dtype=torch.float32, device=dev)
+        losses[:it0] = torch.tensor(done, dtype=torch.float32)
         if n_local:
             q = torch.ones((min(mb, n_local), model.state_dim), dtype=torch.float32, device=dev)
             wbytes = int(lib().dpt_gpt2_train_workspace_bytes(ctypes.byref(net._weights_struct(model, params, [])),
                                                                min(mb, n_local), T))
             work = torch.empty((max(wbytes, 16),), dtype=torch.uint8, device=dev)
-        for it in range(n_iters):
+        for it in range(it0, n_iters):
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)] if timings is not None else []
             mark = lambda i: ev and ev[i].record()   # noqa: E731
             err = None
@@ -332,6 +410,10 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
                 optimizer.step()
                 mark(4)
                 torch.cuda.current_stream().synchronize()
+                # every rank holds the same weights and AdamW state; a failed write makes every rank raise
+                if state_path is not None and rank == 0 and ((it + 1) % save_every == 0 or it + 1 == n_iters):
+                    C.save_state(state_path, C.training_state("interactive", [model], optimizer, args, it + 1,
+                                                              {"losses": losses[:it + 1].tolist()}))
             except Exception as e:   # noqa: BLE001
                 err = e
             _agree(err, ws)                                 # no rank rewrites its slots before every rank has summed them
