@@ -15,7 +15,10 @@
 // Layout: K and V are both [layer][t][channel] (128 B rows, appended coalesced).  Attention maps a
 // lane to (key group lane/8, channel quad lane%8): one LDG.128 instruction covers 4 keys x 32 channels,
 // 8 are kept in flight per lane (32 keys), the 8-lane dot products are combined by a 7-shuffle
-// butterfly transpose-reduce, softmax is a warp reduction, and PV accumulates float4 channel quads.  K/V reads bypass L1 (ld.global.cg) so L1 keeps the ~200 KB of weights that
+// butterfly transpose-reduce, softmax is a warp reduction, and PV accumulates float4 channel quads.  The
+// fp32 attention (attention_f32) is one body for both stagings of the K/V tiles: register-staged global
+// loads (GlobalKv) or bulk-async copies through a per-warp shared-memory ring (KvRing, small batches of
+// the online loop).  K/V reads bypass L1 (ld.global.cg) so L1 keeps the ~200 KB of weights that
 // every warp re-reads; weights are read through the read-only path.  fp32 everywhere, accurate
 // expf/tanhf/sqrtf (the 1e-5 logit parity bar excludes TF32 and .approx forms).
 // Bound: K/V bytes read per token-forward = n_layer * 2 * t * 32 * 4 (HBM once the in-flight caches
@@ -88,8 +91,6 @@ __device__ __forceinline__ float gelu_new(float x) {  // transformers NewGELUAct
   return 0.5f * x * (1.0f + tanhf(0.7978845608028654f * (x + 0.044715f * x * x * x)));
 }
 
-// One token through all layers.  x: this lane's channel of the embedded token (+wpe).  kv: this
-// sequence's cache, [L][2][32][Tpad] floats.  sx[32], sh[128], ssc[Tpad]: per-warp shared scratch.
 constexpr int PF_AHEAD = 3;      // K/V L2 prefetch distance in 32-key iterations (fp32 cache: 4 KB each)
 constexpr int PF_MAX_POS = 192;  // only short (latency-bound) sequences prefetch: +20 % at H=100, -2 % at H=500 without the cap
 
@@ -151,10 +152,233 @@ __global__ void pack_wfrag_kernel(const float* __restrict__ W, uint4* __restrict
 constexpr int GPT2_MINB_F32 = 9;   // 56 registers: 221 ms at C4 against 241 ms (8) / 226 ms (7) / 270 ms (10)
 constexpr int GPT2_MINB_BF16 = 6;
 
-// WS: the projections run on the tensor cores from bf16 weight fragments in shared memory (`wf`, all layers)
-template <bool BF16, bool WS = false>
+// Bytes of one sequence's K/V cache: [L][K, V][Tpad][32 channels], fp32 or bf16 (precision 1)
+__host__ __device__ __forceinline__ size_t kv_seq_bytes(int L, int Tpad, bool bf16) {
+  return (size_t)L * 2 * G_E * Tpad * (bf16 ? 2 : 4);
+}
+
+// Keys 0..pos-1 in tiles of TILE: f(k0, std::false_type) for every full tile, then f(k0, std::true_type) for the last,
+// partial one if there is one.  MASK_ALL: every tile takes the masked (std::true_type) form -- one copy of the tile code
+template <int TILE, bool MASK_ALL = false, class F>
+__device__ __forceinline__ void for_each_key_tile(int pos, F&& f) {
+  if constexpr (MASK_ALL) {
+    for (int k0 = 0; k0 < pos; k0 += TILE) f(k0, std::true_type{});
+  } else {
+    int k0 = 0;
+    for (; k0 + TILE <= pos; k0 += TILE) f(k0, std::false_type{});
+    if (k0 < pos) f(k0, std::true_type{});
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Sources of the fp32 attention's 32-key K / V tiles.  tile(X, k0, pos, lane) returns this lane's channel quad of the
+// tile (X = the layer's K or V cache), load(t, k0, r) reads row r of it (row stride = 8 float4), consumed(lane) follows
+// the last read of a tile, begin_token / end_token bracket each token.
+// ---------------------------------------------------------------------------------------------
+// Register-staged: ld.global.cg straight from the cache, 8 rows in flight per lane; short sequences prefetch to L2 ahead.
+struct GlobalKv {
+  static constexpr bool MASK_ALL = false;
+  __device__ __forceinline__ void begin_token(int, int) {}
+  __device__ __forceinline__ void end_token() {}
+  __device__ __forceinline__ const float4* tile(const float* X, int k0, int pos, int lane) {
+    if (pos <= PF_MAX_POS && k0 + PF_AHEAD * 32 < pos) prefetch_l2(X + (size_t)(k0 + PF_AHEAD * 32 + lane) * G_E);
+    return reinterpret_cast<const float4*>(X) + (lane & 7);
+  }
+  __device__ __forceinline__ float4 load(const float4* t, int k0, int r) const { return __ldcg(t + (size_t)(k0 + r) * 8); }
+  __device__ __forceinline__ void consumed(int) {}
+};
+
+// Bulk-async (TMA engine) staging: cp.async.bulk global -> shared, completion on an mbarrier.  A warp's cached keys of one
+// layer are ONE contiguous run per tensor ([t][32 channels] fp32, 128 B rows), so a tile of 32 keys is a single <= 4 KB
+// bulk copy of exactly the live rows (no padded rows are read).  Each warp owns a ring of KV_STAGES such tiles and walks
+// the token's tile sequence  layer 0 K tiles, layer 0 V tiles, layer 1 K tiles, ...: the copy of tile j + KV_STAGES is
+// issued (one lane, one instruction) the moment tile j has been consumed, so the stream keeps flowing through the softmax
+// between the K and the V pass and through the projections / MLP between layers -- with register-staged loads a warp has
+// nothing in flight during those phases.
+constexpr int TMA_WARPS = 4;
+constexpr int TMA_MINB = 5;   // 96 registers: 20 warps per SM with a 2-deep ring (measured best at 10k envs: 210 ms; 4 CTAs / 128 regs: 257 ms)
+constexpr int KV_STAGES = 2;  // ring depth: measured at 1250 and 10000 envs, 2 stages beat 3, 4 and 6 (DESIGN.md)
+constexpr int KV_TILE_BYTES = 32 * G_E * 4;   // 32 keys x 32 channels fp32
+
+__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+struct KvRing {
+  static constexpr bool MASK_ALL = true;   // every tile masked, K rows past the last key read stale (fewer registers than the split)
+  uint32_t stage0, bar0;        // shared addresses: stage s at stage0 + s * KV_TILE_BYTES, its mbarrier at bar0 + 8 s
+  uint32_t is;                  // stage the next issued tile goes to
+  uint32_t cs, cp;              // stage of the next tile to consume, and the parity of its mbarrier phase
+  int cl, ckv, ct;              // cursor of the next tile to issue: layer, K (0) / V (1), tile
+  int nt, pos, L, Tpad;
+  const float* kv;
+
+  __device__ __forceinline__ void issue_next(int lane) {
+    if (cl >= L) return;
+    if (lane == 0) {
+      const uint32_t s = is;
+      const int nkeys = min(32, pos - 32 * ct);
+      const uint32_t bytes = (uint32_t)nkeys * (G_E * 4);
+      const float* src = kv + ((size_t)(cl * 2 + ckv) * Tpad + (size_t)ct * 32) * G_E;
+      const uint32_t bar = bar0 + 8 * s, dst = stage0 + s * KV_TILE_BYTES;
+      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes),
+                   "r"(bar)
+                   : "memory");
+    }
+    if (++is == KV_STAGES) is = 0;
+    if (++ct == nt) {
+      ct = 0;
+      if (++ckv == 2) ckv = 0, ++cl;
+    }
+  }
+  // start of a token at position `pos` (keys 0 .. pos-1 are cached): fill the ring
+  __device__ __forceinline__ void begin_token(int pos_, int lane) {
+    pos = pos_, nt = (pos_ + 31) >> 5;
+    cl = nt ? 0 : L, ckv = 0, ct = 0;
+    for (int i = 0; i < KV_STAGES; ++i) issue_next(lane);
+  }
+  // this token's appended K/V rows (generic-proxy stores of all lanes) must be visible to the bulk copies (async proxy)
+  // that the next token issues
+  __device__ __forceinline__ void end_token() {
+    __syncwarp();
+    asm volatile("fence.proxy.async;" ::: "memory");
+  }
+  // wait for the next tile in sequence (tiles arrive in the order the attention asks for them; X, k0 and pos are implied)
+  __device__ __forceinline__ const float4* tile(const float*, int, int, int lane) {
+    const uint32_t s = cs, par = cp;
+    const uint32_t bar = bar0 + 8 * s;
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tKVWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t@!p bra KVWAIT_%=;\n\t}" ::"r"(bar), "r"(par)
+        : "memory");
+    return reinterpret_cast<const float4*>(__cvta_shared_to_generic((size_t)(stage0 + s * KV_TILE_BYTES))) + (lane & 7);
+  }
+  __device__ __forceinline__ float4 load(const float4* t, int, int r) const { return t[r * 8]; }   // rows past the last key: stale
+  // every lane has finished reading the tile: its stage is free for the next copy
+  __device__ __forceinline__ void consumed(int lane) {
+    __syncwarp();
+    if (++cs == KV_STAGES) cs = 0, cp ^= 1u;
+    issue_next(lane);
+  }
+};
+
+// fp32 attention of the token at `pos` (query q, key k, value v: this lane's channel) over the cached keys 0..pos-1 and
+// itself; appends k and v to the layer's caches K and V first.  Returns this lane's channel of the attention output.
+// A lane maps to (key group g = lane/8, channel quad b8 = lane%8): one 16 B load covers 4 keys x 32 channels, 8 are kept
+// in flight per lane (32 keys), the 8-lane dot products are combined by a 7-shuffle butterfly transpose-reduce, softmax
+// is a warp reduction, and PV accumulates float4 channel quads.
+template <class Src>
+__device__ __forceinline__ float attention_f32(float q, float k, float v, int pos, float* K, float* V, float* sx, float* ssc,
+                                               int lane, Src& src) {
+  K[(size_t)pos * G_E + lane] = k;   // both caches are [t][channel]: appends are coalesced 128 B rows
+  V[(size_t)pos * G_E + lane] = v;
+  q *= 0.17677669529663687f;  // 1/sqrt(head_dim = 32)
+  sx[lane] = q;
+  __syncwarp();
+  const int g = lane >> 3, b8 = lane & 7;
+  const float4 q4 = reinterpret_cast<const float4*>(sx)[b8];
+  __syncwarp();
+  // TAIL = the last, partial tile: load instruction i covers keys k0 + 4 i .. k0 + 4 i + 3 of all key groups, so
+  // instructions past the last key are skipped with a WARP-UNIFORM predicate (round 2: the padded rows of the last tile
+  // were 4.7 % of the kernel's DRAM traffic; per-lane predication of every tile, which skips 3-5 % of the K/V traffic at
+  // H = 500, cost more issue than the bytes saved)
+  float lmax = -INFINITY;
+  for_each_key_tile<32, Src::MASK_ALL>(pos, [&](const int k0, auto tail_tag) {
+    constexpr bool TAIL = decltype(tail_tag)::value;
+    const int r = pos - k0;
+    const float4* t = src.tile(K, k0, pos, lane);
+    float4 kk[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+      kk[i] = (!TAIL || Src::MASK_ALL || 4 * i < r) ? src.load(t, k0, 4 * i + g) : make_float4(0.f, 0.f, 0.f, 0.f);   // in bounds (Tpad % 32 == 0)
+    float pv[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) pv[i] = fmaf(q4.x, kk[i].x, fmaf(q4.y, kk[i].y, fmaf(q4.z, kk[i].z, q4.w * kk[i].w)));
+    src.consumed(lane);
+    // butterfly transpose-reduce over the 8 lanes of a key group: lane b8 ends with the full dot of chunk i = b8
+    float w4[4], w2[2];
+    const bool u4 = b8 & 4, u2 = b8 & 2, u1 = b8 & 1;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float send = u4 ? pv[j] : pv[j + 4], keep = u4 ? pv[j + 4] : pv[j];
+      w4[j] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
+    }
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {
+      const float send = u2 ? w4[j] : w4[j + 2], keep = u2 ? w4[j + 2] : w4[j];
+      w2[j] = keep + __shfl_xor_sync(0xffffffffu, send, 2);
+    }
+    const float sc = (u1 ? w2[1] : w2[0]) + __shfl_xor_sync(0xffffffffu, u1 ? w2[0] : w2[1], 1);
+    const int key = k0 + 4 * b8 + g;
+    if (!TAIL || key < pos) {
+      ssc[key] = sc;
+      lmax = fmaxf(lmax, sc);
+    }
+  });
+  const float s_self = warp_sum(q * k);  // the token attends to itself (causal mask keeps keys <= pos)
+  lmax = fmaxf(warp_max(lmax), s_self);
+  __syncwarp();
+  float lsum = 0.f;
+  for (int key = lane; key < pos; key += 32) {
+    const float pr = expf(ssc[key] - lmax);
+    ssc[key] = pr;
+    lsum += pr;
+  }
+  const float p_self = expf(s_self - lmax);
+  const float inv = 1.0f / (warp_sum(lsum) + p_self);
+  __syncwarp();
+  float4 oa = make_float4(0.f, 0.f, 0.f, 0.f);
+  for_each_key_tile<32, Src::MASK_ALL>(pos, [&](const int k0, auto tail_tag) {
+    constexpr bool TAIL = decltype(tail_tag)::value;
+    const float4* t = src.tile(V, k0, pos, lane);
+    float4 vv[8];
+    float pr[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      const int key = k0 + 4 * i + g;
+      const bool ok = !TAIL || key < pos;        // rows >= pos are uninitialised or stale: never touch them
+      vv[i] = ok ? src.load(t, k0, 4 * i + g) : make_float4(0.f, 0.f, 0.f, 0.f);
+      pr[i] = ok ? ssc[key] : 0.f;
+    }
+    src.consumed(lane);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      oa.x = fmaf(pr[i], vv[i].x, oa.x);
+      oa.y = fmaf(pr[i], vv[i].y, oa.y);
+      oa.z = fmaf(pr[i], vv[i].z, oa.z);
+      oa.w = fmaf(pr[i], vv[i].w, oa.w);
+    }
+  });
+  // sum the 4 key groups (lanes with equal b8), then hand channel `lane` its value
+#pragma unroll
+  for (int o_ = 8; o_ <= 16; o_ <<= 1) {
+    oa.x += __shfl_xor_sync(0xffffffffu, oa.x, o_);
+    oa.y += __shfl_xor_sync(0xffffffffu, oa.y, o_);
+    oa.z += __shfl_xor_sync(0xffffffffu, oa.z, o_);
+    oa.w += __shfl_xor_sync(0xffffffffu, oa.w, o_);
+  }
+  __syncwarp();
+  if (lane < 8) reinterpret_cast<float4*>(sx)[lane] = oa;
+  __syncwarp();
+  return (sx[lane] + p_self * v) * inv;
+}
+
+// bf16 cache on the tensor cores (mma.sync m16n8k16, fp32 accumulate); same contract as attention_f32.  The decode is a
+// GEMV per env (one query against that env's private keys), so the products are formed transposed -- keys / channels /
+// outputs are the 16 rows of the A tile and the single query (or probability, or activation) vector is column 0 of B;
+// what the MMA buys is instruction count: 2 HMMA replace ~180 unpack / FMA / shuffle instructions per 16 keys.
+//   K cache: one 64 B row per key, channels permuted so that lane (g = lane/4, c = lane%4) reads the B
+//            fragments of key g for both k-steps with ONE 16 B load (kperm below).
+//   V cache: blocks of 16 keys x 32 channels (1 KB) stored as [channel-in-octet g][key pair c][octet j]
+//            [keys 2c, 2c+1, 2c+8, 2c+9]: lane (g, c) reads the B fragments of all four channel octets with
+//            two 16 B loads; a block is zeroed when its first key is appended (P = 0 must meet finite V).
+
+// One token through all layers.  x: this lane's channel of the embedded token (+wpe).  kv: this sequence's cache
+// (kv_seq_bytes).  sx[32], sh[128], ssc[Tpad]: per-warp shared scratch.  WS: the projections run on the tensor cores
+// from bf16 weight fragments in shared memory (`wf`, all layers).  src: where the fp32 attention's K/V tiles come from.
+template <bool BF16, bool WS = false, class Src = GlobalKv>
 __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int pos, void* kv_, int Tpad, float* sx,
-                                               float* sh, float* ssc, int lane, const uint4* wf = nullptr) {
+                                               float* sh, float* ssc, int lane, const uint4* wf = nullptr, Src&& src = {}) {
+  using KvT = std::conditional_t<BF16, __nv_bfloat16, float>;
+  src.begin_token(pos, lane);
   for (int l = 0; l < m.L; ++l) {
     const LayerW& w = m.layer[l];
     // ---- attention ----
@@ -169,127 +393,14 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
     } else {
       matvec_packed<G_E, 3>(sx, w.attn_wP, w.attn_b, lane, qkv);
     }
-    float q = qkv[0];
-    const float k = qkv[1], v = qkv[2];
-    float lmax = -INFINITY, s_self, p_self, inv, osum;
-    if constexpr (!BF16) {
-      __syncwarp();
-      float* K = reinterpret_cast<float*>(kv_) + (size_t)(l * 2) * G_E * Tpad;
-      float* V = K + (size_t)G_E * Tpad;
-      K[(size_t)pos * G_E + lane] = k;   // both caches are [t][channel]: appends are coalesced 128 B rows
-      V[(size_t)pos * G_E + lane] = v;
-      q *= 0.17677669529663687f;  // 1/sqrt(head_dim = 32)
-      sx[lane] = q;
-      __syncwarp();
-      // lane = (key group g = lane/8, channel quad c4 = 4*(lane%8)): one LDG.128 instruction covers 4 keys
-      const int g = lane >> 3, b8 = lane & 7;
-      const float4 q4 = reinterpret_cast<const float4*>(sx)[b8];
-      const float4* K4 = reinterpret_cast<const float4*>(K) + b8;   // row stride = 8 float4
-      const float4* V4 = reinterpret_cast<const float4*>(V) + b8;
-      __syncwarp();
-      // cached keys 0..pos-1, 32 per tile: 8 row loads in flight per lane.  TAIL = the last, partial tile: load instruction i
-      // covers keys k0 + 4 i .. k0 + 4 i + 3 of all key groups, so instructions past the last key are skipped with a
-      // WARP-UNIFORM predicate (round 2: the padded rows of the last tile were 4.7 % of the kernel's DRAM traffic; per-lane
-      // predication of every tile, which skips 3-5 % of the K/V traffic at H = 500, cost more issue than the bytes saved)
-      auto k_tile = [&](const int k0, auto tail_tag) {
-        constexpr bool TAIL = decltype(tail_tag)::value;
-        const int r = pos - k0;
-        if (pos <= PF_MAX_POS && k0 + PF_AHEAD * 32 < pos) prefetch_l2(K + (size_t)(k0 + PF_AHEAD * 32 + lane) * G_E);
-        float4 kk[8];
-  #pragma unroll
-        for (int i = 0; i < 8; ++i)
-          kk[i] = (!TAIL || 4 * i < r) ? __ldcg(K4 + (size_t)(k0 + 4 * i + g) * 8) : make_float4(0.f, 0.f, 0.f, 0.f);   // in bounds (Tpad % 32 == 0)
-        float pv[8];
-  #pragma unroll
-        for (int i = 0; i < 8; ++i) pv[i] = fmaf(q4.x, kk[i].x, fmaf(q4.y, kk[i].y, fmaf(q4.z, kk[i].z, q4.w * kk[i].w)));
-        // butterfly transpose-reduce over the 8 lanes of a key group: lane b8 ends with the full dot of chunk i = b8
-        float w4[4], w2[2];
-        const bool u4 = b8 & 4, u2 = b8 & 2, u1 = b8 & 1;
-  #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const float send = u4 ? pv[j] : pv[j + 4], keep = u4 ? pv[j + 4] : pv[j];
-          w4[j] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
-        }
-  #pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const float send = u2 ? w4[j] : w4[j + 2], keep = u2 ? w4[j + 2] : w4[j];
-          w2[j] = keep + __shfl_xor_sync(0xffffffffu, send, 2);
-        }
-        const float sc = (u1 ? w2[1] : w2[0]) + __shfl_xor_sync(0xffffffffu, u1 ? w2[0] : w2[1], 1);
-        const int key = k0 + 4 * b8 + g;
-        if (!TAIL || key < pos) {
-          ssc[key] = sc;
-          lmax = fmaxf(lmax, sc);
-        }
-      };
-      {
-        int k0 = 0;
-        for (; k0 + 32 <= pos; k0 += 32) k_tile(k0, std::false_type{});
-        if (k0 < pos) k_tile(k0, std::true_type{});
-      }
-      s_self = warp_sum(q * k);  // the token attends to itself (causal mask keeps keys <= pos)
-      lmax = fmaxf(warp_max(lmax), s_self);
-      __syncwarp();
-      float lsum = 0.f;
-      for (int key = lane; key < pos; key += 32) {
-        const float pr = expf(ssc[key] - lmax);
-        ssc[key] = pr;
-        lsum += pr;
-      }
-      p_self = expf(s_self - lmax);
-      inv = 1.0f / (warp_sum(lsum) + p_self);
-      __syncwarp();
-      float4 oa = make_float4(0.f, 0.f, 0.f, 0.f);
-      auto v_tile = [&](const int k0, auto tail_tag) {
-        constexpr bool TAIL = decltype(tail_tag)::value;
-        if (pos <= PF_MAX_POS && k0 + PF_AHEAD * 32 < pos) prefetch_l2(V + (size_t)(k0 + PF_AHEAD * 32 + lane) * G_E);
-        float4 vv[8];
-        float pr[8];
-  #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int key = k0 + 4 * i + g;
-          const bool ok = !TAIL || key < pos;        // rows >= pos are uninitialised: never touch them
-          vv[i] = ok ? __ldcg(V4 + (size_t)key * 8) : make_float4(0.f, 0.f, 0.f, 0.f);
-          pr[i] = ok ? ssc[key] : 0.f;
-        }
-  #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          oa.x = fmaf(pr[i], vv[i].x, oa.x);
-          oa.y = fmaf(pr[i], vv[i].y, oa.y);
-          oa.z = fmaf(pr[i], vv[i].z, oa.z);
-          oa.w = fmaf(pr[i], vv[i].w, oa.w);
-        }
-      };
-      {
-        int k0 = 0;
-        for (; k0 + 32 <= pos; k0 += 32) v_tile(k0, std::false_type{});
-        if (k0 < pos) v_tile(k0, std::true_type{});
-      }
-      // sum the 4 key groups (lanes with equal b8), then hand channel `lane` its value
-  #pragma unroll
-      for (int o_ = 8; o_ <= 16; o_ <<= 1) {
-        oa.x += __shfl_xor_sync(0xffffffffu, oa.x, o_);
-        oa.y += __shfl_xor_sync(0xffffffffu, oa.y, o_);
-        oa.z += __shfl_xor_sync(0xffffffffu, oa.z, o_);
-        oa.w += __shfl_xor_sync(0xffffffffu, oa.w, o_);
-      }
-      __syncwarp();
-      if (lane < 8) reinterpret_cast<float4*>(sx)[lane] = oa;
-      __syncwarp();
-      osum = sx[lane] + p_self * v;
-    } else {
-      __syncwarp();
-      // bf16 cache on the tensor cores (mma.sync m16n8k16, fp32 accumulate).  The decode is a GEMV per env (one
-      // query against that env's private keys), so the products are formed transposed -- keys / channels / outputs are
-      // the 16 rows of the A tile and the single query (or probability, or activation) vector is column 0 of B; what
-      // the MMA buys is instruction count: 2 HMMA replace ~180 unpack / FMA / shuffle instructions per 16 keys.
-      //   K cache: one 64 B row per key, channels permuted so that lane (g = lane/4, c = lane%4) reads the B
-      //            fragments of key g for both k-steps with ONE 16 B load (kperm below).
-      //   V cache: blocks of 16 keys x 32 channels (1 KB) stored as [channel-in-octet g][key pair c][octet j]
-      //            [keys 2c, 2c+1, 2c+8, 2c+9]: lane (g, c) reads the B fragments of all four channel octets with
-      //            two 16 B loads; a block is zeroed when its first key is appended (P = 0 must meet finite V).
-      __nv_bfloat16* K = reinterpret_cast<__nv_bfloat16*>(kv_) + (size_t)(l * 2) * G_E * Tpad;
-      __nv_bfloat16* V = K + (size_t)G_E * Tpad;
+    __syncwarp();
+    KvT* K = reinterpret_cast<KvT*>(kv_) + (size_t)(l * 2) * G_E * Tpad;
+    KvT* V = K + (size_t)G_E * Tpad;
+    float o;
+    if constexpr (BF16)
+    {
+      float q = qkv[0];
+      const float k = qkv[1], v = qkv[2];
       const int g = lane >> 2, c = lane & 3;
       {
         const int r = lane & 15;
@@ -316,16 +427,17 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
       __syncwarp();
       // 64 keys per tile; TAIL = the last, partial tile: load instruction i covers keys k0 + 8 i .. k0 + 8 i + 7, instructions
       // past the last key are skipped with a warp-uniform predicate (the padded rows were 6.2 % of the DRAM traffic)
-      auto k_tile = [&](const int k0, auto tail_tag) {
+      float lmax = -INFINITY;
+      for_each_key_tile<64>(pos, [&](const int k0, auto tail_tag) {
         constexpr bool TAIL = decltype(tail_tag)::value;
         const int r = pos - k0;
         uint4 kk[8];
-#pragma unroll
+    #pragma unroll
         for (int i = 0; i < 8; ++i)
           kk[i] = (!TAIL || 8 * i < r) ? __ldcg(K8 + (size_t)(k0 + 8 * i + g) * 4) : make_uint4(0u, 0u, 0u, 0u);   // in bounds (Tpad % 64 == 0)
         // (an L2 prefetch of the same 64 keys' V blocks here was measured slower: 161 ms with, 155 ms without, C4)
         // scores^T = K q^T: 16 keys are the rows of the A tile (octets 2m and 2m + 1), q is column 0 of B
-#pragma unroll
+    #pragma unroll
         for (int mt = 0; mt < 4; ++mt) {
           if (TAIL && 16 * mt >= r) break;        // (warp-uniform)
           float d[4] = {0.f, 0.f, 0.f, 0.f};
@@ -337,13 +449,8 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
             if (!TAIL || key + 8 < pos) ssc[key + 8] = d[2], lmax = fmaxf(lmax, d[2]);
           }
         }
-      };
-      {
-        int k0 = 0;
-        for (; k0 + 64 <= pos; k0 += 64) k_tile(k0, std::false_type{});
-        if (k0 < pos) k_tile(k0, std::true_type{});
-      }
-      s_self = warp_sum(q * k);
+      });
+      const float s_self = warp_sum(q * k);
       lmax = fmaxf(warp_max(lmax), s_self);
       __syncwarp();
       float lsum = 0.f;
@@ -354,22 +461,22 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
         lsum += pr;
       }
       for (int key = pos + lane; key < ((pos + 15) & ~15); key += 32) ssc[key] = 0.f;   // tail of the last key block
-      p_self = expf(s_self - lmax);
-      inv = 1.0f / (warp_sum(lsum) + p_self);
+      const float p_self = expf(s_self - lmax);
+      const float inv = 1.0f / (warp_sum(lsum) + p_self);
       __syncwarp();
       float oa[2][4];   // out^T = V^T p^T: channel tiles 0..15 and 16..31 are the rows, p is column 0 of B
-#pragma unroll
+    #pragma unroll
       for (int jn = 0; jn < 2; ++jn) oa[jn][0] = oa[jn][1] = oa[jn][2] = oa[jn][3] = 0.f;
       const uint4* VB = reinterpret_cast<const uint4*>(V) + 2 * lane;   // block stride = 64 uint4
       for (int k0 = 0; k0 < pos; k0 += 64) {
         uint4 va[4], vc[4];
-#pragma unroll
+    #pragma unroll
         for (int i = 0; i < 4; ++i) {
           const bool ok = k0 + 16 * i < pos;          // blocks past the last key are uninitialised: never touch them
           va[i] = ok ? __ldcg(VB + (size_t)((k0 >> 4) + i) * 64) : make_uint4(0, 0, 0, 0);
           vc[i] = ok ? __ldcg(VB + (size_t)((k0 >> 4) + i) * 64 + 1) : make_uint4(0, 0, 0, 0);
         }
-#pragma unroll
+    #pragma unroll
         for (int i = 0; i < 4; ++i) {
           uint32_t pa0 = 0, pa2 = 0;
           if (lane < 4 && k0 + 16 * i < pos) {
@@ -383,13 +490,14 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
       }
       __syncwarp();
       if (c == 0) {   // column 0 of the output tiles: lane (g, 0) holds channels 16 jn + g and 16 jn + g + 8
-#pragma unroll
+    #pragma unroll
         for (int jn = 0; jn < 2; ++jn) sx[16 * jn + g] = oa[jn][0], sx[16 * jn + 8 + g] = oa[jn][2];
       }
       __syncwarp();
-      osum = sx[lane] + p_self * v;
+      o = (sx[lane] + p_self * v) * inv;
     }
-    const float o = osum * inv;
+    else
+      o = attention_f32(qkv[0], qkv[1], qkv[2], pos, K, V, sx, ssc, lane, src);
     __syncwarp();
     sx[lane] = o;
     __syncwarp();
@@ -428,193 +536,7 @@ __device__ __forceinline__ float token_forward(const Gpt2Dev& m, float x, int po
     x += y2;
     __syncwarp();
   }
-  return x;
-}
-
-// ---------------------------------------------------------------------------------------------
-// Bulk-async (TMA engine) staging of the fp32 K/V stream: cp.async.bulk global -> shared, completion on an mbarrier.
-// A warp's cached keys of one layer are ONE contiguous run per tensor ([t][32 channels] fp32, 128 B rows), so a tile of
-// 32 keys is a single <= 4 KB bulk copy of exactly the live rows (no padded rows are read).  Each warp owns a ring of
-// KV_STAGES such tiles and walks the token's tile sequence  layer 0 K tiles, layer 0 V tiles, layer 1 K tiles, ...:
-// the copy of tile j + KV_STAGES is issued (one lane, one instruction) the moment tile j has been consumed, so the
-// stream keeps flowing through the softmax between the K and the V pass and through the projections / MLP between
-// layers -- with register-staged loads (token_forward above) a warp has nothing in flight during those phases.
-// ---------------------------------------------------------------------------------------------
-constexpr int TMA_WARPS = 4;
-constexpr int TMA_MINB = 5;   // 96 registers: 20 warps per SM with a 2-deep ring (measured best at 10k envs: 210 ms; 4 CTAs / 128 regs: 257 ms)
-constexpr int KV_STAGES = 2;  // ring depth: measured at 1250 and 10000 envs, 2 stages beat 3, 4 and 6 (DESIGN.md)
-constexpr int KV_TILE_BYTES = 32 * G_E * 4;   // 32 keys x 32 channels fp32
-
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-struct KvRing {
-  uint32_t stage0, bar0;        // shared addresses: stage s at stage0 + s * KV_TILE_BYTES, its mbarrier at bar0 + 8 s
-  uint32_t is;                  // stage the next issued tile goes to
-  uint32_t cs, cp;              // stage of the next tile to consume, and the parity of its mbarrier phase
-  int cl, ckv, ct;              // cursor of the next tile to issue: layer, K (0) / V (1), tile
-  int nt, pos, L, Tpad;
-  const float* kv;
-
-  __device__ __forceinline__ void issue_next(int lane) {
-    if (cl >= L) return;
-    if (lane == 0) {
-      const uint32_t s = is;
-      const int nkeys = min(32, pos - 32 * ct);
-      const uint32_t bytes = (uint32_t)nkeys * (G_E * 4);
-      const float* src = kv + ((size_t)(cl * 2 + ckv) * Tpad + (size_t)ct * 32) * G_E;
-      const uint32_t bar = bar0 + 8 * s, dst = stage0 + s * KV_TILE_BYTES;
-      asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-      asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes),
-                   "r"(bar)
-                   : "memory");
-    }
-    if (++is == KV_STAGES) is = 0;
-    if (++ct == nt) {
-      ct = 0;
-      if (++ckv == 2) ckv = 0, ++cl;
-    }
-  }
-  // start of a token at position `pos` (keys 0 .. pos-1 are cached): fill the ring
-  __device__ __forceinline__ void begin_token(int pos_, int lane) {
-    pos = pos_, nt = (pos_ + 31) >> 5;
-    cl = nt ? 0 : L, ckv = 0, ct = 0;
-    for (int i = 0; i < KV_STAGES; ++i) issue_next(lane);
-  }
-  // wait for the next tile in sequence; returns its shared-memory address as a generic pointer
-  __device__ __forceinline__ const float4* acquire() {
-    const uint32_t s = cs, par = cp;
-    const uint32_t bar = bar0 + 8 * s;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tKVWAIT_%=:\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t@!p bra KVWAIT_%=;\n\t}" ::"r"(bar), "r"(par)
-        : "memory");
-    return reinterpret_cast<const float4*>(__cvta_shared_to_generic((size_t)(stage0 + s * KV_TILE_BYTES)));
-  }
-  // every lane has finished reading the tile: its stage is free for the next copy
-  __device__ __forceinline__ void release(int lane) {
-    __syncwarp();
-    if (++cs == KV_STAGES) cs = 0, cp ^= 1u;
-    issue_next(lane);
-  }
-};
-
-// token_forward with the fp32 K/V stream staged through the ring (same arithmetic, same order of operations)
-__device__ __forceinline__ float token_forward_tma(const Gpt2Dev& m, float x, int pos, float* kvf, int Tpad, float* sx, float* sh, float* ssc,
-                                                   int lane, KvRing& ring) {
-  ring.begin_token(pos, lane);
-  for (int l = 0; l < m.L; ++l) {
-    const LayerW& w = m.layer[l];
-    sx[lane] = layer_norm(x, w.ln1_w, w.ln1_b, lane);
-    __syncwarp();
-    float qkv[3];
-    matvec_packed<G_E, 3>(sx, w.attn_wP, w.attn_b, lane, qkv);
-    float q = qkv[0];
-    const float k = qkv[1], v = qkv[2];
-    __syncwarp();
-    float* K = kvf + (size_t)(l * 2) * G_E * Tpad;
-    float* V = K + (size_t)G_E * Tpad;
-    K[(size_t)pos * G_E + lane] = k;   // appended rows are read (by bulk copies) from the NEXT token on
-    V[(size_t)pos * G_E + lane] = v;
-    q *= 0.17677669529663687f;  // 1/sqrt(head_dim = 32)
-    sx[lane] = q;
-    __syncwarp();
-    const int g = lane >> 3, b8 = lane & 7;
-    const float4 q4 = reinterpret_cast<const float4*>(sx)[b8];
-    __syncwarp();
-    float lmax = -INFINITY;
-    for (int k0 = 0; k0 < pos; k0 += 32) {
-      const float4* Ks = ring.acquire() + b8;   // row stride = 8 float4
-      float4 kk[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) kk[i] = Ks[(4 * i + g) * 8];   // rows past the last key hold stale data: masked below
-      float pv[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) pv[i] = fmaf(q4.x, kk[i].x, fmaf(q4.y, kk[i].y, fmaf(q4.z, kk[i].z, q4.w * kk[i].w)));
-      ring.release(lane);
-      float w4[4], w2[2];
-      const bool u4 = b8 & 4, u2 = b8 & 2, u1 = b8 & 1;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const float send = u4 ? pv[j] : pv[j + 4], keep = u4 ? pv[j + 4] : pv[j];
-        w4[j] = keep + __shfl_xor_sync(0xffffffffu, send, 4);
-      }
-#pragma unroll
-      for (int j = 0; j < 2; ++j) {
-        const float send = u2 ? w4[j] : w4[j + 2], keep = u2 ? w4[j + 2] : w4[j];
-        w2[j] = keep + __shfl_xor_sync(0xffffffffu, send, 2);
-      }
-      const float sc = (u1 ? w2[1] : w2[0]) + __shfl_xor_sync(0xffffffffu, u1 ? w2[0] : w2[1], 1);
-      const int key = k0 + 4 * b8 + g;
-      if (key < pos) {
-        ssc[key] = sc;
-        lmax = fmaxf(lmax, sc);
-      }
-    }
-    const float s_self = warp_sum(q * k);  // the token attends to itself (causal mask keeps keys <= pos)
-    lmax = fmaxf(warp_max(lmax), s_self);
-    __syncwarp();
-    float lsum = 0.f;
-    for (int key = lane; key < pos; key += 32) {
-      const float pr = expf(ssc[key] - lmax);
-      ssc[key] = pr;
-      lsum += pr;
-    }
-    const float p_self = expf(s_self - lmax);
-    const float inv = 1.0f / (warp_sum(lsum) + p_self);
-    __syncwarp();
-    float4 oa = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int k0 = 0; k0 < pos; k0 += 32) {
-      const float4* Vs = ring.acquire() + b8;
-      float4 vv[8];
-      float pr[8];
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        const int key = k0 + 4 * i + g;
-        const bool ok = key < pos;                 // rows >= pos are stale: never let them in
-        vv[i] = ok ? Vs[(4 * i + g) * 8] : make_float4(0.f, 0.f, 0.f, 0.f);
-        pr[i] = ok ? ssc[key] : 0.f;
-      }
-      ring.release(lane);
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        oa.x = fmaf(pr[i], vv[i].x, oa.x);
-        oa.y = fmaf(pr[i], vv[i].y, oa.y);
-        oa.z = fmaf(pr[i], vv[i].z, oa.z);
-        oa.w = fmaf(pr[i], vv[i].w, oa.w);
-      }
-    }
-#pragma unroll
-    for (int o_ = 8; o_ <= 16; o_ <<= 1) {
-      oa.x += __shfl_xor_sync(0xffffffffu, oa.x, o_);
-      oa.y += __shfl_xor_sync(0xffffffffu, oa.y, o_);
-      oa.z += __shfl_xor_sync(0xffffffffu, oa.z, o_);
-      oa.w += __shfl_xor_sync(0xffffffffu, oa.w, o_);
-    }
-    __syncwarp();
-    if (lane < 8) reinterpret_cast<float4*>(sx)[lane] = oa;
-    __syncwarp();
-    const float o = (sx[lane] + p_self * v) * inv;
-    __syncwarp();
-    sx[lane] = o;
-    __syncwarp();
-    float y;
-    matvec_packed<G_E, 1>(sx, w.proj_wP, w.proj_b, lane, &y);
-    x += y;
-    __syncwarp();
-    sx[lane] = layer_norm(x, w.ln2_w, w.ln2_b, lane);
-    __syncwarp();
-    float hh[4];
-    matvec_packed<G_E, 4>(sx, w.fc_wP, w.fc_b, lane, hh);
-    sh[lane] = gelu_new(hh[0]), sh[32 + lane] = gelu_new(hh[1]), sh[64 + lane] = gelu_new(hh[2]), sh[96 + lane] = gelu_new(hh[3]);
-    __syncwarp();
-    float y2;
-    matvec_packed<G_FF, 1>(sh, w.fc2_wP, w.fc2_b, lane, &y2);
-    x += y2;
-    __syncwarp();
-  }
-  // this token's appended K/V rows (generic-proxy stores of all lanes) must be visible to the bulk copies (async proxy)
-  // that the next token issues
-  __syncwarp();
-  asm volatile("fence.proxy.async;" ::: "memory");
+  src.end_token();
   return x;
 }
 
@@ -636,6 +558,7 @@ struct WarpScratch {
   float* sh;
   float* ssc;
 };
+__host__ __device__ __forceinline__ size_t warp_scratch_bytes(int Tpad) { return (size_t)(G_E + G_FF + Tpad) * sizeof(float); }
 __device__ __forceinline__ WarpScratch warp_scratch(float* smem, int warp, int Tpad) {
   float* base = smem + (size_t)warp * (G_E + G_FF + Tpad);
   return WarpScratch{base, base + G_E, base + G_E + G_FF};
@@ -660,7 +583,7 @@ __global__ void __launch_bounds__(G_THREADS) gpt2_forward_kernel(const ForwardPa
   if (b >= p.B) return;
   const Gpt2Dev& m = p.m;
   const WarpScratch ws = warp_scratch(g_smem, warp, p.Tpad);
-  char* kv = reinterpret_cast<char*>(p.kv) + (size_t)b * m.L * 2 * G_E * p.Tpad * (BF16 ? 2 : 4);
+  char* kv = reinterpret_cast<char*>(p.kv) + (size_t)b * kv_seq_bytes(m.L, p.Tpad, BF16);
   const int dx = m.dx, du = m.du, din = m.din;
   for (int pos = 0; pos <= p.T; ++pos) {
     // token = [state | action | next_state | reward]; position 0 = query state, zeros elsewhere (models/net.py:45-53)
@@ -715,7 +638,7 @@ __global__ void __launch_bounds__(G_THREADS) gpt2_decode_step_kernel(const StepP
   if (b >= p.N) return;
   const Gpt2Dev& m = p.m;
   const WarpScratch ws = warp_scratch(g_smem, warp, p.Tpad);
-  char* kv = reinterpret_cast<char*>(p.kv) + (size_t)b * m.L * 2 * G_E * p.Tpad * (BF16 ? 2 : 4);
+  char* kv = reinterpret_cast<char*>(p.kv) + (size_t)b * kv_seq_bytes(m.L, p.Tpad, BF16);
   const float tok = lane < m.din ? p.tokens[(size_t)b * m.din + lane] : 0.f;
   float x = __ldg(m.embed_b + lane) + __ldg(m.wpe + (size_t)p.pos * G_E + lane);
   for (int i = 0; i < m.din; ++i) x = fmaf(__shfl_sync(0xffffffffu, tok, i), __ldg(m.embed_wT + i * G_E + lane), x);
@@ -758,7 +681,7 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
   const Gpt2Dev& m = p.m;
   const uint4* wf = nullptr;
   float* scratch = g_smem;
-  KvRing ring;
+  std::conditional_t<TMA, KvRing, GlobalKv> kv_src;
   if constexpr (TMA) {   // [warps][KV_STAGES] tiles of 4 KB | [warps][KV_STAGES] mbarriers | per-warp scratch
     const int nw = blockDim.x >> 5;
     unsigned char* base = reinterpret_cast<unsigned char*>(g_smem);
@@ -767,10 +690,10 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
       asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_addr(bars + threadIdx.x)) : "memory");
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
-    ring.stage0 = smem_addr(base + (size_t)warp * KV_STAGES * KV_TILE_BYTES);
-    ring.bar0 = smem_addr(bars + warp * KV_STAGES);
-    ring.is = ring.cs = ring.cp = 0;
-    ring.L = m.L, ring.Tpad = p.Tpad;
+    kv_src.stage0 = smem_addr(base + (size_t)warp * KV_STAGES * KV_TILE_BYTES);
+    kv_src.bar0 = smem_addr(bars + warp * KV_STAGES);
+    kv_src.is = kv_src.cs = kv_src.cp = 0;
+    kv_src.L = m.L, kv_src.Tpad = p.Tpad;
     scratch = reinterpret_cast<float*>(bars + ((nw * KV_STAGES + 1) & ~1));   // keep the per-warp scratch 16 B aligned
   }
   if constexpr (WS) {
@@ -784,8 +707,8 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
   const int env = blockIdx.x * (int)(blockDim.x >> 5) + warp;   // WS: the host picks <= GW_WARPS warps per CTA
   if (env >= p.N) return;
   const WarpScratch ws = warp_scratch(scratch, warp, p.Tpad);
-  char* kv = reinterpret_cast<char*>(p.kv) + (size_t)env * m.L * 2 * G_E * p.Tpad * (BF16 ? 2 : 4);
-  if constexpr (TMA) ring.kv = reinterpret_cast<const float*>(kv);
+  char* kv = reinterpret_cast<char*>(p.kv) + (size_t)env * kv_seq_bytes(m.L, p.Tpad, BF16);
+  if constexpr (TMA) kv_src.kv = reinterpret_cast<const float*>(kv);
   const int du = m.du, H = p.H, N = p.N;
   const uint64_t gid = p.env_id0 + (uint64_t)env;
   const float mean_l = lane < du ? p.means[(size_t)env * du + lane] : -INFINITY;
@@ -807,10 +730,7 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
   for (int h = 0; h < H; ++h) {
     float x = e_bias + e_state + __ldg(m.wpe + (size_t)h * G_E + lane);
     if (h > 0) x += __ldg(m.embed_wT + (1 + a_prev) * G_E + lane) + e_next + e_rew * r_prev;
-    if constexpr (TMA)
-      x = token_forward_tma(m, x, h, reinterpret_cast<float*>(kv), p.Tpad, ws.sx, ws.sh, ws.ssc, lane, ring);
-    else
-      x = token_forward<BF16, WS>(m, x, h, kv, p.Tpad, ws.sx, ws.sh, ws.ssc, lane, wf);
+    x = token_forward<BF16, WS>(m, x, h, kv, p.Tpad, ws.sx, ws.sh, ws.ssc, lane, wf, kv_src);
     const float lg = head_logits(m, x, ws.sx, lane);
     if (p.out.logits && lane < du) p.out.logits[((size_t)h * N + env) * du + lane] = lg;
     int a;
@@ -907,9 +827,8 @@ __global__ void __launch_bounds__(G_THREADS, GPT2_MINB_F32) gpt2_explore_exploit
   const Gpt2Dev& me = p.me;
   const Gpt2Dev& mx = p.mx;
   const WarpScratch ws = warp_scratch(g_smem, warp, p.Tpad);
-  const size_t kv_stride_e = (size_t)me.L * 2 * G_E * p.Tpad * 4, kv_stride_x = (size_t)mx.L * 2 * G_E * p.Tpad * 4;
-  char* kve = reinterpret_cast<char*>(p.kv_e) + (size_t)env * kv_stride_e;
-  char* kvx = reinterpret_cast<char*>(p.kv_x) + (size_t)env * kv_stride_x;
+  char* kve = reinterpret_cast<char*>(p.kv_e) + (size_t)env * kv_seq_bytes(me.L, p.Tpad, false);
+  char* kvx = reinterpret_cast<char*>(p.kv_x) + (size_t)env * kv_seq_bytes(mx.L, p.Tpad, false);
   const int du = me.du, K = p.K, N = p.N;
   const uint64_t gid = p.env_id0 + (uint64_t)env;
   const float mean_l = lane < du ? p.means[(size_t)env * du + lane] : -INFINITY;
@@ -930,7 +849,7 @@ __global__ void __launch_bounds__(G_THREADS, GPT2_MINB_F32) gpt2_explore_exploit
     // ---- explorer: logits at position h, sampled arm (recorded) -----------------------------
     float x = ee_bias + ee_state + __ldg(me.wpe + (size_t)h * G_E + lane);
     if (h > 0) x += __ldg(me.embed_wT + (1 + a_prev) * G_E + lane) + ee_next + ee_rew * r_prev;
-    x = token_forward<false, false>(me, x, h, kve, p.Tpad, ws.sx, ws.sh, ws.ssc, lane);
+    x = token_forward<false>(me, x, h, kve, p.Tpad, ws.sx, ws.sh, ws.ssc, lane);
     const float lge = head_logits(me, x, ws.sx, lane);
     if (p.out.logits_explorer && lane < du) p.out.logits_explorer[((size_t)h * N + env) * du + lane] = lge;
     const uint4 w = philox_words(p.key, gid, (uint32_t)h, STREAM_CTRL);
@@ -957,7 +876,7 @@ __global__ void __launch_bounds__(G_THREADS, GPT2_MINB_F32) gpt2_explore_exploit
     // ---- exploiter: logits at position h, cross-entropy against the optimal arm --------------
     float y = ex_bias + ex_state + __ldg(mx.wpe + (size_t)h * G_E + lane);
     if (h > 0) y += __ldg(mx.embed_wT + (1 + a_prev) * G_E + lane) + ex_next + ex_rew * r_prev;
-    y = token_forward<false, false>(mx, y, h, kvx, p.Tpad, ws.sx, ws.sh, ws.ssc, lane);
+    y = token_forward<false>(mx, y, h, kvx, p.Tpad, ws.sx, ws.sh, ws.ssc, lane);
     const float lgx = head_logits(mx, y, ws.sx, lane);
     if (p.out.logits_exploiter && lane < du) p.out.logits_exploiter[((size_t)h * N + env) * du + lane] = lgx;
     const float lmx = warp_max(lane < du ? lgx : -INFINITY);
@@ -1104,17 +1023,22 @@ extern "C" int dpt_gpt2_destroy(dpt_gpt2_t* m) {
 
 extern "C" uint64_t dpt_gpt2_forward_workspace_bytes(const dpt_gpt2_t* m, int B, int T, int precision) {
   if (!m || B <= 0 || T < 0) return 0;
-  return (uint64_t)B * m->dev.L * 2 * G_E * tpad_for(T + 1, precision) * (precision ? 2 : 4);
+  return (uint64_t)B * kv_seq_bytes(m->dev.L, tpad_for(T + 1, precision), precision);
 }
 
-static int launch_smem(const void* kern, size_t smem) {
+// Launch `kern` (one instantiation of a kernel template) with `smem` bytes of dynamic shared memory, raising the
+// kernel's shared-memory limit first when that is over the default 48 KB
+template <class P>
+static int launch(void (*kern)(P), int blocks, int threads, size_t smem, void* stream, const P& p) {
   if (smem > 48 * 1024) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) {
       set_error("sequence too long for the per-warp score scratch (%zu B of shared memory): %s", smem, cudaGetErrorString(e));
       return DPT_ERR_INVALID_ARG;
     }
   }
+  kern<<<blocks, threads, smem, (cudaStream_t)stream>>>(p);
+  DPT_LAUNCH_CHECK();
   return DPT_OK;
 }
 
@@ -1146,16 +1070,8 @@ extern "C" int dpt_gpt2_forward(dpt_gpt2_t* m, const float* query_states, const 
   p.query = query_states, p.cs = ctx_states, p.ca = ctx_actions, p.cns = ctx_next_states, p.cr = ctx_rewards;
   p.B = B, p.T = T, p.Ts = T_stride, p.test = test, p.Tpad = tpad_for(T + 1, precision), p.share = ctx_share;
   p.out = out, p.kv = workspace;
-  const size_t smem = (size_t)G_WARPS * (G_E + G_FF + p.Tpad) * sizeof(float);
-  const void* kern = precision ? (const void*)gpt2_forward_kernel<true> : (const void*)gpt2_forward_kernel<false>;
-  int rc = launch_smem(kern, smem);
-  if (rc != DPT_OK) return rc;
-  if (precision)
-    gpt2_forward_kernel<true><<<(B + G_WARPS - 1) / G_WARPS, G_THREADS, smem, (cudaStream_t)stream>>>(p);
-  else
-    gpt2_forward_kernel<false><<<(B + G_WARPS - 1) / G_WARPS, G_THREADS, smem, (cudaStream_t)stream>>>(p);
-  DPT_LAUNCH_CHECK();
-  return DPT_OK;
+  return launch(precision ? gpt2_forward_kernel<true> : gpt2_forward_kernel<false>, (B + G_WARPS - 1) / G_WARPS, G_THREADS,
+                G_WARPS * warp_scratch_bytes(p.Tpad), stream, p);
 }
 
 extern "C" int dpt_gpt2_decode_step(dpt_gpt2_t* m, const float* tokens, int N, int pos, int T_max, int precision, void* kv_cache,
@@ -1170,21 +1086,13 @@ extern "C" int dpt_gpt2_decode_step(dpt_gpt2_t* m, const float* tokens, int N, i
   StepParams p{};
   p.m = m->dev;
   p.tokens = tokens, p.N = N, p.pos = pos, p.Tpad = tpad_for(T_max, precision), p.out = logits, p.kv = kv_cache;
-  const size_t smem = (size_t)G_WARPS * (G_E + G_FF + p.Tpad) * sizeof(float);
-  const void* kern = precision ? (const void*)gpt2_decode_step_kernel<true> : (const void*)gpt2_decode_step_kernel<false>;
-  int rc = launch_smem(kern, smem);
-  if (rc != DPT_OK) return rc;
-  if (precision)
-    gpt2_decode_step_kernel<true><<<(N + G_WARPS - 1) / G_WARPS, G_THREADS, smem, (cudaStream_t)stream>>>(p);
-  else
-    gpt2_decode_step_kernel<false><<<(N + G_WARPS - 1) / G_WARPS, G_THREADS, smem, (cudaStream_t)stream>>>(p);
-  DPT_LAUNCH_CHECK();
-  return DPT_OK;
+  return launch(precision ? gpt2_decode_step_kernel<true> : gpt2_decode_step_kernel<false>, (N + G_WARPS - 1) / G_WARPS, G_THREADS,
+                G_WARPS * warp_scratch_bytes(p.Tpad), stream, p);
 }
 
 extern "C" uint64_t dpt_gpt2_online_kv_bytes(const dpt_gpt2_t* m, int N, int H, int precision) {
   if (!m || N <= 0 || H <= 0) return 0;
-  return (uint64_t)N * m->dev.L * 2 * G_E * tpad_for(H, precision) * (precision ? 2 : 4);
+  return (uint64_t)N * kv_seq_bytes(m->dev.L, tpad_for(H, precision), precision);
 }
 
 extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double var, int reward_type, int sample, uint64_t seed,
@@ -1215,17 +1123,13 @@ extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double va
   p.cum_means = cum_means, p.regret = regret_sums;
   if (inject) p.in = *inject;
   if (dump) p.out = *dump;
-  const size_t per_warp = (size_t)(G_E + G_FF + p.Tpad) * sizeof(float);
+  const size_t per_warp = warp_scratch_bytes(p.Tpad);
   const size_t smem_ws = (size_t)m->dev.L * WF_UINT4 * 16 + GW_WARPS * per_warp;
   if (precision && smem_ws <= 227 * 1024) {   // weight fragments of all layers + 24 warps' scratch fit one SM
-    int rc = launch_smem((const void*)gpt2_online_kernel<true, true>, smem_ws);
-    if (rc != DPT_OK) return rc;
     // one CTA per SM: keep the wave count of 24-warp CTAs but spread the envs evenly over those waves
     const long per_wave = (long)sm_count() * GW_WARPS, waves = (N + per_wave - 1) / per_wave;
     const int nw = (int)std::min<long>(GW_WARPS, std::max<long>(1, (N + waves * sm_count() - 1) / (waves * sm_count())));
-    gpt2_online_kernel<true, true><<<(N + nw - 1) / nw, nw * 32, smem_ws, (cudaStream_t)stream>>>(p);
-    DPT_LAUNCH_CHECK();
-    return DPT_OK;
+    return launch(gpt2_online_kernel<true, true>, (N + nw - 1) / nw, nw * 32, smem_ws, stream, p);
   }
   // fp32 K/V staged by bulk-async copies (cp.async.bulk + mbarrier ring per warp) when the batch leaves warp slots empty
   // (fewer than ~36 env-warps per SM): there the register-staged kernel cannot keep enough bytes in flight (0.43 of the HBM
@@ -1236,22 +1140,10 @@ extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double va
     // 4-warp CTAs would put 12 warps on some SMs and 8 on the others)
     const int nw = env_warps_per_sm <= 12 ? 1 : (env_warps_per_sm <= 20 ? 2 : TMA_WARPS);
     const size_t smem_tma = (size_t)nw * (KV_STAGES * (KV_TILE_BYTES + 8) + per_warp) + 8;
-    int rc = launch_smem((const void*)gpt2_online_kernel<false, false, true>, smem_tma);
-    if (rc != DPT_OK) return rc;
-    gpt2_online_kernel<false, false, true><<<(N + nw - 1) / nw, nw * 32, smem_tma, (cudaStream_t)stream>>>(p);
-    DPT_LAUNCH_CHECK();
-    return DPT_OK;
+    return launch(gpt2_online_kernel<false, false, true>, (N + nw - 1) / nw, nw * 32, smem_tma, stream, p);
   }
-  const size_t smem = G_WARPS * per_warp;
-  const void* kern = precision ? (const void*)gpt2_online_kernel<true, false> : (const void*)gpt2_online_kernel<false, false>;
-  int rc = launch_smem(kern, smem);
-  if (rc != DPT_OK) return rc;
-  if (precision)
-    gpt2_online_kernel<true, false><<<(N + G_WARPS - 1) / G_WARPS, G_THREADS, smem, (cudaStream_t)stream>>>(p);
-  else
-    gpt2_online_kernel<false, false><<<(N + G_WARPS - 1) / G_WARPS, G_THREADS, smem, (cudaStream_t)stream>>>(p);
-  DPT_LAUNCH_CHECK();
-  return DPT_OK;
+  return launch(precision ? gpt2_online_kernel<true, false> : gpt2_online_kernel<false, false>, (N + G_WARPS - 1) / G_WARPS, G_THREADS,
+                G_WARPS * per_warp, stream, p);
 }
 
 extern "C" int dpt_gpt2_explore_exploit_rollout(dpt_gpt2_t* explorer, dpt_gpt2_t* exploiter, const float* means, double var, int reward_type,
@@ -1282,10 +1174,5 @@ extern "C" int dpt_gpt2_explore_exploit_rollout(dpt_gpt2_t* explorer, dpt_gpt2_t
   p.ctx_s = ctx_states, p.ctx_a = ctx_actions, p.ctx_ns = ctx_next_states, p.ctx_r = ctx_rewards, p.adv = advantages;
   if (inject) p.in = *inject;
   if (dump) p.out = *dump;
-  const size_t smem = (size_t)G_WARPS * (G_E + G_FF + p.Tpad) * sizeof(float);
-  int rc = launch_smem((const void*)gpt2_explore_exploit_kernel, smem);
-  if (rc != DPT_OK) return rc;
-  gpt2_explore_exploit_kernel<<<(N + G_WARPS - 1) / G_WARPS, G_THREADS, smem, (cudaStream_t)stream>>>(p);
-  DPT_LAUNCH_CHECK();
-  return DPT_OK;
+  return launch(gpt2_explore_exploit_kernel, (N + G_WARPS - 1) / G_WARPS, G_THREADS, G_WARPS * warp_scratch_bytes(p.Tpad), stream, p);
 }
