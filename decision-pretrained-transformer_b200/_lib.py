@@ -10,7 +10,7 @@ from ctypes import (POINTER, Structure, c_char_p, c_double, c_float, c_int, c_in
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DPT_B200_LIB") or os.path.join(_HERE, "libdpt_b200.so")   # override: A/B builds of the same ABI
-ABI_VERSION = 7
+ABI_VERSION = 8
 
 OK, ERR_INVALID_ARG, ERR_CUDA, ERR_UNSUPPORTED = 0, -1, -2, -3
 
@@ -150,6 +150,10 @@ PROTOTYPES = {
     "dpt_gpt2_online_loop": (c_int, [c_void_p, c_void_p, c_double, c_int, c_int, c_uint64, c_uint64, c_int, c_int, c_int,
                                      c_void_p, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                      POINTER(Gpt2OnlineInject), POINTER(Gpt2OnlineDump), c_void_p]),
+    "dpt_gpt2_online_loop_population": (c_int, [POINTER(c_void_p), c_int, c_void_p, c_double, c_int, c_int, c_uint64, c_uint64,
+                                                c_int, c_int, c_int, c_void_p, c_uint64, POINTER(c_void_p), POINTER(c_void_p),
+                                                POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p),
+                                                POINTER(Gpt2OnlineInject), POINTER(Gpt2OnlineDump), c_void_p]),
     "dpt_gpt2_explore_exploit_rollout": (c_int, [c_void_p, c_void_p, c_void_p, c_double, c_int, c_uint64, c_uint64, c_int, c_int,
                                                  c_void_p, c_void_p, c_uint64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                                  POINTER(ExploreInject), POINTER(ExploreDump), c_void_p]),

@@ -650,7 +650,36 @@ __global__ void __launch_bounds__(G_THREADS) gpt2_decode_step_kernel(const StepP
 // ---------------------------------------------------------------------------------------------
 // Fused bandit online loop with the transformer controller
 // ---------------------------------------------------------------------------------------------
+// The online loop's launch parameters.  NM: member capacity of the launch -- 1 for dpt_gpt2_online_loop and one-member
+// population calls, ONLINE_POP_MAX for dpt_gpt2_online_loop_population, whose CTA (env block, member = blockIdx.y) takes
+// its member's weights, K/V region and outputs from a table in the kernel parameters (no upload, graph-capturable).  The
+// means, noise and inject arrays are shared: member i computes exactly what a one-model call on its own weights would.
+constexpr int ONLINE_POP_MAX = DPT_GPT2_ONLINE_POPULATION_MAX;
+struct OnlineMember {   // what differs between the members of a population launch
+  Gpt2Dev m;
+  void* kv;
+  float *ctx_s, *ctx_a, *ctx_ns, *ctx_r, *cum_means;
+  double* regret;
+  dpt_gpt2_online_dump_t out;
+};
+template <int NM>
 struct OnlineGptParams {
+  const float* means;
+  double var;
+  int rtype;   // DPT_REWARD_*
+  int sample;
+  Key key;
+  uint64_t env_id0;
+  int N, H, Tpad;
+  dpt_gpt2_online_inject_t in;
+  OnlineMember mem[NM];
+  __device__ __forceinline__ const OnlineMember& member() const { return mem[blockIdx.y]; }
+  OnlineMember& slot(int i) { return mem[i]; }
+};
+static_assert(sizeof(OnlineGptParams<ONLINE_POP_MAX>) <= 32764, "population table exceeds the kernel parameter limit");
+// one model: the fields of OnlineMember and the shared ones in one block (the layout the one-model kernels were tuned with)
+template <>
+struct OnlineGptParams<1> {
   Gpt2Dev m;
   const float* means;
   double var;
@@ -664,6 +693,8 @@ struct OnlineGptParams {
   double* regret;
   dpt_gpt2_online_inject_t in;
   dpt_gpt2_online_dump_t out;
+  __device__ __forceinline__ const OnlineGptParams& member() const { return *this; }
+  OnlineGptParams& slot(int) { return *this; }
 };
 
 // WS (precision 1): ONE CTA of GW_WARPS warps per SM shares the bf16 weight fragments of all layers in shared memory
@@ -672,13 +703,14 @@ constexpr int GW_WARPS = 24;
 constexpr int GW_THREADS = GW_WARPS * 32;
 
 // TMA (precision 0 only): the fp32 K/V stream is staged through a per-warp ring of bulk-async copies (KvRing)
-template <bool BF16, bool WS, bool TMA = false>
+template <bool BF16, bool WS, bool TMA = false, int NM = 1>
 __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_THREADS),
                                   WS ? 1 : (TMA ? TMA_MINB : (BF16 ? GPT2_MINB_BF16 : GPT2_MINB_F32)))
-    gpt2_online_kernel(const OnlineGptParams p) {
+    gpt2_online_kernel(const __grid_constant__ OnlineGptParams<NM> p) {
   extern __shared__ __align__(128) float g_smem[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const Gpt2Dev& m = p.m;
+  const auto& mb = p.member();   // this CTA's member
+  const Gpt2Dev& m = mb.m;
   const uint4* wf = nullptr;
   float* scratch = g_smem;
   std::conditional_t<TMA, KvRing, GlobalKv> kv_src;
@@ -707,16 +739,16 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
   const int env = blockIdx.x * (int)(blockDim.x >> 5) + warp;   // WS: the host picks <= GW_WARPS warps per CTA
   if (env >= p.N) return;
   const WarpScratch ws = warp_scratch(scratch, warp, p.Tpad);
-  char* kv = reinterpret_cast<char*>(p.kv) + (size_t)env * kv_seq_bytes(m.L, p.Tpad, BF16);
+  char* kv = reinterpret_cast<char*>(mb.kv) + (size_t)env * kv_seq_bytes(m.L, p.Tpad, BF16);
   if constexpr (TMA) kv_src.kv = reinterpret_cast<const float*>(kv);
   const int du = m.du, H = p.H, N = p.N;
   const uint64_t gid = p.env_id0 + (uint64_t)env;
   const float mean_l = lane < du ? p.means[(size_t)env * du + lane] : -INFINITY;
   const float mmax = warp_max(mean_l);
-  if (p.ctx_s) {
+  if (mb.ctx_s) {
     for (int h = lane; h < H; h += 32) {
-      p.ctx_s[(size_t)env * H + h] = 1.0f;
-      p.ctx_ns[(size_t)env * H + h] = 1.0f;
+      mb.ctx_s[(size_t)env * H + h] = 1.0f;
+      mb.ctx_ns[(size_t)env * H + h] = 1.0f;
     }
   }
   // constant part of every token: bias + state (== 1) column (+ next_state column for context tokens)
@@ -732,7 +764,7 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
     if (h > 0) x += __ldg(m.embed_wT + (1 + a_prev) * G_E + lane) + e_next + e_rew * r_prev;
     x = token_forward<BF16, WS>(m, x, h, kv, p.Tpad, ws.sx, ws.sh, ws.ssc, lane, wf, kv_src);
     const float lg = head_logits(m, x, ws.sx, lane);
-    if (p.out.logits && lane < du) p.out.logits[((size_t)h * N + env) * du + lane] = lg;
+    if (mb.out.logits && lane < du) mb.out.logits[((size_t)h * N + env) * du + lane] = lg;
     int a;
     if (p.sample) {
       // scipy.special.softmax (float64) + np.random.choice(p): cdf = cumsum(p) / cdf[-1]; searchsorted(u, 'right')
@@ -756,7 +788,7 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
         const uint4 w = philox_words(p.key, gid, (uint32_t)h, STREAM_CTRL);
         u = ((double)(w.x >> 5) * 67108864.0 + (double)(w.y >> 6)) * (1.0 / 9007199254740992.0);
       }
-      if (p.out.ctrl_u && lane == 0) p.out.ctrl_u[(size_t)h * N + env] = u;
+      if (mb.out.ctrl_u && lane == 0) mb.out.ctrl_u[(size_t)h * N + env] = u;
       a = __popc(__ballot_sync(0xffffffffu, lane < du - 1 && cdf <= u));
     } else {  // np.argmax: first maximum
       const float lm = warp_max(lane < du ? lg : -INFINITY);
@@ -778,17 +810,17 @@ __global__ void __launch_bounds__(WS ? GW_THREADS : (TMA ? TMA_WARPS * 32 : G_TH
     const float r = p.rtype == DPT_REWARD_GAUSSIAN ? (float)((double)ma + (0.0 + p.var * (double)z))   // envs/bandit_env.py:59
                                                    : (z < ma ? 1.f : 0.f);                             // :61 Bernoulli(mean)
     if (lane == 0) {
-      if (p.out.reward_z) p.out.reward_z[(size_t)h * N + env] = z;
-      if (p.cum_means) p.cum_means[(size_t)h * N + env] = ma;
-      if (p.regret) {
+      if (mb.out.reward_z) mb.out.reward_z[(size_t)h * N + env] = z;
+      if (mb.cum_means) mb.cum_means[(size_t)h * N + env] = ma;
+      if (mb.regret) {
         const double reg = (double)mmax - (double)ma;
         creg += reg;
-        double* dst = p.regret + 4 * (size_t)h;
+        double* dst = mb.regret + 4 * (size_t)h;
         atomicAdd(dst, reg), atomicAdd(dst + 1, reg * reg), atomicAdd(dst + 2, creg), atomicAdd(dst + 3, creg * creg);
       }
-      if (p.ctx_r) p.ctx_r[(size_t)env * H + h] = r;
+      if (mb.ctx_r) mb.ctx_r[(size_t)env * H + h] = r;
     }
-    if (p.ctx_a && lane < du) p.ctx_a[((size_t)env * H + h) * du + lane] = (lane == a) ? 1.f : 0.f;
+    if (mb.ctx_a && lane < du) mb.ctx_a[((size_t)env * H + h) * du + lane] = (lane == a) ? 1.f : 0.f;
     a_prev = a;
     r_prev = r;
   }
@@ -1029,7 +1061,7 @@ extern "C" uint64_t dpt_gpt2_forward_workspace_bytes(const dpt_gpt2_t* m, int B,
 // Launch `kern` (one instantiation of a kernel template) with `smem` bytes of dynamic shared memory, raising the
 // kernel's shared-memory limit first when that is over the default 48 KB
 template <class P>
-static int launch(void (*kern)(P), int blocks, int threads, size_t smem, void* stream, const P& p) {
+static int launch(void (*kern)(P), dim3 blocks, int threads, size_t smem, void* stream, const P& p) {
   if (smem > 48 * 1024) {
     cudaError_t e = cudaFuncSetAttribute((const void*)kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) {
@@ -1095,6 +1127,36 @@ extern "C" uint64_t dpt_gpt2_online_kv_bytes(const dpt_gpt2_t* m, int N, int H, 
   return (uint64_t)N * kv_seq_bytes(m->dev.L, tpad_for(H, precision), precision);
 }
 
+// Launch the online loop for members 0 .. n-1 of `p` (n = 1: the one-model call).  The kernel variant and the CTA size
+// follow from the launch's total env-warps n * N: WS when the bf16 weight fragments fit, the bulk-copy ring at <= 24 fp32
+// env-warps per SM, register-staged loads otherwise.  Every draw is keyed by (seed, env id, step), so a member's result
+// does not depend on the variant.  Grid: (env blocks, member).
+template <int NM>
+static int online_launch(const OnlineGptParams<NM>& p, int n, int L, int precision, void* stream) {
+  const long N = p.N, total = (long)n * p.N;
+  const size_t per_warp = warp_scratch_bytes(p.Tpad);
+  const size_t smem_ws = (size_t)L * WF_UINT4 * 16 + GW_WARPS * per_warp;
+  if (precision && smem_ws <= 227 * 1024) {   // weight fragments of all layers + 24 warps' scratch fit one SM
+    // one CTA per SM: keep the wave count of 24-warp CTAs but spread the envs evenly over those waves
+    const long per_wave = (long)sm_count() * GW_WARPS, waves = (total + per_wave - 1) / per_wave;
+    const int nw = (int)std::min<long>(GW_WARPS, std::max<long>(1, (total + waves * sm_count() - 1) / (waves * sm_count())));
+    return launch(gpt2_online_kernel<true, true, false, NM>, dim3((N + nw - 1) / nw, n), nw * 32, smem_ws, stream, p);
+  }
+  // fp32 K/V staged by bulk-async copies (cp.async.bulk + mbarrier ring per warp) when the batch leaves warp slots empty
+  // (fewer than ~36 env-warps per SM): there the register-staged kernel cannot keep enough bytes in flight (0.43 of the HBM
+  // bound at 1250 envs) and a ring can (0.8+)
+  const long env_warps_per_sm = (total + sm_count() - 1) / sm_count();
+  if (!precision && env_warps_per_sm <= 24) {
+    // CTA size: small batches get small CTAs so that the SMs carry equal numbers of warps (1250 envs = 8.4 warps per SM:
+    // 4-warp CTAs would put 12 warps on some SMs and 8 on the others)
+    const int nw = env_warps_per_sm <= 12 ? 1 : (env_warps_per_sm <= 20 ? 2 : TMA_WARPS);
+    const size_t smem_tma = (size_t)nw * (KV_STAGES * (KV_TILE_BYTES + 8) + per_warp) + 8;
+    return launch(gpt2_online_kernel<false, false, true, NM>, dim3((N + nw - 1) / nw, n), nw * 32, smem_tma, stream, p);
+  }
+  return launch(precision ? gpt2_online_kernel<true, false, false, NM> : gpt2_online_kernel<false, false, false, NM>,
+                dim3((N + G_WARPS - 1) / G_WARPS, n), G_THREADS, G_WARPS * per_warp, stream, p);
+}
+
 extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double var, int reward_type, int sample, uint64_t seed,
                                     uint64_t env_id0, int N, int H, int precision, void* kv_cache, uint64_t kv_bytes,
                                     float* ctx_states, float* ctx_actions, float* ctx_next_states, float* ctx_rewards,
@@ -1112,7 +1174,7 @@ extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double va
   const bool any = ctx_states || ctx_actions || ctx_next_states || ctx_rewards;
   DPT_CHECK_ARG(!any || (ctx_states && ctx_actions && ctx_next_states && ctx_rewards),
                 "dpt_gpt2_online_loop: context pointers must be all NULL or all non-NULL");
-  OnlineGptParams p{};
+  OnlineGptParams<1> p{};
   p.m = m->dev;
   p.means = means, p.var = var, p.rtype = reward_type, p.sample = sample;
   p.key = Key{(uint32_t)seed, (uint32_t)(seed >> 32)};
@@ -1123,27 +1185,63 @@ extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double va
   p.cum_means = cum_means, p.regret = regret_sums;
   if (inject) p.in = *inject;
   if (dump) p.out = *dump;
-  const size_t per_warp = warp_scratch_bytes(p.Tpad);
-  const size_t smem_ws = (size_t)m->dev.L * WF_UINT4 * 16 + GW_WARPS * per_warp;
-  if (precision && smem_ws <= 227 * 1024) {   // weight fragments of all layers + 24 warps' scratch fit one SM
-    // one CTA per SM: keep the wave count of 24-warp CTAs but spread the envs evenly over those waves
-    const long per_wave = (long)sm_count() * GW_WARPS, waves = (N + per_wave - 1) / per_wave;
-    const int nw = (int)std::min<long>(GW_WARPS, std::max<long>(1, (N + waves * sm_count() - 1) / (waves * sm_count())));
-    return launch(gpt2_online_kernel<true, true>, (N + nw - 1) / nw, nw * 32, smem_ws, stream, p);
+  return online_launch(p, 1, m->dev.L, precision, stream);
+}
+
+extern "C" int dpt_gpt2_online_loop_population(dpt_gpt2_t* const* models, int n_models, const float* means, double var,
+                                               int reward_type, int sample, uint64_t seed, uint64_t env_id0, int N, int H,
+                                               int precision, void* kv_cache, uint64_t kv_bytes, float* const* ctx_states,
+                                               float* const* ctx_actions, float* const* ctx_next_states,
+                                               float* const* ctx_rewards, float* const* cum_means, double* const* regret_sums,
+                                               const dpt_gpt2_online_inject_t* inject, const dpt_gpt2_online_dump_t* dump,
+                                               void* stream) {
+  const char* fn = "dpt_gpt2_online_loop_population";
+  DPT_CHECK_ARG(n_models >= 0 && n_models <= ONLINE_POP_MAX, "%s: n_models=%d outside [0,%d]", fn, n_models, ONLINE_POP_MAX);
+  if (n_models == 0) return DPT_OK;
+  DPT_CHECK_ARG(models, "%s: null models array", fn);
+  DPT_CHECK_ARG(reward_type == DPT_REWARD_GAUSSIAN || reward_type == DPT_REWARD_BERNOULLI,
+                "%s: unknown reward_type %d (0 uniform/gaussian, 1 bernoulli)", fn, reward_type);
+  DPT_CHECK_ARG(precision == 0 || precision == 1, "%s: precision %d (0 = fp32, 1 = bf16 K/V cache)", fn, precision);
+  DPT_CHECK_ARG(N >= 0 && H >= 0, "%s: N=%d H=%d", fn, N, H);
+  auto at = [](auto* const* a, int i) { return a ? a[i] : nullptr; };
+  for (int i = 0; i < n_models; ++i) {
+    DPT_CHECK_ARG(models[i], "%s: member %d is a null model", fn, i);
+    const Gpt2Dev &d = models[i]->dev, &d0 = models[0]->dev;
+    DPT_CHECK_ARG(d.dx == 1, "%s: member %d has state_dim=%d, the bandit loop needs 1", fn, i, d.dx);
+    const struct { const char* name; int v, v0; } f[] = {{"n_layer", d.L, d0.L}, {"action_dim", d.du, d0.du}};
+    for (const auto& x : f)
+      DPT_CHECK_ARG(x.v == x.v0, "%s: member %d has %s=%d, member 0 has %d (members must share one shape)", fn, i, x.name, x.v,
+                    x.v0);
+    DPT_CHECK_ARG(H <= d.n_pos, "%s: member %d: H=%d exceeds n_positions %d", fn, i, H, d.n_pos);
+    const int set = !!at(ctx_states, i) + !!at(ctx_actions, i) + !!at(ctx_next_states, i) + !!at(ctx_rewards, i);
+    DPT_CHECK_ARG(set == 0 || set == 4, "%s: member %d: context pointers must be all NULL or all non-NULL", fn, i);
   }
-  // fp32 K/V staged by bulk-async copies (cp.async.bulk + mbarrier ring per warp) when the batch leaves warp slots empty
-  // (fewer than ~36 env-warps per SM): there the register-staged kernel cannot keep enough bytes in flight (0.43 of the HBM
-  // bound at 1250 envs) and a ring can (0.8+)
-  const long env_warps_per_sm = ((long)N + sm_count() - 1) / sm_count();
-  if (!precision && env_warps_per_sm <= 24) {
-    // CTA size: small batches get small CTAs so that the SMs carry equal numbers of warps (1250 envs = 8.4 warps per SM:
-    // 4-warp CTAs would put 12 warps on some SMs and 8 on the others)
-    const int nw = env_warps_per_sm <= 12 ? 1 : (env_warps_per_sm <= 20 ? 2 : TMA_WARPS);
-    const size_t smem_tma = (size_t)nw * (KV_STAGES * (KV_TILE_BYTES + 8) + per_warp) + 8;
-    return launch(gpt2_online_kernel<false, false, true>, (N + nw - 1) / nw, nw * 32, smem_tma, stream, p);
+  if (N == 0 || H == 0) return DPT_OK;
+  const uint64_t per = dpt_gpt2_online_kv_bytes(models[0], N, H, precision);
+  DPT_CHECK_ARG(means && kv_cache && kv_bytes / n_models >= per, "%s: null means, or kv cache of %llu B below %d x %llu B", fn,
+                (unsigned long long)kv_bytes, n_models, (unsigned long long)per);
+  auto fill = [&](auto& p) {
+    p.means = means, p.var = var, p.rtype = reward_type, p.sample = sample;
+    p.key = Key{(uint32_t)seed, (uint32_t)(seed >> 32)};
+    p.env_id0 = env_id0;
+    p.N = N, p.H = H, p.Tpad = tpad_for(H, precision);
+    if (inject) p.in = *inject;
+    for (int i = 0; i < n_models; ++i) {
+      auto& mb = p.slot(i);
+      mb.m = models[i]->dev;
+      mb.kv = static_cast<char*>(kv_cache) + i * per;
+      mb.ctx_s = at(ctx_states, i), mb.ctx_a = at(ctx_actions, i), mb.ctx_ns = at(ctx_next_states, i), mb.ctx_r = at(ctx_rewards, i);
+      mb.cum_means = at(cum_means, i), mb.regret = at(regret_sums, i);
+      if (dump) mb.out = dump[i];
+    }
+    return online_launch(p, n_models, models[0]->dev.L, precision, stream);
+  };
+  if (n_models == 1) {   // the one-model kernels and parameter block
+    OnlineGptParams<1> p{};
+    return fill(p);
   }
-  return launch(precision ? gpt2_online_kernel<true, false> : gpt2_online_kernel<false, false>, (N + G_WARPS - 1) / G_WARPS, G_THREADS,
-                G_WARPS * per_warp, stream, p);
+  OnlineGptParams<ONLINE_POP_MAX> p{};
+  return fill(p);
 }
 
 extern "C" int dpt_gpt2_explore_exploit_rollout(dpt_gpt2_t* explorer, dpt_gpt2_t* exploiter, const float* means, double var, int reward_type,

@@ -133,6 +133,37 @@ def online(eval_trajs, model, n_eval, horizon, var, bandit_type="uniform"):
     return all_means, regret_stats(all_means)
 
 
+def online_population(eval_trajs, models, n_eval, horizon, var, bandit_type="uniform"):
+    """``online`` for a population of same-shape models (seeds, learning rates, saved epochs): Opt, EmpMean(online),
+    UCB(1.0) and Thompson run once and their arrays are shared by every member's dict; the transformer loop of all
+    members runs in population launches (models.net.online_loop_population) with ONE key for the whole population, so
+    every member sees the same tasks and the same noise.  Keys are drawn in ``online``'s order (opt, Lnr, Emp, UCB,
+    Thomp): member i's result equals ``online(eval_trajs, models[i], ...)`` started from the same rng state, bit for bit.
+    Returns (list of all_means dicts, list of regret statistics), one per member."""
+    from ..models.net import online_loop_population
+    envs = [BanditEnv(eval_trajs[i]["means"], horizon, var=var) for i in range(n_eval)]
+    vec_env = BanditEnvVec(envs)
+    models = list(models)
+    ctrls = [BanditTransformerController(m, sample=True, batch_size=len(envs)) for m in models]
+    if any(_fusable(vec_env, c) is None for c in ctrls):
+        raise NotImplementedError("online_population: every member needs the fused transformer loop (state_dim == 1)")
+    shared = {"opt": deploy_online_vec(vec_env, OptPolicy(envs, batch_size=len(envs)), horizon).T}
+    lnr = online_loop_population(models, vec_env.means, horizon, float(envs[0].var), True, rng.next_key(), 0, materialise=False,
+                                 regret=False, reward_type=envs[0].type)
+    for name, c in (("Emp", EmpMeanPolicy(envs[0], online=True, batch_size=len(envs))),
+                    ("UCB1.0", UCBPolicy(envs[0], const=1.0, batch_size=len(envs))),
+                    ("Thomp", ThompsonSamplingPolicy(envs[0], std=var, sample=True, prior_mean=0.5, prior_var=1 / 12.0,
+                                                     warm_start=False, batch_size=len(envs)))):
+        shared[name] = deploy_online_vec(vec_env, c, horizon).T
+    all_means = []
+    for out in lnr:
+        am = {"opt": shared["opt"], "Lnr": out["cum_means"].cpu().numpy().astype(np.float64).T}
+        am.update((k, shared[k]) for k in ("Emp", "UCB1.0", "Thomp"))
+        assert am["Lnr"].shape[0] == n_eval
+        all_means.append(am)
+    return all_means, [regret_stats(am) for am in all_means]
+
+
 def offline(eval_trajs, model, n_eval, horizon, var, bandit_type="uniform", np_random_compat=False):
     """evals/eval_bandit.py:214-301 without the bar plot: every controller sees the first ``horizon``
     context rows of each eval trajectory and plays ONE noise-free pull (deploy_eval); returns the dict

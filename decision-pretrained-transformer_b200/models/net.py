@@ -208,53 +208,13 @@ class Transformer(nn.Module):
         return _Decoder(self, n_seqs, self.horizon if max_transitions is None else max_transitions)
 
     # ---- fused in-context evaluation loop ---------------------------------------------------
-    @torch.no_grad()
     def online_loop(self, means, horizon, var, sample, seed, env_id0=0, materialise=True, regret=True, inject=None,
                     dump=False, reward_type="uniform"):
         """deploy_online_vec with BanditTransformerController in one launch (KV-cached decode +
-        sampling + env step).  Returns the same dict as kernels.online_loop."""
-        dev = kernels._dev()
-        h = self.handle()
-        means = kernels._as(means, torch.float32, dev)
-        N, d = means.shape
-        assert d == self.action_dim
-        H = horizon
-        out = {"cum_means": torch.empty((H, N), dtype=torch.float32, device=dev)}
-        if regret:
-            out["regret_sums"] = torch.zeros((H, 4), dtype=torch.float64, device=dev)
-        if materialise:
-            out.update(context_states=torch.empty((N, H, 1), dtype=torch.float32, device=dev),
-                       context_actions=torch.empty((N, H, d), dtype=torch.float32, device=dev),
-                       context_next_states=torch.empty((N, H, 1), dtype=torch.float32, device=dev),
-                       context_rewards=torch.empty((N, H, 1), dtype=torch.float32, device=dev))
-        kv_bytes = lib().dpt_gpt2_online_kv_bytes(h, N, H, self.precision)
-        kv = self._scratch(kv_bytes)
-        inj_p, dump_p, keep = None, None, []
-        if inject is not None:
-            s = _lib.Gpt2OnlineInject()
-            for k, dt in (("reward_z", torch.float32), ("ctrl_u", torch.float64)):
-                if inject.get(k) is not None:
-                    t = kernels._as(inject[k], dt, dev)
-                    keep.append(t)
-                    setattr(s, k, ptr(t))
-            inj_p = ctypes.byref(s)
-        noise = None
-        if dump:
-            noise = {"reward_z": torch.empty((H, N), dtype=torch.float32, device=dev),
-                     "ctrl_u": torch.zeros((H, N), dtype=torch.float64, device=dev),
-                     "logits": torch.empty((H, N, d), dtype=torch.float32, device=dev)}
-            s2 = _lib.Gpt2OnlineDump()
-            for k, t in noise.items():
-                setattr(s2, k, ptr(t))
-            dump_p = ctypes.byref(s2)
-        check(lib().dpt_gpt2_online_loop(h, ptr(means), float(var), kernels.REWARD_TYPES[reward_type], 1 if sample else 0, seed, env_id0, N, H, self.precision, ptr(kv),
-                                         kv.numel(), ptr(out.get("context_states")), ptr(out.get("context_actions")),
-                                         ptr(out.get("context_next_states")), ptr(out.get("context_rewards")),
-                                         ptr(out["cum_means"]), ptr(out.get("regret_sums")), inj_p, dump_p, stream_ptr()),
-              "dpt_gpt2_online_loop")
-        if noise is not None:
-            out["noise"] = noise
-        return out
+        sampling + env step).  Returns the same dict as kernels.online_loop.  This is the one-member case of
+        ``online_loop_population``."""
+        return online_loop_population([self], means, horizon, var, sample, seed, env_id0, materialise, regret, inject, dump,
+                                      reward_type)[0]
 
 
 _LAYER_FIELDS = (lambda b: b.ln_1.weight, lambda b: b.ln_1.bias, lambda b: b.attn.c_attn.weight, lambda b: b.attn.c_attn.bias,
@@ -411,6 +371,91 @@ class _PopulationTrainFn(torch.autograd.Function):
                   "dpt_gpt2_train_backward" if k == 1 else "dpt_gpt2_train_population_backward")
         ctx.ws = None
         return (None, None, *[None if douts[i // n] is None else g for i, g in enumerate(grads)])
+
+
+ONLINE_POPULATION_MAX = 16              # DPT_GPT2_ONLINE_POPULATION_MAX: members per population launch of the online loop
+ONLINE_KV_LAUNCH_BYTES = 8 * 1024 ** 3   # K/V scratch one population launch may take (one member may take more on its own)
+_ONLINE_FIELDS = ("horizon", "state_dim", "action_dim", "n_layer", "precision")
+
+
+def online_launch_groups(k, kv_bytes_per_member):
+    """[(first, stop)] member ranges of the population launches for ``k`` members of ``kv_bytes_per_member`` bytes of K/V
+    scratch each: at most ONLINE_POPULATION_MAX members and ONLINE_KV_LAUNCH_BYTES of scratch per launch, at least one
+    member.  At 100 envs x H = 500 fp32 a member takes 52 MB and a launch holds 16; at 10 000 envs it takes 5.2 GB and
+    runs alone -- where one member fills the GPU, grouping gains nothing, and a population must never need more memory
+    than k one-model calls."""
+    per = max(1, min(ONLINE_POPULATION_MAX, ONLINE_KV_LAUNCH_BYTES // max(1, int(kv_bytes_per_member))))
+    return [(a, min(k, a + per)) for a in range(0, k, per)]
+
+
+@torch.no_grad()
+def online_loop_population(models, means, horizon, var, sample, seed, env_id0=0, materialise=True, regret=True, inject=None,
+                           dump=False, reward_type="uniform"):
+    """``[m.online_loop(means, horizon, ...) for m in models]`` in shared launches: the bandit online loop of several
+    same-shape Transformers on the same tasks and the same noise (same means, seed, env ids, inject).  Member i's dict is
+    bit for bit what ``models[i].online_loop`` returns alone (``regret_sums`` are float64 atomics: equal up to their order
+    of addition).  Members must agree on ``horizon``, ``state_dim``, ``action_dim``, ``n_layer``, ``precision`` and the
+    device, else ``ValueError`` naming the member and the field.  Populations are cut into launches by
+    ``online_launch_groups``."""
+    models = list(models)
+    if not models:
+        return []
+    m0 = models[0]
+    devs = [next(m.parameters()).device for m in models]
+    for i, m in enumerate(models):
+        for f in _ONLINE_FIELDS:
+            if getattr(m, f) != getattr(m0, f):
+                raise ValueError("online_loop_population: member %d has %s=%r, member 0 has %r"
+                                 % (i, f, getattr(m, f), getattr(m0, f)))
+        if devs[i] != devs[0]:
+            raise ValueError("online_loop_population: member %d is on %s, member 0 on %s" % (i, devs[i], devs[0]))
+    dev = kernels._dev()
+    hs = [m.handle() for m in models]
+    means = kernels._as(means, torch.float32, dev)
+    N, d = means.shape
+    assert d == m0.action_dim
+    H, k = horizon, len(models)
+    outs = []
+    for _ in models:
+        out = {"cum_means": torch.empty((H, N), dtype=torch.float32, device=dev)}
+        if regret:
+            out["regret_sums"] = torch.zeros((H, 4), dtype=torch.float64, device=dev)
+        if materialise:
+            out.update(context_states=torch.empty((N, H, 1), dtype=torch.float32, device=dev),
+                       context_actions=torch.empty((N, H, d), dtype=torch.float32, device=dev),
+                       context_next_states=torch.empty((N, H, 1), dtype=torch.float32, device=dev),
+                       context_rewards=torch.empty((N, H, 1), dtype=torch.float32, device=dev))
+        if dump:
+            out["noise"] = {"reward_z": torch.empty((H, N), dtype=torch.float32, device=dev),
+                            "ctrl_u": torch.zeros((H, N), dtype=torch.float64, device=dev),
+                            "logits": torch.empty((H, N, d), dtype=torch.float32, device=dev)}
+        outs.append(out)
+    inj_p, keep = None, []
+    if inject is not None:
+        s = _lib.Gpt2OnlineInject()
+        for key, dt in (("reward_z", torch.float32), ("ctrl_u", torch.float64)):
+            if inject.get(key) is not None:
+                t = kernels._as(inject[key], dt, dev)
+                keep.append(t)
+                setattr(s, key, ptr(t))
+        inj_p = ctypes.byref(s)
+    kv_bytes = lib().dpt_gpt2_online_kv_bytes(hs[0], N, H, m0.precision)
+    for a, b in online_launch_groups(k, kv_bytes):
+        n, os_ = b - a, outs[a:b]
+        # one member reuses its model's scratch, as the one-model call always has; a group takes a buffer of its own
+        kv = models[a]._scratch(kv_bytes) if n == 1 else torch.empty((max(n * int(kv_bytes), 1),), dtype=torch.uint8, device=dev)
+        arr = lambda vals: (ctypes.c_void_p * n)(*vals)   # noqa: E731
+        col = lambda key: arr([ptr(o.get(key)) for o in os_])   # noqa: E731
+        dump_p = None
+        if dump:
+            dump_p = (_lib.Gpt2OnlineDump * n)(*[_lib.Gpt2OnlineDump(**{key: ptr(t) for key, t in o["noise"].items()}) for o in os_])
+        check(lib().dpt_gpt2_online_loop_population(arr(hs[a:b]), n, ptr(means), float(var), kernels.REWARD_TYPES[reward_type],
+                                                    1 if sample else 0, seed, env_id0, N, H, m0.precision, ptr(kv), kv.numel(),
+                                                    col("context_states"), col("context_actions"), col("context_next_states"),
+                                                    col("context_rewards"), col("cum_means"), col("regret_sums"), inj_p,
+                                                    dump_p, stream_ptr()),
+              "dpt_gpt2_online_loop" if k == 1 else "dpt_gpt2_online_loop_population")
+    return outs
 
 
 class _Decoder:

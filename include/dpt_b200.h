@@ -35,7 +35,7 @@ extern "C" {
 #define DPT_ERR_CUDA (-2)
 #define DPT_ERR_UNSUPPORTED (-3)
 
-#define DPT_ABI_VERSION 7
+#define DPT_ABI_VERSION 8
 
 /* reward_type of the bandit entry points (envs/bandit_env.py:56-63, envs/gpu_bandit_env.py:53-63):
  * 0 'uniform'  : r = means[a] + var * z, z ~ N(0,1);
@@ -433,6 +433,27 @@ int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double var, int rewa
                          float* ctx_actions, float* ctx_next_states, float* ctx_rewards, float* cum_means,
                          double* regret_sums, const dpt_gpt2_online_inject_t* inject,
                          const dpt_gpt2_online_dump_t* dump, void* stream);
+
+/* Population evaluation: the online loop of n_models same-shape models (members share n_layer and action_dim, have
+ * state_dim == 1 and n_positions >= H) in one launch, on the same tasks and the same noise: member i's outputs are bit for
+ * bit those of dpt_gpt2_online_loop(models[i], ...) with the same means, var, reward_type, sample, seed, env_id0, N, H,
+ * precision and inject, whichever kernel variant the population's total of n_models * N env-warps selects (regret sums
+ * are float64 atomics: equal up to their order of addition).  models, ctx_*, cum_means, regret_sums: HOST arrays of
+ * n_models pointers (device pointers with the shapes of the one-model call); a whole array may be NULL, an entry may be
+ * NULL where the one-model call allows it, and a member's four context pointers are all NULL or all set.  dump: n_models
+ * structs or NULL.  inject is shared by every member.  kv_cache holds n_models regions of
+ * dpt_gpt2_online_kv_bytes(models[0], N, H, precision) bytes, one after another.  The per-member tables travel in the
+ * kernel parameters: no host synchronisation, no upload, capturable in a CUDA graph.
+ * 1 <= n_models <= DPT_GPT2_ONLINE_POPULATION_MAX per call; n_models = 0, N = 0 or H = 0 is a no-op.  n_models outside
+ * [0, max], null pointers, a K/V buffer that is too small and a member of another shape (the message names the member and
+ * the field) return DPT_ERR_INVALID_ARG. */
+#define DPT_GPT2_ONLINE_POPULATION_MAX 16
+int dpt_gpt2_online_loop_population(dpt_gpt2_t* const* models, int n_models, const float* means, double var, int reward_type,
+                                    int sample, uint64_t seed, uint64_t env_id0, int N, int H, int precision, void* kv_cache,
+                                    uint64_t kv_bytes, float* const* ctx_states, float* const* ctx_actions,
+                                    float* const* ctx_next_states, float* const* ctx_rewards, float* const* cum_means,
+                                    double* const* regret_sums, const dpt_gpt2_online_inject_t* inject,
+                                    const dpt_gpt2_online_dump_t* dump, void* stream);
 
 /* One decode step for callers that drive their own loop (the rollout half of train_interactive.py:97-132 /
  * train_explorer_exploiter.py:110-166, where the arm that is pulled is chosen outside): append the token of position
