@@ -10,7 +10,7 @@ from ctypes import (POINTER, Structure, c_char_p, c_double, c_float, c_int, c_in
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("DPT_B200_LIB") or os.path.join(_HERE, "libdpt_b200.so")   # override: A/B builds of the same ABI
-ABI_VERSION = 8
+ABI_VERSION = 9
 
 OK, ERR_INVALID_ARG, ERR_CUDA, ERR_UNSUPPORTED = 0, -1, -2, -3
 
@@ -141,6 +141,12 @@ PROTOTYPES = {
                                                   c_int, POINTER(c_void_p), c_void_p, c_uint64, c_void_p]),
     "dpt_gpt2_train_population_backward": (c_int, [POINTER(Gpt2Weights), c_int, POINTER(c_void_p), c_int, c_int, c_int,
                                                    POINTER(Gpt2Grads), c_void_p, c_uint64, c_void_p]),
+    "dpt_gpt2_train_population_workspace_bytes_ex": (c_uint64, [POINTER(Gpt2Weights), c_int, c_int, c_int, c_int]),
+    "dpt_gpt2_train_population_forward_ex": (c_int, [POINTER(Gpt2Weights), c_int, POINTER(c_void_p), POINTER(c_void_p),
+                                                     POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), c_int, c_int, c_int,
+                                                     c_int, c_int, POINTER(c_void_p), c_void_p, c_uint64, c_void_p]),
+    "dpt_gpt2_train_population_backward_ex": (c_int, [POINTER(Gpt2Weights), c_int, POINTER(c_void_p), c_int, c_int, c_int, c_int,
+                                                      POINTER(Gpt2Grads), c_void_p, c_uint64, c_void_p]),
     "dpt_ordered_sum_f32": (c_int, [POINTER(c_void_p), c_int, c_int64, c_void_p, c_void_p]),
     "dpt_darkroom_policy_rollout": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_uint64, c_uint64, c_int64,
                                             c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,

@@ -48,10 +48,11 @@ def weights(model):
     return OrderedDict(model.state_dict())
 
 
-def train_args(batch_size, lrs, wds, seeds, train_datasets, test_datasets, device):
+def train_args(batch_size, lrs, wds, seeds, train_datasets, test_datasets, device, precision=0):
     """The arguments of ``train`` / ``train_population`` that a resume must repeat: the batch size, the device the batches
-    are drawn on, and per member its lr, weight_decay and seed, the length and shuffle flag of its train and test
-    datasets and which members share them (``train_set`` / ``test_set``: the first member with the same dataset)."""
+    are drawn on, the training precision (``forward_train``'s), and per member its lr, weight_decay and seed, the length
+    and shuffle flag of its train and test datasets and which members share them (``train_set`` / ``test_set``: the first
+    member with the same dataset)."""
     def first(ds, i):
         return next(j for j in range(i + 1) if ds[j] is ds[i])
     members = []
@@ -60,7 +61,7 @@ def train_args(batch_size, lrs, wds, seeds, train_datasets, test_datasets, devic
         for split, ds in (("train", train_datasets), ("test", test_datasets)):
             a.update({split + "_items": len(ds[i]), split + "_shuffle": bool(ds[i].shuffle), split + "_set": first(ds, i)})
         members.append(a)
-    return {"batch_size": int(batch_size), "device": torch.device(device).type, "members": members}
+    return {"batch_size": int(batch_size), "device": torch.device(device).type, "precision": int(precision), "members": members}
 
 
 def interactive_args(dim, n_envs, K, mb, var, env_type, seed, lr, weight_decay):
@@ -134,6 +135,8 @@ def check_state(state, kind, models, optimizer, args, total):
     for i, (m, s) in enumerate(zip(models, saved)):
         _compare(model_config(m), s["config"], "member %d has " % i)
     ours, theirs = dict(args), dict(state["args"])
+    if kind != "interactive":
+        theirs.setdefault("precision", 0)   # states written before the training precision was an argument were fp32
     om, tm = ours.pop("members", None), theirs.pop("members", None)
     _compare(ours, theirs)
     for i, (a, b) in enumerate(zip(om or [], tm or [])):

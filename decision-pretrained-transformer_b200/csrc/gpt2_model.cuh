@@ -108,4 +108,23 @@ template <int NM>
 int gpt2_train_forward_launch(const TrainFwdParams<NM>& p, int n, cudaStream_t st);
 void gpt2_pack_wimg(const float* attn_w, const float* proj_w, const float* fc_w, const float* fc2_w, unsigned char* img,
                     cudaStream_t st);
+
+// bf16 training (precision 1): the tcgen05 dense forward (gpt2_dense.cu, SAVE = true) on the parameter tensors, with the
+// weight images of member i, layer l at wimg[i] + l * WIMG_BYTES (packed from the parameters by gpt2_pack_train_wimg in
+// the same call).  It saves the same fp32 records (TA_* / TF_*) as the fp32 forward of training.
+template <int NM>
+struct TrainFwd16Params {
+  int L, dx, du, din, B, T, Ts, test;
+  TrainFwdMember mem[NM];
+  const uint4* wimg[NM];
+};
+template <int NM>
+int gpt2_train_forward_bf16_launch(const TrainFwd16Params<NM>& p, int n, cudaStream_t st);
+template <int NM>
+struct WimgPackParams {
+  const float* w[NM][G_MAX_L][4];   // attn_w, proj_w, fc_w, fc2_w of member i, layer l
+  unsigned char* img[NM];
+};
+template <int NM>
+int gpt2_pack_train_wimg(const WimgPackParams<NM>& p, int L, int n, cudaStream_t st);
 }  // namespace dpt

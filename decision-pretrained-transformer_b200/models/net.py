@@ -10,7 +10,9 @@ from the config is ignored: the trunk always has ONE head (models/net.py:29), he
 ``forward`` is dpt_gpt2_forward (hand-written CUDA, fp32) under ``torch.no_grad()``.  ``forward_train`` is the
 same computation with a gradient: dpt_gpt2_train_forward / dpt_gpt2_train_backward (hand-written CUDA, fp32) read
 the parameter tensors in place, and autograd receives a gradient for every parameter except ``transformer.wte``
-(which the model never reads, as in the reference).  The class holds no HuggingFace dependency.
+(which the model never reads, as in the reference).  ``forward_train(x, precision=1)`` is bf16 mixed-precision
+training (the *_ex entry points): the tcgen05 forward of ``forward`` at ``model.precision = 1`` and a tensor-core
+attention backward, with fp32 master weights and gradient sums.  The class holds no HuggingFace dependency.
 """
 import ctypes
 
@@ -191,12 +193,20 @@ class Transformer(nn.Module):
             ps += [f(b) for b in t.h]
         return ps
 
-    def forward_train(self, x):
+    def forward_train(self, x, precision=0):
         """``forward(x)`` with an autograd graph: returns ``preds[:, -1, :]`` (test) or ``preds[:, 1:, :]`` with a
-        ``grad_fn``; ``backward`` fills ``.grad`` of every parameter except ``transformer.wte``.  The logits are
-        bit-identical to ``forward(x)``.  The context inputs get no gradient.  fp32, sequences of <= 512 tokens.
-        This is the one-member case of ``forward_train_population``."""
-        return forward_train_population([self], [x])[0]
+        ``grad_fn``; ``backward`` fills ``.grad`` of every parameter except ``transformer.wte``.  The context inputs get
+        no gradient.  Sequences of <= 512 tokens.  This is the one-member case of ``forward_train_population``.
+
+        ``precision`` is the precision of this training step, independent of ``self.precision`` (the precision of
+        ``forward``, of the online loop and of rollouts):
+
+        - 0 (default): fp32 on the CUDA cores; the logits are bit-identical to ``forward(x)`` at ``self.precision = 0``.
+        - 1: bf16 mixed precision.  bf16 operands at the tensor-core inputs, fp32 accumulation, LayerNorm, softmax
+          statistics, residual stream and gradient sums; the parameters (master weights) stay fp32.  The logits are
+          bit-identical to ``forward(x)`` at ``self.precision = 1`` (within 2e-2 of fp32); the gradients are
+          deterministic."""
+        return forward_train_population([self], [x], precision)[0]
 
     # ---- step-by-step K/V-cached decode (callers that choose the pulled arm themselves) -------------
     def decoder(self, n_seqs, max_transitions=None):
@@ -265,14 +275,16 @@ def _train_inputs(x, dev):
 _MEMBER_FIELDS = ("n_layer", "state_dim", "action_dim", "horizon", "test")
 
 
-def forward_train_population(models, batches):
-    """``[m.forward_train(x) for m, x in zip(models, batches)]`` in the same kernel launches: member i's logits, and
+def forward_train_population(models, batches, precision=0):
+    """``[m.forward_train(x, precision) for m, x in zip(models, batches)]`` in the same kernel launches: member i's logits, and
     after ``backward`` the ``.grad`` of its parameters, are bit-identical to training it alone.  The members are
     same-shape Transformers (``n_layer``, ``state_dim``, ``action_dim``, ``horizon`` and ``test`` agree, else
     ``ValueError``) on one device, and the batches share B and T.  All members' parameters go through ONE autograd
     Function; a member whose logits get no gradient keeps ``.grad`` as it was, as if it had not been trained.  At most
     ``POPULATION_MAX`` members per call are launched together; larger populations are cut into such calls."""
     models, batches = list(models), list(batches)
+    if precision not in (0, 1):
+        raise ValueError("forward_train: precision=%r, training supports 0 (fp32) and 1 (bf16)" % (precision,))
     if len(models) != len(batches):
         raise ValueError("forward_train_population: %d models and %d batches" % (len(models), len(batches)))
     if not models:
@@ -305,7 +317,7 @@ def forward_train_population(models, batches):
     for a in range(0, len(models), POPULATION_MAX):
         ms = models[a:a + POPULATION_MAX]
         params = [p for m in ms for p in m._train_params()]
-        out += list(_PopulationTrainFn.apply(ms, ins[a:a + POPULATION_MAX], *params))
+        out += list(_PopulationTrainFn.apply(ms, ins[a:a + POPULATION_MAX], precision, *params))
     return out
 
 
@@ -313,11 +325,11 @@ POPULATION_MAX = 32   # DPT_GPT2_POPULATION_MAX: members per population launch
 
 
 class _PopulationTrainFn(torch.autograd.Function):
-    """dpt_gpt2_train_population_forward / _backward over k members (k = 1: the one-model path).  One workspace holds
-    every member's saved activations between the two."""
+    """dpt_gpt2_train_population_forward / _backward over k members (k = 1: the one-model path), or their _ex forms at
+    precision 1.  One workspace holds every member's saved activations between the two."""
 
     @staticmethod
-    def forward(ctx, models, inputs, *params):
+    def forward(ctx, models, inputs, precision, *params):
         ctx.set_materialize_grads(False)
         k, m0 = len(models), models[0]
         B, T, stride = inputs[0][5:8]
@@ -327,15 +339,22 @@ class _PopulationTrainFn(torch.autograd.Function):
         w = (_lib.Gpt2Weights * k)(*[_weights_struct(m, params[i * n:(i + 1) * n], keep) for i, m in enumerate(models)])
         outs = [torch.empty((B, m0.action_dim) if m0.test else (B, T, m0.action_dim), dtype=torch.float32, device=dev)
                 for _ in range(k)]
-        nbytes = lib().dpt_gpt2_train_population_workspace_bytes(w, k, B, T)
+        nbytes = lib().dpt_gpt2_train_population_workspace_bytes_ex(w, k, B, T, precision)
         ws = torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=dev)
         arr = lambda ts: (ctypes.c_void_p * k)(*[t.data_ptr() if T else None for t in ts])   # noqa: E731
         qs = (ctypes.c_void_p * k)(*[x[0].data_ptr() for x in inputs])
-        check(lib().dpt_gpt2_train_population_forward(w, k, qs, *[arr([x[j] for x in inputs]) for j in range(1, 5)], B, T, stride,
-                                                      1 if m0.test else 0, (ctypes.c_void_p * k)(*[o.data_ptr() for o in outs]),
-                                                      ws.data_ptr(), ws.numel(), stream_ptr()),
-              "dpt_gpt2_train_forward" if k == 1 else "dpt_gpt2_train_population_forward")
+        ins = [arr([x[j] for x in inputs]) for j in range(1, 5)]
+        os_ = (ctypes.c_void_p * k)(*[o.data_ptr() for o in outs])
+        test = 1 if m0.test else 0
+        if precision == 0:
+            check(lib().dpt_gpt2_train_population_forward(w, k, qs, *ins, B, T, stride, test, os_, ws.data_ptr(), ws.numel(),
+                                                          stream_ptr()),
+                  "dpt_gpt2_train_forward" if k == 1 else "dpt_gpt2_train_population_forward")
+        else:
+            check(lib().dpt_gpt2_train_population_forward_ex(w, k, qs, *ins, B, T, stride, test, precision, os_, ws.data_ptr(),
+                                                             ws.numel(), stream_ptr()), "dpt_gpt2_train_population_forward_ex")
         ctx.models, ctx.ws, ctx.B, ctx.T, ctx.test, ctx.out_shape = models, ws, B, T, m0.test, outs[0].shape
+        ctx.precision = precision
         ctx.save_for_backward(*params)
         return tuple(outs)
 
@@ -365,12 +384,18 @@ class _PopulationTrainFn(torch.autograd.Function):
             # a member whose logits got no gradient runs on a zero dout; its gradients are dropped below
             ds = [torch.zeros(ctx.out_shape, dtype=torch.float32, device=dev) if d is None else d.to(torch.float32).contiguous()
                   for d in douts]
-            check(lib().dpt_gpt2_train_population_backward(w, k, (ctypes.c_void_p * k)(*[d.data_ptr() for d in ds]), ctx.B,
-                                                           ctx.T, 1 if ctx.test else 0, gs, ctx.ws.data_ptr(), ctx.ws.numel(),
-                                                           stream_ptr()),
-                  "dpt_gpt2_train_backward" if k == 1 else "dpt_gpt2_train_population_backward")
+            dp = (ctypes.c_void_p * k)(*[d.data_ptr() for d in ds])
+            test = 1 if ctx.test else 0
+            if ctx.precision == 0:
+                check(lib().dpt_gpt2_train_population_backward(w, k, dp, ctx.B, ctx.T, test, gs, ctx.ws.data_ptr(), ctx.ws.numel(),
+                                                               stream_ptr()),
+                      "dpt_gpt2_train_backward" if k == 1 else "dpt_gpt2_train_population_backward")
+            else:
+                check(lib().dpt_gpt2_train_population_backward_ex(w, k, dp, ctx.B, ctx.T, test, ctx.precision, gs, ctx.ws.data_ptr(),
+                                                                  ctx.ws.numel(), stream_ptr()),
+                      "dpt_gpt2_train_population_backward_ex")
         ctx.ws = None
-        return (None, None, *[None if douts[i // n] is None else g for i, g in enumerate(grads)])
+        return (None, None, None, *[None if douts[i // n] is None else g for i, g in enumerate(grads)])
 
 
 ONLINE_POPULATION_MAX = 16              # DPT_GPT2_ONLINE_POPULATION_MAX: members per population launch of the online loop

@@ -40,11 +40,11 @@ def ce_sum_loss(pred, batch):
     return F.cross_entropy(pred.reshape(-1, du), target.reshape(-1, du), reduction="sum")
 
 
-def train_step(model, optimizer, batch, loss_fn=ce_sum_loss):
-    """One optimizer step: ``model.forward_train(batch)``, ``loss_fn(pred, batch)``, backward, ``optimizer.step()``.
-    Returns the loss as a device tensor (no host synchronisation)."""
+def train_step(model, optimizer, batch, loss_fn=ce_sum_loss, precision=0):
+    """One optimizer step: ``model.forward_train(batch, precision)``, ``loss_fn(pred, batch)``, backward,
+    ``optimizer.step()``.  Returns the loss as a device tensor (no host synchronisation)."""
     optimizer.zero_grad()
-    pred = model.forward_train(batch)
+    pred = model.forward_train(batch, precision)
     loss = loss_fn(pred, batch)
     loss.backward()
     optimizer.step()
@@ -71,26 +71,26 @@ def batches(dataset, batch_size, generator, shuffle_items=None):
 
 
 def train(model, train_dataset, test_dataset, num_epochs, batch_size=64, lr=1e-3, weight_decay=1e-4, seed=None,
-          optimizer=None, *, state_path=None, save_every=50, resume=False, weights_dir=None, stems=None):
+          optimizer=None, *, state_path=None, save_every=50, resume=False, weights_dir=None, stems=None, precision=0):
     """The reference's epoch loop.  Returns ``(train_loss, test_loss, optimizer)``: per-epoch lists of floats and the
     AdamW optimizer (its ``state_dict`` is the reference's).  This is the one-member case of ``train_population``, whose
-    docstring describes the checkpoint arguments; ``stems`` is one stem here."""
+    docstring describes the checkpoint arguments and ``precision``; ``stems`` is one stem here."""
     tr, te, optimizer = _population("train", [model], train_dataset, test_dataset, num_epochs, batch_size, lr, weight_decay,
                                     [seed], optimizer, state_path, save_every, resume, weights_dir,
-                                    None if stems is None else [stems])
+                                    None if stems is None else [stems], precision)
     return tr[0], te[0], optimizer
 
 
-def train_population_step(models, optimizer, batches, loss_fn=ce_sum_loss):
+def train_population_step(models, optimizer, batches, loss_fn=ce_sum_loss, precision=0):
     """One optimizer step of every member: ``forward_train_population``, the loss of each member on its own batch, one
     backward and ``optimizer.step()``.  Member i's gradient is the one ``train_step(models[i], ..., batches[i])`` computes,
     bit for bit.  With the default loss the cross-entropy runs once on the stacked logits (per-row reduction, then a sum
     per member), so a member's loss value can differ from ``train_step``'s in the last bits (within 1e-6 relative); with
     one member, or another ``loss_fn``, each member's loss is ``loss_fn(pred, batch)`` as in ``train_step``.  Returns the
-    losses as one device tensor [k] (no host synchronisation)."""
+    losses as one device tensor [k] (no host synchronisation).  ``precision``: that of ``forward_train_population``."""
     from .models.net import forward_train_population
     optimizer.zero_grad()
-    preds = forward_train_population(models, batches)
+    preds = forward_train_population(models, batches, precision)
     if loss_fn is ce_sum_loss and len(preds) > 1:
         pred = torch.stack(preds)
         du, k = pred.shape[-1], pred.shape[0]
@@ -145,7 +145,8 @@ def _population_batches(datasets, batch_size, gens):
 
 
 def train_population(models, train_datasets, test_datasets, num_epochs, batch_size=64, lr=1e-3, weight_decay=1e-4, seeds=None,
-                     optimizer=None, *, state_path=None, save_every=50, resume=False, weights_dir=None, stems=None):
+                     optimizer=None, *, state_path=None, save_every=50, resume=False, weights_dir=None, stems=None,
+                     precision=0):
     """``train`` of k same-shape models at once (``forward_train_population``): the members' forward and backward run in
     the same kernel launches, their batches are gathered together and their AdamW updates go through one optimizer.
 
@@ -172,13 +173,18 @@ def train_population(models, train_datasets, test_datasets, num_epochs, batch_si
       optimizer groups) raises ``ValueError`` before anything is modified.
     - ``weights_dir`` with ``stems`` (k distinct stems, e.g. from ``utils.build_bandit_model_filename``): member i's
       ``state_dict`` goes to ``{weights_dir}/{stems[i]}_epoch{e + 1}.pt`` at the same epochs and to
-      ``{weights_dir}/{stems[i]}.pt`` at the end (``checkpoint.save_weights``), as the reference's train.py writes them."""
+      ``{weights_dir}/{stems[i]}.pt`` at the end (``checkpoint.save_weights``), as the reference's train.py writes them.
+
+    ``precision``: the precision of the training steps (``forward_train``): 0 = fp32 (default), 1 = bf16 mixed precision
+    with fp32 master weights and AdamW state.  The test loss is ``model.forward`` at ``model.precision`` either way.  A
+    resume must repeat it (a state saved at one precision and resumed at the other raises ``ValueError``); states written
+    before this argument existed were fp32 and resume at 0.  The weight files do not depend on it."""
     return _population("population", models, train_datasets, test_datasets, num_epochs, batch_size, lr, weight_decay, seeds,
-                       optimizer, state_path, save_every, resume, weights_dir, stems)
+                       optimizer, state_path, save_every, resume, weights_dir, stems, precision)
 
 
 def _population(kind, models, train_datasets, test_datasets, num_epochs, batch_size, lr, weight_decay, seeds, optimizer,
-                state_path, save_every, resume, weights_dir, stems):
+                state_path, save_every, resume, weights_dir, stems, precision):
     models = list(models)
     k = len(models)
     if k == 0:
@@ -187,6 +193,8 @@ def _population(kind, models, train_datasets, test_datasets, num_epochs, batch_s
     lrs, wds = _per_member(lr, k, "lr"), _per_member(weight_decay, k, "weight_decay")
     seeds = _per_member(seeds, k, "seeds")
     _check_saving(state_path, save_every, resume)
+    if precision not in (0, 1):
+        raise ValueError("train_population: precision=%r, training supports 0 (fp32) and 1 (bf16)" % (precision,))
     if weights_dir is not None:
         stems = _per_member(stems, k, "stems")
         if None in stems or len(set(stems)) != k:
@@ -215,7 +223,7 @@ def _population(kind, models, train_datasets, test_datasets, num_epochs, batch_s
         gens.append(g)
     horizon = models[0].horizon
     train_loss, test_loss = [[] for _ in range(k)], [[] for _ in range(k)]
-    args = C.train_args(batch_size, lrs, wds, seeds, trs, tes, dev)
+    args = C.train_args(batch_size, lrs, wds, seeds, trs, tes, dev, precision)
     e0 = 0
     if resume and os.path.exists(state_path):
         e0, hist = C.load_state(state_path, kind, models, optimizer, args, num_epochs, gens)
@@ -229,9 +237,9 @@ def _population(kind, models, train_datasets, test_datasets, num_epochs, batch_s
         tr = torch.zeros((k,), dtype=torch.float32, device=dev)
         for bs in _population_batches(trs, batch_size, gens):
             if k == 1:
-                tr[0] += train_step(models[0], optimizer, bs[0])
+                tr[0] += train_step(models[0], optimizer, bs[0], precision=precision)
             else:
-                tr += train_population_step(models, optimizer, bs)
+                tr += train_population_step(models, optimizer, bs, precision=precision)
         losses = torch.stack([torch.stack(te) / horizon / len(tes[0]), tr / horizon / len(trs[0])]).tolist()   # one host read
         for i in range(k):
             test_loss[i].append(losses[0][i])

@@ -35,7 +35,7 @@ extern "C" {
 #define DPT_ERR_CUDA (-2)
 #define DPT_ERR_UNSUPPORTED (-3)
 
-#define DPT_ABI_VERSION 8
+#define DPT_ABI_VERSION 9
 
 /* reward_type of the bandit entry points (envs/bandit_env.py:56-63, envs/gpu_bandit_env.py:53-63):
  * 0 'uniform'  : r = means[a] + var * z, z ~ N(0,1);
@@ -401,6 +401,31 @@ int dpt_gpt2_train_population_forward(const dpt_gpt2_weights_t* w, int n_models,
 int dpt_gpt2_train_population_backward(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B, int T,
                                        int test, const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes,
                                        void* stream);
+
+/* Mixed-precision training: the population calls above with a `precision` argument.  precision = 0 runs exactly the
+ * fp32 kernels of the calls without _ex (same results, bit for bit).  precision = 1 is bf16 training: bf16 operands at the
+ * tensor-core inputs, fp32 accumulation, fp32 LayerNorm, softmax statistics, residual stream and gradient sums.
+ * - forward: the tcgen05 dense forward of dpt_gpt2_forward(precision = 1) on the parameter tensors; member i's logits are
+ *   bit-identical to dpt_gpt2_forward(precision = 1) on a handle of the same weights.
+ * - backward: the attention backward on mma.sync tensor-core products (bf16 in, fp32 out), split over ceil((T+1)/64)
+ *   CTAs per sequence; the projection, MLP and LayerNorm backward and every weight-gradient sum in fp32.  Two identical
+ *   calls give bit-identical gradients, and member i's equal the one-member call's.
+ * Workspace at precision 1: dpt_gpt2_train_population_workspace_bytes_ex(w, n_models, B, T, 1) bytes, 16 B aligned, the
+ * same buffer for the forward and the backward.  It is larger than at precision 0: each member region also holds the bf16
+ * weight images the forward packs from the parameters (40 KB per layer) and the attention-output gradients of one layer
+ * (144 B per row); the two precisions' workspaces are not interchangeable.
+ * B = 0 (and n_models = 0) only validates: the same argument checks run, nothing is launched.  precision outside {0, 1},
+ * n_embd != 32, n_layer > 8 and T + 1 > 512 return DPT_ERR_UNSUPPORTED with a message; the other errors are those of the
+ * calls without _ex.  workspace_bytes_ex returns 0 for arguments it cannot size (as the call without _ex does). */
+uint64_t dpt_gpt2_train_population_workspace_bytes_ex(const dpt_gpt2_weights_t* w, int n_models, int B, int T, int precision);
+int dpt_gpt2_train_population_forward_ex(const dpt_gpt2_weights_t* w, int n_models, const float* const* query_states,
+                                         const float* const* ctx_states, const float* const* ctx_actions,
+                                         const float* const* ctx_next_states, const float* const* ctx_rewards, int B, int T,
+                                         int T_stride, int test, int precision, float* const* out, void* workspace,
+                                         uint64_t workspace_bytes, void* stream);
+int dpt_gpt2_train_population_backward_ex(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B, int T,
+                                          int test, int precision, const dpt_gpt2_grads_t* grads, void* workspace,
+                                          uint64_t workspace_bytes, void* stream);
 
 /* Ordered multi-source sum (the gradient exchange of the data-parallel interactive trainer, train_interactive.py:97-139;
  * the reference is single-GPU): dst[i] = (((src[0][i] + src[1][i]) + ...) + src[M-1][i]) for i < n, fp32, added in
