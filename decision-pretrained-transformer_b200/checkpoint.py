@@ -64,10 +64,11 @@ def train_args(batch_size, lrs, wds, seeds, train_datasets, test_datasets, devic
     return {"batch_size": int(batch_size), "device": torch.device(device).type, "precision": int(precision), "members": members}
 
 
-def interactive_args(dim, n_envs, K, mb, var, env_type, seed, lr, weight_decay):
-    """The arguments of ``train_interactive`` / ``dist.train_interactive_sharded`` that a resume must repeat."""
+def interactive_args(dim, n_envs, K, mb, var, env_type, seed, lr, weight_decay, precision=0):
+    """The arguments of ``train_interactive`` / ``dist.train_interactive_sharded`` that a resume must repeat, the training
+    precision of the gradient half among them."""
     return {"dim": int(dim), "n_envs": int(n_envs), "K": int(K), "mb": int(mb), "var": float(var), "env_type": str(env_type),
-            "seed": int(seed), "lr": float(lr), "weight_decay": float(weight_decay)}
+            "seed": int(seed), "lr": float(lr), "weight_decay": float(weight_decay), "precision": int(precision)}
 
 
 def training_state(kind, models, optimizer, args, next_index, history, generators=None):
@@ -135,8 +136,7 @@ def check_state(state, kind, models, optimizer, args, total):
     for i, (m, s) in enumerate(zip(models, saved)):
         _compare(model_config(m), s["config"], "member %d has " % i)
     ours, theirs = dict(args), dict(state["args"])
-    if kind != "interactive":
-        theirs.setdefault("precision", 0)   # states written before the training precision was an argument were fp32
+    theirs.setdefault("precision", 0)   # states written before the training precision was an argument were fp32
     om, tm = ours.pop("members", None), theirs.pop("members", None)
     _compare(ours, theirs)
     for i, (a, b) in enumerate(zip(om or [], tm or [])):

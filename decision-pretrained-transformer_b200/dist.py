@@ -257,7 +257,8 @@ def train_interactive_sharded(model, dim, n_envs_total, K, n_iters, mb=1024, **k
     range of micro-batches (``microbatch_shard``; Philox counters use global env ids, so its contexts are slices of the
     one-GPU rollout), keeps their gradient slots in a ``PeerBuffer``, and every rank sums all slots in micro-batch order
     (``dpt_ordered_sum_f32`` over the peer mappings) before its AdamW step.  The weights after every iteration are
-    bit-identical on every rank and to the one-GPU run, for any world size.  Same arguments and return value; with
+    bit-identical on every rank and to the one-GPU run, for any world size and at either training ``precision`` (0 = fp32,
+    1 = bf16; the rollout runs at ``model.precision``).  Same arguments and return value; with
     ``state_path``, rank 0 writes the training state after the iteration's AdamW step (a failed write makes every rank
     raise), and on ``resume`` every rank reads the same file, which may come from any world size."""
     from . import train

@@ -273,33 +273,40 @@ def interactive_loss(last_logits, target, n_envs):
 
 
 def train_interactive(model, dim, n_envs, K, n_iters, mb=1024, var=0.0, env_type="uniform", seed=0, lr=1e-3,
-                      weight_decay=1e-4, optimizer=None, timings=None, *, state_path=None, save_every=50, resume=False):
+                      weight_decay=1e-4, optimizer=None, timings=None, *, state_path=None, save_every=50, resume=False,
+                      precision=0):
     """On-policy training (train_interactive.py:97-139) on one GPU.  Iteration ``it``:
 
     1. ``env = GPUBanditEnv(dim, n_envs, K, var, env_type, seed=rng.key_for(seed, it))``;
     2. ``env.rollout(model, K, sample=True)``: the fused K-step rollout with the current weights (``model.precision``);
-    3. the last logits on ``context[:, :K-1]`` with a gradient (``dpt_gpt2_train_forward``, last position, whatever
-       ``model.test`` says), ``interactive_loss`` against ``env.opt_a_index`` and ``dpt_gpt2_train_backward``, one
-       micro-batch of ``mb`` envs at a time (micro-batch m is envs ``[m*mb, min(n_envs, (m+1)*mb))``), each into its own
-       gradient slot;
+    3. the last logits on ``context[:, :K-1]`` with a gradient (``dpt_gpt2_train_population_forward_ex`` with one member,
+       last position, whatever ``model.test`` says), ``interactive_loss`` against ``env.opt_a_index`` and
+       ``dpt_gpt2_train_population_backward_ex``, one micro-batch of ``mb`` envs at a time (micro-batch m is envs
+       ``[m*mb, min(n_envs, (m+1)*mb))``), each into its own gradient slot;
     4. the slots summed in micro-batch order into the parameters' ``.grad`` (one flat buffer; ``transformer.wte`` gets
        none), then ``optimizer.step()`` (default ``torch.optim.AdamW(lr, weight_decay)``).
 
-    With ``mb >= n_envs`` an iteration is exactly ``env.rollout`` + ``forward_train`` + ``interactive_loss`` + ``backward``
-    + ``step``.  The result does not depend on how the micro-batches are spread over GPUs (``dist.train_interactive_sharded``),
-    only on ``mb``.  fp32 training, ``dropout == 0`` and K <= 512 (the limits of ``forward_train``).  ``n_envs == 0`` runs
-    nothing.  ``timings``: a list that receives, per iteration, the CUDA-event milliseconds of the rollout, the forward and
-    backward of all micro-batches, the exchange (host barrier to the end of the sum), the optimizer and the whole iteration.
-    Returns ``(losses, optimizer)``: the per-iteration losses (one host read at the end) and the optimizer.
+    ``precision``: the precision of step 3 only, as in ``train``: 0 = fp32 (default), 1 = bf16 mixed precision with fp32
+    master weights, gradient slots, gradient sum and AdamW state.  The rollout of step 2 runs at ``model.precision``
+    whatever ``precision`` is.  Values other than 0 and 1 raise ``ValueError`` before anything else is checked.
+
+    With ``mb >= n_envs`` an iteration is exactly ``env.rollout`` + ``forward_train(b, precision)`` + ``interactive_loss``
+    + ``backward`` + ``step``.  The result does not depend on how the micro-batches are spread over GPUs
+    (``dist.train_interactive_sharded``), only on ``mb``.  ``dropout == 0`` and K <= 512 (the limits of ``forward_train``),
+    checked before the first rollout.  ``n_envs == 0`` runs nothing.  ``timings``: a list that receives, per iteration,
+    the CUDA-event milliseconds of the rollout, the forward and backward of all micro-batches, the exchange (host barrier
+    to the end of the sum), the optimizer and the whole iteration.  Returns ``(losses, optimizer)``: the per-iteration
+    losses (one host read at the end) and the optimizer.
 
     ``state_path``, ``save_every`` and ``resume`` work as in ``train_population``, per iteration: the state is written
     after every iteration it with ``(it + 1) % save_every == 0`` and after the last one, and a resumed call continues at
     the saved iteration with its keys ``rng.key_for(seed, it)``; ``n_iters`` stays the total.  The arguments a resume must
-    repeat are ``dim``, ``n_envs``, ``K``, ``mb``, ``var``, ``env_type``, ``seed``, ``lr`` and ``weight_decay``, not the
-    world size: a state saved by ``dist.train_interactive_sharded`` at one world size resumes at any other."""
+    repeat are ``dim``, ``n_envs``, ``K``, ``mb``, ``var``, ``env_type``, ``seed``, ``lr``, ``weight_decay`` and
+    ``precision`` (states written before ``precision`` existed were fp32 and resume at 0), not the world size: a state
+    saved by ``dist.train_interactive_sharded`` at one world size resumes at any other."""
     return _interactive(model, dim, n_envs, K, n_iters, mb, 0, 1, var=var, env_type=env_type, seed=seed, lr=lr,
                         weight_decay=weight_decay, optimizer=optimizer, timings=timings, state_path=state_path,
-                        save_every=save_every, resume=resume)
+                        save_every=save_every, resume=resume, precision=precision)
 
 
 def _agree(err, ws):
@@ -317,8 +324,10 @@ def _agree(err, ws):
 
 
 def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type="uniform", seed=0, lr=1e-3,
-                 weight_decay=1e-4, optimizer=None, timings=None, state_path=None, save_every=50, resume=False):
+                 weight_decay=1e-4, optimizer=None, timings=None, state_path=None, save_every=50, resume=False, precision=0):
     """train_interactive on rank ``rank`` of ``ws`` (ws == 1: the one-GPU trainer; see dist.train_interactive_sharded)."""
+    if precision not in (0, 1):
+        raise ValueError("train_interactive: precision=%r, training supports 0 (fp32) and 1 (bf16)" % (precision,))
     import ctypes
     from . import _lib, dist as D, kernels, rng
     from ._lib import check, lib, stream_ptr
@@ -344,10 +353,14 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
     P = sum(sizes) + 1                 # a slot: every trained parameter (_train_params order), then the micro-batch's loss
     Ps = (P + 3) & ~3                  # slot stride: 16 B aligned slots
     T, du, st = K - 1, model.action_dim, stream_ptr()
-    # the train kernels' shape checks (n_embd, n_layer, sequence length) before any rollout: a B = 0 call only validates
-    check(lib().dpt_gpt2_train_forward(ctypes.byref(net._weights_struct(model, params, [])), None, None, None, None, None, 0,
-                                       T, K, 1, None, None, 0, st), "dpt_gpt2_train_forward")
-    args = C.interactive_args(dim, n_envs, K, mb, var, env_type, seed, lr, weight_decay)
+    fwd, bwd = "dpt_gpt2_train_population_forward_ex", "dpt_gpt2_train_population_backward_ex"
+    one = lambda *ps: (ctypes.c_void_p * 1)(*ps)   # noqa: E731  (the one-member pointer arrays of the population calls)
+    w = (_lib.Gpt2Weights * 1)(net._weights_struct(model, params, []))
+    # the train kernels' shape and precision checks (n_embd, n_layer, sequence length) before any rollout: a B = 0 call
+    # only validates
+    check(lib().dpt_gpt2_train_population_forward_ex(w, 1, None, None, None, None, None, 0, T, K, 1, precision, None, None, 0,
+                                                     st), fwd)
+    args = C.interactive_args(dim, n_envs, K, mb, var, env_type, seed, lr, weight_decay, precision)
     it0, done = 0, []
     if resume:   # every rank reads the same file; all raise if one fails to
         err = None
@@ -373,8 +386,7 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
         losses[:it0] = torch.tensor(done, dtype=torch.float32)
         if n_local:
             q = torch.ones((min(mb, n_local), model.state_dim), dtype=torch.float32, device=dev)
-            wbytes = int(lib().dpt_gpt2_train_workspace_bytes(ctypes.byref(net._weights_struct(model, params, [])),
-                                                               min(mb, n_local), T))
+            wbytes = int(lib().dpt_gpt2_train_population_workspace_bytes_ex(w, 1, min(mb, n_local), T, precision))
             work = torch.empty((max(wbytes, 16),), dtype=torch.uint8, device=dev)
         for it in range(it0, n_iters):
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)] if timings is not None else []
@@ -387,22 +399,24 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
                     ro = env.rollout(model, K, sample=True, logits=False)
                     mark(1)
                     keep = []
-                    w = net._weights_struct(model, params, keep)
+                    w = (_lib.Gpt2Weights * 1)(net._weights_struct(model, params, keep))
                     ctx = [ro[k] for k in _CTX]
                     for j in range(n_mb):
                         a, b = j * mb, min(n_local, (j + 1) * mb)
                         out = torch.empty((b - a, du), dtype=torch.float32, device=dev)
-                        cp = [c[a:b].data_ptr() if T else None for c in ctx]
-                        check(lib().dpt_gpt2_train_forward(ctypes.byref(w), q.data_ptr(), *cp, b - a, T, K, 1, out.data_ptr(),
-                                                           work.data_ptr(), work.numel(), st), "dpt_gpt2_train_forward")
+                        cp = [one(c[a:b].data_ptr() if T else None) for c in ctx]
+                        check(lib().dpt_gpt2_train_population_forward_ex(w, 1, one(q.data_ptr()), *cp, b - a, T, K, 1, precision,
+                                                                         one(out.data_ptr()), work.data_ptr(), work.numel(), st),
+                              fwd)
                         lg = out.requires_grad_()
                         with torch.enable_grad():
                             loss = interactive_loss(lg, ro["target"][a:b], n_envs)
                             dout, = torch.autograd.grad(loss, lg)
+                        dout = dout.contiguous()
                         g = net._pointer_struct(_lib.Gpt2Grads, model, grad_slots[j], keep)
-                        check(lib().dpt_gpt2_train_backward(ctypes.byref(w), dout.contiguous().data_ptr(), b - a, T, 1,
-                                                            ctypes.byref(g), work.data_ptr(), work.numel(), st),
-                              "dpt_gpt2_train_backward")
+                        check(lib().dpt_gpt2_train_population_backward_ex(w, 1, one(dout.data_ptr()), b - a, T, 1, precision,
+                                                                          ctypes.byref(g), work.data_ptr(), work.numel(), st),
+                              bwd)
                         slots[j, P - 1].copy_(loss.detach())
                 else:
                     mark(1)

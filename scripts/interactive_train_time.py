@@ -1,12 +1,16 @@
 """One iteration of the interactive trainer (train.train_interactive / dist.train_interactive_sharded) at the fork's
 scale, on 1, 2, 4 and 8 GPUs (as many as the box has), each world size under torch.distributed.run:
 
-    python scripts/interactive_train_time.py [--out FILE] [--iters 5] [--warmup 2]
+    python scripts/interactive_train_time.py [--out FILE] [--iters 5] [--warmup 2] [--precision 0 1]
+                                             [--rollout-precision 0 1] [--rounds 3]
 
 Problem: d = 5 arms, 4 layers, n_embd 32, N = 100 000 envs per iteration, micro-batches of 1024 envs, K = 100 and
-K = 500.  Per world size and K: the median over ``--iters`` iterations (after ``--warmup``) of the CUDA-event phases the
-trainer records (rollout, forward + backward of all micro-batches, exchange = host barrier to the end of the ordered sum,
-AdamW, whole iteration), per rank and the slowest rank.  Comparison arm, one GPU, N = 8192: the same iteration composed
+K = 500.  Per world size, K, rollout precision (``model.precision``, ``--rollout-precision``) and training precision
+(the ``precision`` argument, ``--precision``): the median over ``--iters`` iterations (after ``--warmup``) of every round
+of the CUDA-event phases the trainer records (rollout, forward + backward of all micro-batches, exchange = host barrier to
+the end of the ordered sum, AdamW, whole iteration), per rank and the slowest rank.  The training precisions alternate
+within each of ``--rounds`` rounds, in one process, so that they see the same card state; with two of them the ratio of
+their phase times is recorded too.  Comparison arm, one GPU, N = 8192: the same iteration composed
 from the step-by-step pieces (``Transformer.decoder`` + ``GPUBanditEnv.step`` per step, then one whole-batch
 ``forward_train``) against ``train_interactive`` at that N.  The card's name and power limit are read in the same run.
 Writes one JSON file (default: profiles/r06_interactive_train_time.json) and prints it.
@@ -51,6 +55,22 @@ def med(rows):
     return {k: float(np.median([r[k] for r in rows])) for k in PHASES}
 
 
+def case(args, K, rollout_precision):
+    """The timed runs of one K and rollout precision on this rank: {training precision: (timings, losses of round 0)}."""
+    from dpt_b200 import dist as D
+    runs = {p: ([], None) for p in args.precision}
+    for _ in range(args.rounds):
+        for p in args.precision:
+            m, tm = model(K), []
+            m.precision = rollout_precision
+            losses, _ = D.train_interactive_sharded(m, D_ARMS, N, K, args.warmup + args.iters, mb=MB, var=VAR, seed=SEED,
+                                                    timings=tm, precision=p)
+            runs[p] = (runs[p][0] + tm[args.warmup:], runs[p][1] or losses)
+            del m
+            torch.cuda.empty_cache()
+    return runs
+
+
 def worker(args):
     """One rank of one world size (under torch.distributed.run): rank 0 writes the gathered timings to args.worker."""
     import torch.distributed as dist
@@ -60,23 +80,27 @@ def worker(args):
     torch.cuda.set_device(lr)
     dist.init_process_group("nccl", device_id=torch.device("cuda", lr))
     out = {"world": ws}
+    _, _, lo, hi = D.microbatch_shard(N, MB, rank, ws)
+    envs = [None] * ws
+    dist.all_gather_object(envs, hi - lo)
     for K in KS:
-        m, tm = model(K), []
-        t0 = time.perf_counter()
-        losses, _ = D.train_interactive_sharded(m, D_ARMS, N, K, args.warmup + args.iters, mb=MB, var=VAR, seed=SEED, timings=tm)
-        wall = time.perf_counter() - t0
-        per_rank = [None] * ws
-        dist.all_gather_object(per_rank, tm[args.warmup:])
-        meds = [med(r) for r in per_rank]
-        _, _, lo, hi = D.microbatch_shard(N, MB, rank, ws)
-        envs = [None] * ws
-        dist.all_gather_object(envs, hi - lo)
-        out["K%d" % K] = {"median_ms_rank0": meds[0], "median_ms_slowest_rank": {k: max(x[k] for x in meds) for k in PHASES},
-                          "exchange_share_rank0": meds[0]["exchange"] / meds[0]["total"], "envs_per_rank": envs,
-                          "wall_s_all_iterations_rank0": wall, "losses": losses,
-                          "iterations_ms_rank0": per_rank[0]}
-        del m
-        torch.cuda.empty_cache()
+        res = out["K%d" % K] = {"envs_per_rank": envs}
+        for rp in args.rollout_precision:
+            t0 = time.perf_counter()
+            runs = case(args, K, rp)
+            wall = time.perf_counter() - t0
+            r = res["rollout_precision_%d" % rp] = {"wall_s_all_runs_rank0": wall}
+            for p, (tm, losses) in runs.items():
+                per_rank = [None] * ws
+                dist.all_gather_object(per_rank, tm)
+                meds = [med(x) for x in per_rank]
+                r["precision_%d" % p] = {"median_ms_rank0": meds[0],
+                                         "median_ms_slowest_rank": {k: max(x[k] for x in meds) for k in PHASES},
+                                         "exchange_share_rank0": meds[0]["exchange"] / meds[0]["total"], "losses": losses,
+                                         "iterations_ms_rank0": per_rank[0]}
+            if set(args.precision) == {0, 1}:
+                a, b = r["precision_1"]["median_ms_rank0"], r["precision_0"]["median_ms_rank0"]
+                r["precision_1_over_0_rank0"] = {k: a[k] / b[k] for k in PHASES}
     if rank == 0:
         with open(args.worker, "w") as f:
             json.dump(out, f)
@@ -143,6 +167,11 @@ def main():
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r06_interactive_train_time.json"))
     ap.add_argument("--iters", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=2)
+    ap.add_argument("--precision", type=int, nargs="+", default=[0], choices=(0, 1),
+                    help="training precisions, alternated within each round")
+    ap.add_argument("--rollout-precision", type=int, nargs="+", default=[0], choices=(0, 1),
+                    help="model.precision values, the precision of the rollout")
+    ap.add_argument("--rounds", type=int, default=1)
     ap.add_argument("--worker", default=None, help=argparse.SUPPRESS)
     args = ap.parse_args()
     if args.worker:
@@ -151,7 +180,9 @@ def main():
         raise SystemExit("interactive_train_time.py measures on the GPU; no CUDA device found")
     n_gpus = torch.cuda.device_count()
     res = {"gpu": gpu_info(), "config": {"d": D_ARMS, "n_layer": L, "n_embd": 32, "N": N, "mb": MB, "K": list(KS), "var": VAR,
-                                         "iters": args.iters, "warmup": args.warmup, "precision": "fp32"}, "worlds": {}}
+                                         "iters": args.iters, "warmup": args.warmup, "rounds": args.rounds,
+                                         "precision": args.precision, "rollout_precision": args.rollout_precision},
+           "worlds": {}}
     with tempfile.TemporaryDirectory() as tmp:
         for ws in (1, 2, 4, 8):
             if ws > n_gpus:
@@ -163,7 +194,8 @@ def main():
             path = os.path.join(tmp, "w%d.json" % ws)
             cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(ws), "--master-addr",
                    "127.0.0.1", "--master-port", str(port), os.path.abspath(__file__), "--worker", path,
-                   "--iters", str(args.iters), "--warmup", str(args.warmup)]
+                   "--iters", str(args.iters), "--warmup", str(args.warmup), "--rounds", str(args.rounds),
+                   "--precision", *map(str, args.precision), "--rollout-precision", *map(str, args.rollout_precision)]
             r = subprocess.run(cmd, cwd=ROOT, capture_output=True, text=True, timeout=3000)
             if r.returncode != 0:
                 raise SystemExit("world %d failed:\n%s\n%s" % (ws, r.stdout[-3000:], r.stderr[-3000:]))
