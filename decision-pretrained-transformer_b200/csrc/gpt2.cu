@@ -1012,6 +1012,7 @@ extern "C" int dpt_gpt2_create(const dpt_gpt2_weights_t* w, dpt_gpt2_t** out, vo
   d.pred_b = copy(w->pred_b, du);
   d.lnf_w = copy(w->lnf_w, G_E);
   d.lnf_b = copy(w->lnf_b, G_E);
+  WimgPackParams<1> pk{};
   for (int l = 0; l < L; ++l) {
     LayerW& lw = d.layer[l];
     DPT_CHECK_ARG(w->ln1_w[l] && w->attn_w[l] && w->proj_w[l] && w->fc_w[l] && w->fc2_w[l], "dpt_gpt2_create: null layer %d weight", l);
@@ -1029,7 +1030,8 @@ extern "C" int dpt_gpt2_create(const dpt_gpt2_weights_t* w, dpt_gpt2_t** out, vo
     lw.attn_w = copy(w->attn_w[l], G_E * 3 * G_E), lw.proj_w = copy(w->proj_w[l], G_E * G_E);
     lw.fc_w = copy(w->fc_w[l], G_E * G_FF), lw.fc2_w = copy(w->fc2_w[l], G_FF * G_E);
     unsigned char* img = reinterpret_cast<unsigned char*>(take(WIMG_BYTES / 4));   // tcgen05 B-operand image (bf16)
-    gpt2_pack_wimg(w->attn_w[l], w->proj_w[l], w->fc_w[l], w->fc2_w[l], img, st);
+    pk.w[0][l][0] = w->attn_w[l], pk.w[0][l][1] = w->proj_w[l], pk.w[0][l][2] = w->fc_w[l], pk.w[0][l][3] = w->fc2_w[l];
+    pk.img[0][l] = img;
     lw.wimg = reinterpret_cast<const uint4*>(img);
     uint4* frag = reinterpret_cast<uint4*>(take((size_t)WF_UINT4 * 4));                // mma.sync B fragments (bf16)
     auto packf = [&](const float* src, int K, int N, int off) {
@@ -1040,6 +1042,8 @@ extern "C" int dpt_gpt2_create(const dpt_gpt2_weights_t* w, dpt_gpt2_t** out, vo
     packf(w->fc_w[l], G_E, G_FF, WF_FC), packf(w->fc2_w[l], G_FF, G_E, WF_FC2);
     lw.wfrag = frag;
   }
+  const int rc = gpt2_pack_wimg<1>(pk, L, 1, st);   // every layer's image in one launch
+  if (rc != DPT_OK) return rc;
   DPT_LAUNCH_CHECK();
   guard.m = nullptr;
   *out = m;

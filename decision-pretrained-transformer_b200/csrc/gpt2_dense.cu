@@ -1,5 +1,5 @@
 // Dense Transformer.forward(x) on the 5th-generation tensor cores (precision = 1; this kernel: <= 128 tokens,
-// the multi-tile kernel at the end of the file: 129..512 tokens).
+// the multi-tile kernel below: 129..512 tokens).
 //
 // One CTA = one sequence; thread t owns token row t (128 threads = 128 TMEM lanes).  Every contraction of
 // the GPT-2 block is ONE tcgen05.mma chain with M = 128 tokens, bf16 operands in shared memory (K-major,
@@ -18,6 +18,13 @@
 // and copied into shared memory per layer.  The residual stream x stays in fp32 registers (32 per thread).
 // This is the dense path of SURVEY.md §8(d) ("the only place tensor cores are the relevant pipe"); it is
 // opt-in (precision = 1, 2e-2 logit bar) because the 1e-5 bar of the default path excludes bf16 operands.
+//
+// The short pipeline is one row body, dense_short_rows<SAVE>.  SAVE = false is inference (gpt2_dense_kernel).  SAVE = true
+// is the forward of bf16 training (gpt2_train_forward_bf16_kernel, called from gpt2_train.cu): the same rows on the
+// parameter tensors and on weight images packed from them, so the logits are bit-identical to inference, and every row
+// also stores what the backward needs in fp32 (TrainSave, layout TA_* / TF_* in gpt2_model.cuh).  The long pipeline has a
+// training copy, dense_long_rows (see there).  A training launch covers a population of same-shape models: CTA (b,
+// member = blockIdx.y).  pack_wimg_kernel writes the weight images of inference and training.
 #include "common.cuh"
 #include "gpt2_model.cuh"
 #include "umma.cuh"
@@ -91,7 +98,32 @@ __device__ __forceinline__ void run_mma(Pipe& pp, int tid, IssueFn issue) {
   umma::fence_after_sync();
 }
 
-__global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParams p) {
+// rec[at..at+31] = x, rec[st] = mean, rec[st + 1] = 1 / std of x (the statistics of ln_row)
+__device__ __forceinline__ void save_ln_(float* rec, int at, int st, const float* x) {
+  store32_(rec + at, x);
+  float mean = 0.f;
+#pragma unroll
+  for (int c = 0; c < G_E; ++c) mean += x[c];
+  mean *= (1.0f / G_E);
+  float var = 0.f;
+#pragma unroll
+  for (int c = 0; c < G_E; ++c) var = fmaf(x[c] - mean, x[c] - mean, var);
+  rec[st] = mean, rec[st + 1] = 1.0f / sqrtf(var * (1.0f / G_E) + 1e-5f);
+}
+// dst[0..31] = y + bias
+__device__ __forceinline__ void save_bias_(float* dst, const float* y, const float* bias) {
+  float v[G_E];
+#pragma unroll
+  for (int c = 0; c < G_E; ++c) v[c] = y[c] + __ldg(bias + c);
+  store32_(dst, v);
+}
+
+// The rows of sequence b = blockIdx.x (<= 128 tokens), thread t = row t.  SAVE = false: m = sh = the handle (Gpt2Dev), with
+// its transposed embed / pred copies and the layer images m.layer[l].wimg.  SAVE = true: m = TrainW, the parameter tensors
+// as they are (embed_transition.weight [E, din], pred_actions.weight [du, E]); sh gives L, dx, du, din and the images
+// sh.wimg + l * WIMG_BYTES; every row also stores its activations in sv.  p: the inputs, the output and B, T, Ts, test, share.
+template <bool SAVE, class W, class Sh, class P>
+__device__ __forceinline__ void dense_short_rows(const W& m, const Sh& sh, const P& p, const TrainSave& sv) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   __shared__ uint64_t bar;
   __shared__ uint32_t tmem_base_s;
@@ -99,10 +131,9 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
   unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int tid = threadIdx.x, warp = tid >> 5;
   const int b = blockIdx.x;
-  const Gpt2Dev& m = p.m;
   const int S = p.T + 1;                // tokens in the sequence (<= 128)
   const bool valid = tid < S;
-  const int dx = m.dx, du = m.du, din = m.din;
+  const int dx = sh.dx, du = sh.du, din = sh.din;
 
   if (warp == 0) umma::tmem_alloc(&tmem_base_s, TM_COLS);
   if (tid == 0) umma::mbar_init(&bar, 1);
@@ -125,12 +156,18 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
         tok[2 * dx + du] = p.cr[row];
       }
     }
+    if (SAVE && valid) store32_(sv.fin + ((size_t)b * S + tid) * TF_STRIDE + TF_TOK, tok);
 #pragma unroll
     for (int c = 0; c < G_E; ++c) x[c] = valid ? __ldg(m.embed_b + c) + __ldg(m.wpe + (size_t)tid * G_E + c) : 0.f;
     for (int i = 0; i < din; ++i) {
       const float tv = tok[i];
 #pragma unroll
-      for (int c = 0; c < G_E; ++c) x[c] = fmaf(tv, __ldg(m.embed_wT + i * G_E + c), x[c]);
+      for (int c = 0; c < G_E; ++c) {
+        const float* e;
+        if constexpr (SAVE) e = m.embed_w + c * din + i;
+        else e = m.embed_wT + i * G_E + c;
+        x[c] = fmaf(tv, __ldg(e), x[c]);
+      }
     }
   }
   umma::fence_before_sync();
@@ -141,16 +178,20 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
   const uint32_t aVT0 = umma::smem_u32(smem + SM_VT0), aVT1 = umma::smem_u32(smem + SM_VT1), aW = umma::smem_u32(smem + SM_W);
   const uint32_t id32 = umma::make_idesc_bf16(128, 32), id96 = umma::make_idesc_bf16(128, 96), id128 = umma::make_idesc_bf16(128, 128);
 
-  for (int l = 0; l < m.L; ++l) {
-    const LayerW& w = m.layer[l];
+  for (int l = 0; l < sh.L; ++l) {
+    const auto& w = m.layer[l];
+    float* const rec = SAVE && valid ? sv.act + (((size_t)l * p.B + b) * S + tid) * TA_STRIDE : nullptr;   // SAVE: this row's record
     // weight image of this layer -> smem (all MMAs that read the previous image have completed)
     {
-      const uint4* src = w.wimg;
+      const uint4* src;
+      if constexpr (SAVE) src = sh.wimg + (size_t)l * (WIMG_BYTES / 16);
+      else src = w.wimg;
       uint4* dst = reinterpret_cast<uint4*>(smem + SM_W);
       for (int i = tid; i < WIMG_BYTES / 16; i += DN_THREADS) dst[i] = __ldg(src + i);
     }
     float y[G_E];
     // ---- LN1 -> A ; QKV = Xn Wqkv ----
+    if (SAVE && valid) save_ln_(rec, TA_XIN, TA_MU1, x);
     ln_row(x, w.ln1_w, w.ln1_b, y);
     st_row32(smem + SM_A0, tid, y);
     run_mma(pp, tid, [&] {
@@ -162,12 +203,15 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
     umma::tmem_ld32(umma::tmem_addr(tb, warp, 0), y);
 #pragma unroll
     for (int c = 0; c < G_E; ++c) y[c] = (y[c] + __ldg(w.attn_b + c)) * 0.17677669529663687f;
+    if (SAVE && valid) store32_(rec + TA_Q, y);
     st_row32(smem + SM_A0, tid, y);
     umma::tmem_ld32(umma::tmem_addr(tb, warp, 32), y);
 #pragma unroll
     for (int c = 0; c < G_E; ++c) y[c] += __ldg(w.attn_b + G_E + c);
+    if (SAVE && valid) store32_(rec + TA_K, y);
     st_row32(smem + SM_K, tid, y);
     umma::tmem_ld32(umma::tmem_addr(tb, warp, 64), y);
+    if (SAVE && valid) save_bias_(rec + TA_V, y, w.attn_b + 2 * G_E);
     {
       unsigned char* vt = smem + (tid < 64 ? SM_VT0 : SM_VT1);
       const int kk = tid & 63;
@@ -206,6 +250,7 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
       for (int c = 0; c < 4; ++c) umma::st_chunk(tile, tid, ((c0 & 63) >> 3) + c, y + 8 * c);
     }
     const float inv = 1.0f / sum;
+    if (SAVE && valid) rec[TA_LSE] = mx + logf(sum);
     // ---- O = P V ----
     run_mma(pp, tid, [&] {
 #pragma unroll
@@ -216,6 +261,7 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
     umma::tmem_ld32(umma::tmem_addr(tb, warp, 0), y);
 #pragma unroll
     for (int c = 0; c < G_E; ++c) y[c] *= inv;
+    if (SAVE && valid) store32_(rec + TA_O, y);
     st_row32(smem + SM_A0, tid, y);
     // ---- x += o Wproj + b ----
     run_mma(pp, tid, [&] {
@@ -227,6 +273,7 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
 #pragma unroll
     for (int c = 0; c < G_E; ++c) x[c] += y[c] + __ldg(w.proj_b + c);
     // ---- LN2 -> A ; F = Xn Wfc ----
+    if (SAVE && valid) save_ln_(rec, TA_XMID, TA_MU2, x);
     ln_row(x, w.ln2_w, w.ln2_b, y);
     st_row32(smem + SM_A0, tid, y);
     run_mma(pp, tid, [&] {
@@ -237,6 +284,7 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
 #pragma unroll
     for (int c0 = 0; c0 < 128; c0 += 32) {
       umma::tmem_ld32(umma::tmem_addr(tb, warp, 128 + c0), y);
+      if (SAVE && valid) save_bias_(rec + TA_H + c0, y, w.fc_b + c0);
 #pragma unroll
       for (int i = 0; i < 32; ++i) y[i] = gelu_new_d(y[i] + __ldg(w.fc_b + c0 + i));
       unsigned char* tile = smem + (c0 < 64 ? SM_A0 : SM_A1);
@@ -258,6 +306,7 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
   }
 
   // ---- ln_f + pred_actions ----
+  if (SAVE && valid) save_ln_(sv.fin + ((size_t)b * S + tid) * TF_STRIDE, TF_X, TF_MU, x);
   if (p.test ? (tid == p.T) : (tid >= 1 && tid <= p.T)) {
     float y[G_E];
     ln_row(x, m.lnf_w, m.lnf_b, y);
@@ -265,7 +314,12 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
     for (int j = 0; j < du; ++j) {
       float lg = __ldg(m.pred_b + j);
 #pragma unroll
-      for (int c = 0; c < G_E; ++c) lg = fmaf(y[c], __ldg(m.pred_wT + c * du + j), lg);
+      for (int c = 0; c < G_E; ++c) {
+        const float* e;
+        if constexpr (SAVE) e = m.pred_w + j * G_E + c;
+        else e = m.pred_wT + c * du + j;
+        lg = fmaf(y[c], __ldg(e), lg);
+      }
       o[j] = lg;
     }
   }
@@ -274,22 +328,8 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParam
   if (warp == 0) umma::tmem_dealloc(tb, TM_COLS);
 }
 
-// B[n][k] = W[k][n] (W is [In][Out] row-major) as bf16 into K64 tiles of `rows` = Out rows starting at img + off
-__global__ void pack_wimg_kernel(const float* W, unsigned char* img, int off, int In, int Out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= In * Out) return;
-  const int k = i / Out, n = i - k * Out;
-  unsigned char* tile = img + off + (k >> 6) * (Out * 128);
-  *reinterpret_cast<__nv_bfloat16*>(tile + umma::k64_offset(n, k & 63)) = __float2bfloat16_rn(W[i]);
-}
-
-void gpt2_pack_wimg(const float* attn_w, const float* proj_w, const float* fc_w, const float* fc2_w, unsigned char* img,
-                    cudaStream_t st) {
-  cudaMemsetAsync(img, 0, WIMG_BYTES, st);
-  pack_wimg_kernel<<<(32 * 96 + 255) / 256, 256, 0, st>>>(attn_w, img, WIMG_QKV, 32, 96);
-  pack_wimg_kernel<<<(32 * 32 + 255) / 256, 256, 0, st>>>(proj_w, img, WIMG_PROJ, 32, 32);
-  pack_wimg_kernel<<<(32 * 128 + 255) / 256, 256, 0, st>>>(fc_w, img, WIMG_FC, 32, 128);
-  pack_wimg_kernel<<<(128 * 32 + 255) / 256, 256, 0, st>>>(fc2_w, img, WIMG_FC2, 128, 32);
+__global__ void __launch_bounds__(DN_THREADS) gpt2_dense_kernel(const DenseParams p) {
+  dense_short_rows<false>(p.m, p.m, p, TrainSave{});
 }
 
 int gpt2_dense_launch(const DenseParams& p, cudaStream_t st) {
@@ -550,237 +590,11 @@ int gpt2_dense_long_launch(const DenseParams& p, cudaStream_t st) {
   return DPT_OK;
 }
 
-}  // namespace dpt
-
-// =============================================================================================
-// The forward of bf16 training (precision 1): the two pipelines above on the parameter tensors and
-// the weight images packed from them into the workspace (the bytes dpt_gpt2_create packs), so the logits are
-// bit-identical to dpt_gpt2_forward(precision = 1).  Every row also stores what the backward needs in fp32: the TA_* /
-// TF_* records of the fp32 forward of training, which the weight-gradient reduction reads unchanged.  The inference
-// kernels keep their own copy of the pipelines: folding them into these functions moved their register allocation
-// (cuobjdump -sass), and they are the measured inference path.
-// =============================================================================================
-namespace dpt {
-
-// rec[at..at+31] = x, rec[st] = mean, rec[st + 1] = 1 / std of x (the statistics of ln_row)
-__device__ __forceinline__ void save_ln_(float* rec, int at, int st, const float* x) {
-  store32_(rec + at, x);
-  float mean = 0.f;
-#pragma unroll
-  for (int c = 0; c < G_E; ++c) mean += x[c];
-  mean *= (1.0f / G_E);
-  float var = 0.f;
-#pragma unroll
-  for (int c = 0; c < G_E; ++c) var = fmaf(x[c] - mean, x[c] - mean, var);
-  rec[st] = mean, rec[st + 1] = 1.0f / sqrtf(var * (1.0f / G_E) + 1e-5f);
-}
-// dst[0..31] = y + bias
-__device__ __forceinline__ void save_bias_(float* dst, const float* y, const float* bias) {
-  float v[G_E];
-#pragma unroll
-  for (int c = 0; c < G_E; ++c) v[c] = y[c] + __ldg(bias + c);
-  store32_(dst, v);
-}
-
-// The rows of sequence b = blockIdx.x (<= 128 tokens), thread t = row t: gpt2_dense_kernel's pipeline on the parameter
-// tensors m (TrainW: embed_transition.weight [E, din], pred_actions.weight [du, E]) and the weight images sh.wimg; sh
-// gives L, dx, du, din; p the inputs, the output and B, T, Ts, test, share.  Every row also stores its activations
-// (TrainSave, layout TA_* / TF_*) in fp32.
-template <class W, class Sh, class P>
-__device__ __forceinline__ void dense_short_rows(const W& m, const Sh& sh, const P& p, const TrainSave& sv) {
-  extern __shared__ __align__(1024) unsigned char smem_raw[];
-  __shared__ uint64_t bar;
-  __shared__ uint32_t tmem_base_s;
-  // dynamic smem base is only guaranteed 16 B-aligned: round up to 1024 B (the launch adds 1 KB of slack)
-  unsigned char* smem = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int tid = threadIdx.x, warp = tid >> 5;
-  const int b = blockIdx.x;
-  const int S = p.T + 1;                // tokens in the sequence (<= 128)
-  const bool valid = tid < S;
-  const int dx = sh.dx, du = sh.du, din = sh.din;
-
-  if (warp == 0) umma::tmem_alloc(&tmem_base_s, TM_COLS);
-  if (tid == 0) umma::mbar_init(&bar, 1);
-  Pipe pp{&bar, 0};
-
-  // ---- token embedding (models/net.py:45-54): row 0 = query state, rows 1..T = context transitions ----
-  float x[G_E];
-  {
-    float tok[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) tok[i] = 0.f;
-    if (valid) {
-      if (tid == 0) {
-        for (int i = 0; i < dx; ++i) tok[i] = p.query[(size_t)b * dx + i];
-      } else {
-        const size_t row = (size_t)(b / p.share) * p.Ts + (tid - 1);
-        for (int i = 0; i < dx; ++i) tok[i] = p.cs[row * dx + i];
-        for (int i = 0; i < du; ++i) tok[dx + i] = p.ca[row * du + i];
-        for (int i = 0; i < dx; ++i) tok[dx + du + i] = p.cns[row * dx + i];
-        tok[2 * dx + du] = p.cr[row];
-      }
-    }
-    if (valid) store32_(sv.fin + ((size_t)b * S + tid) * TF_STRIDE + TF_TOK, tok);
-#pragma unroll
-    for (int c = 0; c < G_E; ++c) x[c] = valid ? __ldg(m.embed_b + c) + __ldg(m.wpe + (size_t)tid * G_E + c) : 0.f;
-    for (int i = 0; i < din; ++i) {
-      const float tv = tok[i];
-#pragma unroll
-      for (int c = 0; c < G_E; ++c) x[c] = fmaf(tv, __ldg(m.embed_w + c * din + i), x[c]);
-    }
-  }
-  umma::fence_before_sync();
-  __syncthreads();
-  umma::fence_after_sync();
-  const uint32_t tb = tmem_base_s;
-  const uint32_t aA0 = umma::smem_u32(smem + SM_A0), aA1 = umma::smem_u32(smem + SM_A1), aK = umma::smem_u32(smem + SM_K);
-  const uint32_t aVT0 = umma::smem_u32(smem + SM_VT0), aVT1 = umma::smem_u32(smem + SM_VT1), aW = umma::smem_u32(smem + SM_W);
-  const uint32_t id32 = umma::make_idesc_bf16(128, 32), id96 = umma::make_idesc_bf16(128, 96), id128 = umma::make_idesc_bf16(128, 128);
-
-  for (int l = 0; l < sh.L; ++l) {
-    const auto& w = m.layer[l];
-    float* const rec = valid ? sv.act + (((size_t)l * p.B + b) * S + tid) * TA_STRIDE : nullptr;   // this row's record
-    // weight image of this layer -> smem (all MMAs that read the previous image have completed)
-    {
-      const uint4* src = sh.wimg + (size_t)l * (WIMG_BYTES / 16);
-      uint4* dst = reinterpret_cast<uint4*>(smem + SM_W);
-      for (int i = tid; i < WIMG_BYTES / 16; i += DN_THREADS) dst[i] = __ldg(src + i);
-    }
-    float y[G_E];
-    // ---- LN1 -> A ; QKV = Xn Wqkv ----
-    if (valid) save_ln_(rec, TA_XIN, TA_MU1, x);
-    ln_row(x, w.ln1_w, w.ln1_b, y);
-    st_row32(smem + SM_A0, tid, y);
-    run_mma(pp, tid, [&] {
-#pragma unroll
-      for (int ks = 0; ks < 2; ++ks)
-        umma::mma_bf16(tb + 0, umma::make_desc_k64(aA0 + ks * 32), umma::make_desc_k64(aW + WIMG_QKV + ks * 32), id96, ks > 0);
-    });
-    // ---- q (scaled) -> A, k -> B, v -> B^T ----
-    umma::tmem_ld32(umma::tmem_addr(tb, warp, 0), y);
-#pragma unroll
-    for (int c = 0; c < G_E; ++c) y[c] = (y[c] + __ldg(w.attn_b + c)) * 0.17677669529663687f;
-    if (valid) store32_(rec + TA_Q, y);
-    st_row32(smem + SM_A0, tid, y);
-    umma::tmem_ld32(umma::tmem_addr(tb, warp, 32), y);
-#pragma unroll
-    for (int c = 0; c < G_E; ++c) y[c] += __ldg(w.attn_b + G_E + c);
-    if (valid) store32_(rec + TA_K, y);
-    st_row32(smem + SM_K, tid, y);
-    umma::tmem_ld32(umma::tmem_addr(tb, warp, 64), y);
-    if (valid) save_bias_(rec + TA_V, y, w.attn_b + 2 * G_E);
-    {
-      unsigned char* vt = smem + (tid < 64 ? SM_VT0 : SM_VT1);
-      const int kk = tid & 63;
-#pragma unroll
-      for (int c = 0; c < G_E; ++c)
-        *reinterpret_cast<__nv_bfloat16*>(vt + umma::k64_offset(c, kk)) = __float2bfloat16_rn(y[c] + __ldg(w.attn_b + 2 * G_E + c));
-    }
-    // ---- S = Q K^T ----
-    run_mma(pp, tid, [&] {
-#pragma unroll
-      for (int ks = 0; ks < 2; ++ks)
-        umma::mma_bf16(tb + 128, umma::make_desc_k64(aA0 + ks * 32), umma::make_desc_k64(aK + ks * 32), id128, ks > 0);
-    });
-    // ---- causal softmax of row tid (keys <= tid), two passes over the TMEM row ----
-    float mx = -INFINITY;
-#pragma unroll
-    for (int c0 = 0; c0 < 128; c0 += 32) {
-      umma::tmem_ld32(umma::tmem_addr(tb, warp, 128 + c0), y);
-#pragma unroll
-      for (int i = 0; i < 32; ++i)
-        if (c0 + i <= tid) mx = fmaxf(mx, y[i]);
-    }
-    float sum = 0.f;
-#pragma unroll
-    for (int c0 = 0; c0 < 128; c0 += 32) {
-      umma::tmem_ld32(umma::tmem_addr(tb, warp, 128 + c0), y);
-#pragma unroll
-      for (int i = 0; i < 32; ++i) {
-        const float pr = (c0 + i <= tid) ? exp_fast(y[i] - mx) : 0.f;
-        // the normaliser uses the bf16-rounded probabilities that the tensor core will see
-        y[i] = __bfloat162float(__float2bfloat16_rn(pr));
-        sum += y[i];
-      }
-      unsigned char* tile = smem + (c0 < 64 ? SM_A0 : SM_A1);
-#pragma unroll
-      for (int c = 0; c < 4; ++c) umma::st_chunk(tile, tid, ((c0 & 63) >> 3) + c, y + 8 * c);
-    }
-    const float inv = 1.0f / sum;
-    if (valid) rec[TA_LSE] = mx + logf(sum);
-    // ---- O = P V ----
-    run_mma(pp, tid, [&] {
-#pragma unroll
-      for (int ks = 0; ks < 8; ++ks)
-        umma::mma_bf16(tb + 0, umma::make_desc_k64((ks < 4 ? aA0 : aA1) + (ks & 3) * 32),
-                       umma::make_desc_k64((ks < 4 ? aVT0 : aVT1) + (ks & 3) * 32), id32, ks > 0);
-    });
-    umma::tmem_ld32(umma::tmem_addr(tb, warp, 0), y);
-#pragma unroll
-    for (int c = 0; c < G_E; ++c) y[c] *= inv;
-    if (valid) store32_(rec + TA_O, y);
-    st_row32(smem + SM_A0, tid, y);
-    // ---- x += o Wproj + b ----
-    run_mma(pp, tid, [&] {
-#pragma unroll
-      for (int ks = 0; ks < 2; ++ks)
-        umma::mma_bf16(tb + 32, umma::make_desc_k64(aA0 + ks * 32), umma::make_desc_k64(aW + WIMG_PROJ + ks * 32), id32, ks > 0);
-    });
-    umma::tmem_ld32(umma::tmem_addr(tb, warp, 32), y);
-#pragma unroll
-    for (int c = 0; c < G_E; ++c) x[c] += y[c] + __ldg(w.proj_b + c);
-    // ---- LN2 -> A ; F = Xn Wfc ----
-    if (valid) save_ln_(rec, TA_XMID, TA_MU2, x);
-    ln_row(x, w.ln2_w, w.ln2_b, y);
-    st_row32(smem + SM_A0, tid, y);
-    run_mma(pp, tid, [&] {
-#pragma unroll
-      for (int ks = 0; ks < 2; ++ks)
-        umma::mma_bf16(tb + 128, umma::make_desc_k64(aA0 + ks * 32), umma::make_desc_k64(aW + WIMG_FC + ks * 32), id128, ks > 0);
-    });
-#pragma unroll
-    for (int c0 = 0; c0 < 128; c0 += 32) {
-      umma::tmem_ld32(umma::tmem_addr(tb, warp, 128 + c0), y);
-      if (valid) save_bias_(rec + TA_H + c0, y, w.fc_b + c0);
-#pragma unroll
-      for (int i = 0; i < 32; ++i) y[i] = gelu_new_d(y[i] + __ldg(w.fc_b + c0 + i));
-      unsigned char* tile = smem + (c0 < 64 ? SM_A0 : SM_A1);
-#pragma unroll
-      for (int c = 0; c < 4; ++c) umma::st_chunk(tile, tid, ((c0 & 63) >> 3) + c, y + 8 * c);
-    }
-    // ---- x += g Wfc2 + b ----
-    run_mma(pp, tid, [&] {
-#pragma unroll
-      for (int ks = 0; ks < 8; ++ks)
-        umma::mma_bf16(tb + 0, umma::make_desc_k64((ks < 4 ? aA0 : aA1) + (ks & 3) * 32),
-                       umma::make_desc_k64(aW + WIMG_FC2 + (ks < 4 ? 0 : 4096) + (ks & 3) * 32), id32, ks > 0);
-    });
-    umma::tmem_ld32(umma::tmem_addr(tb, warp, 0), y);
-#pragma unroll
-    for (int c = 0; c < G_E; ++c) x[c] += y[c] + __ldg(w.fc2_b + c);
-    umma::fence_before_sync();
-    __syncthreads();   // every thread has drained its TMEM loads and smem reads before the next layer's image copy
-  }
-
-  // ---- ln_f + pred_actions ----
-  if (valid) save_ln_(sv.fin + ((size_t)b * S + tid) * TF_STRIDE, TF_X, TF_MU, x);
-  if (p.test ? (tid == p.T) : (tid >= 1 && tid <= p.T)) {
-    float y[G_E];
-    ln_row(x, m.lnf_w, m.lnf_b, y);
-    float* o = p.test ? p.out + (size_t)b * du : p.out + ((size_t)b * p.T + (tid - 1)) * du;
-    for (int j = 0; j < du; ++j) {
-      float lg = __ldg(m.pred_b + j);
-#pragma unroll
-      for (int c = 0; c < G_E; ++c) lg = fmaf(y[c], __ldg(m.pred_w + j * G_E + c), lg);
-      o[j] = lg;
-    }
-  }
-  umma::fence_before_sync();
-  __syncthreads();
-  if (warp == 0) umma::tmem_dealloc(tb, TM_COLS);
-}
-
-// the rows of sequence b (129..512 tokens): gpt2_dense_long_kernel's pipeline; m, sh, p as in dense_short_rows
+// The rows of sequence b (129..512 tokens) for the forward of bf16 training: gpt2_dense_long_kernel's pipeline on the
+// parameter tensors, saving the activations; m, sh, p and sv as in dense_short_rows with SAVE = true.  Unlike the short
+// pipeline, this one is not shared with the inference kernel: compiled from one SAVE-templated body,
+// gpt2_dense_long_kernel<2> ran 1.1 % slower at B = 1024 x 201 tokens (one B200 at 1000 W).  A change to the pipeline
+// is made in both copies, and the training logits stay bit-identical to gpt2_dense_long_kernel's.
 template <int NT, class W, class Sh, class P>
 __device__ __forceinline__ void dense_long_rows(const W& m, const Sh& sh, const P& p, const TrainSave& sv) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -993,6 +807,7 @@ __device__ __forceinline__ void dense_long_rows(const W& m, const Sh& sh, const 
   if (warp == 0) umma::tmem_dealloc(tb, TM_COLS);
 }
 
+
 // ---- the forward of bf16 training: CTA (b, member = blockIdx.y), on the member's parameters ----
 struct TrainShape16 {
   int L, dx, du, din;
@@ -1016,7 +831,7 @@ __global__ void __launch_bounds__(DN_THREADS) gpt2_train_forward_bf16_kernel(con
   TrainShape16 sh;
   train16_member(p, mb, sh);
   const TrainIo io{mb->query, mb->cs, mb->ca, mb->cns, mb->cr, mb->out, p.B, p.T, p.Ts, p.test, 1};
-  dense_short_rows(mb->w, sh, io, mb->sv);
+  dense_short_rows<true>(mb->w, sh, io, mb->sv);
 }
 
 template <int NT, int NM>
@@ -1052,10 +867,10 @@ int gpt2_train_forward_bf16_launch(const TrainFwd16Params<NM>& p, int n, cudaStr
 template int gpt2_train_forward_bf16_launch<1>(const TrainFwd16Params<1>&, int, cudaStream_t);
 template int gpt2_train_forward_bf16_launch<TRAIN_POP_MAX>(const TrainFwd16Params<TRAIN_POP_MAX>&, int, cudaStream_t);
 
-// the weight images of every member and layer (the same bytes gpt2_pack_wimg writes, k beyond In zero), one launch:
-// CTA (element block, layer, member)
+// The weight images (layout WIMG_* in gpt2_model.cuh) of members 0 .. n-1, layers 0 .. L-1, one launch: CTA (element
+// block, layer, member).  Every byte of an image is written; k beyond In is zero.
 template <int NM>
-__global__ void pack_train_wimg_kernel(const __grid_constant__ WimgPackParams<NM> p) {
+__global__ void pack_wimg_kernel(const __grid_constant__ WimgPackParams<NM> p) {
   const int z = NM == 1 ? 0 : blockIdx.z, l = blockIdx.y;
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= WIMG_BYTES / 2) return;
@@ -1065,21 +880,23 @@ __global__ void pack_train_wimg_kernel(const __grid_constant__ WimgPackParams<NM
   while (i >= Out[seg] * max(64, In[seg])) i -= Out[seg] * max(64, In[seg]), ++seg;
   const int kp = max(64, In[seg]), n = i / kp, k = i % kp;
   const float v = k < In[seg] ? p.w[z][l][seg][k * Out[seg] + n] : 0.f;
-  unsigned char* tile = p.img[z] + (size_t)l * WIMG_BYTES + Off[seg] + (k >> 6) * (Out[seg] * 128);
+  unsigned char* tile = p.img[z][l] + Off[seg] + (k >> 6) * (Out[seg] * 128);
   *reinterpret_cast<__nv_bfloat16*>(tile + umma::k64_offset(n, k & 63)) = __float2bfloat16_rn(v);
 }
+static_assert(sizeof(WimgPackParams<TRAIN_POP_MAX>) <= 32764 && sizeof(TrainFwd16Params<TRAIN_POP_MAX>) <= 32764,
+              "the per-member tables of TRAIN_POP_MAX members must fit the kernel parameter limit");
 
 template <int NM>
-int gpt2_pack_train_wimg(const WimgPackParams<NM>& p, int L, int n, cudaStream_t st) {
-  pack_train_wimg_kernel<NM><<<dim3((WIMG_BYTES / 2 + 255) / 256, L, n), 256, 0, st>>>(p);
+int gpt2_pack_wimg(const WimgPackParams<NM>& p, int L, int n, cudaStream_t st) {
+  pack_wimg_kernel<NM><<<dim3((WIMG_BYTES / 2 + 255) / 256, L, n), 256, 0, st>>>(p);
   const cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) {
-    set_error("pack_train_wimg launch failed: %s", cudaGetErrorString(e));
+    set_error("pack_wimg launch failed: %s", cudaGetErrorString(e));
     return DPT_ERR_CUDA;
   }
   return DPT_OK;
 }
-template int gpt2_pack_train_wimg<1>(const WimgPackParams<1>&, int, int, cudaStream_t);
-template int gpt2_pack_train_wimg<TRAIN_POP_MAX>(const WimgPackParams<TRAIN_POP_MAX>&, int, int, cudaStream_t);
+template int gpt2_pack_wimg<1>(const WimgPackParams<1>&, int, int, cudaStream_t);
+template int gpt2_pack_wimg<TRAIN_POP_MAX>(const WimgPackParams<TRAIN_POP_MAX>&, int, int, cudaStream_t);
 
 }  // namespace dpt

@@ -23,8 +23,8 @@
 //
 // bf16 training (precision = 1, the *_ex entry points): bf16 operands at the tensor-core inputs, fp32 accumulation,
 // LayerNorm, softmax statistics, residual stream, loss, master weights and gradient sums.
-//   forward : the weight images of every member and layer are packed from the parameters (pack_train_wimg_kernel), then
-//             the tcgen05 dense forward (gpt2_dense.cu, SAVE = true) runs and saves the same fp32 records as the fp32
+//   forward : the weight images of every member and layer are packed from the parameters (pack_wimg_kernel), then
+//             the tcgen05 dense forward (gpt2_dense.cu) runs and saves the same fp32 records as the fp32
 //             forward of training; its logits are bit-identical to dpt_gpt2_forward(precision = 1).
 //   backward: 2 L + 1 launches, then the same weight-gradient reduction as fp32.
 //     gpt2_train_rows_bf16_kernel (phase l = L-1 .. -1, one thread per row of all B*S rows): the ln_1 backward of layer
@@ -994,13 +994,13 @@ static int population_forward16(const char* fn, const dpt_gpt2_weights_t* w, int
     float* mws = ws + (size_t)i * lay.total;
     m.sv = TrainSave{mws + lay.act, mws + lay.fin};
     p.wimg[i] = reinterpret_cast<const uint4*>(mws + lay.wimg);
-    pk.img[i] = reinterpret_cast<unsigned char*>(mws + lay.wimg);
     for (int l = 0; l < p.L; ++l) {
       const TrainLayerW& lw = m.w.layer[l];
       pk.w[i][l][0] = lw.attn_w, pk.w[i][l][1] = lw.proj_w, pk.w[i][l][2] = lw.fc_w, pk.w[i][l][3] = lw.fc2_w;
+      pk.img[i][l] = reinterpret_cast<unsigned char*>(mws + lay.wimg) + (size_t)l * WIMG_BYTES;
     }
   }
-  const int rc = gpt2_pack_train_wimg<NM>(pk, p.L, n, st);
+  const int rc = gpt2_pack_wimg<NM>(pk, p.L, n, st);
   if (rc != DPT_OK) return rc;
   return gpt2_train_forward_bf16_launch<NM>(p, n, st);
 }

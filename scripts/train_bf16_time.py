@@ -28,7 +28,7 @@ from dpt_b200.models.net import Transformer
 
 CASES = [("bandit_b64", 1, 5, 500, 4, 64, 1), ("darkroom_b64", 2, 5, 100, 4, 64, 1), ("bandit_b1024", 1, 5, 500, 4, 1024, 1),
          ("bandit_b64_population_k8", 1, 5, 500, 4, 64, 8)]
-PHASES = {"forward": ["gpt2_train_forward", "pack_train_wimg"],
+PHASES = {"forward": ["gpt2_train_forward", "pack_wimg"],
           "backward": ["gpt2_train_backward_kernel", "gpt2_train_rows_bf16", "gpt2_train_attn_bf16"],
           "reduction": ["weight_grad_partial_kernel", "weight_grad_reduce_kernel", "wpe_grad_kernel"]}
 
