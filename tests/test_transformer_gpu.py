@@ -458,10 +458,11 @@ def test_darkroom_offline_eval(dpt, name):
 def test_bf16_decode_fallback_geometry(dpt):
     """precision = 1 beyond what one SM's shared memory holds (weight fragments of all layers + 24 warps of score
     scratch): the loop falls back to 4-warp CTAs with the weights read through L1.  Same 2e-2 bar: the logits the loop
-    saw at the last steps against a fp32 forward (token-sequential kernel, > 512 tokens) over the context it built."""
+    saw at the last steps against a fp32 forward (token-sequential kernel, > 512 tokens) over the context it built.
+    At L = 4 the fallback starts at Tpad = 1280 (H > 1216): 4 x 24 KB of fragments + 24 x (160 + Tpad) x 4 B > 227 KB."""
     from dpt_b200.models.net import Transformer
     torch.manual_seed(11)
-    H, d, L, N = 1210, 5, 4, 6
+    H, d, L, N = 1300, 5, 4, 6
     m = Transformer({"horizon": H, "state_dim": 1, "action_dim": d, "n_layer": L, "n_embd": 32, "n_head": 1, "dropout": 0.0, "test": True})
     with torch.no_grad():
         for k, p in m.named_parameters():
