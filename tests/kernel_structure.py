@@ -1,6 +1,7 @@
 """Helpers of the structural kernel tests (test_kernel_structure_cpu.py, test_kernel_structure_gpu.py): the model they
-use, a batch whose sequences differ from a base sequence in exactly one token each, and the check that an output row
-depends on a token exactly when causality says it must.
+use, a batch whose sequences differ from a base sequence in exactly one token each, the check that an output row
+depends on a token exactly when causality says it must, and the online-loop cases (one per kernel variant) that
+test_sharp_attention_gpu.py shares.
 
 Token convention (the reference's models/net.py): token 0 is the query, token t >= 1 is context row t - 1.  With
 ``test=False`` output row r is token r + 1; with ``test=True`` the only output is token T."""
@@ -117,3 +118,23 @@ def wpe_grad_violations(g, r):
     if len(leak):
         bad.append("r=%d: wpe.grad rows %s are nonzero past r + 1" % (r, leak.tolist()[:8]))
     return bad
+
+
+def online_cases():
+    """(precision, L, N, H, variant) of the online loop, one per instantiation of gpt2_online_kernel: gpt2.cu
+    online_launch picks the variant from the env-warps per SM (one env per warp) at precision 0 and from the shared
+    memory the weight fragments need at precision 1.  test_kernel_structure_gpu.py checks with the profiler that each
+    case launches the variant it is named after."""
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    return [(0, 2, 37, 100, "fp32 bulk-copy ring, 1-warp CTAs"),
+            (0, 2, 16 * sms, 100, "fp32 bulk-copy ring, 2-warp CTAs"),
+            (0, 2, 24 * sms, 100, "fp32 bulk-copy ring, 4-warp CTAs"),
+            (0, 2, 24 * sms + 1, 100, "fp32 register-staged"),
+            (1, 2, 37, 100, "bf16 warp-specialised"),
+            (1, 4, 6, 1300, "bf16 fallback")]
+
+
+# (BF16, WS, TMA) template arguments of gpt2_online_kernel per variant of online_cases
+ONLINE_VARIANT_ARGS = {"fp32 bulk-copy ring": ("false", "false", "true"),
+                       "fp32 register-staged": ("false", "false", "false"),
+                       "bf16 warp-specialised": ("true", "true", "false"), "bf16 fallback": ("true", "false", "false")}

@@ -225,10 +225,6 @@ def test_decoder_scratch_independent(dpt, filled_runs, precision):
     _same(*filled_runs(lambda: _decode(m, x, 130)), "decoder")
 
 
-def _sm_count():
-    return torch.cuda.get_device_properties(0).multi_processor_count
-
-
 def _bf16_ws_fits(L, H):
     """The online loop's choice at precision 1 (gpt2.cu online_launch): the warp-specialised kernel when L layers of
     weight fragments (24 KB each) and 24 warps of score scratch ((32 + 128 + Tpad) floats, Tpad = H rounded up to 64)
@@ -236,27 +232,10 @@ def _bf16_ws_fits(L, H):
     return L * 24576 + 24 * (32 + 128 + (H + 63) // 64 * 64) * 4 <= 227 * 1024
 
 
-def _online_cases():
-    """(precision, L, N, H, variant) of the online loop: gpt2.cu online_launch picks the variant from the env-warps per
-    SM (one env per warp) at precision 0 and from the shared memory the weight fragments need at precision 1."""
-    sms = _sm_count()
-    return [(0, 2, 37, 100, "fp32 bulk-copy ring, 1-warp CTAs"),
-            (0, 2, 16 * sms, 100, "fp32 bulk-copy ring, 2-warp CTAs"),
-            (0, 2, 24 * sms, 100, "fp32 bulk-copy ring, 4-warp CTAs"),
-            (0, 2, 24 * sms + 1, 100, "fp32 register-staged"),
-            (1, 2, 37, 100, "bf16 warp-specialised"),
-            (1, 4, 6, 1300, "bf16 fallback")]
-
-
-# (BF16, WS, TMA) template arguments of gpt2_online_kernel per variant
-_VARIANT_ARGS = {"fp32 bulk-copy ring": ("false", "false", "true"), "fp32 register-staged": ("false", "false", "false"),
-                 "bf16 warp-specialised": ("true", "true", "false"), "bf16 fallback": ("true", "false", "false")}
-
-
 def test_online_loop_cases_reach_their_variants(dpt):
     """The N / H of the scratch cases launch the kernel variant they are named after (kernel names from the profiler).
     At L = 4 a horizon of 1210 (Tpad 1216) still fits the warp-specialised kernel; 1300 is past it."""
-    for precision, L, N, H, variant in _online_cases() + [(1, 4, 6, 1210, "bf16 warp-specialised")]:
+    for precision, L, N, H, variant in KS.online_cases() + [(1, 4, 6, 1210, "bf16 warp-specialised")]:
         assert _bf16_ws_fits(L, H) == (variant == "bf16 warp-specialised") or precision == 0
         m = KS.model(1, 5, L, H, True).cuda()
         m.precision = precision
@@ -267,7 +246,7 @@ def test_online_loop_cases_reach_their_variants(dpt):
             torch.cuda.synchronize()
         names = [e.name for e in prof.events() if "gpt2_online_kernel" in e.name]
         args = {re.search(r"gpt2_online_kernel<(\w+), ?(\w+), ?(\w+)", n).groups() for n in names}
-        assert args == {_VARIANT_ARGS[variant.split(",")[0]]}, (variant, names)
+        assert args == {KS.ONLINE_VARIANT_ARGS[variant.split(",")[0]]}, (variant, names)
 
 
 @pytest.mark.parametrize("case", range(6))
@@ -275,7 +254,7 @@ def test_online_loop_scratch_independent(dpt, filled_runs, case):
     """online_loop with dump=True in every kernel variant, and a two-member online_loop_population: context, cumulative
     means, regret sums, reward noise, uniforms and logits."""
     from dpt_b200.models.net import online_loop_population
-    precision, L, N, H, variant = _online_cases()[case]
+    precision, L, N, H, variant = KS.online_cases()[case]
     ms = [KS.model(1, 5, L, H, True, seed=i).cuda() for i in range(2)]
     for mm in ms:
         mm.precision = precision

@@ -31,10 +31,15 @@ def tokens(q, cs, ca, cns, cr):
     return torch.cat([first, rest], 1)
 
 
-def forward(P, n_layer, q, cs, ca, cns, cr, test, sdpa=False):
+def forward(P, n_layer, q, cs, ca, cns, cr, test, sdpa=False, record=None, rnd=None):
     """Transformer.forward in the dtype of P (float64 for the yardstick; float32 with sdpa=True is the eager torch
-    training step that scripts/train_time.py times)."""
+    training step that scripts/train_time.py times).
+
+    record: a list that receives each layer's (scores, probabilities), [B, S, S] with -inf / 0 above the diagonal.
+    rnd: a function applied to q, k, v, the attention probabilities and both operands of every projection inside the
+    layers (the places where the bf16 kernels hold bf16 values); None leaves every value in the dtype of P."""
     dt = P["embed_transition.weight"].dtype
+    r = rnd or (lambda t: t)
     seq = tokens(*(t.to(dt) for t in (q, cs, ca, cns, cr)))
     S = seq.shape[1]
     x = seq @ P["embed_transition.weight"].T + P["embed_transition.bias"] + P["transformer.wpe.weight"][:S]
@@ -43,16 +48,20 @@ def forward(P, n_layer, q, cs, ca, cns, cr, test, sdpa=False):
     for l in range(n_layer):
         p = "transformer.h.%d." % l
         h = _ln(x, P[p + "ln_1.weight"], P[p + "ln_1.bias"])
-        qkv = h @ P[p + "attn.c_attn.weight"] + P[p + "attn.c_attn.bias"]
-        qq, k, v = qkv[..., :E], qkv[..., E:2 * E], qkv[..., 2 * E:]
+        qkv = r(h) @ r(P[p + "attn.c_attn.weight"]) + P[p + "attn.c_attn.bias"]
+        qq, k, v = r(qkv[..., :E]), r(qkv[..., E:2 * E]), r(qkv[..., 2 * E:])
         if sdpa:
             a = torch.nn.functional.scaled_dot_product_attention(qq, k, v, is_causal=True)
         else:
             s = (qq @ k.transpose(-1, -2)) / math.sqrt(E)
-            a = torch.softmax(s.masked_fill(~mask, float("-inf")), -1) @ v
-        x = x + a @ P[p + "attn.c_proj.weight"] + P[p + "attn.c_proj.bias"]
+            pr = torch.softmax(s.masked_fill(~mask, float("-inf")), -1)
+            if record is not None:
+                record.append((s.masked_fill(~mask, float("-inf")), pr))
+            a = r(pr) @ v
+        x = x + r(a) @ r(P[p + "attn.c_proj.weight"]) + P[p + "attn.c_proj.bias"]
         h = _ln(x, P[p + "ln_2.weight"], P[p + "ln_2.bias"])
-        x = x + _gelu_new(h @ P[p + "mlp.c_fc.weight"] + P[p + "mlp.c_fc.bias"]) @ P[p + "mlp.c_proj.weight"] + P[p + "mlp.c_proj.bias"]
+        f = _gelu_new(r(h) @ r(P[p + "mlp.c_fc.weight"]) + P[p + "mlp.c_fc.bias"])
+        x = x + r(f) @ r(P[p + "mlp.c_proj.weight"]) + P[p + "mlp.c_proj.bias"]
     x = _ln(x, P["transformer.ln_f.weight"], P["transformer.ln_f.bias"])
     preds = x @ P["pred_actions.weight"].T + P["pred_actions.bias"]
     return preds[:, -1, :] if test else preds[:, 1:, :]
