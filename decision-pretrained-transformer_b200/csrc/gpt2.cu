@@ -650,10 +650,10 @@ __global__ void __launch_bounds__(G_THREADS) gpt2_decode_step_kernel(const StepP
 // ---------------------------------------------------------------------------------------------
 // Fused bandit online loop with the transformer controller
 // ---------------------------------------------------------------------------------------------
-// The online loop's launch parameters.  NM: member capacity of the launch -- 1 for dpt_gpt2_online_loop and one-member
-// population calls, ONLINE_POP_MAX for dpt_gpt2_online_loop_population, whose CTA (env block, member = blockIdx.y) takes
-// its member's weights, K/V region and outputs from a table in the kernel parameters (no upload, graph-capturable).  The
-// means, noise and inject arrays are shared: member i computes exactly what a one-model call on its own weights would.
+// The online loop's launch parameters.  NM: member capacity of the launch -- 1 for a one-model dpt_gpt2_online_loop call,
+// ONLINE_POP_MAX for a population call, whose CTA (env block, member = blockIdx.y) takes its member's weights, K/V region
+// and outputs from a table in the kernel parameters (no upload, graph-capturable).  The means, noise and inject arrays
+// are shared: member i computes exactly what a one-model call on its own weights would.
 constexpr int ONLINE_POP_MAX = DPT_GPT2_ONLINE_POPULATION_MAX;
 struct OnlineMember {   // what differs between the members of a population launch
   Gpt2Dev m;
@@ -1161,45 +1161,13 @@ static int online_launch(const OnlineGptParams<NM>& p, int n, int L, int precisi
                 dim3((N + G_WARPS - 1) / G_WARPS, n), G_THREADS, G_WARPS * per_warp, stream, p);
 }
 
-extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double var, int reward_type, int sample, uint64_t seed,
-                                    uint64_t env_id0, int N, int H, int precision, void* kv_cache, uint64_t kv_bytes,
-                                    float* ctx_states, float* ctx_actions, float* ctx_next_states, float* ctx_rewards,
-                                    float* cum_means, double* regret_sums, const dpt_gpt2_online_inject_t* inject,
+extern "C" int dpt_gpt2_online_loop(dpt_gpt2_t* const* models, int n_models, const float* means, double var, int reward_type,
+                                    int sample, uint64_t seed, uint64_t env_id0, int N, int H, int precision, void* kv_cache,
+                                    uint64_t kv_bytes, float* const* ctx_states, float* const* ctx_actions,
+                                    float* const* ctx_next_states, float* const* ctx_rewards, float* const* cum_means,
+                                    double* const* regret_sums, const dpt_gpt2_online_inject_t* inject,
                                     const dpt_gpt2_online_dump_t* dump, void* stream) {
-  DPT_CHECK_ARG(m, "dpt_gpt2_online_loop: null model");
-  DPT_CHECK_ARG(reward_type == DPT_REWARD_GAUSSIAN || reward_type == DPT_REWARD_BERNOULLI,
-                "dpt_gpt2_online_loop: unknown reward_type %d (0 uniform/gaussian, 1 bernoulli)", reward_type);
-  DPT_CHECK_ARG(precision == 0 || precision == 1, "dpt_gpt2_online_loop: precision %d (0 = fp32, 1 = bf16 K/V cache)", precision);
-  DPT_CHECK_ARG(m->dev.dx == 1, "dpt_gpt2_online_loop: bandit loop needs state_dim == 1 (got %d)", m->dev.dx);
-  DPT_CHECK_ARG(N >= 0 && H >= 0, "dpt_gpt2_online_loop: N=%d H=%d", N, H);
-  DPT_CHECK_ARG(H <= m->dev.n_pos, "dpt_gpt2_online_loop: H=%d exceeds n_positions %d", H, m->dev.n_pos);
-  if (N == 0 || H == 0) return DPT_OK;
-  DPT_CHECK_ARG(means && kv_cache && kv_bytes >= dpt_gpt2_online_kv_bytes(m, N, H, precision), "dpt_gpt2_online_loop: null means or kv cache too small");
-  const bool any = ctx_states || ctx_actions || ctx_next_states || ctx_rewards;
-  DPT_CHECK_ARG(!any || (ctx_states && ctx_actions && ctx_next_states && ctx_rewards),
-                "dpt_gpt2_online_loop: context pointers must be all NULL or all non-NULL");
-  OnlineGptParams<1> p{};
-  p.m = m->dev;
-  p.means = means, p.var = var, p.rtype = reward_type, p.sample = sample;
-  p.key = Key{(uint32_t)seed, (uint32_t)(seed >> 32)};
-  p.env_id0 = env_id0;
-  p.N = N, p.H = H, p.Tpad = tpad_for(H, precision);
-  p.kv = kv_cache;
-  p.ctx_s = ctx_states, p.ctx_a = ctx_actions, p.ctx_ns = ctx_next_states, p.ctx_r = ctx_rewards;
-  p.cum_means = cum_means, p.regret = regret_sums;
-  if (inject) p.in = *inject;
-  if (dump) p.out = *dump;
-  return online_launch(p, 1, m->dev.L, precision, stream);
-}
-
-extern "C" int dpt_gpt2_online_loop_population(dpt_gpt2_t* const* models, int n_models, const float* means, double var,
-                                               int reward_type, int sample, uint64_t seed, uint64_t env_id0, int N, int H,
-                                               int precision, void* kv_cache, uint64_t kv_bytes, float* const* ctx_states,
-                                               float* const* ctx_actions, float* const* ctx_next_states,
-                                               float* const* ctx_rewards, float* const* cum_means, double* const* regret_sums,
-                                               const dpt_gpt2_online_inject_t* inject, const dpt_gpt2_online_dump_t* dump,
-                                               void* stream) {
-  const char* fn = "dpt_gpt2_online_loop_population";
+  const char* fn = "dpt_gpt2_online_loop";
   DPT_CHECK_ARG(n_models >= 0 && n_models <= ONLINE_POP_MAX, "%s: n_models=%d outside [0,%d]", fn, n_models, ONLINE_POP_MAX);
   if (n_models == 0) return DPT_OK;
   DPT_CHECK_ARG(models, "%s: null models array", fn);

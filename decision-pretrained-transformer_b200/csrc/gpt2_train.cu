@@ -1,5 +1,6 @@
 // Training of the GPT-2 (models/net.py:9-60) in fp32 on the CUDA cores, sequences of <= 512 tokens.
 //
+// At precision 0:
 //   dpt_gpt2_train_forward : the dense fp32 forward (gpt2_dense_fp32.cu, SAVE = true) on the parameter tensors as
 //                            they are -- no handle, no repack -- which also stores each row's activations (TA_* / TF_*).
 //   dpt_gpt2_train_backward: three launches on the caller's stream.
@@ -15,14 +16,14 @@
 //        the position gradients over the batch in sequence order (rows past T are zero).
 //   Every sum has a fixed order, so two identical calls give bit-identical gradients.
 //
-// Population training (dpt_gpt2_train_population_*): n same-shape models in the same launches.  Every kernel takes its
-// member from the grid (forward / backward: blockIdx.y, partial sums and reduction: blockIdx.z, wpe: blockIdx.y); member i
-// uses workspace region i (train_layout(...).total floats each) and its own pointer table in the kernel parameters.  The
-// chunking depends on B and T only, so each member runs exactly the arithmetic of the one-model call; the one-model entry
-// points are the n = 1 case (kernels instantiated with a member capacity NM of 1, so their parameter blocks stay small).
+// Population training (n_models > 1): n same-shape models in the same launches.  Every kernel takes its member from the
+// grid (forward / backward: blockIdx.y, partial sums and reduction: blockIdx.z, wpe: blockIdx.y); member i uses workspace
+// region i (train_layout(...).total floats each) and its own pointer table in the kernel parameters.  The chunking depends
+// on B and T only, so each member runs exactly the arithmetic of a one-model call.  n = 1 launches the kernels
+// instantiated with a member capacity NM of 1, so that their parameter blocks stay small; n > 1 those with TRAIN_POP_MAX.
 //
-// bf16 training (precision = 1, the *_ex entry points): bf16 operands at the tensor-core inputs, fp32 accumulation,
-// LayerNorm, softmax statistics, residual stream, loss, master weights and gradient sums.
+// bf16 training (precision = 1): bf16 operands at the tensor-core inputs, fp32 accumulation, LayerNorm, softmax
+// statistics, residual stream, loss, master weights and gradient sums.
 //   forward : the weight images of every member and layer are packed from the parameters (pack_wimg_kernel), then
 //             the tcgen05 dense forward (gpt2_dense.cu) runs and saves the same fp32 records as the fp32
 //             forward of training; its logits are bit-identical to dpt_gpt2_forward(precision = 1).
@@ -851,7 +852,7 @@ static int params_per_slot(int L, int din, int du) {
   return (p + 3) & ~3;
 }
 
-static TrainLayout train_layout(int L, int din, int du, int B, int T, int precision = 0) {
+static TrainLayout train_layout(int L, int din, int du, int B, int T, int precision) {
   TrainLayout t{};
   t.L = L, t.S = T + 1, t.din = din, t.du = du;
   t.NR = (size_t)B * t.S;
@@ -876,7 +877,7 @@ static TrainLayout train_layout(int L, int din, int du, int B, int T, int precis
   return t;
 }
 
-// `mem`: the member's index in a population call (its messages name it), -1 for the one-model entry points
+// `mem`: the member's index in a population call (its messages name it), -1 for a one-model call
 static int check_model(const char* fn, int mem, const dpt_gpt2_weights_t* w, int B, int T) {
   char who[96];
   if (mem < 0) snprintf(who, sizeof who, "%s", fn);
@@ -910,9 +911,9 @@ static int check_model(const char* fn, int mem, const dpt_gpt2_weights_t* w, int
   return DPT_OK;
 }
 
-// The checks of a population call: 0 <= n <= TRAIN_POP_MAX, every member valid (check_model) and of member 0's shape.
+// The checks of a training call: 0 <= n <= TRAIN_POP_MAX, every member valid (check_model) and of member 0's shape.
 // Returns DPT_OK with *done = true when there is nothing to compute (n = 0 or B = 0).
-static int check_population(const char* fn, const dpt_gpt2_weights_t* w, int n, int B, int T, bool* done, int precision = 0) {
+static int check_population(const char* fn, const dpt_gpt2_weights_t* w, int n, int B, int T, bool* done, int precision) {
   *done = true;
   if (precision != 0 && precision != 1) {
     set_error("%s: precision=%d, training supports 0 (fp32) and 1 (bf16 tensor cores)", fn, precision);
@@ -949,7 +950,7 @@ static TrainW train_w(const dpt_gpt2_weights_t* w) {
   return d;
 }
 
-static uint64_t member_bytes(const dpt_gpt2_weights_t* w, int B, int T, int precision = 0) {
+static uint64_t member_bytes(const dpt_gpt2_weights_t* w, int B, int T, int precision) {
   return train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T, precision).total * sizeof(float);
 }
 
@@ -957,7 +958,7 @@ template <int NM>
 static int population_forward(const char* fn, const dpt_gpt2_weights_t* w, int n, const float* const* query,
                               const float* const* cs, const float* const* ca, const float* const* cns, const float* const* cr,
                               int B, int T, int T_stride, int test, float* const* out, float* ws, cudaStream_t st) {
-  const TrainLayout lay = train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T);
+  const TrainLayout lay = train_layout(w->n_layer, 2 * w->state_dim + w->action_dim + 1, w->action_dim, B, T, 0);
   TrainFwdParams<NM> p{};
   p.L = w->n_layer, p.dx = w->state_dim, p.du = w->action_dim, p.din = lay.din;
   p.B = B, p.T = T, p.Ts = T_stride, p.test = test ? 1 : 0;
@@ -1122,11 +1123,21 @@ static int population_backward(const char* fn, const dpt_gpt2_weights_t* w, int 
   return DPT_OK;
 }
 
-// the argument checks and launches shared by the one-model and the population entry points (one = the one-model call)
-static int train_forward(const char* fn, bool one, const dpt_gpt2_weights_t* w, int n, const float* const* query,
-                         const float* const* cs, const float* const* ca, const float* const* cns, const float* const* cr, int B,
-                         int T, int T_stride, int test, float* const* out, void* workspace, uint64_t workspace_bytes,
-                         void* stream, int precision = 0) {
+}  // namespace dpt
+
+using namespace dpt;
+
+extern "C" uint64_t dpt_gpt2_train_workspace_bytes(const dpt_gpt2_weights_t* w, int n_models, int B, int T, int precision) {
+  if (!w || n_models <= 0 || n_models > TRAIN_POP_MAX || B <= 0 || T < 0 || w->n_layer < 1 || (precision != 0 && precision != 1))
+    return 0;
+  return (uint64_t)n_models * member_bytes(w, B, T, precision);
+}
+
+extern "C" int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, int n, const float* const* query, const float* const* cs,
+                                      const float* const* ca, const float* const* cns, const float* const* cr, int B, int T,
+                                      int T_stride, int test, int precision, float* const* out, void* workspace,
+                                      uint64_t workspace_bytes, void* stream) {
+  const char* fn = "dpt_gpt2_train_forward";
   bool done;
   int rc = check_population(fn, w, n, B, T, &done, precision);
   if (rc != DPT_OK) return rc;
@@ -1136,7 +1147,7 @@ static int train_forward(const char* fn, bool one, const dpt_gpt2_weights_t* w, 
   DPT_CHECK_ARG(query && out && (T == 0 || (cs && ca && cns && cr)), "%s: null input or output pointer array", fn);
   for (int i = 0; i < n; ++i)
     DPT_CHECK_ARG(query[i] && out[i] && (T == 0 || (cs[i] && ca[i] && cns[i] && cr[i])),
-                  one ? "%s: null input or output pointer" : "%s: member %d: null input or output pointer", fn, i);
+                  n == 1 ? "%s: null input or output pointer" : "%s: member %d: null input or output pointer", fn, i);
   const uint64_t need = (uint64_t)n * member_bytes(w, B, T, precision);
   DPT_CHECK_ARG(workspace && workspace_bytes >= need && aligned16(workspace), "%s: workspace of %llu B, needs %llu B (16 B aligned)",
                 fn, (unsigned long long)workspace_bytes, (unsigned long long)need);
@@ -1149,9 +1160,10 @@ static int train_forward(const char* fn, bool one, const dpt_gpt2_weights_t* w, 
                 : population_forward<TRAIN_POP_MAX>(fn, w, n, query, cs, ca, cns, cr, B, T, T_stride, test, out, ws, st);
 }
 
-static int train_backward(const char* fn, bool one, const dpt_gpt2_weights_t* w, int n, const float* const* dout, int B, int T,
-                          int test, const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream,
-                          int precision = 0) {
+extern "C" int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, int n, const float* const* dout, int B, int T, int test,
+                                       int precision, const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes,
+                                       void* stream) {
+  const char* fn = "dpt_gpt2_train_backward";
   bool done;
   int rc = check_population(fn, w, n, B, T, &done, precision);
   if (rc != DPT_OK || done) return rc;
@@ -1162,11 +1174,11 @@ static int train_backward(const char* fn, bool one, const dpt_gpt2_weights_t* w,
   const int L = w->n_layer;
   for (int i = 0; i < n; ++i) {
     const dpt_gpt2_grads_t* g = grads + i;
-    DPT_CHECK_ARG(dout[i], one ? "%s: null dout or grads" : "%s: member %d: null dout", fn, i);
+    DPT_CHECK_ARG(dout[i], n == 1 ? "%s: null dout or grads" : "%s: member %d: null dout", fn, i);
     DPT_CHECK_ARG(g->wpe && g->embed_w && g->embed_b && g->pred_w && g->pred_b && g->lnf_w && g->lnf_b && g->ln1_w && g->ln1_b &&
                       g->attn_w && g->attn_b && g->proj_w && g->proj_b && g->ln2_w && g->ln2_b && g->fc_w && g->fc_b &&
                       g->fc2_w && g->fc2_b,
-                  one ? "%s: null gradient pointer" : "%s: member %d: null gradient pointer", fn, i);
+                  n == 1 ? "%s: null gradient pointer" : "%s: member %d: null gradient pointer", fn, i);
     for (int l = 0; l < L; ++l)
       DPT_CHECK_ARG(g->ln1_w[l] && g->ln1_b[l] && g->attn_w[l] && g->attn_b[l] && g->proj_w[l] && g->proj_b[l] && g->ln2_w[l] &&
                         g->ln2_b[l] && g->fc_w[l] && g->fc_b[l] && g->fc2_w[l] && g->fc2_b[l],
@@ -1176,69 +1188,4 @@ static int train_backward(const char* fn, bool one, const dpt_gpt2_weights_t* w,
   cudaStream_t st = (cudaStream_t)stream;
   return n == 1 ? population_backward<1>(fn, w, n, dout, B, T, test, grads, ws, st, precision)
                 : population_backward<TRAIN_POP_MAX>(fn, w, n, dout, B, T, test, grads, ws, st, precision);
-}
-
-}  // namespace dpt
-
-using namespace dpt;
-
-extern "C" uint64_t dpt_gpt2_train_population_workspace_bytes_ex(const dpt_gpt2_weights_t* w, int n_models, int B, int T,
-                                                                  int precision) {
-  if (!w || n_models <= 0 || n_models > TRAIN_POP_MAX || B <= 0 || T < 0 || w->n_layer < 1 || (precision != 0 && precision != 1))
-    return 0;
-  return (uint64_t)n_models * member_bytes(w, B, T, precision);
-}
-
-extern "C" uint64_t dpt_gpt2_train_population_workspace_bytes(const dpt_gpt2_weights_t* w, int n_models, int B, int T) {
-  return dpt_gpt2_train_population_workspace_bytes_ex(w, n_models, B, T, 0);
-}
-
-extern "C" uint64_t dpt_gpt2_train_workspace_bytes(const dpt_gpt2_weights_t* w, int B, int T) {
-  return dpt_gpt2_train_population_workspace_bytes(w, 1, B, T);
-}
-
-extern "C" int dpt_gpt2_train_population_forward(const dpt_gpt2_weights_t* w, int n_models, const float* const* query_states,
-                                                 const float* const* ctx_states, const float* const* ctx_actions,
-                                                 const float* const* ctx_next_states, const float* const* ctx_rewards, int B,
-                                                 int T, int T_stride, int test, float* const* out, void* workspace,
-                                                 uint64_t workspace_bytes, void* stream) {
-  return train_forward("dpt_gpt2_train_population_forward", false, w, n_models, query_states, ctx_states, ctx_actions,
-                       ctx_next_states, ctx_rewards, B, T, T_stride, test, out, workspace, workspace_bytes, stream);
-}
-
-extern "C" int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, const float* query_states, const float* ctx_states,
-                                      const float* ctx_actions, const float* ctx_next_states, const float* ctx_rewards, int B,
-                                      int T, int T_stride, int test, float* out, void* workspace, uint64_t workspace_bytes,
-                                      void* stream) {
-  return train_forward("dpt_gpt2_train_forward", true, w, 1, &query_states, &ctx_states, &ctx_actions, &ctx_next_states,
-                       &ctx_rewards, B, T, T_stride, test, &out, workspace, workspace_bytes, stream);
-}
-
-extern "C" int dpt_gpt2_train_population_forward_ex(const dpt_gpt2_weights_t* w, int n_models, const float* const* query_states,
-                                                    const float* const* ctx_states, const float* const* ctx_actions,
-                                                    const float* const* ctx_next_states, const float* const* ctx_rewards, int B,
-                                                    int T, int T_stride, int test, int precision, float* const* out,
-                                                    void* workspace, uint64_t workspace_bytes, void* stream) {
-  return train_forward("dpt_gpt2_train_population_forward_ex", n_models == 1, w, n_models, query_states, ctx_states,
-                       ctx_actions, ctx_next_states, ctx_rewards, B, T, T_stride, test, out, workspace, workspace_bytes, stream,
-                       precision);
-}
-
-extern "C" int dpt_gpt2_train_population_backward_ex(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B,
-                                                     int T, int test, int precision, const dpt_gpt2_grads_t* grads,
-                                                     void* workspace, uint64_t workspace_bytes, void* stream) {
-  return train_backward("dpt_gpt2_train_population_backward_ex", n_models == 1, w, n_models, dout, B, T, test, grads, workspace,
-                        workspace_bytes, stream, precision);
-}
-
-extern "C" int dpt_gpt2_train_population_backward(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B,
-                                                  int T, int test, const dpt_gpt2_grads_t* grads, void* workspace,
-                                                  uint64_t workspace_bytes, void* stream) {
-  return train_backward("dpt_gpt2_train_population_backward", false, w, n_models, dout, B, T, test, grads, workspace,
-                        workspace_bytes, stream);
-}
-
-extern "C" int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float* dout, int B, int T, int test,
-                                       const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream) {
-  return train_backward("dpt_gpt2_train_backward", true, w, 1, &dout, B, T, test, grads, workspace, workspace_bytes, stream);
 }

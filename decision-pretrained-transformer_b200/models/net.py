@@ -11,8 +11,8 @@ from the config is ignored: the trunk always has ONE head (models/net.py:29), he
 same computation with a gradient: dpt_gpt2_train_forward / dpt_gpt2_train_backward (hand-written CUDA, fp32) read
 the parameter tensors in place, and autograd receives a gradient for every parameter except ``transformer.wte``
 (which the model never reads, as in the reference).  ``forward_train(x, precision=1)`` is bf16 mixed-precision
-training (the *_ex entry points): the tcgen05 forward of ``forward`` at ``model.precision = 1`` and a tensor-core
-attention backward, with fp32 master weights and gradient sums.  The class holds no HuggingFace dependency.
+training (the same entry points at precision 1): the tcgen05 forward of ``forward`` at ``model.precision = 1`` and a
+tensor-core attention backward, with fp32 master weights and gradient sums.  The class holds no HuggingFace dependency.
 """
 import ctypes
 
@@ -109,33 +109,11 @@ class Transformer(nn.Module):
         if self._handle is not None and ver == self._handle_version:
             return self._handle
         self._free()
-        t = self.transformer
-        f = lambda p: p.detach().float().contiguous()   # noqa: E731
-        keep = []
-
-        def P(p):
-            x = f(p)
-            keep.append(x)
-            return x.data_ptr()
-
-        def arr(fn):
-            a = (ctypes.c_void_p * self.n_layer)(*[P(fn(b)) for b in t.h])
-            keep.append(a)
-            return ctypes.cast(a, ctypes.POINTER(ctypes.c_void_p))
-        w = _lib.Gpt2Weights(
-            horizon=self.horizon, state_dim=self.state_dim, action_dim=self.action_dim, n_layer=self.n_layer,
-            n_embd=self.n_embd, n_positions=t.wpe.weight.shape[0],
-            wpe=P(t.wpe.weight), embed_w=P(self.embed_transition.weight), embed_b=P(self.embed_transition.bias),
-            pred_w=P(self.pred_actions.weight), pred_b=P(self.pred_actions.bias), lnf_w=P(t.ln_f.weight), lnf_b=P(t.ln_f.bias),
-            ln1_w=arr(lambda b: b.ln_1.weight), ln1_b=arr(lambda b: b.ln_1.bias),
-            attn_w=arr(lambda b: b.attn.c_attn.weight), attn_b=arr(lambda b: b.attn.c_attn.bias),
-            proj_w=arr(lambda b: b.attn.c_proj.weight), proj_b=arr(lambda b: b.attn.c_proj.bias),
-            ln2_w=arr(lambda b: b.ln_2.weight), ln2_b=arr(lambda b: b.ln_2.bias),
-            fc_w=arr(lambda b: b.mlp.c_fc.weight), fc_b=arr(lambda b: b.mlp.c_fc.bias),
-            fc2_w=arr(lambda b: b.mlp.c_proj.weight), fc2_b=arr(lambda b: b.mlp.c_proj.bias))
+        ps, keep = [p.detach().float().contiguous() for p in self._train_params()], []
+        w = _weights_struct(self, ps, keep)
         h = ctypes.c_void_p()
         check(lib().dpt_gpt2_create(ctypes.byref(w), ctypes.byref(h), stream_ptr()), "dpt_gpt2_create")
-        torch.cuda.current_stream().synchronize()      # the D2D repack read `keep`
+        torch.cuda.current_stream().synchronize()      # the D2D repack read `ps`
         self._handle, self._handle_version = h, ver
         return h
 
@@ -161,19 +139,7 @@ class Transformer(nn.Module):
         """``ctx_share`` > 1: ``query_states`` has ctx_share rows per context row (see dpt_gpt2_forward)."""
         dev = kernels._dev()
         h = self.handle()
-        f = lambda t: t.to(device=dev, dtype=torch.float32)   # noqa: E731
-        q = f(x["query_states"]).contiguous()
-        cs, ca, cns, cr = f(x["context_states"]), f(x["context_actions"]), f(x["context_next_states"]), f(x["context_rewards"])
-        B, T = ca.shape[0] * ctx_share, ca.shape[1]
-        Bc = ca.shape[0]
-        assert q.shape[0] == B
-        # context views [:, :h] of a [B,H,.] buffer are passed with their row stride, without a copy
-        stride = ca.stride(0) // max(1, ca.shape[2]) if T > 0 else 0
-        ok = T > 0 and stride >= T and all(t.stride(-1) == 1 and t.stride(1) == t.shape[2] and t.stride(0) == stride * t.shape[2]
-                           for t in (cs, ca, cns, cr.reshape(Bc, T, 1) if cr.dim() == 2 else cr))
-        if not ok:
-            cs, ca, cns, cr = cs.contiguous(), ca.contiguous(), cns.contiguous(), cr.contiguous()
-            stride = T
+        q, cs, ca, cns, cr, B, T, stride = _batch_inputs(x, dev, ctx_share)
         out = torch.empty((B, self.action_dim) if self.test else (B, T, self.action_dim), dtype=torch.float32, device=dev)
         nbytes = lib().dpt_gpt2_forward_workspace_bytes(h, B, T, self.precision)
         ws = self._scratch(nbytes)
@@ -235,7 +201,8 @@ _TOP_NAMES = ("wpe", "embed_w", "embed_b", "pred_w", "pred_b", "lnf_w", "lnf_b")
 
 
 def _pointer_struct(cls, model, tensors, keep, **extra):
-    """dpt_gpt2_weights_t / dpt_gpt2_grads_t over `tensors` (ordered as Transformer._train_params)."""
+    """dpt_gpt2_weights_t / dpt_gpt2_grads_t over `tensors` (ordered as Transformer._train_params); the per-layer pointer
+    arrays go to `keep`."""
     L = model.n_layer
     for t in tensors:
         if t.dtype != torch.float32 or not t.is_contiguous() or not t.is_cuda:
@@ -255,17 +222,18 @@ def _weights_struct(model, params, keep):
                            n_positions=model.transformer.wpe.weight.shape[0])
 
 
-def _train_inputs(x, dev):
-    """(q, cs, ca, cns, cr, B, T, stride) of a batch dict; context views [:, :h] of a [B,H,.] buffer keep their row
-    stride, other layouts are made contiguous."""
+def _batch_inputs(x, dev, ctx_share=1):
+    """(q, cs, ca, cns, cr, B, T, stride) of a batch dict, B = ctx_share * context rows (see dpt_gpt2_forward); context
+    views [:, :h] of a [B,H,.] buffer keep their row stride, other layouts are made contiguous."""
     f = lambda t: t.to(device=dev, dtype=torch.float32)   # noqa: E731
     q = f(x["query_states"]).contiguous()
     cs, ca, cns, cr = f(x["context_states"]), f(x["context_actions"]), f(x["context_next_states"]), f(x["context_rewards"])
-    B, T = ca.shape[0], ca.shape[1]
+    Bc, T = ca.shape[0], ca.shape[1]
+    B = Bc * ctx_share
     assert q.shape[0] == B, "query_states and the context disagree on the batch size"
     stride = ca.stride(0) // max(1, ca.shape[2]) if T > 0 else 0
     ok = T > 0 and stride >= T and all(t.stride(-1) == 1 and t.stride(1) == t.shape[2] and t.stride(0) == stride * t.shape[2]
-                                       for t in (cs, ca, cns, cr.reshape(B, T, 1) if cr.dim() == 2 else cr))
+                                       for t in (cs, ca, cns, cr.reshape(Bc, T, 1) if cr.dim() == 2 else cr))
     if not ok:
         cs, ca, cns, cr = cs.contiguous(), ca.contiguous(), cns.contiguous(), cr.contiguous()
         stride = T
@@ -304,7 +272,7 @@ def forward_train_population(models, batches, precision=0):
     if devs[0] != dev:
         for m in models:
             m.to(dev)
-    ins = [_train_inputs(x, dev) for x in batches]
+    ins = [_batch_inputs(x, dev) for x in batches]
     for i, x in enumerate(ins):
         if x[5:7] != ins[0][5:7]:
             raise ValueError("forward_train_population: batch %d has B, T = %d, %d, batch 0 has %d, %d"
@@ -324,9 +292,52 @@ def forward_train_population(models, batches, precision=0):
 POPULATION_MAX = 32   # DPT_GPT2_POPULATION_MAX: members per population launch
 
 
+class _TrainCall:
+    """The arguments of dpt_gpt2_train_forward / dpt_gpt2_train_backward for k same-shape members: the weights array over
+    the members' parameter tensors, the HOST arrays of k device pointers (refilled by every call, never reallocated) and
+    the workspace that holds the saved activations from a forward to its backward."""
+
+    def __init__(self, models, params, precision):
+        k = len(models)
+        n = len(params) // k
+        self.models, self.k, self.precision, self._keep = models, k, precision, []
+        self.w = (_lib.Gpt2Weights * k)(*[_weights_struct(m, params[i * n:(i + 1) * n], self._keep)
+                                          for i, m in enumerate(models)])
+        self._arrays = [(ctypes.c_void_p * k)() for _ in range(6)]   # query, the four context inputs, out / dout
+        self.ws = None
+
+    def reserve(self, B, T, dev):
+        """Allocate the workspace for calls of up to B sequences of T transitions."""
+        nbytes = lib().dpt_gpt2_train_workspace_bytes(self.w, self.k, B, T, self.precision)
+        self.ws = torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=dev)
+
+    def _fill(self, j, ptrs):
+        a = self._arrays[j]
+        a[:] = ptrs
+        return a
+
+    def grads(self, tensors):
+        """dpt_gpt2_grads_t of every member over ``tensors[i]`` (ordered as Transformer._train_params)."""
+        return (_lib.Gpt2Grads * self.k)(*[_pointer_struct(_lib.Gpt2Grads, m, ts, self._keep)
+                                           for m, ts in zip(self.models, tensors)])
+
+    def forward(self, inputs, outs, B, T, stride, test):
+        """``inputs[i]``: member i's query states and four context tensors; ``outs[i]``: its logits."""
+        ins = [self._fill(j, [x[j].data_ptr() if j == 0 or T else None for x in inputs]) for j in range(5)]
+        check(lib().dpt_gpt2_train_forward(self.w, self.k, *ins, B, T, stride, 1 if test else 0, self.precision,
+                                           self._fill(5, [o.data_ptr() for o in outs]), self.ws.data_ptr(), self.ws.numel(),
+                                           stream_ptr()), "dpt_gpt2_train_forward")
+
+    def backward(self, douts, grads, B, T, test):
+        """``douts[i]``: the gradient of member i's logits; ``grads``: from ``self.grads``."""
+        check(lib().dpt_gpt2_train_backward(self.w, self.k, self._fill(5, [d.data_ptr() for d in douts]), B, T, 1 if test else 0,
+                                            self.precision, grads, self.ws.data_ptr(), self.ws.numel(), stream_ptr()),
+              "dpt_gpt2_train_backward")
+
+
 class _PopulationTrainFn(torch.autograd.Function):
-    """dpt_gpt2_train_population_forward / _backward over k members (k = 1: the one-model path), or their _ex forms at
-    precision 1.  One workspace holds every member's saved activations between the two."""
+    """dpt_gpt2_train_forward / dpt_gpt2_train_backward over k members.  One workspace holds every member's saved
+    activations between the two."""
 
     @staticmethod
     def forward(ctx, models, inputs, precision, *params):
@@ -334,27 +345,12 @@ class _PopulationTrainFn(torch.autograd.Function):
         k, m0 = len(models), models[0]
         B, T, stride = inputs[0][5:8]
         dev = inputs[0][0].device
-        n = len(params) // k
-        keep = []
-        w = (_lib.Gpt2Weights * k)(*[_weights_struct(m, params[i * n:(i + 1) * n], keep) for i, m in enumerate(models)])
+        call = _TrainCall(models, params, precision)
+        call.reserve(B, T, dev)
         outs = [torch.empty((B, m0.action_dim) if m0.test else (B, T, m0.action_dim), dtype=torch.float32, device=dev)
                 for _ in range(k)]
-        nbytes = lib().dpt_gpt2_train_population_workspace_bytes_ex(w, k, B, T, precision)
-        ws = torch.empty((max(int(nbytes), 16),), dtype=torch.uint8, device=dev)
-        arr = lambda ts: (ctypes.c_void_p * k)(*[t.data_ptr() if T else None for t in ts])   # noqa: E731
-        qs = (ctypes.c_void_p * k)(*[x[0].data_ptr() for x in inputs])
-        ins = [arr([x[j] for x in inputs]) for j in range(1, 5)]
-        os_ = (ctypes.c_void_p * k)(*[o.data_ptr() for o in outs])
-        test = 1 if m0.test else 0
-        if precision == 0:
-            check(lib().dpt_gpt2_train_population_forward(w, k, qs, *ins, B, T, stride, test, os_, ws.data_ptr(), ws.numel(),
-                                                          stream_ptr()),
-                  "dpt_gpt2_train_forward" if k == 1 else "dpt_gpt2_train_population_forward")
-        else:
-            check(lib().dpt_gpt2_train_population_forward_ex(w, k, qs, *ins, B, T, stride, test, precision, os_, ws.data_ptr(),
-                                                             ws.numel(), stream_ptr()), "dpt_gpt2_train_population_forward_ex")
-        ctx.models, ctx.ws, ctx.B, ctx.T, ctx.test, ctx.out_shape = models, ws, B, T, m0.test, outs[0].shape
-        ctx.precision = precision
+        call.forward([x[:5] for x in inputs], outs, B, T, stride, m0.test)
+        ctx.call, ctx.B, ctx.T, ctx.test, ctx.out_shape = call, B, T, m0.test, outs[0].shape
         ctx.save_for_backward(*params)
         return tuple(outs)
 
@@ -362,7 +358,7 @@ class _PopulationTrainFn(torch.autograd.Function):
     @torch.autograd.function.once_differentiable
     def backward(ctx, *douts):
         params = ctx.saved_tensors
-        models, k = ctx.models, len(ctx.models)
+        call, k = ctx.call, ctx.call.k
         n = len(params) // k
         dev = params[0].device
         grads = []
@@ -377,24 +373,11 @@ class _PopulationTrainFn(torch.autograd.Function):
             for g in grads:
                 g.zero_()
         else:
-            keep = []
-            w = (_lib.Gpt2Weights * k)(*[_weights_struct(m, params[i * n:(i + 1) * n], keep) for i, m in enumerate(models)])
-            gs = (_lib.Gpt2Grads * k)(*[_pointer_struct(_lib.Gpt2Grads, m, grads[i * n:(i + 1) * n], keep)
-                                        for i, m in enumerate(models)])
             # a member whose logits got no gradient runs on a zero dout; its gradients are dropped below
             ds = [torch.zeros(ctx.out_shape, dtype=torch.float32, device=dev) if d is None else d.to(torch.float32).contiguous()
                   for d in douts]
-            dp = (ctypes.c_void_p * k)(*[d.data_ptr() for d in ds])
-            test = 1 if ctx.test else 0
-            if ctx.precision == 0:
-                check(lib().dpt_gpt2_train_population_backward(w, k, dp, ctx.B, ctx.T, test, gs, ctx.ws.data_ptr(), ctx.ws.numel(),
-                                                               stream_ptr()),
-                      "dpt_gpt2_train_backward" if k == 1 else "dpt_gpt2_train_population_backward")
-            else:
-                check(lib().dpt_gpt2_train_population_backward_ex(w, k, dp, ctx.B, ctx.T, test, ctx.precision, gs, ctx.ws.data_ptr(),
-                                                                  ctx.ws.numel(), stream_ptr()),
-                      "dpt_gpt2_train_population_backward_ex")
-        ctx.ws = None
+            call.backward(ds, call.grads([grads[i * n:(i + 1) * n] for i in range(k)]), ctx.B, ctx.T, ctx.test)
+        ctx.call = None
         return (None, None, None, *[None if douts[i // n] is None else g for i, g in enumerate(grads)])
 
 
@@ -474,12 +457,11 @@ def online_loop_population(models, means, horizon, var, sample, seed, env_id0=0,
         dump_p = None
         if dump:
             dump_p = (_lib.Gpt2OnlineDump * n)(*[_lib.Gpt2OnlineDump(**{key: ptr(t) for key, t in o["noise"].items()}) for o in os_])
-        check(lib().dpt_gpt2_online_loop_population(arr(hs[a:b]), n, ptr(means), float(var), kernels.REWARD_TYPES[reward_type],
-                                                    1 if sample else 0, seed, env_id0, N, H, m0.precision, ptr(kv), kv.numel(),
-                                                    col("context_states"), col("context_actions"), col("context_next_states"),
-                                                    col("context_rewards"), col("cum_means"), col("regret_sums"), inj_p,
-                                                    dump_p, stream_ptr()),
-              "dpt_gpt2_online_loop" if k == 1 else "dpt_gpt2_online_loop_population")
+        check(lib().dpt_gpt2_online_loop(arr(hs[a:b]), n, ptr(means), float(var), kernels.REWARD_TYPES[reward_type],
+                                         1 if sample else 0, seed, env_id0, N, H, m0.precision, ptr(kv), kv.numel(),
+                                         col("context_states"), col("context_actions"), col("context_next_states"),
+                                         col("context_rewards"), col("cum_means"), col("regret_sums"), inj_p, dump_p,
+                                         stream_ptr()), "dpt_gpt2_online_loop")
     return outs
 
 

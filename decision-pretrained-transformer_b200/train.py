@@ -279,9 +279,9 @@ def train_interactive(model, dim, n_envs, K, n_iters, mb=1024, var=0.0, env_type
 
     1. ``env = GPUBanditEnv(dim, n_envs, K, var, env_type, seed=rng.key_for(seed, it))``;
     2. ``env.rollout(model, K, sample=True)``: the fused K-step rollout with the current weights (``model.precision``);
-    3. the last logits on ``context[:, :K-1]`` with a gradient (``dpt_gpt2_train_population_forward_ex`` with one member,
-       last position, whatever ``model.test`` says), ``interactive_loss`` against ``env.opt_a_index`` and
-       ``dpt_gpt2_train_population_backward_ex``, one micro-batch of ``mb`` envs at a time (micro-batch m is envs
+    3. the last logits on ``context[:, :K-1]`` with a gradient (``dpt_gpt2_train_forward`` with one member, last
+       position, whatever ``model.test`` says), ``interactive_loss`` against ``env.opt_a_index`` and
+       ``dpt_gpt2_train_backward``, one micro-batch of ``mb`` envs at a time (micro-batch m is envs
        ``[m*mb, min(n_envs, (m+1)*mb))``), each into its own gradient slot;
     4. the slots summed in micro-batch order into the parameters' ``.grad`` (one flat buffer; ``transformer.wte`` gets
        none), then ``optimizer.step()`` (default ``torch.optim.AdamW(lr, weight_decay)``).
@@ -329,7 +329,7 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
     if precision not in (0, 1):
         raise ValueError("train_interactive: precision=%r, training supports 0 (fp32) and 1 (bf16)" % (precision,))
     import ctypes
-    from . import _lib, dist as D, kernels, rng
+    from . import dist as D, kernels, rng
     from ._lib import check, lib, stream_ptr
     from .envs.gpu_bandit_env import GPUBanditEnv
     from .models import net
@@ -353,13 +353,11 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
     P = sum(sizes) + 1                 # a slot: every trained parameter (_train_params order), then the micro-batch's loss
     Ps = (P + 3) & ~3                  # slot stride: 16 B aligned slots
     T, du, st = K - 1, model.action_dim, stream_ptr()
-    fwd, bwd = "dpt_gpt2_train_population_forward_ex", "dpt_gpt2_train_population_backward_ex"
-    one = lambda *ps: (ctypes.c_void_p * 1)(*ps)   # noqa: E731  (the one-member pointer arrays of the population calls)
-    w = (_lib.Gpt2Weights * 1)(net._weights_struct(model, params, []))
+    call = net._TrainCall([model], params, precision)
     # the train kernels' shape and precision checks (n_embd, n_layer, sequence length) before any rollout: a B = 0 call
     # only validates
-    check(lib().dpt_gpt2_train_population_forward_ex(w, 1, None, None, None, None, None, 0, T, K, 1, precision, None, None, 0,
-                                                     st), fwd)
+    check(lib().dpt_gpt2_train_forward(call.w, 1, None, None, None, None, None, 0, T, K, 1, precision, None, None, 0, st),
+          "dpt_gpt2_train_forward")
     args = C.interactive_args(dim, n_envs, K, mb, var, env_type, seed, lr, weight_decay, precision)
     it0, done = 0, []
     if resume:   # every rank reads the same file; all raise if one fails to
@@ -386,8 +384,8 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
         losses[:it0] = torch.tensor(done, dtype=torch.float32)
         if n_local:
             q = torch.ones((min(mb, n_local), model.state_dim), dtype=torch.float32, device=dev)
-            wbytes = int(lib().dpt_gpt2_train_population_workspace_bytes_ex(w, 1, min(mb, n_local), T, precision))
-            work = torch.empty((max(wbytes, 16),), dtype=torch.uint8, device=dev)
+            call.reserve(min(mb, n_local), T, dev)
+            slot_grads = [call.grads([g]) for g in grad_slots]
         for it in range(it0, n_iters):
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)] if timings is not None else []
             mark = lambda i: ev and ev[i].record()   # noqa: E731
@@ -398,25 +396,16 @@ def _interactive(model, dim, n_envs, K, n_iters, mb, rank, ws, var=0.0, env_type
                     env = GPUBanditEnv(dim, n_local, K, var, env_type, device=dev, seed=rng.key_for(seed, it), env_id0=lo)
                     ro = env.rollout(model, K, sample=True, logits=False)
                     mark(1)
-                    keep = []
-                    w = (_lib.Gpt2Weights * 1)(net._weights_struct(model, params, keep))
                     ctx = [ro[k] for k in _CTX]
                     for j in range(n_mb):
                         a, b = j * mb, min(n_local, (j + 1) * mb)
                         out = torch.empty((b - a, du), dtype=torch.float32, device=dev)
-                        cp = [one(c[a:b].data_ptr() if T else None) for c in ctx]
-                        check(lib().dpt_gpt2_train_population_forward_ex(w, 1, one(q.data_ptr()), *cp, b - a, T, K, 1, precision,
-                                                                         one(out.data_ptr()), work.data_ptr(), work.numel(), st),
-                              fwd)
+                        call.forward([[q] + [c[a:b] for c in ctx]], [out], b - a, T, K, True)
                         lg = out.requires_grad_()
                         with torch.enable_grad():
                             loss = interactive_loss(lg, ro["target"][a:b], n_envs)
                             dout, = torch.autograd.grad(loss, lg)
-                        dout = dout.contiguous()
-                        g = net._pointer_struct(_lib.Gpt2Grads, model, grad_slots[j], keep)
-                        check(lib().dpt_gpt2_train_population_backward_ex(w, 1, one(dout.data_ptr()), b - a, T, 1, precision,
-                                                                          ctypes.byref(g), work.data_ptr(), work.numel(), st),
-                              bwd)
+                        call.backward([dout.contiguous()], slot_grads[j], b - a, T, True)
                         slots[j, P - 1].copy_(loss.detach())
                 else:
                     mark(1)

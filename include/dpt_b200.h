@@ -35,7 +35,7 @@ extern "C" {
 #define DPT_ERR_CUDA (-2)
 #define DPT_ERR_UNSUPPORTED (-3)
 
-#define DPT_ABI_VERSION 9
+#define DPT_ABI_VERSION 10
 
 /* reward_type of the bandit entry points (envs/bandit_env.py:56-63, envs/gpu_bandit_env.py:53-63):
  * 0 'uniform'  : r = means[a] + var * z, z ~ N(0,1);
@@ -341,14 +341,32 @@ int dpt_gpt2_forward(dpt_gpt2_t* m, const float* query_states, const float* ctx_
                      const float* ctx_next_states, const float* ctx_rewards, int B, int T, int T_stride, int ctx_share,
                      int test, int precision, float* out, void* workspace, uint64_t workspace_bytes, void* stream);
 
-/* Training (train.py:252-331 with Transformer.forward, models/net.py:41-60): fp32, sequences of <= 512 tokens, the
- * parameter tensors read in place through dpt_gpt2_weights_t (no handle, no repack, no host synchronisation).
- * dpt_gpt2_train_forward computes the same logits as dpt_gpt2_forward(precision = 0), bit for bit, and saves the
- * activations the backward needs in `workspace` (dpt_gpt2_train_workspace_bytes(w, B, T) bytes, 16 B aligned, the same
- * buffer for both calls).  dpt_gpt2_train_backward takes dout, the gradient of the logits ([B,du] if test, else
- * [B,T,du]), and OVERWRITES every gradient of `grads` (transformer.wte is not an input and has none): weight gradients
- * are sums over all B*(T+1) rows reduced in a fixed order (two identical calls give bit-identical gradients); wpe's
- * gradient has n_positions rows, zero past row T.  The context inputs get no gradient.  B = 0 is a no-op.  n_embd != 32,
+/* Training (train.py:252-331 with Transformer.forward, models/net.py:41-60): sequences of <= 512 tokens, the parameter
+ * tensors read in place through dpt_gpt2_weights_t (no handle, no repack, no host synchronisation).  One call trains
+ * n_models same-shape models in the same launches (members share n_layer, state_dim, action_dim and n_positions): w and
+ * grads are arrays of n_models structs; query_states, ctx_*, out and dout are HOST arrays of n_models DEVICE pointers,
+ * with the shapes of dpt_gpt2_forward; B, T, T_stride, test and precision are shared.  Member i's logits and gradients are
+ * bit-identical to those of a one-member call on its own weights, inputs and dout (same row chunking, same fixed-order
+ * sums).  The per-member tables travel in the kernel parameters: no upload, capturable in a CUDA graph.
+ * dpt_gpt2_train_forward computes the logits of dpt_gpt2_forward at the same precision, bit for bit, and saves the
+ * activations the backward needs in `workspace`.  dpt_gpt2_train_backward takes dout, the gradient of the logits ([B,du]
+ * if test, else [B,T,du]), and OVERWRITES every gradient of `grads` (transformer.wte is not an input and has none): weight
+ * gradients are sums over all B*(T+1) rows reduced in a fixed order (two identical calls give bit-identical gradients);
+ * wpe's gradient has n_positions rows, zero past row T.  The context inputs get no gradient.
+ * precision:
+ * - 0: fp32 on the CUDA cores.
+ * - 1: bf16 training: bf16 operands at the tensor-core inputs, fp32 accumulation, fp32 LayerNorm, softmax statistics,
+ *   residual stream and gradient sums.  The forward is the tcgen05 dense forward on the parameter tensors; the backward
+ *   runs the attention backward on mma.sync tensor-core products (bf16 in, fp32 out), split over ceil((T+1)/64) CTAs per
+ *   sequence, and the projection, MLP and LayerNorm backward and every weight-gradient sum in fp32.
+ * Workspace: dpt_gpt2_train_workspace_bytes(w, n_models, B, T, precision) = n_models times the bytes of one member,
+ * 16 B aligned, the same buffer for the forward and the backward; member regions follow one another.  At precision 1 each
+ * region also holds the bf16 weight images the forward packs from the parameters (40 KB per layer) and the
+ * attention-output gradients of one layer (144 B per row), so the two precisions' workspaces are not interchangeable.
+ * dpt_gpt2_train_workspace_bytes returns 0 for arguments it cannot size.
+ * 1 <= n_models <= DPT_GPT2_POPULATION_MAX per call; n_models = 0 or B = 0 only validates: the argument checks run,
+ * nothing is launched.  n_models < 0 or above the limit, null pointers and a member of another shape (the message names
+ * the member and the field when n_models > 1) return DPT_ERR_INVALID_ARG; precision outside {0, 1}, n_embd != 32,
  * n_layer > 8 and T + 1 > 512 return DPT_ERR_UNSUPPORTED. */
 typedef struct {
   float* wpe;
@@ -373,59 +391,16 @@ typedef struct {
   float* const* fc2_b;
 } dpt_gpt2_grads_t;
 
-uint64_t dpt_gpt2_train_workspace_bytes(const dpt_gpt2_weights_t* w, int B, int T);
-int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, const float* query_states, const float* ctx_states,
-                           const float* ctx_actions, const float* ctx_next_states, const float* ctx_rewards, int B, int T,
-                           int T_stride, int test, float* out, void* workspace, uint64_t workspace_bytes, void* stream);
-int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, const float* dout, int B, int T, int test,
-                            const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes, void* stream);
-
-/* Population training: n_models same-shape models (members share n_layer, state_dim, action_dim and n_positions) trained
- * in the same launches, each exactly as dpt_gpt2_train_forward / dpt_gpt2_train_backward would train it alone: member i's
- * logits and gradients are bit-identical to the one-model calls on its own weights, inputs and dout (same row chunking,
- * same fixed-order sums).  w and grads are arrays of n_models structs; query_states, ctx_*, out and dout are HOST arrays
- * of n_models DEVICE pointers, with the shapes of the one-model calls; B, T, T_stride and test are shared.  The workspace
- * holds one member region after another: dpt_gpt2_train_population_workspace_bytes(w, n_models, B, T) =
- * n_models * dpt_gpt2_train_workspace_bytes(w, B, T) bytes, 16 B aligned, the same buffer for both calls.  The per-member
- * tables travel in the kernel parameters: no host synchronisation, no upload, capturable in a CUDA graph.
- * 1 <= n_models <= DPT_GPT2_POPULATION_MAX per call; n_models = 0 or B = 0 is a no-op.  n_models < 0 or above the limit,
- * null pointers and a member of another shape (the message names the member and the field) return DPT_ERR_INVALID_ARG;
- * n_embd != 32, n_layer > 8 and T + 1 > 512 return DPT_ERR_UNSUPPORTED. */
 #define DPT_GPT2_POPULATION_MAX 32
-uint64_t dpt_gpt2_train_population_workspace_bytes(const dpt_gpt2_weights_t* w, int n_models, int B, int T);
-int dpt_gpt2_train_population_forward(const dpt_gpt2_weights_t* w, int n_models, const float* const* query_states,
-                                      const float* const* ctx_states, const float* const* ctx_actions,
-                                      const float* const* ctx_next_states, const float* const* ctx_rewards, int B, int T,
-                                      int T_stride, int test, float* const* out, void* workspace, uint64_t workspace_bytes,
-                                      void* stream);
-int dpt_gpt2_train_population_backward(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B, int T,
-                                       int test, const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes,
-                                       void* stream);
-
-/* Mixed-precision training: the population calls above with a `precision` argument.  precision = 0 runs exactly the
- * fp32 kernels of the calls without _ex (same results, bit for bit).  precision = 1 is bf16 training: bf16 operands at the
- * tensor-core inputs, fp32 accumulation, fp32 LayerNorm, softmax statistics, residual stream and gradient sums.
- * - forward: the tcgen05 dense forward of dpt_gpt2_forward(precision = 1) on the parameter tensors; member i's logits are
- *   bit-identical to dpt_gpt2_forward(precision = 1) on a handle of the same weights.
- * - backward: the attention backward on mma.sync tensor-core products (bf16 in, fp32 out), split over ceil((T+1)/64)
- *   CTAs per sequence; the projection, MLP and LayerNorm backward and every weight-gradient sum in fp32.  Two identical
- *   calls give bit-identical gradients, and member i's equal the one-member call's.
- * Workspace at precision 1: dpt_gpt2_train_population_workspace_bytes_ex(w, n_models, B, T, 1) bytes, 16 B aligned, the
- * same buffer for the forward and the backward.  It is larger than at precision 0: each member region also holds the bf16
- * weight images the forward packs from the parameters (40 KB per layer) and the attention-output gradients of one layer
- * (144 B per row); the two precisions' workspaces are not interchangeable.
- * B = 0 (and n_models = 0) only validates: the same argument checks run, nothing is launched.  precision outside {0, 1},
- * n_embd != 32, n_layer > 8 and T + 1 > 512 return DPT_ERR_UNSUPPORTED with a message; the other errors are those of the
- * calls without _ex.  workspace_bytes_ex returns 0 for arguments it cannot size (as the call without _ex does). */
-uint64_t dpt_gpt2_train_population_workspace_bytes_ex(const dpt_gpt2_weights_t* w, int n_models, int B, int T, int precision);
-int dpt_gpt2_train_population_forward_ex(const dpt_gpt2_weights_t* w, int n_models, const float* const* query_states,
-                                         const float* const* ctx_states, const float* const* ctx_actions,
-                                         const float* const* ctx_next_states, const float* const* ctx_rewards, int B, int T,
-                                         int T_stride, int test, int precision, float* const* out, void* workspace,
-                                         uint64_t workspace_bytes, void* stream);
-int dpt_gpt2_train_population_backward_ex(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B, int T,
-                                          int test, int precision, const dpt_gpt2_grads_t* grads, void* workspace,
-                                          uint64_t workspace_bytes, void* stream);
+uint64_t dpt_gpt2_train_workspace_bytes(const dpt_gpt2_weights_t* w, int n_models, int B, int T, int precision);
+int dpt_gpt2_train_forward(const dpt_gpt2_weights_t* w, int n_models, const float* const* query_states,
+                           const float* const* ctx_states, const float* const* ctx_actions,
+                           const float* const* ctx_next_states, const float* const* ctx_rewards, int B, int T,
+                           int T_stride, int test, int precision, float* const* out, void* workspace,
+                           uint64_t workspace_bytes, void* stream);
+int dpt_gpt2_train_backward(const dpt_gpt2_weights_t* w, int n_models, const float* const* dout, int B, int T, int test,
+                            int precision, const dpt_gpt2_grads_t* grads, void* workspace, uint64_t workspace_bytes,
+                            void* stream);
 
 /* Ordered multi-source sum (the gradient exchange of the data-parallel interactive trainer, train_interactive.py:97-139;
  * the reference is single-GPU): dst[i] = (((src[0][i] + src[1][i]) + ...) + src[M-1][i]) for i < n, fp32, added in
@@ -438,8 +413,20 @@ int dpt_ordered_sum_f32(const float* const* src, int M, int64_t n, float* dst, v
 /* Fused bandit online loop with the transformer controller: evals/eval_bandit.py:56-103 +
  * ctrls/ctrl_bandit.py:383-444 (BanditTransformerController, sample != 0 -> softmax + categorical
  * draw, else argmax) + env step, with a per-env KV cache (valid because the bandit query token is
- * constant, SURVEY.md §3.3).  kv_cache: device scratch of dpt_gpt2_online_kv_bytes(...) bytes.
- * inject: reward_z [H,N] fp32, ctrl_u f64 [H,N] (uniforms of the categorical draw). */
+ * constant, SURVEY.md §3.3).  inject: reward_z [H,N] fp32, ctrl_u f64 [H,N] (uniforms of the categorical draw).
+ * One call runs the loop of n_models same-shape models (members share n_layer and action_dim, have state_dim == 1 and
+ * n_positions >= H) in one launch, on the same tasks and the same noise: member i's outputs are bit for bit those of a
+ * one-member call on models[i] with the same means, var, reward_type, sample, seed, env_id0, N, H, precision and inject,
+ * whichever kernel variant the call's total of n_models * N env-warps selects (regret sums are float64 atomics: equal up
+ * to their order of addition).  models, ctx_*, cum_means, regret_sums: HOST arrays of n_models pointers (device pointers;
+ * ctx_* [N,H,.], cum_means [H,N] fp32, regret_sums [H,4] f64 as in dpt_online_loop); a whole array may be NULL, an entry
+ * may be NULL (not written), and a member's four context pointers are all NULL or all set.  dump: n_models structs or
+ * NULL.  inject is shared by every member.  kv_cache holds n_models regions of
+ * dpt_gpt2_online_kv_bytes(models[0], N, H, precision) bytes, one after another.  The per-member tables travel in the
+ * kernel parameters: no host synchronisation, no upload, capturable in a CUDA graph.
+ * 1 <= n_models <= DPT_GPT2_ONLINE_POPULATION_MAX per call; n_models = 0, N = 0 or H = 0 is a no-op.  n_models outside
+ * [0, max], null pointers, a K/V buffer that is too small and a member of another shape (the message names the member and
+ * the field) return DPT_ERR_INVALID_ARG. */
 typedef struct {
   const float* reward_z;
   const double* ctrl_u;
@@ -452,40 +439,21 @@ typedef struct {
 } dpt_gpt2_online_dump_t;
 
 uint64_t dpt_gpt2_online_kv_bytes(const dpt_gpt2_t* m, int N, int H, int precision);
-int dpt_gpt2_online_loop(dpt_gpt2_t* m, const float* means, double var, int reward_type, int sample, uint64_t seed,
-                         uint64_t env_id0,
-                         int N, int H, int precision, void* kv_cache, uint64_t kv_bytes, float* ctx_states,
-                         float* ctx_actions, float* ctx_next_states, float* ctx_rewards, float* cum_means,
-                         double* regret_sums, const dpt_gpt2_online_inject_t* inject,
-                         const dpt_gpt2_online_dump_t* dump, void* stream);
-
-/* Population evaluation: the online loop of n_models same-shape models (members share n_layer and action_dim, have
- * state_dim == 1 and n_positions >= H) in one launch, on the same tasks and the same noise: member i's outputs are bit for
- * bit those of dpt_gpt2_online_loop(models[i], ...) with the same means, var, reward_type, sample, seed, env_id0, N, H,
- * precision and inject, whichever kernel variant the population's total of n_models * N env-warps selects (regret sums
- * are float64 atomics: equal up to their order of addition).  models, ctx_*, cum_means, regret_sums: HOST arrays of
- * n_models pointers (device pointers with the shapes of the one-model call); a whole array may be NULL, an entry may be
- * NULL where the one-model call allows it, and a member's four context pointers are all NULL or all set.  dump: n_models
- * structs or NULL.  inject is shared by every member.  kv_cache holds n_models regions of
- * dpt_gpt2_online_kv_bytes(models[0], N, H, precision) bytes, one after another.  The per-member tables travel in the
- * kernel parameters: no host synchronisation, no upload, capturable in a CUDA graph.
- * 1 <= n_models <= DPT_GPT2_ONLINE_POPULATION_MAX per call; n_models = 0, N = 0 or H = 0 is a no-op.  n_models outside
- * [0, max], null pointers, a K/V buffer that is too small and a member of another shape (the message names the member and
- * the field) return DPT_ERR_INVALID_ARG. */
 #define DPT_GPT2_ONLINE_POPULATION_MAX 16
-int dpt_gpt2_online_loop_population(dpt_gpt2_t* const* models, int n_models, const float* means, double var, int reward_type,
-                                    int sample, uint64_t seed, uint64_t env_id0, int N, int H, int precision, void* kv_cache,
-                                    uint64_t kv_bytes, float* const* ctx_states, float* const* ctx_actions,
-                                    float* const* ctx_next_states, float* const* ctx_rewards, float* const* cum_means,
-                                    double* const* regret_sums, const dpt_gpt2_online_inject_t* inject,
-                                    const dpt_gpt2_online_dump_t* dump, void* stream);
+int dpt_gpt2_online_loop(dpt_gpt2_t* const* models, int n_models, const float* means, double var, int reward_type,
+                         int sample, uint64_t seed, uint64_t env_id0, int N, int H, int precision, void* kv_cache,
+                         uint64_t kv_bytes, float* const* ctx_states, float* const* ctx_actions,
+                         float* const* ctx_next_states, float* const* ctx_rewards, float* const* cum_means,
+                         double* const* regret_sums, const dpt_gpt2_online_inject_t* inject,
+                         const dpt_gpt2_online_dump_t* dump, void* stream);
 
 /* One decode step for callers that drive their own loop (the rollout half of train_interactive.py:97-132 /
  * train_explorer_exploiter.py:110-166, where the arm that is pulled is chosen outside): append the token of position
  * `pos` (tokens [N, 2*dx+du+1] = [state | action | next_state | reward]; position 0 is the query token
  * [query_state, 0, ...], models/net.py:45-53) to every sequence's K/V cache and write the logits at that position
  * (= Transformer.forward(...)[:, -1] over the pos transitions appended so far) to logits [N, du].  Positions must be
- * appended in order 0, 1, 2, ...; kv_cache as for dpt_gpt2_online_loop: dpt_gpt2_online_kv_bytes(m, N, T_max, precision). */
+ * appended in order 0, 1, 2, ...; kv_cache: dpt_gpt2_online_kv_bytes(m, N, T_max, precision) bytes, one member region of
+ * dpt_gpt2_online_loop. */
 int dpt_gpt2_decode_step(dpt_gpt2_t* m, const float* tokens, int N, int pos, int T_max, int precision, void* kv_cache,
                          uint64_t kv_bytes, float* logits, void* stream);
 

@@ -233,8 +233,9 @@ def _bf16_ws_fits(L, H):
 
 
 def test_online_loop_cases_reach_their_variants(dpt):
-    """The N / H of the scratch cases launch the kernel variant they are named after (kernel names from the profiler).
-    At L = 4 a horizon of 1210 (Tpad 1216) still fits the warp-specialised kernel; 1300 is past it."""
+    """The N / H of the scratch cases launch the kernel variant they are named after (kernel names from the profiler),
+    with the one-model parameter block (member capacity NM = 1).  At L = 4 a horizon of 1210 (Tpad 1216) still fits the
+    warp-specialised kernel; 1300 is past it."""
     for precision, L, N, H, variant in KS.online_cases() + [(1, 4, 6, 1210, "bf16 warp-specialised")]:
         assert _bf16_ws_fits(L, H) == (variant == "bf16 warp-specialised") or precision == 0
         m = KS.model(1, 5, L, H, True).cuda()
@@ -245,8 +246,34 @@ def test_online_loop_cases_reach_their_variants(dpt):
             m.online_loop(means, H, 0.3, True, 1, 0)
             torch.cuda.synchronize()
         names = [e.name for e in prof.events() if "gpt2_online_kernel" in e.name]
-        args = {re.search(r"gpt2_online_kernel<(\w+), ?(\w+), ?(\w+)", n).groups() for n in names}
-        assert args == {KS.ONLINE_VARIANT_ARGS[variant.split(",")[0]]}, (variant, names)
+        args = {re.search(r"gpt2_online_kernel<(\w+), ?(\w+), ?(\w+), ?(\w+)", n).groups() for n in names}
+        assert args == {KS.ONLINE_VARIANT_ARGS[variant.split(",")[0]] + ("1",)}, (variant, names)
+
+
+# the training kernels, each templated on the member capacity NM of its launch (its last template argument)
+TRAIN_KERNELS = {0: {"gpt2_train_forward_kernel", "gpt2_train_backward_kernel", "weight_grad_reduce_kernel", "wpe_grad_kernel"},
+                 1: {"pack_wimg_kernel", "gpt2_train_forward_bf16_kernel", "gpt2_train_rows_bf16_kernel",
+                     "gpt2_train_attn_bf16_kernel", "weight_grad_reduce_kernel", "wpe_grad_kernel"}}
+
+
+@pytest.mark.parametrize("precision", [0, 1])
+def test_training_launches_reach_their_member_capacity(dpt, precision):
+    """A one-model forward_train + backward launches the NM = 1 instances of the training kernels (small parameter
+    blocks), a two-member population the NM = 32 ones (kernel names from the profiler)."""
+    from dpt_b200.models.net import POPULATION_MAX, forward_train_population
+    ms = [_model(1, 5, 2, seed=i) for i in range(2)]
+    x = KS.base_batch(1, 5, 4, 100, seed=1, device="cuda")
+    pat = re.compile(r"(%s)<([^<>]*)>" % "|".join(TRAIN_KERNELS[precision]))
+    for members, nm in ((ms[:1], "1"), (ms, str(POPULATION_MAX))):
+        def step():
+            outs = forward_train_population(members, [x] * len(members), precision)
+            sum(KS.row_weighted_ce(o, x["optimal_actions"], slice(None)) for o in outs).backward()
+        step()   # module load outside the profile
+        with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+            step()
+            torch.cuda.synchronize()
+        found = {(m.group(1), m.group(2).split(",")[-1].strip()) for m in map(pat.search, (e.name for e in prof.events())) if m}
+        assert found == {(k, nm) for k in TRAIN_KERNELS[precision]}, (len(members), sorted(found))
 
 
 @pytest.mark.parametrize("case", range(6))

@@ -1,4 +1,4 @@
-"""CPU tier of population evaluation: argument checks of dpt_gpt2_online_loop_population that run before any launch (no
+"""CPU tier of population evaluation: argument checks of dpt_gpt2_online_loop that run before any launch (no
 GPU needed), the ValueErrors of online_loop_population for members that do not line up, and how a population is cut into
 launches by member capacity and by the K/V scratch bound."""
 import ctypes
@@ -12,8 +12,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _call(lib, models, n, N=100, H=50, kv=None, kv_bytes=0):
-    return lib.dpt_gpt2_online_loop_population(models, n, None, 0.3, 0, 1, 7, 0, N, H, 0, kv, kv_bytes, None, None, None,
-                                               None, None, None, None, None, None)
+    return lib.dpt_gpt2_online_loop(models, n, None, 0.3, 0, 1, 7, 0, N, H, 0, kv, kv_bytes, None, None, None, None, None,
+                                    None, None, None, None)
 
 
 def test_population_online_entry_point_rejects_bad_arguments(dpt):
@@ -30,8 +30,8 @@ def test_population_online_entry_point_rejects_bad_arguments(dpt):
     # no member: nothing to check, nothing to launch
     assert _call(lib, None, 0) == 0
     assert _call(lib, nulls, 0, N=0, H=0) == 0
-    with pytest.raises(ValueError, match="dpt_gpt2_online_loop_population"):
-        dpt._lib.check(_call(lib, nulls, -1), "dpt_gpt2_online_loop_population")
+    with pytest.raises(ValueError, match="dpt_gpt2_online_loop"):
+        dpt._lib.check(_call(lib, nulls, -1), "dpt_gpt2_online_loop")
 
 
 def _model(**over):

@@ -92,35 +92,6 @@ def test_injected_noise_is_shared(dpt, members):
         assert torch.equal(ref["noise"]["reward_z"], inject["reward_z"]) and torch.equal(ref["noise"]["ctrl_u"], inject["ctrl_u"])
 
 
-def _c_online_loop(dpt, m, means, H, seed, env_id0):
-    """The one-model C entry point called directly (Transformer.online_loop goes through the population entry point)."""
-    from dpt_b200._lib import lib, ptr, stream_ptr
-    N, d = means.shape
-    out = {"cum_means": torch.empty((H, N), device="cuda"), "regret_sums": torch.zeros((H, 4), dtype=torch.float64, device="cuda"),
-           "context_states": torch.empty((N, H, 1), device="cuda"), "context_actions": torch.empty((N, H, d), device="cuda"),
-           "context_next_states": torch.empty((N, H, 1), device="cuda"), "context_rewards": torch.empty((N, H, 1), device="cuda"),
-           "noise": {"reward_z": torch.empty((H, N), device="cuda"), "ctrl_u": torch.zeros((H, N), dtype=torch.float64, device="cuda"),
-                     "logits": torch.empty((H, N, d), device="cuda")}}
-    h = m.handle()
-    nb = lib().dpt_gpt2_online_kv_bytes(h, N, H, m.precision)
-    kv = torch.empty((nb,), dtype=torch.uint8, device="cuda")
-    dump = dpt._lib.Gpt2OnlineDump(**{k: ptr(t) for k, t in out["noise"].items()})
-    dpt._lib.check(lib().dpt_gpt2_online_loop(h, ptr(means), 0.3, 0, 1, seed, env_id0, N, H, m.precision, ptr(kv), nb,
-                                              *[ptr(out[k]) for k in CTX], ptr(out["cum_means"]), ptr(out["regret_sums"]), None,
-                                              ctypes.byref(dump), stream_ptr()), "dpt_gpt2_online_loop")
-    return out
-
-
-@pytest.mark.parametrize("precision", [0, 1])
-def test_one_member_equals_the_one_model_entry_point(dpt, members, precision):
-    from dpt_b200.models.net import online_loop_population
-    m = members(1, precision)[0]
-    means, _, _ = dpt.kernels.bandit_sample_means(500, 5, 3, 2)
-    ref = _c_online_loop(dpt, m, means, 90, 3, 2)
-    _same(online_loop_population([m], means, 90, 0.3, True, 3, 2, dump=True)[0], ref)
-    _same(m.online_loop(means, 90, 0.3, True, 3, 2, dump=True), ref)
-
-
 def test_population_above_one_launch(dpt, members):
     from dpt_b200.models import net
     k = net.ONLINE_POPULATION_MAX + 2
@@ -174,8 +145,8 @@ def test_empty_population_and_empty_shapes(dpt, members):
     means, _, _ = dpt.kernels.bandit_sample_means(16, 5, 1, 0)
     assert online_loop_population([], means, 10, 0.3, True, 1) == []
     lib = dpt._lib.lib()
-    assert lib.dpt_gpt2_online_loop_population(None, 0, None, 0.3, 0, 1, 1, 0, 16, 10, 0, None, 0, None, None, None, None, None,
-                                               None, None, None, None) == 0
+    assert lib.dpt_gpt2_online_loop(None, 0, None, 0.3, 0, 1, 1, 0, 16, 10, 0, None, 0, None, None, None, None, None, None, None,
+                                    None, None) == 0
     zero_n = online_loop_population(ms, means[:0], 10, 0.3, True, 1)
     assert [o["cum_means"].shape for o in zero_n] == [(10, 0)] * 2
     zero_h = online_loop_population(ms, means, 0, 0.3, True, 1)
@@ -194,19 +165,19 @@ def test_mismatched_members_raise_in_python_and_c(dpt, members):
             online_loop_population(ms + [odd], means, 10, 0.3, True, 1)
         hs = (ctypes.c_void_p * 3)(*[m.handle() for m in ms + [odd]])
         kv = torch.empty((1 << 24,), dtype=torch.uint8, device="cuda")
-        rc = lib().dpt_gpt2_online_loop_population(hs, 3, ptr(means), 0.3, 0, 1, 1, 0, 16, 10, 0, ptr(kv), kv.numel(), None, None,
-                                                   None, None, None, None, None, None, None)
+        rc = lib().dpt_gpt2_online_loop(hs, 3, ptr(means), 0.3, 0, 1, 1, 0, 16, 10, 0, ptr(kv), kv.numel(), None, None, None, None,
+                                        None, None, None, None, None)
         assert rc == dpt._lib.ERR_INVALID_ARG and ("member 2 has %s" % field) in lib().dpt_last_error().decode()
     hs = (ctypes.c_void_p * 2)(*[m.handle() for m in ms])
     per = lib().dpt_gpt2_online_kv_bytes(ms[0].handle(), 16, 10, 0)
     kv = torch.empty((2 * per,), dtype=torch.uint8, device="cuda")
     args = (ptr(means), 0.3, 0, 1, 1, 0, 16, 10, 0, ptr(kv))
-    assert lib().dpt_gpt2_online_loop_population(hs, 2, *args, 2 * per - 1, None, None, None, None, None, None, None, None,
-                                                 None) == dpt._lib.ERR_INVALID_ARG
+    assert lib().dpt_gpt2_online_loop(hs, 2, *args, 2 * per - 1, None, None, None, None, None, None, None, None,
+                                      None) == dpt._lib.ERR_INVALID_ARG
     assert "kv cache" in lib().dpt_last_error().decode()
     cs = (ctypes.c_void_p * 2)(None, ptr(torch.empty(16 * 10, device="cuda")))
-    assert lib().dpt_gpt2_online_loop_population(hs, 2, *args, 2 * per, cs, None, None, None, None, None, None, None,
-                                                 None) == dpt._lib.ERR_INVALID_ARG
+    assert lib().dpt_gpt2_online_loop(hs, 2, *args, 2 * per, cs, None, None, None, None, None, None, None,
+                                      None) == dpt._lib.ERR_INVALID_ARG
     assert "member 1: context pointers" in lib().dpt_last_error().decode()
 
 

@@ -1,6 +1,6 @@
-"""CPU tier of bf16 training (precision = 1): the ABI version, the argument checks of the dpt_gpt2_train_population_*_ex
-entry points (a B = 0 call only validates, so no GPU is needed), and the training precision in the resume arguments of
-checkpoint.train_args, including states written before it was recorded."""
+"""CPU tier of bf16 training (precision = 1): the ABI version, the precision argument of dpt_gpt2_train_workspace_bytes /
+_forward / _backward (a B = 0 call only validates, so no GPU is needed), and the training precision in the resume
+arguments of checkpoint.train_args, including states written before it was recorded."""
 import ctypes
 
 import pytest
@@ -22,7 +22,7 @@ def _weights(dpt, keep, n_layer=2, n_embd=32, n_positions=2004):
 
 
 def test_abi_version(dpt):
-    assert dpt._lib.ABI_VERSION == 9 == dpt._lib.lib().dpt_version()
+    assert dpt._lib.ABI_VERSION == 10 == dpt._lib.lib().dpt_version()
 
 
 @pytest.mark.parametrize("case,kw,T,precision,msg", [
@@ -31,31 +31,31 @@ def test_abi_version(dpt):
     ("tokens", {}, 512, 1, "512 tokens"),
     ("precision", {}, 10, 2, "precision=2"),
 ])
-def test_ex_entry_points_validate_at_b0(dpt, case, kw, T, precision, msg):
+def test_precision_entry_points_validate_at_b0(dpt, case, kw, T, precision, msg):
     lib = dpt._lib.lib()
     keep = []
     w = (dpt._lib.Gpt2Weights * 1)(_weights(dpt, keep, **kw))
     p = (ctypes.c_void_p * 1)(4096)
-    assert lib.dpt_gpt2_train_population_forward_ex(w, 1, p, p, p, p, p, 0, T, T, 0, precision, p, None, 0, None) == E_UNSUP
+    assert lib.dpt_gpt2_train_forward(w, 1, p, p, p, p, p, 0, T, T, 0, precision, p, None, 0, None) == E_UNSUP
     assert msg in lib.dpt_last_error().decode()
-    assert lib.dpt_gpt2_train_population_backward_ex(w, 1, p, 0, T, 0, precision, None, None, 0, None) == E_UNSUP
+    assert lib.dpt_gpt2_train_backward(w, 1, p, 0, T, 0, precision, None, None, 0, None) == E_UNSUP
     assert msg in lib.dpt_last_error().decode()
 
 
-def test_ex_workspace_and_valid_b0_calls(dpt):
+def test_precision_workspace_and_valid_b0_calls(dpt):
     lib = dpt._lib.lib()
     keep = []
     w = (dpt._lib.Gpt2Weights * 2)(_weights(dpt, keep), _weights(dpt, keep))
     p = (ctypes.c_void_p * 2)(4096, 4096)
-    fp32 = lib.dpt_gpt2_train_population_workspace_bytes(w, 2, 64, 500)
-    assert lib.dpt_gpt2_train_population_workspace_bytes_ex(w, 2, 64, 500, 0) == fp32 > 0
+    fp32 = lib.dpt_gpt2_train_workspace_bytes(w, 2, 64, 500, 0)
+    assert fp32 > 0
     # precision 1 also holds the packed weight images (40 KB per layer) and one layer's attention-output gradients
-    bf16 = lib.dpt_gpt2_train_population_workspace_bytes_ex(w, 2, 64, 500, 1)
+    bf16 = lib.dpt_gpt2_train_workspace_bytes(w, 2, 64, 500, 1)
     assert bf16 == fp32 + 2 * (2 * 40960 + 64 * 501 * 36 * 4)
-    assert lib.dpt_gpt2_train_population_workspace_bytes_ex(w, 2, 64, 500, 2) == 0
+    assert lib.dpt_gpt2_train_workspace_bytes(w, 2, 64, 500, 2) == 0
     for prec in (0, 1):   # a valid shape at B = 0: nothing to do
-        assert lib.dpt_gpt2_train_population_forward_ex(w, 2, p, p, p, p, p, 0, 10, 10, 0, prec, p, None, 0, None) == 0
-        assert lib.dpt_gpt2_train_population_backward_ex(w, 2, p, 0, 10, 0, prec, None, None, 0, None) == 0
+        assert lib.dpt_gpt2_train_forward(w, 2, p, p, p, p, p, 0, 10, 10, 0, prec, p, None, 0, None) == 0
+        assert lib.dpt_gpt2_train_backward(w, 2, p, 0, 10, 0, prec, None, None, 0, None) == 0
 
 
 def test_python_rejects_unknown_precision(dpt):

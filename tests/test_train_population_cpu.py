@@ -1,6 +1,6 @@
-"""CPU tier of population training: argument checks of dpt_gpt2_train_population_* (they run before any launch, so no GPU
-is needed) and the ValueErrors of forward_train_population / train_population for members or datasets that do not line
-up."""
+"""CPU tier of population training: argument checks of dpt_gpt2_train_forward / _backward over several members at
+precision 0 (they run before any launch, so no GPU is needed) and the ValueErrors of forward_train_population /
+train_population for members or datasets that do not line up."""
 import ctypes
 
 import pytest
@@ -23,7 +23,7 @@ def _weights(dpt, keep, n_layer=2, state_dim=1, action_dim=5, n_embd=32, n_posit
 
 def _fwd(lib, w, n, ptrs=None, B=4, T=10):
     p = ptrs if ptrs is not None else (ctypes.c_void_p * max(n, 1))(*[4096] * max(n, 1))
-    return lib.dpt_gpt2_train_population_forward(w, n, p, p, p, p, p, B, T, T, 0, p, None, 0, None)
+    return lib.dpt_gpt2_train_forward(w, n, p, p, p, p, p, B, T, T, 0, 0, p, None, 0, None)
 
 
 def test_population_entry_points_reject_bad_arguments(dpt):
@@ -36,24 +36,24 @@ def test_population_entry_points_reject_bad_arguments(dpt):
     # member count
     for n in (-1, limit + 1):
         assert _fwd(lib, two, n) == E_ARG and ("n_models=%d" % n) in err()
-        assert lib.dpt_gpt2_train_population_backward(two, n, None, 4, 10, 0, None, None, 0, None) == E_ARG
-    assert lib.dpt_gpt2_train_population_workspace_bytes(two, limit + 1, 4, 10) == 0
+        assert lib.dpt_gpt2_train_backward(two, n, None, 4, 10, 0, 0, None, None, 0, None) == E_ARG
+    assert lib.dpt_gpt2_train_workspace_bytes(two, limit + 1, 4, 10, 0) == 0
     # null pointers
     assert _fwd(lib, None, 2) == E_ARG and "null weights" in err()
-    assert lib.dpt_gpt2_train_population_forward(two, 2, None, None, None, None, None, 4, 10, 10, 0, None, None, 0, None) == E_ARG
+    assert lib.dpt_gpt2_train_forward(two, 2, None, None, None, None, None, 4, 10, 10, 0, 0, None, None, 0, None) == E_ARG
     assert "null input or output pointer array" in err()
     nulls = (ctypes.c_void_p * 2)(4096, None)
     assert _fwd(lib, two, 2, nulls) == E_ARG and "member 1: null input or output pointer" in err()
-    assert lib.dpt_gpt2_train_population_backward(two, 2, None, 4, 10, 0, None, None, 0, None) == E_ARG and "null dout" in err()
-    ws_needed = lib.dpt_gpt2_train_population_workspace_bytes(two, 2, 4, 10)
-    assert ws_needed == 2 * lib.dpt_gpt2_train_workspace_bytes(two, 4, 10) > 0
+    assert lib.dpt_gpt2_train_backward(two, 2, None, 4, 10, 0, 0, None, None, 0, None) == E_ARG and "null dout" in err()
+    ws_needed = lib.dpt_gpt2_train_workspace_bytes(two, 2, 4, 10, 0)
+    assert ws_needed == 2 * lib.dpt_gpt2_train_workspace_bytes(two, 1, 4, 10, 0) > 0
     assert _fwd(lib, two, 2) == E_ARG and "workspace" in err()
     # a member of another shape: the message names the member and the field
     for field, kw in (("n_layer", {"n_layer": 3}), ("state_dim", {"state_dim": 2}), ("action_dim", {"action_dim": 4}),
                       ("n_positions", {"n_positions": 404})):
         odd = (dpt._lib.Gpt2Weights * 3)(_weights(dpt, keep), _weights(dpt, keep), _weights(dpt, keep, **kw))
         assert _fwd(lib, odd, 3) == E_ARG and ("member 2 has %s" % field) in err(), field
-        assert lib.dpt_gpt2_train_population_backward(odd, 3, None, 4, 10, 0, None, None, 0, None) == E_ARG
+        assert lib.dpt_gpt2_train_backward(odd, 3, None, 4, 10, 0, 0, None, None, 0, None) == E_ARG
     # the one-model limits, per member
     wide = (dpt._lib.Gpt2Weights * 2)(_weights(dpt, keep), _weights(dpt, keep, n_embd=64))
     assert _fwd(lib, wide, 2) == E_UNSUP and "member 1: n_embd=64" in err()
@@ -62,11 +62,11 @@ def test_population_entry_points_reject_bad_arguments(dpt):
     assert _fwd(lib, deep, 1) == E_UNSUP
     # no-ops: no member, or an empty batch
     assert _fwd(lib, None, 0) == 0
-    assert lib.dpt_gpt2_train_population_backward(None, 0, None, 4, 10, 0, None, None, 0, None) == 0
+    assert lib.dpt_gpt2_train_backward(None, 0, None, 4, 10, 0, 0, None, None, 0, None) == 0
     assert _fwd(lib, two, 2, B=0) == 0
-    assert lib.dpt_gpt2_train_population_backward(two, 2, None, 0, 10, 0, None, None, 0, None) == 0
-    with pytest.raises(ValueError, match="dpt_gpt2_train_population_forward"):
-        dpt._lib.check(_fwd(lib, two, -1), "dpt_gpt2_train_population_forward")
+    assert lib.dpt_gpt2_train_backward(two, 2, None, 0, 10, 0, 0, None, None, 0, None) == 0
+    with pytest.raises(ValueError, match="dpt_gpt2_train_forward"):
+        dpt._lib.check(_fwd(lib, two, -1), "dpt_gpt2_train_forward")
 
 
 def _model(**over):
